@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- HIMG encode+decode throughput on B200 (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--dump-outputs DIR]
 
 Workload (config.workload): BASELINE.json configs[3] "batch of 4096 1920x1080 RGB images encode+decode
 sharded across 1/2/4/8 B200" -- STRONG scaling: the job is always the 4096 images with seeds 1..4096 at
@@ -24,6 +24,8 @@ Printed JSON (one line, rank 0):
                sample of every other rank's images on its own GPU and compares bitstreams byte for byte
   c2 / c3 / c5 sub-records of the other BASELINE.json configurations (N=1 only)
   cpu_baseline the unmodified reference (oracle/_ref) on the host cores, bounded sample
+
+--dump-outputs DIR (e.g. bench_outputs) writes what the last timed step computed, see dump_outputs().
 """
 from __future__ import annotations
 
@@ -177,6 +179,45 @@ def driver_times(args_list):
         return None
 
 
+DUMP_IMAGES = 8                # images of the shard whose outputs --dump-outputs writes
+DUMP_PIXELS_PER_IMAGE = 1 << 19
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(path, first, out, sizes, table, decoded, status):
+    """--dump-outputs: what the timed step returned in its last step, as float arrays, so that two builds can
+    be compared output for output.  The whole size / offset table of the job and the decode status of every
+    image of the shard; for a fixed, seeded sample of the shard's images (always its first and last) their
+    whole bitstreams (-1 past the end) and their decoded pixels at a fixed, seeded set of positions (flat
+    indices into H x W x NCH, the same in every image).  About 50 MB."""
+    import numpy as np
+    import torch
+
+    B = sizes.numel()
+    rng = np.random.default_rng(20261020)
+    idx = sorted({0, B - 1} | {int(i) for i in rng.choice(B, min(B, DUMP_IMAGES - 2), replace=False)})
+    pos = np.sort(rng.choice(H * W * NCH, min(H * W * NCH, DUMP_PIXELS_PER_IMAGE), replace=False))
+    sizes_h = sizes.cpu().numpy()
+    streams = np.full((len(idx), int(sizes_h[idx].max())), -1, np.float32)
+    for k, i in enumerate(idx):
+        streams[k, : sizes_h[i]] = out[i, : int(sizes_h[i])].cpu().numpy()
+    sel = torch.tensor(idx, device=decoded.device)
+    pixels = decoded[sel].reshape(len(idx), -1)[:, torch.from_numpy(pos).to(decoded.device)].cpu().numpy()
+    arrays = {
+        "sizes": table[0].cpu().numpy().astype(np.float64),
+        "offsets": table[1].cpu().numpy().astype(np.float64),
+        "status": status.cpu().numpy().astype(np.float64),
+        "sample_images": np.asarray(idx, np.float64) + first,
+        "sample_bitstreams": streams,
+        "sample_pixel_positions": pos.astype(np.float64),
+        "sample_pixels": pixels.astype(np.float32),
+    }
+    assert sum(a.nbytes for a in arrays.values()) <= DUMP_LIMIT_BYTES
+    os.makedirs(path, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(path, name + ".npy"), a)
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
@@ -188,7 +229,10 @@ def main():
     ap.add_argument("--cpu-images-per-core", type=int, default=24)
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-subrecords", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the outputs of the last timed step as DIR/<name>.npy (rank 0)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
 
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
@@ -197,6 +241,8 @@ def main():
 
     # ---- reference arm: the reference's CPU implementation, rank 0 only --------------------------
     if args.impl == "reference":
+        if args.dump_outputs:
+            ap.error("--dump-outputs writes the outputs of --impl b200")
         if rank != 0:
             return 0
         per = max(1, min(args.cpu_images_per_core, 12))  # bounded sample per step
@@ -355,6 +401,8 @@ def main():
     ctx.profile(False)
     ctx.encode_status()
     assert int(status.abs().sum()) == 0 and int(table[0].numel()) == total_images
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, first, out, sizes, table, decoded, status)
 
     # encode-only / decode-only splits (device resident), same timing discipline
     def timed(fn, reps):

@@ -76,7 +76,10 @@ struct himgcu_ctx {
   std::vector<std::string> prof_names;
   uint64_t launches = 0;
   size_t max_workspace = (size_t)24 << 30;
-  int item_lists = 1;  // hand the item lists of k_huff_hist2 to the packer (option "item_lists")
+  int item_lists = 1;  // hand the item lists of the histogram pass to the packer (option "item_lists")
+  // framed chunks without parts, option "huff_warp_teams": 1 = k_huff_hist4 / k_huff_pack4 when the batch has a
+  // wave of segments, 2 = whenever possible (tests), 0 = never (k_huff_hist2 / k_huff_pack3)
+  int huff_warp_teams = 1;
   size_t host_sub_bytes = (size_t)192 << 20;  // staged bytes per sub-batch of the host-buffer calls (measured best: 128-192 MB)
   bool force_generic = false;  // tests: route everything through the generic kernels
   int xform_variant = 0;       // experiments: 0 = newest fast kernels, 1 = previous generation
@@ -601,6 +604,7 @@ int huff_encode_items(himgcu_ctx *ctx, int n, HuffChunkArgs *chunks, int nchunks
   TreeParams TP;
   memset(&TP, 0, sizeof(TP));
   ItemLists lists[2];
+  bool teams[2] = {false, false};
   for (int k = 0; k < nchunks; ++k) {
     HuffGeom &hg = chunks[k].hg;
     // Parts per segment: only worth it when the segments alone cannot fill the GPU (the low-res chunk
@@ -617,6 +621,12 @@ int huff_encode_items(himgcu_ctx *ctx, int n, HuffChunkArgs *chunks, int nchunks
       hg.sub_size = sub;
       hg.nsub = (hg.seg_size + sub - 1) / sub;
     }
+    // Warp teams (a warp per segment, eight segments per CTA) for framed chunks whose segments have no parts,
+    // when the segments fill every SM with warps: a single 8K image (1024 segments) measured 0.52 ms encode
+    // with a CTA per segment, 0.88 ms with a warp per segment.
+    const long long wave = 148LL * kTeamWarps * kP4MinCtas;  // resident warps of k_huff_pack4
+    teams[k] = !ctx->force_generic && hg.nseg > 1 && hg.nsub == 1 &&
+               (ctx->huff_warp_teams == 2 || (ctx->huff_warp_teams == 1 && (long long)n * hg.nseg >= wave));
     const std::string tag = chunks[k].tag;
     ENSURE((tag + "_seghist").c_str(), (size_t)n * hg.nseg * hg.nsub * kSyms * sizeof(uint32_t), d_seghist[k]);
     ENSURE((tag + "_partstart").c_str(), (size_t)n * hg.nseg * hg.nsub * sizeof(uint32_t), d_part[k]);
@@ -642,6 +652,9 @@ int huff_encode_items(himgcu_ctx *ctx, int n, HuffChunkArgs *chunks, int nchunks
       CK(cudaMemsetAsync(d_total, 0, (size_t)n * kSyms * sizeof(uint32_t), ctx->stream));
     }
     if (ctx->force_generic) LAUNCH("k_huff_hist", k_huff_hist, grid, kHuffThreads, 0, chunks[k].d_in, hg, d_seghist[k]);
+    else if (teams[k])
+      LAUNCH("k_huff_hist", k_huff_hist4, dim3((hg.nseg + kTeamWarps - 1) / kTeamWarps, n), kTeamThreads, 0, chunks[k].d_in,
+             hg, d_seghist[k], il, d_total);
     else LAUNCH("k_huff_hist", k_huff_hist2, grid, kTokThreads, 0, chunks[k].d_in, hg, d_seghist[k], il, d_total);
     TP.total[k] = d_total;
     TP.seghist[k] = d_seghist[k];
@@ -671,12 +684,16 @@ int huff_encode_items(himgcu_ctx *ctx, int n, HuffChunkArgs *chunks, int nchunks
   const size_t win_bytes = (kWinWords + 2) * sizeof(uint32_t);
   if (ctx->force_generic)  // static + dynamic shared memory of the first-generation packer exceed 48 KiB
     CK(cudaFuncSetAttribute(k_huff_pack, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)win_bytes));
+  if (teams[0] || teams[1]) CK(cudaFuncSetAttribute(k_huff_pack4, cudaFuncAttributeMaxDynamicSharedMemorySize, kP4Smem));
   for (int k = 0; k < nchunks; ++k) {
     const HuffGeom &hg = chunks[k].hg;
     dim3 grid(hg.nseg * hg.nsub, n);
     if (ctx->force_generic)
       LAUNCH("k_huff_pack", k_huff_pack, grid, kHuffThreads, win_bytes, chunks[k].d_in, hg, d_trees[k], d_bits[k],
              d_pos[k], d_sizes, d_out, (unsigned long long)out_stride, d_err);
+    else if (teams[k])
+      LAUNCH("k_huff_pack", k_huff_pack4, dim3((hg.nseg + kTeamWarps - 1) / kTeamWarps, n), kTeamThreads, kP4Smem, chunks[k].d_in,
+             hg, d_trees[k], d_bits[k], d_pos[k], d_sizes, d_out, (unsigned long long)out_stride, d_err, lists[k]);
     else
       LAUNCH("k_huff_pack", k_huff_pack3, grid, kTokThreads, 0, chunks[k].d_in, hg, d_trees[k], d_bits[k], d_pos[k],
              d_part[k], d_sizes, d_out, (unsigned long long)out_stride, d_err, lists[k]);
@@ -1001,6 +1018,8 @@ int prepare_lanes(himgcu_ctx *ctx, int K, int *count) {
   }
   for (himgcu_ctx *l : ctx->lanes) {
     l->force_generic = ctx->force_generic;
+    l->item_lists = ctx->item_lists;
+    l->huff_warp_teams = ctx->huff_warp_teams;
     l->max_workspace = ctx->max_workspace;
   }
   *count = S;
@@ -1775,6 +1794,7 @@ int himgcu_set_option(himgcu_ctx *ctx, const char *name, long long value) {
   else if (!strcmp(name, "xform_variant")) ctx->xform_variant = (int)value;
   else if (!strcmp(name, "max_workspace_bytes")) ctx->max_workspace = (size_t)value;
   else if (!strcmp(name, "item_lists")) ctx->item_lists = value != 0;
+  else if (!strcmp(name, "huff_warp_teams")) ctx->huff_warp_teams = (int)std::max<long long>(0, std::min<long long>(value, 2));
   else if (!strcmp(name, "host_sub_batch_bytes")) ctx->host_sub_bytes = (size_t)std::max<long long>(value, 1 << 20);
   else if (!strcmp(name, "host_lanes")) ctx->host_lanes = (int)std::max<long long>(1, std::min<long long>(value, himgcu_ctx::kMaxLanes));
   else return fail(ctx, HIMGCU_ERR_ARG, "unknown option %s", name);

@@ -8,6 +8,8 @@
 //                  prefix sum of (header + payload) sizes -> absolute byte offsets; container headers
 //   k_huff_pack3   CTA per segment (or part): tokens built once in registers -> scan of bit totals ->
 //                  word-wise accumulation into a shared-memory bit window -> bytes to the final position
+//   k_huff_hist4 / k_huff_pack4 warp teams for framed chunks without parts: a warp per segment, one
+//                  contiguous item list per segment, __syncwarp only
 //   k_huff_hist / k_huff_pack   first-generation kernels (per-thread chunk walks): the force_generic path
 //   k_huff_stale   the reference's uncleared scratch buffer leaks "stale" bits into the padding of
 //                  every segment's last byte (SURVEY A.3 step 5); reproduced as a fix-up pass
@@ -1122,6 +1124,394 @@ __global__ void __launch_bounds__(kTokThreads, kP3MinCtas)
       else dst[gbyte] = (uint8_t)win[0];
     }
     if (gbits != end_bit) atomicMax(err, 99);  // internal consistency
+  }
+}
+
+// =================================================================================================
+// Warp teams (v4) for framed chunks whose segments are not split into parts.  A CTA holds eight
+// consecutive segments of one item, one warp per segment, and a warp synchronises with __syncwarp
+// only: the block scans and barriers of every 8 KiB piece of k_huff_hist2 / k_huff_pack3 go away, and
+// the item list of a segment is one contiguous list without piece boundaries.
+// =================================================================================================
+constexpr int kTeamWarps = 8;
+constexpr int kTeamThreads = kTeamWarps * 32;
+constexpr int kWalkStep = 32 * 16;  // bytes per warp step: 16 per lane
+
+__device__ __forceinline__ uint4 load16(const uint8_t *__restrict__ seg, int seg_size, int off, bool aligned) {
+  if (aligned && off + 16 <= seg_size) return __ldg(reinterpret_cast<const uint4 *>(seg + off));
+  uint32_t w[4] = {0, 0, 0, 0};
+#pragma unroll
+  for (int k = 0; k < 16; ++k)
+    if (off + k < seg_size) w[k >> 2] |= (uint32_t)seg[off + k] << (8 * (k & 3));
+  return make_uint4(w[0], w[1], w[2], w[3]);
+}
+
+// Walks a segment in 512-byte warp steps and appends the position and value of every non-zero byte
+// ("item") to a per-warp queue in shared memory: qpos[1 + k] / qval[1 + k] is item k of the queue,
+// qpos[0] the position of the item before it (-1 at the segment start), so that the zero run in front
+// of item k is qpos[1 + k] - qpos[k] - 1.  Whenever kRound items are queued, consume(k0, cnt, g0)
+// takes items k0 .. k0 + cnt of the queue (g0: their index in the segment); the last call may take
+// fewer.  Queues hold kRound + kWalkStep entries.  Returns the position of the segment's last item, or
+// -1.  Warp-uniform call.
+template <int kRound, class Consume>
+__device__ __forceinline__ int warp_walk_items(const uint8_t *__restrict__ seg, int seg_size, int *qpos, uint8_t *qval,
+                                               Consume &&consume) {
+  const int lane = threadIdx.x & 31;
+  const bool aligned = (reinterpret_cast<uintptr_t>(seg) & 15) == 0;
+  if (lane == 0) qpos[0] = -1;
+  __syncwarp();
+  int qn = 0, g0 = 0;
+  uint4 nxt = load16(seg, seg_size, 16 * lane, aligned);
+  for (int base = 0; base < seg_size; base += kWalkStep) {
+    const int off = base + 16 * lane;
+    const uint4 w = nxt;
+    nxt = load16(seg, seg_size, off + kWalkStep, aligned);  // (nothing past the segment end)
+    uint32_t m = nonzero_nibble(w.x) | nonzero_nibble(w.y) << 4 | nonzero_nibble(w.z) << 8 | nonzero_nibble(w.w) << 12;
+    const uint32_t c = __popc(m);
+    uint32_t inc = c;
+#pragma unroll
+    for (int d = 1; d < 32; d <<= 1) {
+      const uint32_t t = __shfl_up_sync(0xffffffffu, inc, d);
+      if (lane >= d) inc += t;
+    }
+    const int step_items = (int)__shfl_sync(0xffffffffu, inc, 31);
+    if (step_items == 0) continue;
+    int k = 1 + qn + (int)(inc - c);
+    while (m) {
+      const int j = __ffs(m) - 1;
+      m &= m - 1;
+      const uint32_t word = j < 4 ? w.x : (j < 8 ? w.y : (j < 12 ? w.z : w.w));
+      qpos[k] = off + j;
+      qval[k] = (uint8_t)(word >> (8 * (j & 3)));
+      ++k;
+    }
+    qn += step_items;
+    __syncwarp();
+    if (qn >= kRound) {
+      int done = 0;
+      for (; qn - done >= kRound; done += kRound) consume(done, kRound, g0 + done);
+      // the last consumed item and the rest move to the front (the ranges do not overlap: done >= kRound > rest)
+      __syncwarp();
+      for (int i = lane; i <= qn - done; i += 32) {
+        qpos[i] = qpos[done + i];
+        qval[i] = qval[done + i];
+      }
+      g0 += done;
+      qn -= done;
+      __syncwarp();
+    }
+  }
+  if (qn) consume(0, qn, g0);
+  return qpos[qn];
+}
+
+// Item list of a segment, handed from k_huff_hist4 to k_huff_pack4: the zero run in front of each item
+// (u16) and its byte value, ItemLists::pieces_per_part * kItemCap entries per segment (the capacity of
+// the per-piece lists of the same segment).  A segment with more items, or a run of 65536 zeros or
+// more, is marked kItemsNotStored and the packer walks its planes again.
+__device__ __forceinline__ size_t seg_list_base(const ItemLists &L, int nseg, int item, int b) {
+  return ((size_t)item * nseg + b) * ((size_t)L.pieces_per_part * kItemCap);
+}
+
+// grid (ceil(nseg / 8), n), block 256: warp w codes segment 8 * blockIdx.x + w of item blockIdx.y.
+// seghist: [n][nseg][261]; total: [n][261] (atomics).
+__global__ void __launch_bounds__(kTeamThreads)
+    k_huff_hist4(const uint8_t *__restrict__ in, HuffGeom hg, uint32_t *__restrict__ seghist, ItemLists lists,
+                 uint32_t *__restrict__ total) {
+  constexpr int kQ = 32 + kWalkStep;
+  __shared__ uint32_t sh[kTeamWarps][kSyms];
+  __shared__ int qpos_all[kTeamWarps][kQ];
+  __shared__ uint8_t qval_all[kTeamWarps][kQ];
+  const int wid = threadIdx.x >> 5, lane = threadIdx.x & 31, item = blockIdx.y;
+  const int b = blockIdx.x * kTeamWarps + wid;
+  if (b >= hg.nseg) return;
+  uint32_t *h = sh[wid];
+  int *qpos = qpos_all[wid];
+  uint8_t *qval = qval_all[wid];
+  for (int i = lane; i < kSyms; i += 32) h[i] = 0;
+  __syncwarp();
+  const uint8_t *seg = in + (size_t)item * hg.in_stride + (size_t)b * hg.seg_size;
+  const bool lists_on = lists.pieces_per_part != 0;
+  const int cap = lists.pieces_per_part * kItemCap;
+  unsigned short *lpos = lists_on ? lists.pos + seg_list_base(lists, hg.nseg, item, b) : nullptr;
+  uint8_t *lval = lists_on ? lists.val + seg_list_base(lists, hg.nseg, item, b) : nullptr;
+  bool long_gap = false;  // a run that the u16 list entry cannot hold
+  auto run = [&](uint32_t z) {
+    if (z >= (uint32_t)kMaxRun) {
+      atomicAdd(&h[260], z / kMaxRun);
+      z %= kMaxRun;
+    }
+    uint32_t ex;
+    if (z) atomicAdd(&h[run_symbol(z, &ex)], 1u);
+  };
+  int nitems = 0;
+  // one item per lane
+  const int last = warp_walk_items<32>(seg, hg.seg_size, qpos, qval, [&](int k0, int cnt, int g0) {
+    nitems = g0 + cnt;
+    if (lane < cnt) {
+      const int k = k0 + lane;
+      const uint32_t gap = (uint32_t)(qpos[1 + k] - qpos[k] - 1), v = qval[1 + k];
+      run(gap);
+      atomicAdd(&h[v], 1u);
+      long_gap |= gap > 0xffffu;
+      if (lists_on && g0 + lane < cap) {
+        lpos[g0 + lane] = (unsigned short)gap;
+        lval[g0 + lane] = (uint8_t)v;
+      }
+    }
+  });
+  if (lane == 0) run((uint32_t)(hg.seg_size - 1 - last));  // the run still open at the segment end
+  __syncwarp();
+  if (lists_on) {
+    const bool stored = nitems <= cap && !__any_sync(0xffffffffu, long_gap);
+    if (lane == 0) lists.count[(size_t)item * hg.nseg + b] = stored ? (uint32_t)nitems : kItemsNotStored;
+  }
+  uint32_t *dst = seghist + ((size_t)item * hg.nseg + b) * kSyms;
+  for (int i = lane; i < kSyms; i += 32) {
+    const uint32_t v = h[i];
+    dst[i] = v;
+    if (total && v) atomicAdd(&total[(size_t)item * kSyms + i], v);
+  }
+}
+
+// grid (ceil(nseg / 8), n), block 256: warp w packs segment 8 * blockIdx.x + w of item blockIdx.y.  Rounds of
+// 32 lanes x 8 consecutive items in segment order; bit offsets from a warp scan; the bits go into a per-warp
+// window in shared memory through a 64-bit accumulator (one atomicOr per word), and the warp writes the
+// window out when the next round does not fit.
+constexpr int kP4Items = 8;
+constexpr int kP4Round = 32 * kP4Items;
+constexpr int kWin4Words = 512;  // 2 KiB per warp (a q50 segment is ~6 KB)
+constexpr int kWin4Bits = kWin4Words * 32;
+constexpr int kP4Queue = kP4Round + kWalkStep;
+constexpr int kP4MinCtas = 4;  // 64 registers, 49 KiB of shared memory per CTA
+// dynamic shared memory: per warp a window, and a queue for the segments without a stored list
+constexpr int kP4Smem = kTeamWarps * ((kWin4Words + 4) * 4 + kP4Queue * 5);
+
+__global__ void __launch_bounds__(kTeamThreads, kP4MinCtas)
+    k_huff_pack4(const uint8_t *__restrict__ in, HuffGeom hg, const TreeOut *__restrict__ trees,
+                 const uint32_t *__restrict__ seg_bits, const uint32_t *__restrict__ seg_pos,
+                 const uint32_t *__restrict__ sizes, uint8_t *__restrict__ out, unsigned long long out_stride, int *err,
+                 ItemLists lists) {
+  extern __shared__ uint32_t p4_smem[];
+  __shared__ uint2 s_tab[kSyms];
+  const int wid = threadIdx.x >> 5, lane = threadIdx.x & 31, item = blockIdx.y;
+  if (sizes[item] == 0) return;  // did not fit (k_huff_layout)
+  const TreeOut *tr = trees + item;
+  for (int s = threadIdx.x; s < kSyms; s += blockDim.x) {
+    const uint32_t l = tr->len[s];
+    s_tab[s] = make_uint2(tr->code[s], l | ((l + (uint32_t)sym_extra_bits(s)) << 8));
+  }
+  __syncthreads();
+  const int b = blockIdx.x * kTeamWarps + wid;
+  if (b >= hg.nseg) return;
+  uint32_t *win = p4_smem + wid * (kWin4Words + 4);
+  int *qpos = reinterpret_cast<int *>(p4_smem + kTeamWarps * (kWin4Words + 4)) + wid * kP4Queue;
+  uint8_t *qval = reinterpret_cast<uint8_t *>(p4_smem + kTeamWarps * (kWin4Words + 4 + kP4Queue)) + wid * kP4Queue;
+  for (int i = lane; i < kWin4Words + 4; i += 32) win[i] = 0;
+  __syncwarp();
+  const uint8_t *seg = in + (size_t)item * hg.in_stride + (size_t)b * hg.seg_size;
+  uint8_t *dst = out + (size_t)item * out_stride + seg_pos[(size_t)item * hg.nseg + b];
+  const uint32_t full_bits = s_tab[260].y >> 8;  // one maximal run token
+  const uint64_t full_tok = (uint64_t)s_tab[260].x | ((uint64_t)(kMaxRun - 279) << (s_tab[260].y & 255u));
+
+  uint32_t gbyte = 0;  // complete bytes already written to dst
+  uint32_t wfill = 0;  // bits in the window; window bit 0 = bit 0 of byte gbyte
+  // Writes the complete bytes of the window to dst and keeps the unfinished byte.  Warp-uniform call.
+  auto flush = [&]() {
+    __syncwarp();
+    const uint32_t nbytes = wfill >> 3;
+    const uint8_t *wb = reinterpret_cast<const uint8_t *>(win);
+    for (uint32_t i = lane; i < nbytes; i += 32) dst[gbyte + i] = wb[i];
+    const uint32_t keep = (wfill & 7) ? wb[nbytes] : 0u;
+    __syncwarp();
+    const uint32_t used = min((wfill >> 5) + 4u, (uint32_t)(kWin4Words + 4));
+    for (uint32_t i = lane; i < used; i += 32) win[i] = i == 0 ? keep : 0u;
+    __syncwarp();
+    gbyte += nbytes;
+    wfill &= 7;
+  };
+  // Token by token, lane 0 writing: maximal runs, runs, literals that are out of the ordinary.  Uniform calls.
+  auto put_uniform = [&](uint64_t v, uint32_t n) {
+    if (wfill + n > (uint32_t)kWin4Bits) flush();
+    if (lane == 0) put64(win, wfill, v, n);
+    wfill += n;
+  };
+  auto run_uniform = [&](uint32_t z) {
+    for (uint32_t nfull = z / kMaxRun; nfull;) {
+      const uint32_t cap = ((uint32_t)kWin4Bits - wfill) / full_bits;
+      if (cap == 0) {
+        flush();
+        continue;
+      }
+      const uint32_t n = min(nfull, cap);
+      if (lane == 0)
+        for (uint32_t i = 0; i < n; ++i) put64(win, wfill + i * full_bits, full_tok, full_bits);
+      wfill += n * full_bits;
+      nfull -= n;
+    }
+    const uint32_t rest = z % kMaxRun;
+    if (rest) {
+      uint64_t rt;
+      uint32_t rb;
+      run_token(s_tab, rest, &rt, &rb);
+      put_uniform(rt, rb);
+    }
+  };
+  // One round: lane i takes items 8i .. 8i + m - 1 of the round.  fetch8(gap, val) gives the zero run in
+  // front of them and their byte values; fetch1(k, gap, val) item k of the round, for the rare paths (so
+  // that the common one holds only the tokens in registers).
+  auto round = [&](int m, auto &&fetch8, auto &&fetch1) {
+    uint64_t tok[kP4Items];
+    uint32_t tl[kP4Items];
+    uint32_t tbits = 0;
+    bool wide = false;  // an item of more than 32 bits: this lane bypasses the accumulator
+    uint32_t gap[kP4Items], val[kP4Items];
+    fetch8(gap, val);
+#pragma unroll
+    for (int j = 0; j < kP4Items; ++j) {
+      tok[j] = 0;
+      tl[j] = 0;
+      if (j < m) {
+        const uint2 lr = s_tab[val[j]];
+        uint64_t tk = lr.x;
+        uint32_t l = lr.y & 255u;
+        const uint32_t nfull = gap[j] / kMaxRun, z = gap[j] - nfull * kMaxRun;
+        if (z) {
+          uint64_t rt;
+          uint32_t rb;
+          run_token(s_tab, z, &rt, &rb);
+          tk = rt | (tk << rb);  // (only used when it fits 32 bits)
+          l += rb;
+        }
+        wide |= l > 32 || nfull;
+        l += nfull * full_bits;
+        tok[j] = tk;
+        tl[j] = l;
+        tbits += l;
+      }
+    }
+    uint32_t inc = tbits;
+#pragma unroll
+    for (int d = 1; d < 32; d <<= 1) {
+      const uint32_t t = __shfl_up_sync(0xffffffffu, inc, d);
+      if (lane >= d) inc += t;
+    }
+    const uint32_t total = __shfl_sync(0xffffffffu, inc, 31);
+    if (wfill + total > (uint32_t)kWin4Bits) flush();
+    if (wfill + total > (uint32_t)kWin4Bits) {
+      // does not fit even the empty window (long zero runs, or very long codes): item by item
+      for (int L = 0; L < 32; ++L) {
+        const int mL = __shfl_sync(0xffffffffu, m, L);
+#pragma unroll
+        for (int j = 0; j < mL; ++j) {
+          uint32_t g, v;
+          fetch1(kP4Items * L + j, g, v);
+          run_uniform(g);
+          put_uniform(s_tab[v].x, s_tab[v].y & 255u);
+        }
+      }
+      return;
+    }
+    uint32_t pos = wfill + inc - tbits;
+    if (!wide) {
+      uint32_t word = pos >> 5, fill = pos & 31;
+      uint64_t acc = 0;
+#pragma unroll
+      for (int j = 0; j < kP4Items; ++j) {
+        acc |= tok[j] << fill;  // tl <= 32 and fill < 32
+        fill += tl[j];
+        if (fill >= 32) {
+          atomicOr(&win[word], (uint32_t)acc);
+          acc >>= 32;
+          fill -= 32;
+          ++word;
+        }
+      }
+      if ((uint32_t)acc) atomicOr(&win[word], (uint32_t)acc);
+    } else {
+#pragma unroll
+      for (int j = 0; j < kP4Items; ++j) {
+        if (j < m) {
+          uint32_t g, v;
+          fetch1(kP4Items * lane + j, g, v);
+          const uint32_t nfull = g / kMaxRun, z = g - nfull * kMaxRun;
+          for (uint32_t f = 0; f < nfull; ++f, pos += full_bits) put64(win, pos, full_tok, full_bits);
+          if (z) {
+            uint64_t rt;
+            uint32_t rb;
+            run_token(s_tab, z, &rt, &rb);
+            put64(win, pos, rt, rb);
+            pos += rb;
+          }
+          const uint2 lr = s_tab[v];
+          put64(win, pos, lr.x, lr.y & 255u);
+          pos += lr.y & 255u;
+        }
+      }
+    }
+    wfill += total;
+  };
+
+  int last;  // position of the segment's last item
+  const uint32_t cnt = lists.pieces_per_part ? lists.count[(size_t)item * hg.nseg + b] : kItemsNotStored;
+  if (cnt != kItemsNotStored) {
+    // the list of k_huff_hist4: 16 + 8 bytes per lane and round, the next round's loads in flight
+    const size_t lb = seg_list_base(lists, hg.nseg, item, b);
+    const uint4 *gp = reinterpret_cast<const uint4 *>(lists.pos + lb);
+    const uint2 *gv = reinterpret_cast<const uint2 *>(lists.val + lb);
+    uint32_t span = 0;  // bytes covered by this lane's items (run + literal)
+    uint4 np = make_uint4(0, 0, 0, 0);
+    uint2 nv = make_uint2(0, 0);
+    if (kP4Items * lane < (int)cnt) np = __ldg(gp + lane), nv = __ldg(gv + lane);
+    for (int r0 = 0; r0 < (int)cnt; r0 += kP4Round) {
+      const int k0 = r0 + kP4Items * lane, m = min(max((int)cnt - k0, 0), kP4Items);
+      const uint4 p = np;
+      const uint2 v = nv;
+      if (k0 + kP4Round < (int)cnt) np = __ldg(gp + (k0 + kP4Round) / kP4Items), nv = __ldg(gv + (k0 + kP4Round) / kP4Items);
+      round(
+          m,
+          [&](uint32_t(&gap)[kP4Items], uint32_t(&val)[kP4Items]) {
+            const uint32_t pw[4] = {p.x, p.y, p.z, p.w}, vw[2] = {v.x, v.y};
+#pragma unroll
+            for (int j = 0; j < kP4Items; ++j) {
+              gap[j] = (pw[j >> 1] >> (16 * (j & 1))) & 0xffffu;
+              val[j] = (vw[j >> 2] >> (8 * (j & 3))) & 0xffu;
+              if (j < m) span += gap[j] + 1;
+            }
+          },
+          [&](int k, uint32_t &g, uint32_t &val) {
+            g = lists.pos[lb + r0 + k];
+            val = lists.val[lb + r0 + k];
+          });
+    }
+    last = (int)__reduce_add_sync(0xffffffffu, span) - 1;
+  } else {
+    // no list: the items again from the planes, with the walk of k_huff_hist4
+    last = warp_walk_items<kP4Round>(seg, hg.seg_size, qpos, qval, [&](int k0, int n, int) {
+      const int m = min(max(n - kP4Items * lane, 0), kP4Items);
+      auto fetch1 = [&](int k, uint32_t &g, uint32_t &val) {
+        g = (uint32_t)(qpos[1 + k0 + k] - qpos[k0 + k] - 1);
+        val = qval[1 + k0 + k];
+      };
+      round(
+          m,
+          [&](uint32_t(&gap)[kP4Items], uint32_t(&val)[kP4Items]) {
+#pragma unroll
+            for (int j = 0; j < kP4Items; ++j) {
+              gap[j] = 0;
+              val[j] = 0;
+              if (j < m) fetch1(kP4Items * lane + j, gap[j], val[j]);
+            }
+          },
+          fetch1);
+    });
+  }
+  run_uniform((uint32_t)(hg.seg_size - 1 - last));  // the run still open at the segment end
+  flush();
+  // final partial byte (its padding bits are zero here; k_huff_stale adds the stale ones)
+  if (lane == 0) {
+    if (wfill) dst[gbyte] = (uint8_t)win[0];
+    if (gbyte * 8u + wfill != seg_bits[(size_t)item * hg.nseg + b]) atomicMax(err, 99);  // internal consistency
   }
 }
 

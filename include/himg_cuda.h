@@ -177,7 +177,10 @@ uint64_t himgcu_launch_count(himgcu_ctx *ctx);
 /* Tuning / test knobs: "force_generic" (1 = always use the generic kernels instead of the aligned
  * fast paths), "max_workspace_bytes", "host_sub_batch_bytes" (bytes staged per sub-batch of the
  * *_batch_host calls), "host_lanes" (1..4 sub-batches coded concurrently by those calls), "item_lists" (default 1:
- * the packer reads the item lists stored by the histogram pass; 0: it rebuilds them from the planes -- same bytes). */
+ * the packer reads the item lists stored by the histogram pass; 0: it rebuilds them from the planes -- same bytes),
+ * "huff_warp_teams" (entropy coder of framed chunks: 1 = a warp per segment when the batch has enough segments to
+ * fill the GPU, default; 2 = a warp per segment whenever the segments have no parts; 0 = a CTA per segment --
+ * same bytes). */
 int himgcu_set_option(himgcu_ctx *ctx, const char *name, long long value);
 
 #ifdef __cplusplus

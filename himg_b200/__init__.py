@@ -132,6 +132,20 @@ class Context:
                                                 C.byref(h), C.byref(n)), allow=(_native.REJECT,))
         return None if rc == _native.REJECT else out
 
+    def decode_region(self, data: bytes, x: int, y: int, w: int, h: int, flags=STRICT):
+        """Rectangle [x, x+w) x [y, y+h) of the image: the [h][w][nch] array equal to decode(data)[y:y+h, x:x+w],
+        or None where the stream is rejected.  Raises HimgError for an empty rectangle or one outside the image."""
+        buf = np.frombuffer(data, np.uint8)
+        W, H, n = C.c_int(), C.c_int(), C.c_int()
+        if self.lib.himgcu_decode_info(_ptr(buf), buf.size, C.byref(W), C.byref(H), C.byref(n)) != _native.OK:
+            return None
+        if n.value < 1:
+            return None
+        out = np.empty((max(h, 1), max(w, 1), n.value), np.uint8)
+        rc = self._check(self.lib.himgcu_decode_region(self.h, _ptr(buf), buf.size, flags, x, y, w, h, _ptr(out), out.size,
+                                                       C.byref(W), C.byref(H), C.byref(n)), allow=(_native.REJECT,))
+        return None if rc == _native.REJECT else out
+
     # ---- batch, device tensors --------------------------------------------------------------
     def encode_batch(self, pixels, quality=50, use_ycbcr=True, out=None, sizes=None):
         """pixels: CUDA uint8 tensor [n][h][w][nch].  Returns (out [n][stride] u8, sizes [n] i32)."""
@@ -162,6 +176,25 @@ class Context:
             status = torch.empty((n,), dtype=torch.int32, device=himg.device)
         self._check(self.lib.himgcu_decode_batch(self.h, _ptr(himg), _ptr(offsets), _ptr(sizes), n, w, h, nch, flags,
                                                  _ptr(out), _ptr(status)))
+        return out, status
+
+    def decode_batch_region(self, himg, offsets, sizes, w, h, nch, origins, crop_w, crop_h, flags=STRICT, out=None,
+                            status=None):
+        """decode_batch of a crop_w x crop_h rectangle per image: origins is a CUDA int32 [n][2] tensor of (x, y).
+        Returns (pixels [n][crop_h][crop_w][nch], status); status[i] is ERR_ARG where the origin puts the
+        rectangle outside the image (that image's pixels are not written)."""
+        import torch
+
+        n = offsets.numel()
+        if origins.dtype != torch.int32 or origins.numel() != 2 * n:
+            raise ValueError("origins must be an int32 tensor [n][2]")
+        self._bind(himg, offsets, sizes, origins, out, status)
+        if out is None:
+            out = torch.empty((n, crop_h, crop_w, nch), dtype=torch.uint8, device=himg.device)
+        if status is None:
+            status = torch.empty((n,), dtype=torch.int32, device=himg.device)
+        self._check(self.lib.himgcu_decode_batch_region(self.h, _ptr(himg), _ptr(offsets), _ptr(sizes), n, w, h, nch, flags,
+                                                        _ptr(origins), crop_w, crop_h, _ptr(out), _ptr(status)))
         return out, status
 
     # ---- batch, host buffers (numpy arrays or pinned CPU torch tensors) -------------------------

@@ -23,6 +23,7 @@
 #include "xform_avg2.cuh"
 #include "xform_inv4.cuh"
 #include "xform_kernels.cuh"
+#include "xform_region.cuh"
 
 using namespace himgcu;
 
@@ -810,15 +811,27 @@ int launch_stream_cluster(himgcu_ctx *ctx, const char *name, int n, const uint8_
   return HIMGCU_OK;
 }
 
-// Whole-image decode of n streams resident on the device.
-int decode_device(himgcu_ctx *ctx, const uint8_t *d_himg, const unsigned long long *d_offsets,
-                  const uint32_t *d_sizes, int n, const Geom &g, int flags, uint8_t *d_pixels, int *d_status) {
-  const int lenient = (flags & HIMGCU_LENIENT) ? 1 : 0;
+// Device scratch of a decode (whole image or region) that decode_front fills.
+struct DecFront {
+  const ChunkDesc *fcd;
+  const DecTree *ftree;
+  const DecTables *tabs;
+  SegRef *fseg;  // [n][rows]
+  uint8_t *R;    // decoded low-res images
+  bool fork;     // the low-res branch runs on ctx->aux_stream: wait for ctx->ev_join before reading R
+};
+
+// What every decode does before the coefficient planes: container, tables and both trees of n streams, then
+// the low-res branch (segment table, stream, DPCM into R).  The caller ensures its planes buffer before: a
+// workspace that grows is freed after a stream synchronisation, which must not happen while the two branches
+// of a single image run on two streams.
+int decode_front(himgcu_ctx *ctx, const uint8_t *d_himg, const unsigned long long *d_offsets, const uint32_t *d_sizes, int n,
+                 const Geom &g, int lenient, int *d_status, DecFront *f) {
   ChunkDesc *d_lcd, *d_fcd;
   DecTables *d_tabs;
   DecTree *d_ltree, *d_ftree;
   SegRef *d_lseg, *d_fseg;
-  uint8_t *d_lres, *d_planes, *d_R;
+  uint8_t *d_lres, *d_R;
   ENSURE("dec_lcd", (size_t)n * sizeof(ChunkDesc), d_lcd);
   ENSURE("dec_fcd", (size_t)n * sizeof(ChunkDesc), d_fcd);
   ENSURE("dec_tabs", (size_t)n * sizeof(DecTables), d_tabs);
@@ -827,8 +840,8 @@ int decode_device(himgcu_ctx *ctx, const uint8_t *d_himg, const unsigned long lo
   ENSURE("dec_lseg", (size_t)n * sizeof(SegRef), d_lseg);
   ENSURE("dec_fseg", (size_t)n * g.rows * sizeof(SegRef), d_fseg);
   ENSURE("lres", (size_t)n * g.lres_stride, d_lres);
-  ENSURE("planes", (size_t)n * g.planes_bytes, d_planes);
   ENSURE("L", (size_t)n * g.nch * g.rows * g.cols, d_R);
+  *f = DecFront{d_fcd, d_ftree, d_tabs, d_fseg, d_R, n == 1 && !ctx->profile};
   const unsigned nb = (unsigned)((n + 127) / 128);
   LAUNCH("k_dec_parse", k_dec_parse, (unsigned)((n + 3) / 4), 128, 0, d_himg, d_offsets, d_sizes, n, g.w, g.h, g.nch, d_lcd,
          d_fcd, d_tabs, d_status);
@@ -837,7 +850,7 @@ int decode_device(himgcu_ctx *ctx, const uint8_t *d_himg, const unsigned long lo
   // segment table -> coefficient planes) share nothing until the inverse transform, so they run on
   // two streams.  Batches fill the GPU on one stream (and device-side event waits are kept out of
   // the multi-context host pipelines, see run_pipeline).
-  const bool fork = n == 1 && !ctx->profile;
+  const bool fork = f->fork;
   cudaStream_t main_stream = ctx->stream;
   if (fork) {
     if (!ctx->aux_stream) {
@@ -877,7 +890,26 @@ int decode_device(himgcu_ctx *ctx, const uint8_t *d_himg, const unsigned long lo
     CK(cudaEventRecord(ctx->ev_join, ctx->aux_stream));
     if (rc_l) CK(cudaStreamWaitEvent(main_stream, ctx->ev_join, 0));
   }
-  if (rc_l) return rc_l;
+  return rc_l;
+}
+
+// Whole-image decode of n streams resident on the device.
+int decode_device(himgcu_ctx *ctx, const uint8_t *d_himg, const unsigned long long *d_offsets,
+                  const uint32_t *d_sizes, int n, const Geom &g, int flags, uint8_t *d_pixels, int *d_status) {
+  const int lenient = (flags & HIMGCU_LENIENT) ? 1 : 0;
+  uint8_t *d_planes;
+  ENSURE("planes", (size_t)n * g.planes_bytes, d_planes);
+  DecFront f;
+  int rc = decode_front(ctx, d_himg, d_offsets, d_sizes, n, g, lenient, d_status, &f);
+  if (rc) return rc;
+  const ChunkDesc *d_fcd = f.fcd;
+  const DecTree *d_ftree = f.ftree;
+  const DecTables *d_tabs = f.tabs;
+  SegRef *d_fseg = f.fseg;
+  const uint8_t *d_R = f.R;
+  const bool fork = f.fork;
+  cudaStream_t main_stream = ctx->stream;
+  const unsigned nb = (unsigned)((n + 127) / 128);
   // a warp per block row when the batch alone fills the GPU, wider teams for few streams
   const int fres_team = decode_team((long long)n * g.rows, g.seg, kParFresThreads);
   // Few streams (single images): the serial walk over the segment headers runs inside the decode kernel
@@ -901,6 +933,69 @@ int decode_device(himgcu_ctx *ctx, const uint8_t *d_himg, const unsigned long lo
   }
   if (fork) CK(cudaStreamWaitEvent(main_stream, ctx->ev_join, 0));
   return stage_inverse(ctx, d_planes, d_R, n, g, d_tabs, sizeof(DecTables), d_pixels);
+}
+
+// Compact block rows a region decode keeps per image: the most a rectangle of rh rows can touch.
+int region_rows(const Geom &g, int rh) { return std::min((rh + 14) / 8, g.rows); }
+
+// K-inv of a region decode (xform_region.cuh) from the compact planes [n][kr][seg].
+int stage_inverse_region(himgcu_ctx *ctx, const uint8_t *d_planes, const uint8_t *d_R, int n, const Geom &g,
+                         const DecTables *d_tabs, const int32_t *d_origins, int rw, int rh, int kr, uint8_t *d_pixels) {
+  // lane-pair fast path: the shapes k_inverse4 takes, except that the rectangle clips rows and columns
+  if (!ctx->force_generic && (g.cols % 16) == 0 && (g.nch == 1 || g.nch == 3) && (reinterpret_cast<uintptr_t>(d_planes) & 15) == 0 &&
+      (reinterpret_cast<uintptr_t>(d_R) & 1) == 0) {
+    InvTables *d_inv;
+    ENSURE("inv_tables", (size_t)n * sizeof(InvTables), d_inv);
+    LAUNCH("k_inv_tables", k_inv_tables, n, 256, 0, d_tabs, (unsigned long long)sizeof(DecTables), d_inv);
+    const int span = region_span_pairs(rw, g.cols);
+    constexpr int TP = kInv4ThreadsRgb;
+    static_assert(kInv4ThreadsGray == TP, "one tile width for both channel counts");
+    dim3 grid((unsigned)(((long long)kr * span + TP - 1) / TP), 1, n);
+    const int smem = g.nch * 64 * 2 * TP + kInvTableBytes;
+    if (g.nch == 1) {
+      CK(cudaFuncSetAttribute((k_inverse_region4<1, TP>), cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
+      LAUNCH("k_inverse_region4", (k_inverse_region4<1, TP>), grid, TP, smem, d_planes, d_R, g, d_inv,
+             (unsigned long long)sizeof(InvTables), d_origins, rw, rh, kr, span, d_pixels, 1u);
+    } else {
+      CK(cudaFuncSetAttribute((k_inverse_region4<3, TP>), cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
+      LAUNCH("k_inverse_region4", (k_inverse_region4<3, TP>), grid, TP, smem, d_planes, d_R, g, d_inv,
+             (unsigned long long)sizeof(InvTables), d_origins, rw, rh, kr, span, d_pixels, 1u);
+    }
+    return HIMGCU_OK;
+  }
+  const int kb = (rw + 14) / 8;
+  LAUNCH("k_inverse_region", k_inverse_region, dim3((kb + kTile - 1) / kTile, kr, n), kTile, 0, d_planes, d_R, g, d_tabs,
+         (unsigned long long)sizeof(DecTables), d_origins, rw, rh, kr, d_pixels);
+  return HIMGCU_OK;
+}
+
+// Region decode of n streams resident on the device: image i's rectangle rw x rh at (d_origins[2i], d_origins[2i+1])
+// to d_pixels + i * rw * rh * nch.  Only the FRES segments of the block rows the rectangle touches are decoded.
+int decode_region_device(himgcu_ctx *ctx, const uint8_t *d_himg, const unsigned long long *d_offsets, const uint32_t *d_sizes,
+                         int n, const Geom &g, int flags, const int32_t *d_origins, int rw, int rh, uint8_t *d_pixels,
+                         int *d_status) {
+  const int lenient = (flags & HIMGCU_LENIENT) ? 1 : 0;
+  const int kr = region_rows(g, rh);
+  uint8_t *d_planes;
+  SegRef *d_rseg;
+  ENSURE("planes", (size_t)n * kr * g.seg, d_planes);
+  ENSURE("dec_rseg", (size_t)n * kr * sizeof(SegRef), d_rseg);
+  DecFront f;
+  int rc = decode_front(ctx, d_himg, d_offsets, d_sizes, n, g, lenient, d_status, &f);
+  if (rc) return rc;
+  const unsigned long long stride = (unsigned long long)kr * g.seg;
+  LAUNCH("k_dec_segtab_region", k_dec_segtab_region, (unsigned)((n + 127) / 128), 128, 0, d_himg, f.fcd, f.ftree, n, g, lenient,
+         d_origins, rw, rh, kr, f.fseg, d_rseg, d_status);
+  const int team = decode_team((long long)n * kr, g.seg, kParFresThreads);
+  if (team == 32) {
+    LAUNCH("k_dec_stream_fres", k_dec_stream_par<true>, dim3((kr + kParWarpTeams - 1) / kParWarpTeams, n), 32 * kParWarpTeams, 0,
+           d_himg, f.fcd, f.ftree, d_rseg, kr, g.seg, d_planes, stride, d_status);
+  } else {
+    LAUNCH("k_dec_stream_fres", k_dec_stream_par<false>, dim3(kr, n), team, 0, d_himg, f.fcd, f.ftree, d_rseg, kr, g.seg,
+           d_planes, stride, d_status);
+  }
+  if (f.fork) CK(cudaStreamWaitEvent(ctx->stream, ctx->ev_join, 0));
+  return stage_inverse_region(ctx, d_planes, f.R, n, g, f.tabs, d_origins, rw, rh, kr, d_pixels);
 }
 
 }  // namespace
@@ -1442,6 +1537,83 @@ int himgcu_decode(himgcu_ctx *ctx, const uint8_t *himg, size_t size, int flags, 
   // costs one wasted copy, an accepted one (the common case) saves a synchronisation.
   CK(cudaMemcpyAsync(h_status, d_status, sizeof(int), cudaMemcpyDeviceToHost, ctx->stream));
   if ((rc = copy_to_host(ctx, out, d_px, g.out_img_bytes))) return rc;
+  if (*h_status) return fail(ctx, HIMGCU_REJECT, "stream rejected");
+  return HIMGCU_OK;
+}
+
+int himgcu_decode_batch_region(himgcu_ctx *ctx, const uint8_t *d_himg, const uint64_t *d_offsets, const uint32_t *d_sizes, int n,
+                               int w, int h, int nch, int flags, const int32_t *d_origins, int rw, int rh, uint8_t *d_pixels_out,
+                               int32_t *d_status) {
+  if (!ctx || !d_himg || !d_offsets || !d_sizes || !d_origins || !d_pixels_out || !d_status || n < 0)
+    return fail(ctx, HIMGCU_ERR_ARG, "bad argument");
+  if (!shape_ok(w, h, nch)) return fail(ctx, HIMGCU_ERR_UNSUPPORTED, "unsupported shape %dx%dx%d", w, h, nch);
+  if (rw < 1 || rh < 1 || rw > w || rh > h) return fail(ctx, HIMGCU_ERR_ARG, "region %dx%d does not fit a %dx%d image", rw, rh, w, h);
+  if (n == 0) return HIMGCU_OK;
+  CK(cudaSetDevice(ctx->device));
+  const Geom g = make_geom(w, h, nch, nch);
+  const int kr = region_rows(g, rh);
+  const size_t out_bytes = (size_t)rw * rh * nch;
+  const size_t per = per_image_encode_ws(g) - g.planes_bytes + (size_t)kr * (g.seg + sizeof(SegRef)) + sizeof(DecTables) +
+                     2 * sizeof(DecTree) + sizeof(InvTables);
+  int sub = (int)std::min<size_t>((size_t)n, std::max<size_t>(1, ctx->max_workspace / per));
+  sub = std::min(sub, 65535);
+  for (int i0 = 0; i0 < n; i0 += sub) {
+    const int m = std::min(sub, n - i0);
+    int rc = decode_region_device(ctx, d_himg, reinterpret_cast<const unsigned long long *>(d_offsets) + i0, d_sizes + i0, m, g,
+                                  flags, d_origins + 2 * (size_t)i0, rw, rh, d_pixels_out + (size_t)i0 * out_bytes, d_status + i0);
+    if (rc) return rc;
+  }
+  return HIMGCU_OK;
+}
+
+int himgcu_decode_region(himgcu_ctx *ctx, const uint8_t *himg, size_t size, int flags, int x, int y, int rw, int rh, uint8_t *out,
+                         size_t out_cap, int *w, int *h, int *nch) {
+  if (!ctx || !himg || !out) return fail(ctx, HIMGCU_ERR_ARG, "bad argument");
+  int W = 0, H = 0, N = 0;
+  if (himgcu_decode_info(himg, size, &W, &H, &N) != HIMGCU_OK) return fail(ctx, HIMGCU_REJECT, "not a HIMG stream");
+  if (w) *w = W;
+  if (h) *h = H;
+  if (nch) *nch = N;
+  if (W < 1 || H < 1 || N < 1) return fail(ctx, HIMGCU_REJECT, "bad dimensions");
+  if (!shape_ok(W, H, N)) return fail(ctx, HIMGCU_ERR_UNSUPPORTED, "unsupported shape %dx%dx%d", W, H, N);
+  if (size > 0xffffffffull) return fail(ctx, HIMGCU_ERR_UNSUPPORTED, "stream too large");
+  if (rw < 1 || rh < 1 || x < 0 || y < 0 || x > W - rw || y > H - rh)
+    return fail(ctx, HIMGCU_ERR_ARG, "region %dx%d at (%d, %d) is empty or outside the %dx%d image", rw, rh, x, y, W, H);
+  CK(cudaSetDevice(ctx->device));
+  const Geom g = make_geom(W, H, N, N);
+  const size_t out_bytes = (size_t)rw * rh * N;
+  if (out_bytes > out_cap) return fail(ctx, HIMGCU_ERR_CAPACITY, "output buffer too small");
+  uint8_t *d_in, *d_px;
+  unsigned long long *d_off;
+  uint32_t *d_sz;
+  int *d_status;
+  int32_t *d_org;
+  ENSURE("single_in", size + 16, d_in);
+  ENSURE("single_rpx", out_bytes, d_px);
+  ENSURE("single_off", sizeof(unsigned long long), d_off);
+  ENSURE("single_size", sizeof(uint32_t), d_sz);
+  ENSURE("single_status", sizeof(int), d_status);
+  ENSURE("single_origin", 2 * sizeof(int32_t), d_org);
+  int rc = ensure_pinned(ctx, 64);
+  if (rc) return rc;
+  // offset / size / status / origin travel through the context's page-locked scratch, as in himgcu_decode
+  unsigned long long *h_off = reinterpret_cast<unsigned long long *>(ctx->pinned);
+  uint32_t *h_sz = reinterpret_cast<uint32_t *>(h_off + 1);
+  int *h_status = reinterpret_cast<int *>(h_off + 2);
+  int32_t *h_org = reinterpret_cast<int32_t *>(h_off + 3);
+  CK(cudaStreamSynchronize(ctx->stream));
+  *h_off = 0;
+  *h_sz = (uint32_t)size;
+  h_org[0] = x;
+  h_org[1] = y;
+  if ((rc = copy_to_device(ctx, d_in, himg, size))) return rc;
+  CK(cudaMemcpyAsync(d_off, h_off, sizeof(*h_off), cudaMemcpyHostToDevice, ctx->stream));
+  CK(cudaMemcpyAsync(d_sz, h_sz, sizeof(*h_sz), cudaMemcpyHostToDevice, ctx->stream));
+  CK(cudaMemcpyAsync(d_org, h_org, 2 * sizeof(int32_t), cudaMemcpyHostToDevice, ctx->stream));
+  rc = decode_region_device(ctx, d_in, d_off, d_sz, 1, g, flags, d_org, rw, rh, d_px, d_status);
+  if (rc) return rc;
+  CK(cudaMemcpyAsync(h_status, d_status, sizeof(int), cudaMemcpyDeviceToHost, ctx->stream));
+  if ((rc = copy_to_host(ctx, out, d_px, out_bytes))) return rc;
   if (*h_status) return fail(ctx, HIMGCU_REJECT, "stream rejected");
   return HIMGCU_OK;
 }

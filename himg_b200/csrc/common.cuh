@@ -61,6 +61,15 @@ __host__ __device__ constexpr int scan_coef(int i) {
 
 __device__ __forceinline__ int clamp255(int x) { return min(max(x, 0), 255); }
 
+// Region decode: origin (x, y) of image i's rw x rh rectangle (origins [n][2], device memory).  False when the
+// rectangle does not lie inside the image (rw, rh >= 1 are checked on the host).
+__device__ __forceinline__ bool region_origin(const int32_t *__restrict__ origins, int i, const Geom &g, int rw, int rh,
+                                              int &x, int &y) {
+  x = origins[2 * i];
+  y = origins[2 * i + 1];
+  return x >= 0 && y >= 0 && x <= g.w - rw && y <= g.h - rh;
+}
+
 // Sequency-ordered 8-point Walsh-Hadamard butterflies (hadamard.cpp:18-44), in place.
 __device__ __forceinline__ void wht8(int &x0, int &x1, int &x2, int &x3, int &x4, int &x5, int &x6,
                                      int &x7) {

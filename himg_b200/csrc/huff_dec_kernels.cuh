@@ -515,6 +515,32 @@ __global__ void k_dec_segtab(const uint8_t *__restrict__ data, const ChunkDesc *
   segtab_walk<false>(data, cd[i], trees + i, nseg, seg_size, mode, lenient, segs + (size_t)i * nseg, status + i);
 }
 
+// Region decode (framed FRES chunk): the segment table of the block rows r0 = y / 8 .. r1 = (y + rh - 1) / 8 that
+// image i's rectangle touches, compacted to kr entries per image: entry k is row min(r0 + k, r1), so a rectangle
+// that touches fewer than kr rows decodes its last row again instead of needing a "skip" entry.  The header
+// chain is walked only to r1 (into the scratch table `full` [n][rows]; the walk has no end-of-chunk check, so
+// these entries are those of a whole-image walk), and at least to row 1 of a multi-row image so that the lenient
+// framing decision ("more than one segment") is the whole image's.  An origin that puts the rectangle outside
+// the image makes the image's status 2 (HIMGCU_ERR_ARG) and all its entries invalid.
+__global__ void k_dec_segtab_region(const uint8_t *__restrict__ data, const ChunkDesc *__restrict__ cd,
+                                    const DecTree *__restrict__ trees, int n, Geom g, int lenient,
+                                    const int32_t *__restrict__ origins, int rw, int rh, int kr,
+                                    SegRef *__restrict__ full, SegRef *__restrict__ segs, int *__restrict__ status) {
+  const int i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= n) return;
+  SegRef *S = segs + (size_t)i * kr;
+  int x, y;
+  if (!region_origin(origins, i, g, rw, rh, x, y)) {
+    for (int k = 0; k < kr; ++k) seg_store<false>(S + k, 0, 0xffffffffu);
+    atomicMax(status + i, 2);
+    return;
+  }
+  const int r0 = y >> 3, r1 = (y + rh - 1) >> 3;
+  SegRef *F = full + (size_t)i * g.rows;
+  segtab_walk<false>(data, cd[i], trees + i, g.rows > 1 ? max(r1 + 1, 2) : 1, g.seg, 1, lenient, F, status + i);
+  for (int k = 0; k < kr; ++k) S[k] = F[min(r0 + k, r1)];
+}
+
 // ---- subsequence-parallel stream decode ---------------------------------------------------------
 // A team of threads (one CTA) decodes ONE stream.  The bit stream is cut into equal subsequences;
 // thread t starts decoding at a guessed position (the subsequence boundary, usually in the middle

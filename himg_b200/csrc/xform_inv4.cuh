@@ -230,14 +230,32 @@ __device__ __forceinline__ void inv4_corners(const uint8_t *__restrict__ R, int 
   }
 }
 
+// Pixel row y of a block pair (wa: the 8 * NCH bytes of block A, wb: those of block B) to dst0 + y * row_bytes
+// as 16-byte stores: whole pairs of a whole image.
+template <int NCH>
+struct Inv4Store16 {
+  uint8_t *dst0;
+  size_t row_bytes;
+  __device__ __forceinline__ void operator()(int y, const uint32_t (&wa)[2 * NCH], const uint32_t (&wb)[2 * NCH]) const {
+    uint4 *dst = reinterpret_cast<uint4 *>(dst0 + (size_t)y * row_bytes);
+    if (NCH == 1) {
+      dst[0] = make_uint4(wa[0], wa[1], wb[0], wb[1]);
+    } else {
+      dst[0] = make_uint4(wa[0], wa[1], wa[2], wa[3]);
+      dst[1] = make_uint4(wa[4], wa[5], wb[0], wb[1]);
+      dst[2] = make_uint4(wb[2], wb[3], wb[4], wb[5]);
+    }
+  }
+};
+
 // The inverse proper for ONE thread = one block pair: codes in the thread's two byte columns `col` of a
 // shared-memory tile whose rows
-// (scan positions, channel-major) are PITCH bytes apart; the image's tables in sDq / sTab; pixels to
-// dst0 (row 0 of the pair) + y * row_bytes.  No barrier inside.
-template <int NCH, int PITCH>
+// (scan positions, channel-major) are PITCH bytes apart; the image's tables in sDq / sTab; pixel row y of
+// the pair goes out through store(y, ...) (active threads only).  No barrier inside.
+template <int NCH, int PITCH, class STORE = Inv4Store16<NCH>>
 __device__ __forceinline__ void inv4_compute(uint8_t *col, const uint8_t *sDq, const uint32_t *sTab, int pre, int tab_bias,
                                              bool overflow, bool ycbcr, bool active, const uint32_t (&top)[NCH],
-                                             const uint32_t (&bot)[NCH], uint8_t *dst0, size_t row_bytes, uint32_t one) {
+                                             const uint32_t (&bot)[NCH], const STORE &store, uint32_t one) {
 #ifdef HIMG_FORCE_PRE3  // (instruction counting only)
   const bool pre3 = true;
 #else
@@ -364,16 +382,7 @@ __device__ __forceinline__ void inv4_compute(uint8_t *col, const uint8_t *sDq, c
         wa[m] = __byte_perm(pq, q, 0x5410);
         wb[m] = __byte_perm(pq, q, 0x7632);
       }
-      if (active) {
-        uint4 *dst = reinterpret_cast<uint4 *>(dst0 + (size_t)y * row_bytes);
-        if (NCH == 1) {
-          dst[0] = make_uint4(wa[0], wa[1], wb[0], wb[1]);
-        } else {
-          dst[0] = make_uint4(wa[0], wa[1], wa[2], wa[3]);
-          dst[1] = make_uint4(wa[4], wa[5], wb[0], wb[1]);
-          dst[2] = make_uint4(wb[2], wb[3], wb[4], wb[5]);
-        }
-      }
+      if (active) store(y, wa, wb);
     }
   }
 }
@@ -455,7 +464,7 @@ __global__ void __launch_bounds__(TP, NCH == 1 ? 3 : 2)
   cp_async_wait_all();
   __syncthreads();  // the only barrier: from here on a thread touches its own two byte columns only
   inv4_compute<NCH, PITCH>(sPl + 2 * t, sDq, sTab, pre, tab_bias, overflow, ycbcr, active, top, bot,
-                           img + ((size_t)(8 * v) * g.w + (size_t)u * 8) * NCH, (size_t)g.w * NCH, one);
+                           Inv4Store16<NCH>{img + ((size_t)(8 * v) * g.w + (size_t)u * 8) * NCH, (size_t)g.w * NCH}, one);
 }
 
 }  // namespace himgcu

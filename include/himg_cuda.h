@@ -101,6 +101,35 @@ int himgcu_decode_batch(himgcu_ctx *ctx, const uint8_t *d_himg, const uint64_t *
                         const uint32_t *d_sizes, int n, int width, int height, int num_channels,
                         int flags, uint8_t *d_pixels_out, int32_t *d_status);
 
+/* ---- region decode: a rectangle [x, x+rw) x [y, y+rh) of an image ------------------------
+ * Pixel (yy, xx) of the output equals pixel (y+yy, x+xx) of himgcu_decode on the same stream with
+ * the same flags, for every shape himgcu_decode accepts; the output is [rh][rw][num_channels]
+ * tightly packed.  The low-res chunk is decoded in full, but of the FRES chunk only the segment
+ * headers up to the rectangle's last 8-pixel block row (at least the first two) and the segments of
+ * the block rows the rectangle touches are read.  Everything a whole decode checks is checked where the region reads
+ * it: the container, the tables, both trees, the low-res stream, the FRES framing decision, those
+ * segment headers and those segments.  So a stream the whole decode accepts is accepted and its
+ * pixels are the crop, and a stream the region decode rejects is rejected by the whole decode too;
+ * a stream whose corruption lies only in rows below the rectangle, or in segments it does not
+ * touch, may decode as a region.
+ *
+ * Single image, host buffers (as himgcu_decode): HIMGCU_ERR_ARG for an empty rectangle or one
+ * outside the image. */
+int himgcu_decode_region(himgcu_ctx *ctx, const uint8_t *himg, size_t size, int flags, int x, int y,
+                         int rw, int rh, uint8_t *out, size_t out_cap, int *width, int *height,
+                         int *num_channels);
+
+/* n same-shaped streams as himgcu_decode_batch, one rectangle size rw x rh for the batch (checked
+ * here: HIMGCU_ERR_ARG if empty or larger than the image) and one origin per image in DEVICE memory
+ * (d_origins[2i] = x, d_origins[2i+1] = y), so that a caller can draw them on the GPU.  Image i's
+ * rectangle goes to d_pixels_out + i*rw*rh*num_channels.  d_status[i]: HIMGCU_OK / HIMGCU_REJECT as
+ * in himgcu_decode_batch, or HIMGCU_ERR_ARG if the origin puts the rectangle outside the image (its
+ * output is then not written).  Asynchronous on the context's stream. */
+int himgcu_decode_batch_region(himgcu_ctx *ctx, const uint8_t *d_himg, const uint64_t *d_offsets,
+                               const uint32_t *d_sizes, int n, int width, int height, int num_channels,
+                               int flags, const int32_t *d_origins, int rw, int rh,
+                               uint8_t *d_pixels_out, int32_t *d_status);
+
 /* ---- batch, HOST pointers (what a file/stream based caller uses; basis of the e2e figure) ----
  * Same work as the device batch calls with the transfers included: pixels (or bitstreams) are
  * copied host->device in sub-batches, coded, and the results copied back.  Pinned host memory

@@ -197,6 +197,28 @@ class Context:
                                                         _ptr(origins), crop_w, crop_h, _ptr(out), _ptr(status)))
         return out, status
 
+    def decode_batch_region_mixed(self, himg, offsets, sizes, dims, nch, origins, crop_w, crop_h, max_w, max_h, flags=STRICT,
+                                  out=None, status=None):
+        """decode_batch_region of streams with their own sizes: dims is a CUDA int32 [n][2] tensor of (width, height),
+        each at most max_w x max_h, and origins one of (x, y).  Returns (pixels [n][crop_h][crop_w][nch], status);
+        status[i] is REJECT where the stream is rejected or its shape is not dims[i] x nch, and ERR_ARG where dims[i]
+        is < 1 or exceeds the bounds or the origin puts the rectangle outside the image (those pixels are not written)."""
+        import torch
+
+        n = offsets.numel()
+        for name, t in (("dims", dims), ("origins", origins)):
+            if t.dtype != torch.int32 or t.numel() != 2 * n:
+                raise ValueError(name + " must be an int32 tensor [n][2]")
+        self._bind(himg, offsets, sizes, dims, origins, out, status)
+        if out is None:
+            out = torch.empty((n, crop_h, crop_w, nch), dtype=torch.uint8, device=himg.device)
+        if status is None:
+            status = torch.empty((n,), dtype=torch.int32, device=himg.device)
+        self._check(self.lib.himgcu_decode_batch_region_mixed(self.h, _ptr(himg), _ptr(offsets), _ptr(sizes), n, _ptr(dims), max_w,
+                                                              max_h, nch, flags, _ptr(origins), crop_w, crop_h, _ptr(out),
+                                                              _ptr(status)))
+        return out, status
+
     # ---- batch, host buffers (numpy arrays or pinned CPU torch tensors) -------------------------
     def encode_batch_host(self, pixels, quality=50, use_ycbcr=True, out=None, offsets=None, sizes=None):
         """pixels: host uint8 [n][h][w][nch].  Returns (out u8 buffer, offsets u64 [n+1], sizes u32 [n])."""

@@ -196,26 +196,6 @@ void resolve_profile(himgcu_ctx *ctx) {
   ctx->pending.clear();
 }
 
-Geom make_geom(int w, int h, int nch, int pstride) {
-  Geom g;
-  g.w = w;
-  g.h = h;
-  g.nch = nch;
-  g.pstride = pstride;
-  g.rows = (h + 7) >> 3;
-  g.cols = (w + 7) >> 3;
-  g.mrows = (g.rows + 15) / 16;
-  g.mcols = (g.cols + 15) / 16;
-  g.seg = g.cols * 64 * nch;
-  g.lres_ch = g.mrows * g.mcols + g.rows * g.cols;
-  g.lres_size = g.lres_ch * nch;
-  g.img_bytes = (unsigned long long)w * h * pstride;
-  g.out_img_bytes = (unsigned long long)w * h * nch;
-  g.lres_stride = ((unsigned long long)g.lres_size + 63) & ~63ull;
-  g.planes_bytes = (unsigned long long)g.rows * g.seg;
-  return g;
-}
-
 bool shape_ok(int w, int h, int nch) {
   if (w < 1 || h < 1 || nch < 1 || nch > 255) return false;  // (the container stores the channel count in one byte)
   const unsigned long long px = (unsigned long long)w * h * nch;
@@ -804,7 +784,7 @@ int launch_stream_cluster(himgcu_ctx *ctx, const char *name, int n, const uint8_
   {
     LaunchScope ls_(ctx, name);
     e = cudaLaunchKernelEx(&cfg, k_dec_stream_par<false, kDecCluster>, d_in, d_cd, d_tree, const_cast<SegRef *>(d_seg), 1, out_seg,
-                           d_out, out_stride, d_status, 0, 0);
+                           d_out, out_stride, d_status, 0, 0, MixedDims{});
   }
   if (e != cudaSuccess) return fail(ctx, HIMGCU_ERR_CUDA, "launch %s failed: %s", name, cudaGetErrorString(e));
   *launched = true;
@@ -824,9 +804,10 @@ struct DecFront {
 // What every decode does before the coefficient planes: container, tables and both trees of n streams, then
 // the low-res branch (segment table, stream, DPCM into R).  The caller ensures its planes buffer before: a
 // workspace that grows is freed after a stream synchronisation, which must not happen while the two branches
-// of a single image run on two streams.
+// of a single image run on two streams.  With `md` the batch has mixed geometry (see MixedDims): g is then the
+// bounding geometry, which sizes the scratch, and the low-res stream of an image is never given to a cluster.
 int decode_front(himgcu_ctx *ctx, const uint8_t *d_himg, const unsigned long long *d_offsets, const uint32_t *d_sizes, int n,
-                 const Geom &g, int lenient, int *d_status, DecFront *f) {
+                 const Geom &g, int lenient, int *d_status, DecFront *f, const MixedDims *md = nullptr) {
   ChunkDesc *d_lcd, *d_fcd;
   DecTables *d_tabs;
   DecTree *d_ltree, *d_ftree;
@@ -843,8 +824,13 @@ int decode_front(himgcu_ctx *ctx, const uint8_t *d_himg, const unsigned long lon
   ENSURE("L", (size_t)n * g.nch * g.rows * g.cols, d_R);
   *f = DecFront{d_fcd, d_ftree, d_tabs, d_fseg, d_R, n == 1 && !ctx->profile};
   const unsigned nb = (unsigned)((n + 127) / 128);
-  LAUNCH("k_dec_parse", k_dec_parse, (unsigned)((n + 3) / 4), 128, 0, d_himg, d_offsets, d_sizes, n, g.w, g.h, g.nch, d_lcd,
-         d_fcd, d_tabs, d_status);
+  if (md) {
+    LAUNCH("k_dec_parse", k_dec_parse<true>, (unsigned)((n + 3) / 4), 128, 0, d_himg, d_offsets, d_sizes, n, g.w, g.h, g.nch, d_lcd,
+           d_fcd, d_tabs, d_status, *md);
+  } else {
+    LAUNCH("k_dec_parse", k_dec_parse, (unsigned)((n + 3) / 4), 128, 0, d_himg, d_offsets, d_sizes, n, g.w, g.h, g.nch, d_lcd,
+           d_fcd, d_tabs, d_status);
+  }
   LAUNCH("k_dec_tree", k_dec_tree, dim3(n, 2), kDecTreeThreads, 0, d_himg, d_lcd, d_fcd, lenient, d_ltree, d_ftree, d_status);
   // A single image is a chain of latency-bound kernels: its two branches (low-res stream -> DPCM, and
   // segment table -> coefficient planes) share nothing until the inverse transform, so they run on
@@ -869,19 +855,27 @@ int decode_front(himgcu_ctx *ctx, const uint8_t *d_himg, const unsigned long lon
     // wider teams (or a cluster of CTAs) when there are few streams (single images).
     const int lres_team = decode_team(n, g.lres_size, kParLresThreads);
     bool clustered = false;
-    if (use_decode_cluster(n, g.lres_size) && !ctx->force_generic) {
+    if (!md && use_decode_cluster(n, g.lres_size) && !ctx->force_generic) {
       int rc = launch_stream_cluster(ctx, "k_dec_stream_lres", n, d_himg, d_lcd, d_ltree, d_lseg, g.lres_size, d_lres,
                                      (unsigned long long)g.lres_stride, d_status, &clustered);
       if (rc) return rc;
     }
-    if (!clustered) {
+    if (md) {
+      LAUNCH("k_dec_stream_lres", (k_dec_stream_par<false, 1, kMixLres>), dim3(1, n), lres_team, 0, d_himg, d_lcd, d_ltree, d_lseg,
+             1, g.lres_size, d_lres, g.lres_stride, d_status, 0, 0, *md);
+    } else if (!clustered) {
       LAUNCH("k_dec_stream_lres", k_dec_stream_par<false>, dim3(1, n), lres_team, 0, d_himg, d_lcd, d_ltree, d_lseg, 1,
              g.lres_size, d_lres, g.lres_stride, d_status);
     }
     const long long nmb = (long long)n * g.nch * g.mrows * g.mcols;
     const unsigned blocks = (unsigned)((nmb + kLresWarps * 2 - 1) / (kLresWarps * 2));
-    LAUNCH("k_lres_dpcm_dec", (k_lres_dpcm<false>), blocks, kLresWarps * 32, 0, (const uint8_t *)nullptr, d_lres, d_R,
-           g, n, (const uint8_t *)nullptr, d_tabs->low_unmap, (unsigned long long)sizeof(DecTables));
+    if (md) {
+      LAUNCH("k_lres_dpcm_dec", (k_lres_dpcm<false, true>), blocks, kLresWarps * 32, 0, (const uint8_t *)nullptr, d_lres, d_R,
+             g, n, (const uint8_t *)nullptr, d_tabs->low_unmap, (unsigned long long)sizeof(DecTables), *md);
+    } else {
+      LAUNCH("k_lres_dpcm_dec", (k_lres_dpcm<false>), blocks, kLresWarps * 32, 0, (const uint8_t *)nullptr, d_lres, d_R,
+             g, n, (const uint8_t *)nullptr, d_tabs->low_unmap, (unsigned long long)sizeof(DecTables));
+    }
     return HIMGCU_OK;
   };
   int rc_l = lres_branch();
@@ -938,9 +932,17 @@ int decode_device(himgcu_ctx *ctx, const uint8_t *d_himg, const unsigned long lo
 // Compact block rows a region decode keeps per image: the most a rectangle of rh rows can touch.
 int region_rows(const Geom &g, int rh) { return std::min((rh + 14) / 8, g.rows); }
 
-// K-inv of a region decode (xform_region.cuh) from the compact planes [n][kr][seg].
+// K-inv of a region decode (xform_region.cuh) from the compact planes [n][kr][seg].  A mixed-geometry batch (md) takes
+// the generic kernel.
 int stage_inverse_region(himgcu_ctx *ctx, const uint8_t *d_planes, const uint8_t *d_R, int n, const Geom &g,
-                         const DecTables *d_tabs, const int32_t *d_origins, int rw, int rh, int kr, uint8_t *d_pixels) {
+                         const DecTables *d_tabs, const int32_t *d_origins, int rw, int rh, int kr, uint8_t *d_pixels,
+                         const MixedDims *md = nullptr) {
+  const int kb = (rw + 14) / 8;
+  if (md) {
+    LAUNCH("k_inverse_region", k_inverse_region<true>, dim3((kb + kTile - 1) / kTile, kr, n), kTile, 0, d_planes, d_R, g, d_tabs,
+           (unsigned long long)sizeof(DecTables), d_origins, rw, rh, kr, d_pixels, *md);
+    return HIMGCU_OK;
+  }
   // lane-pair fast path: the shapes k_inverse4 takes, except that the rectangle clips rows and columns
   if (!ctx->force_generic && (g.cols % 16) == 0 && (g.nch == 1 || g.nch == 3) && (reinterpret_cast<uintptr_t>(d_planes) & 15) == 0 &&
       (reinterpret_cast<uintptr_t>(d_R) & 1) == 0) {
@@ -963,7 +965,6 @@ int stage_inverse_region(himgcu_ctx *ctx, const uint8_t *d_planes, const uint8_t
     }
     return HIMGCU_OK;
   }
-  const int kb = (rw + 14) / 8;
   LAUNCH("k_inverse_region", k_inverse_region, dim3((kb + kTile - 1) / kTile, kr, n), kTile, 0, d_planes, d_R, g, d_tabs,
          (unsigned long long)sizeof(DecTables), d_origins, rw, rh, kr, d_pixels);
   return HIMGCU_OK;
@@ -971,9 +972,10 @@ int stage_inverse_region(himgcu_ctx *ctx, const uint8_t *d_planes, const uint8_t
 
 // Region decode of n streams resident on the device: image i's rectangle rw x rh at (d_origins[2i], d_origins[2i+1])
 // to d_pixels + i * rw * rh * nch.  Only the FRES segments of the block rows the rectangle touches are decoded.
+// With `md` the batch has mixed geometry and g is its bounding geometry (see MixedDims).
 int decode_region_device(himgcu_ctx *ctx, const uint8_t *d_himg, const unsigned long long *d_offsets, const uint32_t *d_sizes,
                          int n, const Geom &g, int flags, const int32_t *d_origins, int rw, int rh, uint8_t *d_pixels,
-                         int *d_status) {
+                         int *d_status, const MixedDims *md = nullptr) {
   const int lenient = (flags & HIMGCU_LENIENT) ? 1 : 0;
   const int kr = region_rows(g, rh);
   uint8_t *d_planes;
@@ -981,12 +983,25 @@ int decode_region_device(himgcu_ctx *ctx, const uint8_t *d_himg, const unsigned 
   ENSURE("planes", (size_t)n * kr * g.seg, d_planes);
   ENSURE("dec_rseg", (size_t)n * kr * sizeof(SegRef), d_rseg);
   DecFront f;
-  int rc = decode_front(ctx, d_himg, d_offsets, d_sizes, n, g, lenient, d_status, &f);
+  int rc = decode_front(ctx, d_himg, d_offsets, d_sizes, n, g, lenient, d_status, &f, md);
   if (rc) return rc;
   const unsigned long long stride = (unsigned long long)kr * g.seg;
+  const int team = decode_team((long long)n * kr, g.seg, kParFresThreads);
+  if (md) {
+    LAUNCH("k_dec_segtab_region", k_dec_segtab_region<true>, (unsigned)((n + 127) / 128), 128, 0, d_himg, f.fcd, f.ftree, n, g,
+           lenient, d_origins, rw, rh, kr, f.fseg, d_rseg, d_status, *md);
+    if (team == 32) {
+      LAUNCH("k_dec_stream_fres", (k_dec_stream_par<true, 1, kMixFres>), dim3((kr + kParWarpTeams - 1) / kParWarpTeams, n),
+             32 * kParWarpTeams, 0, d_himg, f.fcd, f.ftree, d_rseg, kr, g.seg, d_planes, stride, d_status, 0, 0, *md);
+    } else {
+      LAUNCH("k_dec_stream_fres", (k_dec_stream_par<false, 1, kMixFres>), dim3(kr, n), team, 0, d_himg, f.fcd, f.ftree, d_rseg, kr,
+             g.seg, d_planes, stride, d_status, 0, 0, *md);
+    }
+    if (f.fork) CK(cudaStreamWaitEvent(ctx->stream, ctx->ev_join, 0));
+    return stage_inverse_region(ctx, d_planes, f.R, n, g, f.tabs, d_origins, rw, rh, kr, d_pixels, md);
+  }
   LAUNCH("k_dec_segtab_region", k_dec_segtab_region, (unsigned)((n + 127) / 128), 128, 0, d_himg, f.fcd, f.ftree, n, g, lenient,
          d_origins, rw, rh, kr, f.fseg, d_rseg, d_status);
-  const int team = decode_team((long long)n * kr, g.seg, kParFresThreads);
   if (team == 32) {
     LAUNCH("k_dec_stream_fres", k_dec_stream_par<true>, dim3((kr + kParWarpTeams - 1) / kParWarpTeams, n), 32 * kParWarpTeams, 0,
            d_himg, f.fcd, f.ftree, d_rseg, kr, g.seg, d_planes, stride, d_status);
@@ -1561,6 +1576,36 @@ int himgcu_decode_batch_region(himgcu_ctx *ctx, const uint8_t *d_himg, const uin
     const int m = std::min(sub, n - i0);
     int rc = decode_region_device(ctx, d_himg, reinterpret_cast<const unsigned long long *>(d_offsets) + i0, d_sizes + i0, m, g,
                                   flags, d_origins + 2 * (size_t)i0, rw, rh, d_pixels_out + (size_t)i0 * out_bytes, d_status + i0);
+    if (rc) return rc;
+  }
+  return HIMGCU_OK;
+}
+
+int himgcu_decode_batch_region_mixed(himgcu_ctx *ctx, const uint8_t *d_himg, const uint64_t *d_offsets, const uint32_t *d_sizes,
+                                     int n, const int32_t *d_dims, int max_width, int max_height, int nch, int flags,
+                                     const int32_t *d_origins, int rw, int rh, uint8_t *d_pixels_out, int32_t *d_status) {
+  if (!ctx || !d_himg || !d_offsets || !d_sizes || !d_dims || !d_origins || !d_pixels_out || !d_status || n < 0)
+    return fail(ctx, HIMGCU_ERR_ARG, "bad argument");
+  if (!shape_ok(max_width, max_height, nch))
+    return fail(ctx, HIMGCU_ERR_UNSUPPORTED, "unsupported bounding shape %dx%dx%d", max_width, max_height, nch);
+  if (rw < 1 || rh < 1 || rw > max_width || rh > max_height)
+    return fail(ctx, HIMGCU_ERR_ARG, "region %dx%d does not fit the %dx%d bounds", rw, rh, max_width, max_height);
+  if (n == 0) return HIMGCU_OK;
+  CK(cudaSetDevice(ctx->device));
+  // every per-image scratch slot has the bounding geometry's size; the kernels lay each image out in its own
+  const Geom g = make_geom(max_width, max_height, nch, nch);
+  const int kr = region_rows(g, rh);
+  const size_t out_bytes = (size_t)rw * rh * nch;
+  const size_t per = per_image_encode_ws(g) - g.planes_bytes + (size_t)kr * (g.seg + sizeof(SegRef)) + sizeof(DecTables) +
+                     2 * sizeof(DecTree);
+  int sub = (int)std::min<size_t>((size_t)n, std::max<size_t>(1, ctx->max_workspace / per));
+  sub = std::min(sub, 65535);
+  for (int i0 = 0; i0 < n; i0 += sub) {
+    const int m = std::min(sub, n - i0);
+    const MixedDims md{d_dims + 2 * (size_t)i0, max_width, max_height, nch};
+    int rc = decode_region_device(ctx, d_himg, reinterpret_cast<const unsigned long long *>(d_offsets) + i0, d_sizes + i0, m, g,
+                                  flags, d_origins + 2 * (size_t)i0, rw, rh, d_pixels_out + (size_t)i0 * out_bytes, d_status + i0,
+                                  &md);
     if (rc) return rc;
   }
   return HIMGCU_OK;

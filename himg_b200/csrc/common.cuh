@@ -59,6 +59,43 @@ __host__ __device__ constexpr int scan_coef(int i) {
   return 0;
 }
 
+__host__ __device__ inline Geom make_geom(int w, int h, int nch, int pstride) {
+  Geom g;
+  g.w = w;
+  g.h = h;
+  g.nch = nch;
+  g.pstride = pstride;
+  g.rows = (h + 7) >> 3;
+  g.cols = (w + 7) >> 3;
+  g.mrows = (g.rows + 15) / 16;
+  g.mcols = (g.cols + 15) / 16;
+  g.seg = g.cols * 64 * nch;
+  g.lres_ch = g.mrows * g.mcols + g.rows * g.cols;
+  g.lres_size = g.lres_ch * nch;
+  g.img_bytes = (unsigned long long)w * h * pstride;
+  g.out_img_bytes = (unsigned long long)w * h * nch;
+  g.lres_stride = ((unsigned long long)g.lres_size + 63) & ~63ull;
+  g.planes_bytes = (unsigned long long)g.rows * g.seg;
+  return g;
+}
+
+// Mixed-geometry batch: image i is dims[2i] x dims[2i+1] (device memory), bounded by max_w x max_h.  Every
+// per-image scratch buffer keeps the slot stride of the bounding geometry make_geom(max_w, max_h, nch); inside
+// its slot an image is laid out with its own geometry.
+struct MixedDims {
+  const int32_t *dims;
+  int max_w, max_h, nch;
+};
+
+// Geometry of image i of a mixed batch.  False when its dims are < 1 or exceed the bounds: the image is then
+// HIMGCU_ERR_ARG and nothing of it is decoded (gi is a 1 x 1 placeholder).
+__device__ __forceinline__ bool image_geom(const MixedDims &m, int i, Geom &gi) {
+  const int w = m.dims[2 * i], h = m.dims[2 * i + 1];
+  const bool ok = w >= 1 && h >= 1 && w <= m.max_w && h <= m.max_h;
+  gi = make_geom(ok ? w : 1, ok ? h : 1, m.nch, m.nch);
+  return ok;
+}
+
 __device__ __forceinline__ int clamp255(int x) { return min(max(x, 0), 255); }
 
 // Region decode: origin (x, y) of image i's rw x rh rectangle (origins [n][2], device memory).  False when the

@@ -113,13 +113,23 @@ __device__ __forceinline__ bool parse_mapfun_warp(const uint8_t *in, int size, i
 // grid: ceil(n / 4) x 128 threads; one WARP per image: lane 0 walks the RIFF chunk headers (a short chain of
 // dependent loads), then the lanes parse the three tables side by side -- one thread doing it all was 125 us
 // for a batch, whatever its size, and the first 26 us of every single-image decode.
+// MIXED: the FRMT shape is checked against image i's dims of `md` (w, h are then unused), and dims that are < 1 or
+// exceed the bounds make the image's status 2 (HIMGCU_ERR_ARG) and its chunks invalid.
+template <bool MIXED = false>
 __global__ void __launch_bounds__(128)
     k_dec_parse(const uint8_t *__restrict__ data, const unsigned long long *__restrict__ offsets,
                 const uint32_t *__restrict__ sizes, int n, int w, int h, int nch,
                 ChunkDesc *__restrict__ lres, ChunkDesc *__restrict__ fres,
-                DecTables *__restrict__ tabs, int *__restrict__ status) {
+                DecTables *__restrict__ tabs, int *__restrict__ status, MixedDims md = {}) {
   const int i = (int)((blockIdx.x * blockDim.x + threadIdx.x) >> 5), lane = threadIdx.x & 31;
   if (i >= n) return;
+  bool bad_dims = false;
+  if (MIXED) {
+    Geom gi;
+    bad_dims = !image_geom(md, i, gi);
+    w = gi.w;
+    h = gi.h;
+  }
   const unsigned long long base = offsets[i];
   const uint8_t *p = data + base;
   const long long size = sizes[i];
@@ -130,6 +140,7 @@ __global__ void __launch_bounds__(128)
   int ok = 0;
   if (lane == 0) {
     ok = 1;
+    if (MIXED && bad_dims) ok = 0;
     if (size < 12 || rd_u32(p) != 0x46464952u /*RIFF*/ || rd_u32(p + 8) != 0x474d4948u /*HIMG*/) ok = 0;
     if (ok && (long long)(int)rd_u32(p + 4) + 8 != size) ok = 0;
     long long idx = 12;
@@ -192,7 +203,7 @@ __global__ void __launch_bounds__(128)
     fres[i].off = base + (ok ? (unsigned long long)coff[5] : 0ull);
     fres[i].size = ok ? (uint32_t)csz[5] : 0u;
     fres[i].ok = ok ? 1u : 0u;
-    status[i] = ok ? 0 : 1;
+    status[i] = MIXED && bad_dims ? 2 : (ok ? 0 : 1);
   }
 }
 
@@ -522,22 +533,28 @@ __global__ void k_dec_segtab(const uint8_t *__restrict__ data, const ChunkDesc *
 // these entries are those of a whole-image walk), and at least to row 1 of a multi-row image so that the lenient
 // framing decision ("more than one segment") is the whole image's.  An origin that puts the rectangle outside
 // the image makes the image's status 2 (HIMGCU_ERR_ARG) and all its entries invalid.
+// MIXED: g is the bounding geometry (the stride of `full`); image i's header chain and origin are those of its own
+// geometry from `md`, and dims out of bounds are treated as an origin outside the image.
+template <bool MIXED = false>
 __global__ void k_dec_segtab_region(const uint8_t *__restrict__ data, const ChunkDesc *__restrict__ cd,
                                     const DecTree *__restrict__ trees, int n, Geom g, int lenient,
                                     const int32_t *__restrict__ origins, int rw, int rh, int kr,
-                                    SegRef *__restrict__ full, SegRef *__restrict__ segs, int *__restrict__ status) {
+                                    SegRef *__restrict__ full, SegRef *__restrict__ segs, int *__restrict__ status,
+                                    MixedDims md = {}) {
   const int i = blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= n) return;
   SegRef *S = segs + (size_t)i * kr;
+  Geom gi = g;
+  const bool dims_ok = !MIXED || image_geom(md, i, gi);
   int x, y;
-  if (!region_origin(origins, i, g, rw, rh, x, y)) {
+  if (!dims_ok || !region_origin(origins, i, gi, rw, rh, x, y)) {
     for (int k = 0; k < kr; ++k) seg_store<false>(S + k, 0, 0xffffffffu);
     atomicMax(status + i, 2);
     return;
   }
   const int r0 = y >> 3, r1 = (y + rh - 1) >> 3;
   SegRef *F = full + (size_t)i * g.rows;
-  segtab_walk<false>(data, cd[i], trees + i, g.rows > 1 ? max(r1 + 1, 2) : 1, g.seg, 1, lenient, F, status + i);
+  segtab_walk<false>(data, cd[i], trees + i, gi.rows > 1 ? max(r1 + 1, 2) : 1, gi.seg, 1, lenient, F, status + i);
   for (int k = 0; k < kr; ++k) S[k] = F[min(r0 + k, r1)];
 }
 
@@ -657,11 +674,14 @@ constexpr int kParWarpTeams = 8;  // WARP_TEAMS: streams (one warp each) per CTA
 //   flags and scan totals are exchanged through distributed shared memory, team barriers are
 //   cluster barriers.  This is what a single large image needs: its low-res chunk is ONE stream,
 //   and one CTA (one SM) was the whole machine for it.
-template <bool WARP_TEAMS, int CL = 1>
+// MIX (mixed-geometry batches, one CTA per stream or warp teams, no inline walk): the output size of a stream is
+//   its image's own (from `md`): the low-res chunk (kMixLres) or a block row (kMixFres); out_seg is unused.
+constexpr int kMixLres = 1, kMixFres = 2;
+template <bool WARP_TEAMS, int CL = 1, int MIX = 0>
 __global__ void k_dec_stream_par(const uint8_t *__restrict__ data, const ChunkDesc *__restrict__ cd,
                                  const DecTree *__restrict__ trees, SegRef *__restrict__ segs, int nseg,
                                  int out_seg, uint8_t *__restrict__ out, unsigned long long out_stride,
-                                 int *__restrict__ status, int inline_walk = 0, int lenient = 0) {
+                                 int *__restrict__ status, int inline_walk = 0, int lenient = 0, MixedDims md = {}) {
   __shared__ __align__(16) uint2 lut2[kLutSize];  // the single-token LUT stays in global memory (rare path)
   __shared__ uint32_t s_nodes[kMaxNodes + 1];
   __shared__ uint32_t s_sub[kSubCap << kSubBits];
@@ -673,8 +693,15 @@ __global__ void k_dec_stream_par(const uint8_t *__restrict__ data, const ChunkDe
   // than eight warps (wide teams for a few large streams) write their literals directly
   __shared__ uint32_t s_line[kParWarpTeams * 8 * 32];
   static_assert(!(WARP_TEAMS && CL > 1), "clusters are for the one-stream-per-team variant");
+  static_assert(MIX == 0 || CL == 1, "mixed geometry has no cluster decode");
   namespace cg = cooperative_groups;
   const int item = blockIdx.y;
+  if (MIX) {  // (an image with dims out of bounds has an invalid chunk: its tree is not ok and nothing is written)
+    Geom gi;
+    image_geom(md, item, gi);
+    out_seg = MIX == kMixLres ? gi.lres_size : gi.seg;
+    inline_walk = 0;
+  }
   // inline_walk (one CTA per stream only): CTA 0 of every item walks the segment headers of the framed
   // chunk and publishes the table (see segtab_walk); the stream of CTA x is segment x - 1
   if (!WARP_TEAMS && CL == 1 && inline_walk && blockIdx.x == 0) {

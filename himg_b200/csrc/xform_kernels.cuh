@@ -193,13 +193,17 @@ struct LowResTables {
 
 constexpr int kLresWarps = 4;
 
-template <bool ENCODE>
+// MIXED (decode of a mixed-geometry batch): g is the bounding geometry, which sets the grid and the slot strides
+// (lres_stride and nch * rows * cols bytes per image); image img's macroblocks and its layout inside the slots are
+// those of its own geometry from `md`.  Macroblocks outside it, and images with dims out of bounds, are idle.
+template <bool ENCODE, bool MIXED = false>
 __global__ void __launch_bounds__(kLresWarps * 32)
     k_lres_dpcm(const uint8_t *__restrict__ Lin,   // ENCODE: L [n][nch][rows][cols]; else unused
                 uint8_t *__restrict__ lres,        // ENCODE: out; DECODE: in  ([n][lres_stride])
                 uint8_t *__restrict__ Rout,        // DECODE: R [n][nch][rows][cols]
                 Geom g, int n, const uint8_t *__restrict__ map_lut, const int16_t *__restrict__ unmap,
-                unsigned long long unmap_stride) {
+                unsigned long long unmap_stride, MixedDims md = {}) {
+  static_assert(!(ENCODE && MIXED), "mixed geometry is decode only");
   __shared__ uint8_t sL[kLresWarps * 2][16][16];
   __shared__ uint8_t sR[kLresWarps * 2][16][17];
   // The codes of a macroblock are contiguous in memory but the wavefront touches them along
@@ -209,7 +213,7 @@ __global__ void __launch_bounds__(kLresWarps * 32)
   const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5, half = lane >> 4, hl = lane & 15;
   const long long nmb = (long long)n * g.nch * g.mrows * g.mcols;
   const long long mb = ((long long)blockIdx.x * kLresWarps + wid) * 2 + half;
-  const bool active = mb < nmb;
+  bool active = mb < nmb;
   const int slot = wid * 2 + half;
   int img = 0, c = 0, mv = 0, mu = 0;
   if (active) {
@@ -221,18 +225,24 @@ __global__ void __launch_bounds__(kLresWarps * 32)
     c = (int)(t % g.nch);
     img = (int)(t / g.nch);
   }
-  const int bh = min(16, g.rows - 16 * mv), bw = min(16, g.cols - 16 * mu);
+  Geom gi = g;  // image img's geometry
+  if (MIXED) {
+    active = active && image_geom(md, img, gi) && mv < gi.mrows && mu < gi.mcols;
+    if (!active) mv = mu = 0;
+  }
+  const int bh = min(16, gi.rows - 16 * mv), bw = min(16, gi.cols - 16 * mu);
   const int16_t *un = reinterpret_cast<const int16_t *>(reinterpret_cast<const char *>(unmap) + (size_t)img * unmap_stride);
-  const size_t plane = ((size_t)img * g.nch + c) * g.rows * g.cols;
-  uint8_t *chan = lres + (size_t)img * g.lres_stride + (size_t)c * g.lres_ch;
-  uint8_t *selp = chan + mv * g.mcols + mu;
-  uint8_t *dp = chan + g.mrows * g.mcols + (size_t)mv * 16 * g.cols + (size_t)mu * 16 * bh;
+  const size_t plane = MIXED ? (size_t)img * g.nch * g.rows * g.cols + (size_t)c * gi.rows * gi.cols
+                             : ((size_t)img * g.nch + c) * g.rows * g.cols;
+  uint8_t *chan = lres + (size_t)img * g.lres_stride + (size_t)c * gi.lres_ch;
+  uint8_t *selp = chan + mv * gi.mcols + mu;
+  uint8_t *dp = chan + gi.mrows * gi.mcols + (size_t)mv * 16 * gi.cols + (size_t)mu * 16 * bh;
 
   int p = 0;
   if (ENCODE) {
     // stage the macroblock (row hl) and pick the predictor
     if (active && hl < bw)  // lane = column: every load instruction reads one row of consecutive bytes
-      for (int dv = 0; dv < bh; ++dv) sL[slot][dv][hl] = __ldg(Lin + plane + (size_t)(16 * mv + dv) * g.cols + 16 * mu + hl);
+      for (int dv = 0; dv < bh; ++dv) sL[slot][dv][hl] = __ldg(Lin + plane + (size_t)(16 * mv + dv) * gi.cols + 16 * mu + hl);
     __syncwarp();
     int err[5] = {0, 0, 0, 0, 0};
     if (active && hl < bh) {
@@ -312,7 +322,7 @@ __global__ void __launch_bounds__(kLresWarps * 32)
     if (ENCODE) {
       for (int i = hl; i < bh * bw; i += 16) dp[i] = sC[slot][i];
     } else if (hl < bw) {
-      for (int dv = 0; dv < bh; ++dv) Rout[plane + (size_t)(16 * mv + dv) * g.cols + 16 * mu + hl] = sR[slot][dv][hl];
+      for (int dv = 0; dv < bh; ++dv) Rout[plane + (size_t)(16 * mv + dv) * gi.cols + 16 * mu + hl] = sR[slot][dv][hl];
     }
   }
 }

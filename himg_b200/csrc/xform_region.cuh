@@ -133,16 +133,22 @@ __global__ void __launch_bounds__(TP, NCH == 1 ? 3 : 2)
 
 // grid (ceil(kb / kTile), kr, n), block kTile (kb = (rw + 14) / 8 block columns): thread = block column x / 8 + i of
 // compact slot blockIdx.y.  Same arithmetic as k_inverse.
+// MIXED: g is the bounding geometry, which sets the slot strides (kr * g.seg bytes of planes and nch * rows * cols
+// bytes of R per image); image item's planes (kr segments of its own size), low-res image, corners and origin check
+// use its own geometry from `md`.  An image with dims out of bounds is not written.
+template <bool MIXED = false>
 __global__ void __launch_bounds__(kTile)
     k_inverse_region(const uint8_t *__restrict__ planes, const uint8_t *__restrict__ R, Geom g,
                      const DecTables *__restrict__ tabs, unsigned long long tab_stride, const int32_t *__restrict__ origins,
-                     int rw, int rh, int kr, uint8_t *__restrict__ pixels) {
+                     int rw, int rh, int kr, uint8_t *__restrict__ pixels, MixedDims md = {}) {
   __shared__ int16_t sUn[256];
   __shared__ uint8_t sShift[2][64];
   __shared__ uint32_t sOut[3][kTile][17];  // channels 0-2 of a thread's block (the colour map needs all three)
   const int item = blockIdx.z, slot = blockIdx.y;
+  Geom gi = g;  // the image's geometry
+  if (MIXED && !image_geom(md, item, gi)) return;
   int x, y;
-  if (!region_origin(origins, item, g, rw, rh, x, y)) return;  // (the whole CTA)
+  if (!region_origin(origins, item, gi, rw, rh, x, y)) return;  // (the whole CTA)
   const int v = (y >> 3) + slot;
   if (v > (y + rh - 1) >> 3) return;  // a repeated slot
   const DecTables *T = reinterpret_cast<const DecTables *>(reinterpret_cast<const char *>(tabs) + (size_t)item * tab_stride);
@@ -153,7 +159,7 @@ __global__ void __launch_bounds__(kTile)
   __syncthreads();
   const int u = (x >> 3) + blockIdx.x * kTile + threadIdx.x;
   if (u > (x + rw - 1) >> 3) return;
-  const uint8_t *seg = planes + ((size_t)item * kr + slot) * g.seg;
+  const uint8_t *seg = MIXED ? planes + (size_t)item * kr * g.seg + (size_t)slot * gi.seg : planes + ((size_t)item * kr + slot) * g.seg;
   uint8_t *img = pixels + (size_t)item * rw * rh * nch;
   // pixels of the block inside the rectangle: rows [ya, yb), columns [xa, xb) of the block
   const int ya = max(0, y - 8 * v), yb = min(8, y + rh - 8 * v), xa = max(0, x - 8 * u), xb = min(8, x + rw - 8 * u);
@@ -162,10 +168,10 @@ __global__ void __launch_bounds__(kTile)
 #pragma unroll 1
   for (int c = 0; c < nch; ++c) {
     int xv[64];
-    const uint8_t *src = seg + (size_t)c * g.cols * 64 + u;
+    const uint8_t *src = seg + (size_t)c * gi.cols * 64 + u;
     const uint8_t *sh = sShift[(ycbcr && (c == 1 || c == 2)) ? 1 : 0];
 #pragma unroll
-    for (int j = 0; j < 64; ++j) xv[j] = (int)(short)(sUn[__ldg(src + (size_t)scan_pos(j) * g.cols)] * (1 << sh[j]));
+    for (int j = 0; j < 64; ++j) xv[j] = (int)(short)(sUn[__ldg(src + (size_t)scan_pos(j) * gi.cols)] * (1 << sh[j]));
 #pragma unroll
     for (int r = 0; r < 8; ++r) {
       wht8(xv[r * 8 + 0], xv[r * 8 + 1], xv[r * 8 + 2], xv[r * 8 + 3], xv[r * 8 + 4], xv[r * 8 + 5], xv[r * 8 + 6], xv[r * 8 + 7]);
@@ -179,7 +185,9 @@ __global__ void __launch_bounds__(kTile)
       for (int i = 0; i < 8; ++i) xv[i * 8 + q] >>= 3;
     }
     {
-      const LowCorners k = load_corners(R + ((size_t)item * nch + c) * g.rows * g.cols, g, u, v);
+      const LowCorners k =
+          load_corners(MIXED ? R + (size_t)item * nch * g.rows * g.cols + (size_t)c * gi.rows * gi.cols : R + ((size_t)item * nch + c) * g.rows * g.cols,
+                       gi, u, v);
       int lf[9], rt[9];
       nine(k.x11, k.x21, lf);
       nine(k.x12, k.x22, rt);

@@ -130,6 +130,22 @@ int himgcu_decode_batch_region(himgcu_ctx *ctx, const uint8_t *d_himg, const uin
                                int flags, const int32_t *d_origins, int rw, int rh,
                                uint8_t *d_pixels_out, int32_t *d_status);
 
+/* n streams of one channel count but each of its own size, as a data loader reads them: d_dims[2i]
+ * = width, d_dims[2i+1] = height of image i (DEVICE memory, as d_origins).  max_width x max_height
+ * (host) bounds every image and sizes the workspace (HIMGCU_ERR_UNSUPPORTED if it is not a shape
+ * himgcu_decode_batch takes).  One rectangle size rw x rh for the batch (HIMGCU_ERR_ARG if empty or
+ * larger than the bounds), origins as in himgcu_decode_batch_region; image i's rectangle goes to
+ * d_pixels_out + i*rw*rh*num_channels.  Image i's output and status are those of
+ * himgcu_decode_region on its stream alone with the same origin and flags, and a batch whose dims
+ * are all equal gives what himgcu_decode_batch_region gives.  d_status[i]: HIMGCU_OK; HIMGCU_REJECT
+ * where the stream is rejected, including a FRMT shape other than its dims and num_channels; or
+ * HIMGCU_ERR_ARG when its dims are < 1 or exceed the bounds, or the origin puts the rectangle
+ * outside the image (its output is then not written).  Asynchronous on the context's stream. */
+int himgcu_decode_batch_region_mixed(himgcu_ctx *ctx, const uint8_t *d_himg, const uint64_t *d_offsets,
+                                     const uint32_t *d_sizes, int n, const int32_t *d_dims, int max_width,
+                                     int max_height, int num_channels, int flags, const int32_t *d_origins,
+                                     int rw, int rh, uint8_t *d_pixels_out, int32_t *d_status);
+
 /* ---- batch, HOST pointers (what a file/stream based caller uses; basis of the e2e figure) ----
  * Same work as the device batch calls with the transfers included: pixels (or bitstreams) are
  * copied host->device in sub-batches, coded, and the results copied back.  Pinned host memory

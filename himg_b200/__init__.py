@@ -219,6 +219,32 @@ class Context:
                                                               _ptr(status)))
         return out, status
 
+    def encode_batch_mixed(self, pixels, offsets, dims, nch, max_w, max_h, quality=50, use_ycbcr=True, out=None, sizes=None):
+        """encode_batch of images with their own sizes: pixels is a flat CUDA uint8 buffer holding image i as
+        [h_i][w_i][nch] at byte offsets[i] (int64 [n]), dims a CUDA int32 [n][2] tensor of (w_i, h_i), each at most
+        max_w x max_h.  Returns (out [n][stride] u8, sizes [n] i32); image i's stream is what encode_batch gives for it
+        alone.  sizes[i] is 0 where dims[i] is < 1 or exceeds the bounds (encode_status then raises ERR_ARG) or the
+        stream does not fit the stride (ERR_CAPACITY); nothing is written to such an image's row of out."""
+        import torch
+
+        n = offsets.numel()
+        if pixels.dtype != torch.uint8:
+            raise ValueError("pixels must be uint8")
+        if offsets.dtype != torch.int64:
+            raise ValueError("offsets must be an int64 tensor [n]")
+        if dims.dtype != torch.int32 or dims.numel() != 2 * n:
+            raise ValueError("dims must be an int32 tensor [n][2]")
+        self._bind(pixels, offsets, dims, out, sizes)
+        stride = (encode_bound(max_w, max_h, nch) + 255) & ~255
+        if out is None:
+            out = torch.empty((n, stride), dtype=torch.uint8, device=pixels.device)
+        if sizes is None:
+            sizes = torch.empty((n,), dtype=torch.int32, device=pixels.device)
+        self._check(self.lib.himgcu_encode_batch_mixed(self.h, _ptr(pixels), _ptr(offsets), _ptr(dims), n, max_w, max_h, nch,
+                                                       quality, int(use_ycbcr), _ptr(out), out.stride(0),
+                                                       _ptr(sizes)))
+        return out, sizes
+
     # ---- batch, host buffers (numpy arrays or pinned CPU torch tensors) -------------------------
     def encode_batch_host(self, pixels, quality=50, use_ycbcr=True, out=None, offsets=None, sizes=None):
         """pixels: host uint8 [n][h][w][nch].  Returns (out u8 buffer, offsets u64 [n+1], sizes u32 [n])."""

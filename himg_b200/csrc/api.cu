@@ -307,11 +307,17 @@ QuantParams make_quant(const EncodeTables &t) {
 // ---- stage launchers (device pointers, asynchronous) -------------------------------------------
 
 // cbase / ctotal: the channel group [cbase, cbase + NCH) of an image with ctotal channels (see k_lowres_avg);
-// d_pixels points at the group's first channel.
+// d_pixels points at the group's first channel.  With `md` the batch has mixed geometry (g is the bounding one) and
+// image i starts at d_pixels + px_off[i].
 template <int NCH>
 int launch_avg(himgcu_ctx *ctx, const uint8_t *d_pixels, int n, const Geom &g, bool ycbcr, uint8_t *d_avg, int cbase = 0,
-               int ctotal = NCH) {
+               int ctotal = NCH, const MixedDims *md = nullptr, const unsigned long long *px_off = nullptr) {
   dim3 grid((g.cols + kTile - 1) / kTile, g.rows, n);
+  if (md) {
+    if (ycbcr) LAUNCH("k_lowres_avg", (k_lowres_avg<NCH, true, true>), grid, kTile, 0, d_pixels, g, d_avg, cbase, ctotal, *md, px_off);
+    else LAUNCH("k_lowres_avg", (k_lowres_avg<NCH, false, true>), grid, kTile, 0, d_pixels, g, d_avg, cbase, ctotal, *md, px_off);
+    return HIMGCU_OK;
+  }
   if (ycbcr) LAUNCH("k_lowres_avg", (k_lowres_avg<NCH, true>), grid, kTile, 0, d_pixels, g, d_avg, cbase, ctotal);
   else LAUNCH("k_lowres_avg", (k_lowres_avg<NCH, false>), grid, kTile, 0, d_pixels, g, d_avg, cbase, ctotal);
   return HIMGCU_OK;
@@ -328,13 +334,15 @@ int launch_avg2(himgcu_ctx *ctx, const uint8_t *d_pixels, int n, const Geom &g, 
   return HIMGCU_OK;
 }
 
-int stage_lowres(himgcu_ctx *ctx, const uint8_t *d_pixels, int n, const Geom &g, bool ycbcr, uint8_t *d_L) {
+// With `md` the batch has mixed geometry (see launch_avg) and takes the generic kernels.
+int stage_lowres(himgcu_ctx *ctx, const uint8_t *d_pixels, int n, const Geom &g, bool ycbcr, uint8_t *d_L,
+                 const MixedDims *md = nullptr, const unsigned long long *px_off = nullptr) {
   uint8_t *d_avg;
   const size_t nlow = (size_t)n * g.nch * g.rows * g.cols;
   ENSURE("avg", nlow, d_avg);
   int rc;
   // lane-pair fast path: whole 16-pixel block pairs, tightly packed pixels, 16-byte aligned rows
-  const bool fast = !ctx->force_generic && !(ctx->xform_variant & 1) && g.pstride == g.nch && (g.w % 16) == 0 &&
+  const bool fast = !md && !ctx->force_generic && !(ctx->xform_variant & 1) && g.pstride == g.nch && (g.w % 16) == 0 &&
                     (reinterpret_cast<uintptr_t>(d_pixels) & 15) == 0 && (g.img_bytes & 15) == 0 &&
                     (reinterpret_cast<uintptr_t>(d_avg) & 1) == 0 && (g.nch == 1 || g.nch == 3 || g.nch == 4);
   if (fast) {
@@ -345,19 +353,20 @@ int stage_lowres(himgcu_ctx *ctx, const uint8_t *d_pixels, int n, const Geom &g,
     }
   } else
   switch (g.nch) {
-    case 1: rc = launch_avg<1>(ctx, d_pixels, n, g, false, d_avg); break;
-    case 2: rc = launch_avg<2>(ctx, d_pixels, n, g, false, d_avg); break;
-    case 3: rc = launch_avg<3>(ctx, d_pixels, n, g, ycbcr, d_avg); break;
-    case 4: rc = launch_avg<4>(ctx, d_pixels, n, g, ycbcr, d_avg); break;
+    case 1: rc = launch_avg<1>(ctx, d_pixels, n, g, false, d_avg, 0, 1, md, px_off); break;
+    case 2: rc = launch_avg<2>(ctx, d_pixels, n, g, false, d_avg, 0, 2, md, px_off); break;
+    case 3: rc = launch_avg<3>(ctx, d_pixels, n, g, ycbcr, d_avg, 0, 3, md, px_off); break;
+    case 4: rc = launch_avg<4>(ctx, d_pixels, n, g, ycbcr, d_avg, 0, 4, md, px_off); break;
     default:  // more than four channels: the first three, then one launch per further channel
-      rc = launch_avg<3>(ctx, d_pixels, n, g, ycbcr, d_avg, 0, g.nch);
-      for (int c = 3; c < g.nch && !rc; ++c) rc = launch_avg<1>(ctx, d_pixels + c, n, g, false, d_avg, c, g.nch);
+      rc = launch_avg<3>(ctx, d_pixels, n, g, ycbcr, d_avg, 0, g.nch, md, px_off);
+      for (int c = 3; c < g.nch && !rc; ++c) rc = launch_avg<1>(ctx, d_pixels + c, n, g, false, d_avg, c, g.nch, md, px_off);
       break;
   }
   if (rc) return rc;
   const int threads = std::min(256, (g.cols + 31) & ~31);
-  LAUNCH("k_lowres_comp", k_lowres_comp, dim3((unsigned)(n * g.nch), (g.rows + kCompRows - 1) / kCompRows), threads, 0, d_avg,
-         n * g.nch, g.rows, g.cols, d_L);
+  const dim3 grid((unsigned)(n * g.nch), (g.rows + kCompRows - 1) / kCompRows);
+  if (md) LAUNCH("k_lowres_comp", k_lowres_comp<true>, grid, threads, 0, d_avg, n * g.nch, g.rows, g.cols, d_L, *md);
+  else LAUNCH("k_lowres_comp", k_lowres_comp<false>, grid, threads, 0, d_avg, n * g.nch, g.rows, g.cols, d_L);
   return HIMGCU_OK;
 }
 
@@ -384,12 +393,18 @@ int upload_lowres_tables(himgcu_ctx *ctx, const EncodeTables *enc, const int16_t
   return HIMGCU_OK;
 }
 
-int stage_lres_encode(himgcu_ctx *ctx, const uint8_t *d_L, int n, const Geom &g, const EncodeTables &t, uint8_t *d_lres) {
+int stage_lres_encode(himgcu_ctx *ctx, const uint8_t *d_L, int n, const Geom &g, const EncodeTables &t, uint8_t *d_lres,
+                      const MixedDims *md = nullptr) {
   LowResTables *d_tabs;
   int rc = upload_lowres_tables(ctx, &t, nullptr, &d_tabs);
   if (rc) return rc;
   const long long nmb = (long long)n * g.nch * g.mrows * g.mcols;
   const unsigned blocks = (unsigned)((nmb + kLresWarps * 2 - 1) / (kLresWarps * 2));
+  if (md) {
+    LAUNCH("k_lres_dpcm_enc", (k_lres_dpcm<true, true>), blocks, kLresWarps * 32, 0, d_L, d_lres, (uint8_t *)nullptr, g, n,
+           d_tabs->map_lut, d_tabs->unmap, (unsigned long long)0, *md);
+    return HIMGCU_OK;
+  }
   LAUNCH("k_lres_dpcm_enc", (k_lres_dpcm<true>), blocks, kLresWarps * 32, 0, d_L, d_lres, (uint8_t *)nullptr, g, n,
          d_tabs->map_lut, d_tabs->unmap, (unsigned long long)0);
   return HIMGCU_OK;
@@ -397,9 +412,17 @@ int stage_lres_encode(himgcu_ctx *ctx, const uint8_t *d_L, int n, const Geom &g,
 
 template <int NCH>
 int launch_fwd(himgcu_ctx *ctx, const uint8_t *d_pixels, const uint8_t *d_L, int n, const Geom &g, bool ycbcr,
-               const QuantParams &qp, uint8_t *d_planes, int cbase = 0, int ctotal = NCH) {
+               const QuantParams &qp, uint8_t *d_planes, int cbase = 0, int ctotal = NCH, const MixedDims *md = nullptr,
+               const unsigned long long *px_off = nullptr) {
   dim3 grid((g.cols + kTile - 1) / kTile, g.rows, n);
   const uint8_t *lut = (const uint8_t *)ctx->full_lut.p;
+  if (md) {
+    if (ycbcr)
+      LAUNCH("k_forward", (k_forward<NCH, true, true>), grid, kTile, 0, d_pixels, d_L, g, qp, lut, d_planes, cbase, ctotal, *md, px_off);
+    else
+      LAUNCH("k_forward", (k_forward<NCH, false, true>), grid, kTile, 0, d_pixels, d_L, g, qp, lut, d_planes, cbase, ctotal, *md, px_off);
+    return HIMGCU_OK;
+  }
   if (ycbcr) LAUNCH("k_forward", (k_forward<NCH, true>), grid, kTile, 0, d_pixels, d_L, g, qp, lut, d_planes, cbase, ctotal);
   else LAUNCH("k_forward", (k_forward<NCH, false>), grid, kTile, 0, d_pixels, d_L, g, qp, lut, d_planes, cbase, ctotal);
   return HIMGCU_OK;
@@ -428,10 +451,12 @@ int launch_fwd3(himgcu_ctx *ctx, const uint8_t *d_pixels, const uint8_t *d_L, in
   return HIMGCU_OK;
 }
 
+// With `md` the batch has mixed geometry (see launch_avg) and takes the generic kernels.
 int stage_forward(himgcu_ctx *ctx, const uint8_t *d_pixels, const uint8_t *d_L, int n, const Geom &g,
-                  const EncodeTables &t, uint8_t *d_planes) {
+                  const EncodeTables &t, uint8_t *d_planes, const MixedDims *md = nullptr,
+                  const unsigned long long *px_off = nullptr) {
   // fast path: whole 16-pixel-wide block pairs, tightly packed pixels, 16-byte aligned rows
-  if (!ctx->force_generic && !(ctx->xform_variant & 1) && g.pstride == g.nch && (g.w % 16) == 0 && (g.h % 8) == 0 &&
+  if (!md && !ctx->force_generic && !(ctx->xform_variant & 1) && g.pstride == g.nch && (g.w % 16) == 0 && (g.h % 8) == 0 &&
       (reinterpret_cast<uintptr_t>(d_pixels) & 15) == 0 && (reinterpret_cast<uintptr_t>(d_L) & 1) == 0 &&
       (g.nch == 1 || g.nch == 3 || g.nch == 4)) {
     Fwd3Params P;
@@ -454,14 +479,15 @@ int stage_forward(himgcu_ctx *ctx, const uint8_t *d_pixels, const uint8_t *d_L, 
   if (rc) return rc;
   const QuantParams qp = make_quant(t);
   switch (g.nch) {
-    case 1: return launch_fwd<1>(ctx, d_pixels, d_L, n, g, false, qp, d_planes);
-    case 2: return launch_fwd<2>(ctx, d_pixels, d_L, n, g, false, qp, d_planes);
-    case 3: return launch_fwd<3>(ctx, d_pixels, d_L, n, g, t.ycbcr, qp, d_planes);
-    case 4: return launch_fwd<4>(ctx, d_pixels, d_L, n, g, t.ycbcr, qp, d_planes);
+    case 1: return launch_fwd<1>(ctx, d_pixels, d_L, n, g, false, qp, d_planes, 0, 1, md, px_off);
+    case 2: return launch_fwd<2>(ctx, d_pixels, d_L, n, g, false, qp, d_planes, 0, 2, md, px_off);
+    case 3: return launch_fwd<3>(ctx, d_pixels, d_L, n, g, t.ycbcr, qp, d_planes, 0, 3, md, px_off);
+    case 4: return launch_fwd<4>(ctx, d_pixels, d_L, n, g, t.ycbcr, qp, d_planes, 0, 4, md, px_off);
     default: break;
   }
-  rc = launch_fwd<3>(ctx, d_pixels, d_L, n, g, t.ycbcr, qp, d_planes, 0, g.nch);
-  for (int c = 3; c < g.nch && !rc; ++c) rc = launch_fwd<1>(ctx, d_pixels + c, d_L, n, g, false, qp, d_planes, c, g.nch);
+  rc = launch_fwd<3>(ctx, d_pixels, d_L, n, g, t.ycbcr, qp, d_planes, 0, g.nch, md, px_off);
+  for (int c = 3; c < g.nch && !rc; ++c)
+    rc = launch_fwd<1>(ctx, d_pixels + c, d_L, n, g, false, qp, d_planes, c, g.nch, md, px_off);
   return rc;
 }
 
@@ -546,10 +572,14 @@ struct HuffChunkArgs {
   int size_patch;
 };
 
+// With `md` the items are the images of a mixed-geometry batch (chunk 0 LRES, chunk 1 FRES, each HuffGeom the
+// bounding one; see MixedHuff).  Their chunks have no parts, and force_generic does not apply: the first-generation
+// coder has no mixed variant.
 int huff_encode_items(himgcu_ctx *ctx, int n, HuffChunkArgs *chunks, int nchunks, bool riff, uint8_t *d_out,
-                      size_t out_stride, uint32_t *d_sizes) {
+                      size_t out_stride, uint32_t *d_sizes, const MixedDims *md = nullptr) {
+  const bool generic = ctx->force_generic && !md;
   // Device error flag of the encoder (5: code longer than 32 bits, 4: output does not fit, 99: internal
-  // mismatch).  Sticky per context: cleared when it is read (take_enc_err), not per call, so that an
+  // mismatch, kEncErrDims: dims out of bounds in a mixed batch).  Sticky per context: cleared when it is read (take_enc_err), not per call, so that an
   // error in an earlier sub-batch of an asynchronous call is not lost.
   int *d_err;
   const bool fresh = ctx->bufs.find("enc_err") == ctx->bufs.end() || ctx->bufs["enc_err"].p == nullptr;
@@ -596,7 +626,7 @@ int huff_encode_items(himgcu_ctx *ctx, int n, HuffChunkArgs *chunks, int nchunks
     // CTA per block row and only get parts when even those are few (measured: more parts cost more
     // in the layout and look-back steps than they gain)
     const long long ctas = (long long)n * hg.nseg, fill = hg.nseg == 1 ? 148 * 8 : 148 * 2;
-    if (!ctx->force_generic && ctas < fill && hg.seg_size > 2 * kTokPiece) {
+    if (!generic && !md && ctas < fill && hg.seg_size > 2 * kTokPiece) {
       const int want = (int)std::min<long long>(64, (fill + ctas - 1) / ctas);
       const int sub = (int)((((long long)hg.seg_size + want - 1) / want + kTokPiece - 1) / kTokPiece) * kTokPiece;
       hg.sub_size = sub;
@@ -606,7 +636,7 @@ int huff_encode_items(himgcu_ctx *ctx, int n, HuffChunkArgs *chunks, int nchunks
     // when the segments fill every SM with warps: a single 8K image (1024 segments) measured 0.52 ms encode
     // with a CTA per segment, 0.88 ms with a warp per segment.
     const long long wave = 148LL * kTeamWarps * kP4MinCtas;  // resident warps of k_huff_pack4
-    teams[k] = !ctx->force_generic && hg.nseg > 1 && hg.nsub == 1 &&
+    teams[k] = !generic && hg.nseg > 1 && hg.nsub == 1 &&
                (ctx->huff_warp_teams == 2 || (ctx->huff_warp_teams == 1 && (long long)n * hg.nseg >= wave));
     const std::string tag = chunks[k].tag;
     ENSURE((tag + "_seghist").c_str(), (size_t)n * hg.nseg * hg.nsub * kSyms * sizeof(uint32_t), d_seghist[k]);
@@ -618,7 +648,7 @@ int huff_encode_items(himgcu_ctx *ctx, int n, HuffChunkArgs *chunks, int nchunks
     // item lists of the pieces, handed from the histogram pass to the packer (see ItemLists)
     ItemLists &il = lists[k];
     il = ItemLists{nullptr, nullptr, nullptr, 0};
-    if (!ctx->force_generic && ctx->item_lists) {
+    if (!generic && ctx->item_lists) {
       const int ppp = (hg.sub_size + kTokPiece - 1) / kTokPiece;
       const size_t slots = (size_t)n * hg.nseg * hg.nsub * ppp;
       ENSURE((tag + "_itpos").c_str(), slots * kItemCap * sizeof(unsigned short), il.pos);
@@ -628,15 +658,20 @@ int huff_encode_items(himgcu_ctx *ctx, int n, HuffChunkArgs *chunks, int nchunks
     }
     ENSURE((tag + "_partbits").c_str(), (size_t)n * hg.nseg * hg.nsub * sizeof(uint32_t), d_pbits[k]);
     uint32_t *d_total = nullptr;
-    if (!ctx->force_generic) {  // chunk histograms summed by the histogram kernel itself
+    if (!generic) {  // chunk histograms summed by the histogram kernel itself
       ENSURE((tag + "_histtotal").c_str(), (size_t)n * kSyms * sizeof(uint32_t), d_total);
       CK(cudaMemsetAsync(d_total, 0, (size_t)n * kSyms * sizeof(uint32_t), ctx->stream));
     }
-    if (ctx->force_generic) LAUNCH("k_huff_hist", k_huff_hist, grid, kHuffThreads, 0, chunks[k].d_in, hg, d_seghist[k]);
+    const dim3 team_grid((hg.nseg + kTeamWarps - 1) / kTeamWarps, n);
+    if (md) {
+      const MixedHuff mh{*md, k};
+      if (teams[k])
+        LAUNCH("k_huff_hist", k_huff_hist4<true>, team_grid, kTeamThreads, 0, chunks[k].d_in, hg, d_seghist[k], il, d_total, mh);
+      else LAUNCH("k_huff_hist", k_huff_hist2<true>, grid, kTokThreads, 0, chunks[k].d_in, hg, d_seghist[k], il, d_total, mh);
+    } else if (generic) LAUNCH("k_huff_hist", k_huff_hist, grid, kHuffThreads, 0, chunks[k].d_in, hg, d_seghist[k]);
     else if (teams[k])
-      LAUNCH("k_huff_hist", k_huff_hist4, dim3((hg.nseg + kTeamWarps - 1) / kTeamWarps, n), kTeamThreads, 0, chunks[k].d_in,
-             hg, d_seghist[k], il, d_total);
-    else LAUNCH("k_huff_hist", k_huff_hist2, grid, kTokThreads, 0, chunks[k].d_in, hg, d_seghist[k], il, d_total);
+      LAUNCH("k_huff_hist", k_huff_hist4<false>, team_grid, kTeamThreads, 0, chunks[k].d_in, hg, d_seghist[k], il, d_total);
+    else LAUNCH("k_huff_hist", k_huff_hist2<false>, grid, kTokThreads, 0, chunks[k].d_in, hg, d_seghist[k], il, d_total);
     TP.total[k] = d_total;
     TP.seghist[k] = d_seghist[k];
     TP.trees[k] = d_trees[k];
@@ -661,25 +696,43 @@ int huff_encode_items(himgcu_ctx *ctx, int n, HuffChunkArgs *chunks, int nchunks
     const int rows = chunks[k].hg.nseg * chunks[k].hg.nsub;
     LAUNCH("k_huff_layout", k_huff_segbits, dim3((rows + 7) / 8, n), 256, 0, d_seghist[k], d_trees[k], rows, d_pbits[k]);
   }
-  LAUNCH("k_huff_layout", k_huff_layout, n, kLayoutThreads, 0, P);
+  if (md) LAUNCH("k_huff_layout", k_huff_layout_mixed, n, kLayoutThreads, 0, P, *md, ContainerTemplate::kDimsAt);
+  else LAUNCH("k_huff_layout", k_huff_layout, n, kLayoutThreads, 0, P);
   const size_t win_bytes = (kWinWords + 2) * sizeof(uint32_t);
-  if (ctx->force_generic)  // static + dynamic shared memory of the first-generation packer exceed 48 KiB
+  if (generic)  // static + dynamic shared memory of the first-generation packer exceed 48 KiB
     CK(cudaFuncSetAttribute(k_huff_pack, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)win_bytes));
-  if (teams[0] || teams[1]) CK(cudaFuncSetAttribute(k_huff_pack4, cudaFuncAttributeMaxDynamicSharedMemorySize, kP4Smem));
+  if (teams[0] || teams[1]) {
+    if (md) CK(cudaFuncSetAttribute(k_huff_pack4<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, kP4Smem));
+    else CK(cudaFuncSetAttribute(k_huff_pack4<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, kP4Smem));
+  }
   for (int k = 0; k < nchunks; ++k) {
     const HuffGeom &hg = chunks[k].hg;
     dim3 grid(hg.nseg * hg.nsub, n);
-    if (ctx->force_generic)
+    if (md) {
+      const MixedHuff mh{*md, k};
+      if (teams[k])
+        LAUNCH("k_huff_pack", k_huff_pack4<true>, dim3((hg.nseg + kTeamWarps - 1) / kTeamWarps, n), kTeamThreads, kP4Smem,
+               chunks[k].d_in, hg, d_trees[k], d_bits[k], d_pos[k], d_sizes, d_out, (unsigned long long)out_stride, d_err, lists[k],
+               mh);
+      else
+        LAUNCH("k_huff_pack", k_huff_pack3<true>, grid, kTokThreads, 0, chunks[k].d_in, hg, d_trees[k], d_bits[k], d_pos[k],
+               d_part[k], d_sizes, d_out, (unsigned long long)out_stride, d_err, lists[k], mh);
+      if (hg.nseg > 1)
+        LAUNCH("k_huff_stale", k_huff_stale<true>, dim3((hg.nseg + 255) / 256, n), 256, 0, n, hg.nseg, d_bits[k], d_pos[k], d_sizes,
+               d_out, (unsigned long long)out_stride, *md);
+      continue;
+    }
+    if (generic)
       LAUNCH("k_huff_pack", k_huff_pack, grid, kHuffThreads, win_bytes, chunks[k].d_in, hg, d_trees[k], d_bits[k],
              d_pos[k], d_sizes, d_out, (unsigned long long)out_stride, d_err);
     else if (teams[k])
-      LAUNCH("k_huff_pack", k_huff_pack4, dim3((hg.nseg + kTeamWarps - 1) / kTeamWarps, n), kTeamThreads, kP4Smem, chunks[k].d_in,
+      LAUNCH("k_huff_pack", k_huff_pack4<false>, dim3((hg.nseg + kTeamWarps - 1) / kTeamWarps, n), kTeamThreads, kP4Smem, chunks[k].d_in,
              hg, d_trees[k], d_bits[k], d_pos[k], d_sizes, d_out, (unsigned long long)out_stride, d_err, lists[k]);
     else
-      LAUNCH("k_huff_pack", k_huff_pack3, grid, kTokThreads, 0, chunks[k].d_in, hg, d_trees[k], d_bits[k], d_pos[k],
+      LAUNCH("k_huff_pack", k_huff_pack3<false>, grid, kTokThreads, 0, chunks[k].d_in, hg, d_trees[k], d_bits[k], d_pos[k],
              d_part[k], d_sizes, d_out, (unsigned long long)out_stride, d_err, lists[k]);
     if (hg.nseg > 1) {
-      LAUNCH("k_huff_stale", k_huff_stale, dim3((hg.nseg + 255) / 256, n), 256, 0, n, hg.nseg, d_bits[k], d_pos[k], d_sizes,
+      LAUNCH("k_huff_stale", k_huff_stale<false>, dim3((hg.nseg + 255) / 256, n), 256, 0, n, hg.nseg, d_bits[k], d_pos[k], d_sizes,
              d_out, (unsigned long long)out_stride);
     }
   }
@@ -699,6 +752,7 @@ int read_err_flag(himgcu_ctx *ctx, const char *name, int *value) {
 int enc_err_status(himgcu_ctx *ctx, int err) {
   if (err == 5) return fail(ctx, HIMGCU_ERR_UNSUPPORTED, "Huffman code longer than 32 bits");
   if (err == 99) return fail(ctx, HIMGCU_ERR_CUDA, "internal: packed size mismatch");
+  if (err == kEncErrDims) return fail(ctx, HIMGCU_ERR_ARG, "image dims below 1 or above the bounds");
   if (err) return fail(ctx, HIMGCU_ERR_CAPACITY, "internal output bound exceeded");
   return HIMGCU_OK;
 }
@@ -711,9 +765,11 @@ size_t per_image_encode_ws(const Geom &g) {
              (kItemCap * 3 + 4);
 }
 
-// Whole-image encode of a sub-batch already resident on the device.
+// Whole-image encode of a sub-batch already resident on the device.  With `md` the batch has mixed geometry: g is
+// the bounding geometry, image i starts at d_pixels + px_off[i] and has its own size (see MixedDims).
 int encode_device(himgcu_ctx *ctx, const uint8_t *d_pixels, int n, const Geom &g, int quality, bool ycbcr,
-                  uint8_t *d_out, size_t out_stride, uint32_t *d_sizes) {
+                  uint8_t *d_out, size_t out_stride, uint32_t *d_sizes, const MixedDims *md = nullptr,
+                  const unsigned long long *px_off = nullptr) {
   EncodeTables t;
   BuildEncodeTables(quality, ycbcr, &t);
   ContainerTemplate ct;
@@ -722,11 +778,11 @@ int encode_device(himgcu_ctx *ctx, const uint8_t *d_pixels, int n, const Geom &g
   ENSURE("L", (size_t)n * g.nch * g.rows * g.cols, d_L);
   ENSURE("lres", (size_t)n * g.lres_stride, d_lres);
   ENSURE("planes", (size_t)n * g.planes_bytes, d_planes);
-  int rc = stage_lowres(ctx, d_pixels, n, g, ycbcr, d_L);
+  int rc = stage_lowres(ctx, d_pixels, n, g, ycbcr, d_L, md, px_off);
   if (rc) return rc;
-  rc = stage_lres_encode(ctx, d_L, n, g, t, d_lres);
+  rc = stage_lres_encode(ctx, d_L, n, g, t, d_lres, md);
   if (rc) return rc;
-  rc = stage_forward(ctx, d_pixels, d_L, n, g, t, d_planes);
+  rc = stage_forward(ctx, d_pixels, d_L, n, g, t, d_planes, md, px_off);
   if (rc) return rc;
   HuffChunkArgs ch[2];
   ch[0].d_in = d_lres;
@@ -739,7 +795,7 @@ int encode_device(himgcu_ctx *ctx, const uint8_t *d_pixels, int n, const Geom &g
   ch[1].tag = "fres";
   ch[1].prefix = ct.mid;
   ch[1].size_patch = (int)ct.mid.size() - 4;
-  return huff_encode_items(ctx, n, ch, 2, true, d_out, out_stride, d_sizes);
+  return huff_encode_items(ctx, n, ch, 2, true, d_out, out_stride, d_sizes, md);
 }
 
 // Threads per stream for k_dec_stream_par: grow the team until ~128k threads are in flight, but keep
@@ -1345,6 +1401,30 @@ int himgcu_encode_batch(himgcu_ctx *ctx, const uint8_t *d_pixels, int n, int w, 
     const int m = std::min(sub, n - i0);
     int rc = encode_device(ctx, d_pixels + (size_t)i0 * g.img_bytes, m, g, quality, ycbcr,
                            d_out + (size_t)i0 * out_stride, out_stride, d_sizes + i0);
+    if (rc) return rc;
+  }
+  return HIMGCU_OK;
+}
+
+int himgcu_encode_batch_mixed(himgcu_ctx *ctx, const uint8_t *d_pixels, const uint64_t *d_pixel_offsets, const int32_t *d_dims,
+                              int n, int max_width, int max_height, int nch, int quality, int use_ycbcr, uint8_t *d_out,
+                              size_t out_stride, uint32_t *d_sizes) {
+  if (!ctx || !d_pixels || !d_pixel_offsets || !d_dims || !d_out || !d_sizes || n < 0) return fail(ctx, HIMGCU_ERR_ARG, "bad argument");
+  if (!shape_ok(max_width, max_height, nch))
+    return fail(ctx, HIMGCU_ERR_UNSUPPORTED, "unsupported bounding shape %dx%dx%d", max_width, max_height, nch);
+  if (n == 0) return HIMGCU_OK;
+  CK(cudaSetDevice(ctx->device));
+  // every per-image scratch slot has the bounding geometry's size; the kernels lay each image out in its own
+  const Geom g = make_geom(max_width, max_height, nch, nch);
+  const bool ycbcr = use_ycbcr && nch >= 3;
+  const size_t per = per_image_encode_ws(g);
+  int sub = (int)std::min<size_t>((size_t)n, std::max<size_t>(1, ctx->max_workspace / per));
+  sub = std::min(sub, 65535);
+  for (int i0 = 0; i0 < n; i0 += sub) {
+    const int m = std::min(sub, n - i0);
+    const MixedDims md{d_dims + 2 * (size_t)i0, max_width, max_height, nch};
+    int rc = encode_device(ctx, d_pixels, m, g, quality, ycbcr, d_out + (size_t)i0 * out_stride, out_stride, d_sizes + i0, &md,
+                           reinterpret_cast<const unsigned long long *>(d_pixel_offsets) + i0);
     if (rc) return rc;
   }
   return HIMGCU_OK;

@@ -88,7 +88,7 @@ struct MixedDims {
 };
 
 // Geometry of image i of a mixed batch.  False when its dims are < 1 or exceed the bounds: the image is then
-// HIMGCU_ERR_ARG and nothing of it is decoded (gi is a 1 x 1 placeholder).
+// HIMGCU_ERR_ARG and nothing of it is decoded or encoded (gi is a 1 x 1 placeholder).
 __device__ __forceinline__ bool image_geom(const MixedDims &m, int i, Geom &gi) {
   const int w = m.dims[2 * i], h = m.dims[2 * i + 1];
   const bool ok = w >= 1 && h >= 1 && w <= m.max_w && h <= m.max_h;

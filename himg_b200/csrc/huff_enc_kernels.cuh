@@ -42,6 +42,31 @@ struct HuffGeom {
   int sub_size;
 };
 
+// Mixed-geometry batch (encode): the chunk of item i belongs to an image of its own size, laid out with its own
+// geometry at the start of a slot of the bounding geometry.  The kernels keep the bounding HuffGeom for the slot
+// strides of every per-segment table (nseg, nsub) and take the item's own chunk geometry from mixed_chunk: the LRES
+// chunk is one unframed segment of gi.lres_size bytes, the FRES chunk gi.rows segments of gi.seg bytes.  Mixed
+// chunks have no parts (nsub = 1).  Segments past an item's own, and every segment of an image whose dims are out of
+// bounds, are idle: the histogram pass writes zero rows for them and nothing reads or writes their bytes.
+struct MixedHuff {
+  MixedDims md;
+  int fres;  // 0: the LRES chunk, 1: the FRES chunk
+};
+// Item `item`'s chunk geometry (hg: the bounding one on entry).  False when the image's dims are out of bounds.
+__device__ __forceinline__ bool mixed_chunk(const MixedHuff &m, int item, HuffGeom &hg) {
+  Geom gi;
+  const bool ok = image_geom(m.md, item, gi);
+  if (m.fres) {
+    hg.seg_size = hg.sub_size = gi.seg;
+    hg.nseg = gi.rows;
+    hg.in_size = gi.rows * gi.seg;
+  } else {
+    hg.seg_size = hg.sub_size = hg.in_size = gi.lres_size;
+    hg.nseg = 1;
+  }
+  return ok;
+}
+
 struct TreeOut {
   uint32_t code[kSyms];
   uint32_t hist[kSyms];
@@ -319,10 +344,11 @@ __device__ __forceinline__ size_t item_slot(const ItemLists &L, const HuffGeom &
   return ((size_t)item * hg.nseg * hg.nsub + blockIdx.x) * L.pieces_per_part + piece;
 }
 
-// grid (nseg * nsub, n), block kTokThreads.  seghist: [n][nseg * nsub][261].
+// grid (nseg * nsub, n), block kTokThreads.  seghist: [n][nseg * nsub][261].  MIXED: see MixedHuff.
+template <bool MIXED = false>
 __global__ void __launch_bounds__(kTokThreads, 8)
     k_huff_hist2(const uint8_t *__restrict__ in, HuffGeom hg, uint32_t *__restrict__ seghist, ItemLists lists,
-                 uint32_t *__restrict__ total) {
+                 uint32_t *__restrict__ total, MixedHuff mh = {}) {
   __shared__ uint32_t sh[kSyms];
   __shared__ uint32_t ws[kTokWarps + 1];
   __shared__ uint32_t rows[kTokThreads * kRowWords];
@@ -331,8 +357,10 @@ __global__ void __launch_bounds__(kTokThreads, 8)
   for (int i = threadIdx.x; i < kSyms; i += blockDim.x) sh[i] = 0;
   __syncthreads();
   const int b = blockIdx.x / hg.nsub, part = blockIdx.x - b * hg.nsub;
-  const uint8_t *seg0 = in + (size_t)blockIdx.y * hg.in_stride + (size_t)b * hg.seg_size;
-  const int p0 = part * hg.sub_size, plen = min(hg.sub_size, hg.seg_size - p0);
+  HuffGeom ig = hg;  // this item's chunk
+  const bool idle = MIXED && !(mixed_chunk(mh, blockIdx.y, ig) && b < ig.nseg);  // (a zero histogram row)
+  const uint8_t *seg0 = in + (size_t)blockIdx.y * hg.in_stride + (size_t)b * ig.seg_size;
+  const int p0 = part * ig.sub_size, plen = idle ? 0 : min(ig.sub_size, ig.seg_size - p0);
   const uint8_t *seg = seg0 + p0;
   uint32_t carry = part ? zeros_before(seg0, p0, &s_last) : 0u;
   for (int base = 0; base < plen; base += kTokPiece) {
@@ -738,6 +766,131 @@ __global__ void __launch_bounds__(kLayoutThreads) k_huff_layout(const __grid_con
   }
 }
 
+// Device error flag value of an image whose dims are out of bounds (a mixed batch): below the others (4, 5, 99), so
+// that under atomicMax a worse error of the same call still wins.
+constexpr int kEncErrDims = 1;
+
+// k_huff_layout of a mixed-geometry batch, grid (n).  Chunk 0 is the LRES chunk, chunk 1 the FRES chunk; C.nseg is the bounding segment
+// count, the slot stride of the segment tables; item i's chunks have their own segment counts (1, gi.rows) and the
+// FRES chunk is framed only when gi.rows > 1.  Its width and height go into the two u32 at offset frmt_at of chunk 0's
+// prefix.  An image whose dims are out of bounds gets size 0 and the flag kEncErrDims.  (A kernel of its own: the
+// smallest change to k_huff_layout's source moves its register allocation.)
+__global__ void __launch_bounds__(kLayoutThreads)
+    k_huff_layout_mixed(const __grid_constant__ LayoutParams P, MixedDims md, int frmt_at) {
+  __shared__ uint32_t ws[kLayoutThreads / 32 + 1];
+  __shared__ unsigned long long s_chunk_bytes[2];
+  __shared__ int s_too_long;
+  const int item = blockIdx.x, t = threadIdx.x, lane = t & 31;
+  uint8_t *out = P.out + (size_t)item * P.out_stride;
+  if (t == 0) s_too_long = 0;
+  Geom gi;
+  if (!image_geom(md, item, gi)) {
+    if (t == 0) {
+      P.sizes[item] = 0;
+      atomicMax(P.err, kEncErrDims);
+    }
+    return;
+  }
+
+  // pass 1: segment bit lengths and chunk sizes
+  for (int k = 0; k < P.nchunks; ++k) {
+    const LayoutChunk &C = P.ch[k];
+    const TreeOut *tr = C.trees + item;
+    __syncthreads();
+    for (int s = t; s < kSyms; s += blockDim.x)
+      if (tr->len[s] > 32) s_too_long = 1;  // the reference's codes are uint32_t (huffman_enc.cpp:179): unsupported
+    if (t == 0) s_chunk_bytes[k] = 0;
+    __syncthreads();
+    unsigned long long mine = 0;
+    const int nseg = k ? gi.rows : 1, framed = k && gi.rows > 1;  // this item's chunk
+    for (int b = t; b < nseg; b += kLayoutThreads) {  // a thread per segment: running sum over its parts
+      unsigned long long bits = 0;
+      for (int part = 0; part < C.nsub; ++part) {
+        const size_t pi = ((size_t)item * C.nseg + b) * C.nsub + part;
+        C.part_start[pi] = (uint32_t)bits;
+        bits += C.part_bits[pi];
+      }
+      C.seg_bits[(size_t)item * C.nseg + b] = (uint32_t)bits;
+      const unsigned long long sz = (bits + 7) >> 3;
+      mine += sz + (framed ? (sz <= 0x7fff ? 2 : 4) : 0);
+    }
+#pragma unroll
+    for (int d = 16; d >= 1; d >>= 1) mine += __shfl_xor_sync(0xffffffffu, mine, d);
+    if (lane == 0 && mine) atomicAdd(&s_chunk_bytes[k], mine);
+  }
+  __syncthreads();
+  unsigned long long total = 0;
+  for (int k = 0; k < P.nchunks; ++k)
+    total += (unsigned long long)P.ch[k].prefix_len + ((P.ch[k].trees[item].tree_bits + 7) >> 3) + s_chunk_bytes[k];
+  if (s_too_long || total > P.out_stride || total > 0xffffffffull) {
+    // size 0 marks the item as not encoded (the packer skips it, the host calls report it); the flag
+    // says why: 5 = a Huffman code longer than 32 bits, 4 = the output does not fit
+    if (t == 0) {
+      P.sizes[item] = 0;
+      atomicMax(P.err, s_too_long ? 5 : 4);
+    }
+    return;
+  }
+
+  // pass 2: emit prefixes, trees, segment headers; record payload positions
+  uint32_t pos = 0;
+  for (int k = 0; k < P.nchunks; ++k) {
+    const LayoutChunk &C = P.ch[k];
+    const TreeOut *tr = C.trees + item;
+    const uint32_t prefix_at = pos;
+    for (int i = t; i < C.prefix_len; i += blockDim.x) out[pos + i] = C.prefix[i];
+    pos += C.prefix_len;
+    const uint32_t tree_bytes = (tr->tree_bits + 7) >> 3;
+    for (int i = t; i < (int)tree_bytes; i += blockDim.x) out[pos + i] = tr->tree[i];
+    const uint32_t chunk_bytes = tree_bytes + (uint32_t)s_chunk_bytes[k];
+    __syncthreads();  // prefix bytes written before the patch below
+    if (t == 0 && C.size_patch >= 0) put_u32le(out + prefix_at + C.size_patch, chunk_bytes);
+    if (t == 0 && k == 0) {
+      put_u32le(out + prefix_at + frmt_at, (uint32_t)gi.w);
+      put_u32le(out + prefix_at + frmt_at + 4, (uint32_t)gi.h);
+    }
+    pos += tree_bytes;
+    // exclusive scan of (header + payload) over the segments, kLayoutThreads at a time
+    uint32_t run = 0;
+    const int nseg = k ? gi.rows : 1, framed = k && gi.rows > 1;  // this item's chunk
+    for (int b0 = 0; b0 < nseg; b0 += kLayoutThreads) {
+      const int b = b0 + t;
+      uint32_t sz = 0, hdr = 0;
+      if (b < nseg) {
+        sz = (C.seg_bits[(size_t)item * C.nseg + b] + 7) >> 3;
+        hdr = framed ? (sz <= 0x7fff ? 2u : 4u) : 0u;
+      }
+      uint32_t tot;
+      const uint32_t ex = block_exscan_u32(sz + hdr, ws, &tot);
+      if (b < nseg) {
+        uint8_t *h = out + pos + run + ex;
+        if (hdr == 2) {
+          h[0] = (uint8_t)sz;
+          h[1] = (uint8_t)(sz >> 8);
+        } else if (hdr == 4) {
+          const uint32_t lo = (sz & 0x7fff) | 0x8000, hi = sz >> 15;
+          h[0] = (uint8_t)lo;
+          h[1] = (uint8_t)(lo >> 8);
+          h[2] = (uint8_t)hi;
+          h[3] = (uint8_t)(hi >> 8);
+        }
+        C.seg_pos[(size_t)item * C.nseg + b] = pos + run + ex + hdr;
+        // a byte shared by two parts is written with atomicOr from both sides: clear it
+        for (int part = 1; part < C.nsub; ++part) {
+          const uint32_t st = C.part_start[((size_t)item * C.nseg + b) * C.nsub + part];
+          if (st & 7) out[pos + run + ex + hdr + (st >> 3)] = 0;
+        }
+      }
+      run += tot;
+    }
+    pos += run;
+  }
+  if (t == 0) {
+    P.sizes[item] = pos;
+    if (P.riff_patch) put_u32le(out + 4, pos - 8);
+  }
+}
+
 // ---- K-pack ----------------------------------------------------------------------------------
 struct SizeSink {
   const uint32_t *lenx;  // len + extra bits per symbol
@@ -905,12 +1058,13 @@ __device__ __forceinline__ void put64(uint32_t *win, uint32_t pos, uint64_t val,
   if (hi) atomicOr(&win[word + 2], hi);
 }
 
-// grid (nseg, n), block kTokThreads.
+// grid (nseg, n), block kTokThreads.  MIXED: see MixedHuff.
+template <bool MIXED = false>
 __global__ void __launch_bounds__(kTokThreads, kP3MinCtas)
     k_huff_pack3(const uint8_t *__restrict__ in, HuffGeom hg, const TreeOut *__restrict__ trees,
                  const uint32_t *__restrict__ seg_bits, const uint32_t *__restrict__ seg_pos,
                  const uint32_t *__restrict__ part_start, const uint32_t *__restrict__ sizes,
-                 uint8_t *__restrict__ out, unsigned long long out_stride, int *err, ItemLists lists) {
+                 uint8_t *__restrict__ out, unsigned long long out_stride, int *err, ItemLists lists, MixedHuff mh = {}) {
   __shared__ uint32_t win[kWin2Words + 4];
   __shared__ uint2 s_tab[kSyms];
   __shared__ int s_last;
@@ -928,8 +1082,10 @@ __global__ void __launch_bounds__(kTokThreads, kP3MinCtas)
   }
   for (int i = t; i < kWin2Words + 4; i += blockDim.x) win[i] = 0;
   __syncthreads();
-  const uint8_t *seg0 = in + (size_t)item * hg.in_stride + (size_t)b * hg.seg_size;
-  const int p0 = part * hg.sub_size, plen = min(hg.sub_size, hg.seg_size - p0);
+  HuffGeom ig = hg;  // this item's chunk
+  if (MIXED && !(mixed_chunk(mh, item, ig) && b < ig.nseg)) return;  // (uniform)
+  const uint8_t *seg0 = in + (size_t)item * hg.in_stride + (size_t)b * ig.seg_size;
+  const int p0 = part * ig.sub_size, plen = min(ig.sub_size, ig.seg_size - p0);
   const uint8_t *seg = seg0 + p0;
   // this part's bits start at bit `first_bit` of the segment and end where the next part starts
   const size_t pidx = ((size_t)item * hg.nseg + b) * hg.nsub + part;
@@ -1214,10 +1370,11 @@ __device__ __forceinline__ size_t seg_list_base(const ItemLists &L, int nseg, in
 }
 
 // grid (ceil(nseg / 8), n), block 256: warp w codes segment 8 * blockIdx.x + w of item blockIdx.y.
-// seghist: [n][nseg][261]; total: [n][261] (atomics).
+// seghist: [n][nseg][261]; total: [n][261] (atomics).  MIXED: see MixedHuff.
+template <bool MIXED = false>
 __global__ void __launch_bounds__(kTeamThreads)
     k_huff_hist4(const uint8_t *__restrict__ in, HuffGeom hg, uint32_t *__restrict__ seghist, ItemLists lists,
-                 uint32_t *__restrict__ total) {
+                 uint32_t *__restrict__ total, MixedHuff mh = {}) {
   constexpr int kQ = 32 + kWalkStep;
   __shared__ uint32_t sh[kTeamWarps][kSyms];
   __shared__ int qpos_all[kTeamWarps][kQ];
@@ -1225,12 +1382,17 @@ __global__ void __launch_bounds__(kTeamThreads)
   const int wid = threadIdx.x >> 5, lane = threadIdx.x & 31, item = blockIdx.y;
   const int b = blockIdx.x * kTeamWarps + wid;
   if (b >= hg.nseg) return;
+  HuffGeom ig = hg;  // this item's chunk
+  if (MIXED && !(mixed_chunk(mh, item, ig) && b < ig.nseg)) {  // idle segment: a zero histogram row
+    for (int i = lane; i < kSyms; i += 32) seghist[((size_t)item * hg.nseg + b) * kSyms + i] = 0;
+    return;
+  }
   uint32_t *h = sh[wid];
   int *qpos = qpos_all[wid];
   uint8_t *qval = qval_all[wid];
   for (int i = lane; i < kSyms; i += 32) h[i] = 0;
   __syncwarp();
-  const uint8_t *seg = in + (size_t)item * hg.in_stride + (size_t)b * hg.seg_size;
+  const uint8_t *seg = in + (size_t)item * hg.in_stride + (size_t)b * ig.seg_size;
   const bool lists_on = lists.pieces_per_part != 0;
   const int cap = lists.pieces_per_part * kItemCap;
   unsigned short *lpos = lists_on ? lists.pos + seg_list_base(lists, hg.nseg, item, b) : nullptr;
@@ -1246,7 +1408,7 @@ __global__ void __launch_bounds__(kTeamThreads)
   };
   int nitems = 0;
   // one item per lane
-  const int last = warp_walk_items<32>(seg, hg.seg_size, qpos, qval, [&](int k0, int cnt, int g0) {
+  const int last = warp_walk_items<32>(seg, ig.seg_size, qpos, qval, [&](int k0, int cnt, int g0) {
     nitems = g0 + cnt;
     if (lane < cnt) {
       const int k = k0 + lane;
@@ -1260,7 +1422,7 @@ __global__ void __launch_bounds__(kTeamThreads)
       }
     }
   });
-  if (lane == 0) run((uint32_t)(hg.seg_size - 1 - last));  // the run still open at the segment end
+  if (lane == 0) run((uint32_t)(ig.seg_size - 1 - last));  // the run still open at the segment end
   __syncwarp();
   if (lists_on) {
     const bool stored = nitems <= cap && !__any_sync(0xffffffffu, long_gap);
@@ -1287,11 +1449,13 @@ constexpr int kP4MinCtas = 4;  // 64 registers, 49 KiB of shared memory per CTA
 // dynamic shared memory: per warp a window, and a queue for the segments without a stored list
 constexpr int kP4Smem = kTeamWarps * ((kWin4Words + 4) * 4 + kP4Queue * 5);
 
+// MIXED: see MixedHuff.
+template <bool MIXED = false>
 __global__ void __launch_bounds__(kTeamThreads, kP4MinCtas)
     k_huff_pack4(const uint8_t *__restrict__ in, HuffGeom hg, const TreeOut *__restrict__ trees,
                  const uint32_t *__restrict__ seg_bits, const uint32_t *__restrict__ seg_pos,
                  const uint32_t *__restrict__ sizes, uint8_t *__restrict__ out, unsigned long long out_stride, int *err,
-                 ItemLists lists) {
+                 ItemLists lists, MixedHuff mh = {}) {
   extern __shared__ uint32_t p4_smem[];
   __shared__ uint2 s_tab[kSyms];
   const int wid = threadIdx.x >> 5, lane = threadIdx.x & 31, item = blockIdx.y;
@@ -1304,12 +1468,14 @@ __global__ void __launch_bounds__(kTeamThreads, kP4MinCtas)
   __syncthreads();
   const int b = blockIdx.x * kTeamWarps + wid;
   if (b >= hg.nseg) return;
+  HuffGeom ig = hg;  // this item's chunk
+  if (MIXED && !(mixed_chunk(mh, item, ig) && b < ig.nseg)) return;
   uint32_t *win = p4_smem + wid * (kWin4Words + 4);
   int *qpos = reinterpret_cast<int *>(p4_smem + kTeamWarps * (kWin4Words + 4)) + wid * kP4Queue;
   uint8_t *qval = reinterpret_cast<uint8_t *>(p4_smem + kTeamWarps * (kWin4Words + 4 + kP4Queue)) + wid * kP4Queue;
   for (int i = lane; i < kWin4Words + 4; i += 32) win[i] = 0;
   __syncwarp();
-  const uint8_t *seg = in + (size_t)item * hg.in_stride + (size_t)b * hg.seg_size;
+  const uint8_t *seg = in + (size_t)item * hg.in_stride + (size_t)b * ig.seg_size;
   uint8_t *dst = out + (size_t)item * out_stride + seg_pos[(size_t)item * hg.nseg + b];
   const uint32_t full_bits = s_tab[260].y >> 8;  // one maximal run token
   const uint64_t full_tok = (uint64_t)s_tab[260].x | ((uint64_t)(kMaxRun - 279) << (s_tab[260].y & 255u));
@@ -1487,7 +1653,7 @@ __global__ void __launch_bounds__(kTeamThreads, kP4MinCtas)
     last = (int)__reduce_add_sync(0xffffffffu, span) - 1;
   } else {
     // no list: the items again from the planes, with the walk of k_huff_hist4
-    last = warp_walk_items<kP4Round>(seg, hg.seg_size, qpos, qval, [&](int k0, int n, int) {
+    last = warp_walk_items<kP4Round>(seg, ig.seg_size, qpos, qval, [&](int k0, int n, int) {
       const int m = min(max(n - kP4Items * lane, 0), kP4Items);
       auto fetch1 = [&](int k, uint32_t &g, uint32_t &val) {
         g = (uint32_t)(qpos[1 + k0 + k] - qpos[k0 + k] - 1);
@@ -1506,7 +1672,7 @@ __global__ void __launch_bounds__(kTeamThreads, kP4MinCtas)
           fetch1);
     });
   }
-  run_uniform((uint32_t)(hg.seg_size - 1 - last));  // the run still open at the segment end
+  run_uniform((uint32_t)(ig.seg_size - 1 - last));  // the run still open at the segment end
   flush();
   // final partial byte (its padding bits are zero here; k_huff_stale adds the stale ones)
   if (lane == 0) {
@@ -1521,15 +1687,25 @@ __global__ void __launch_bounds__(kTeamThreads, kP4MinCtas)
 // block's segments and of the 1024 before them sit in shared memory (the walk back over earlier segments
 // was a chain of dependent global loads; it rarely goes further, and then reads global memory again).
 // grid (ceil(nseg / 256), n), block 256.
+// MIXED (the FRES chunk of a mixed-geometry batch): nseg is the bounding segment count (the slot stride of the
+// segment tables); item i has gi.rows segments.
 constexpr int kStaleWindow = 1024;
+template <bool MIXED = false>
 __global__ void __launch_bounds__(256)
     k_huff_stale(int n, int nseg, const uint32_t *__restrict__ seg_bits, const uint32_t *__restrict__ seg_pos,
-                 const uint32_t *__restrict__ sizes, uint8_t *__restrict__ out, unsigned long long out_stride) {
+                 const uint32_t *__restrict__ sizes, uint8_t *__restrict__ out, unsigned long long out_stride,
+                 MixedDims md = {}) {
   __shared__ uint32_t sb[kStaleWindow + 256];
   const int item = blockIdx.y, b0 = blockIdx.x * 256, b = b0 + (int)threadIdx.x;
   if (sizes[item] == 0) return;  // (uniform)
   const uint32_t *bits = seg_bits + (size_t)item * nseg;
   const uint32_t *pos = seg_pos + (size_t)item * nseg;
+  if (MIXED) {
+    Geom gi;
+    image_geom(md, item, gi);  // (dims out of bounds: size 0 above)
+    nseg = gi.rows;
+    if (b0 >= nseg) return;  // (uniform)
+  }
   const int w0 = max(0, b0 - kStaleWindow), w1 = min(nseg, b0 + 256);
   for (int i = threadIdx.x; i < w1 - w0; i += 256) sb[i] = bits[w0 + i];
   __syncthreads();

@@ -47,6 +47,8 @@ bool ParseMapFun(const uint8_t *in, int size, int16_t unmap[256]);
 struct ContainerTemplate {
   std::vector<uint8_t> head;  // "RIFF" size "HIMG" FRMT LMAP "LRES" size   (sizes patched on device)
   std::vector<uint8_t> mid;   // QCFG FMAP "FRES" size
+  // offset in `head` of the FRMT width and height (u32 each): "RIFF" size "HIMG", "FRMT" size, version byte
+  static constexpr int kDimsAt = 12 + 8 + 1;
 };
 void BuildContainerTemplate(const EncodeTables &t, int width, int height, int nch,
                             ContainerTemplate *out);

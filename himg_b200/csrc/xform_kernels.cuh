@@ -79,12 +79,19 @@ __device__ __forceinline__ int colour_fwd(const Row8<NCH> &r, int i, int c) {
 // ycbcr.cpp:24-52, encoder.cpp:69) is handled as its first three channels (colour mapped or not) plus one
 // launch per further channel.  `pixels` then points at the group's first channel (g.pstride = all channels)
 // and cbase / ctotal place the group's planes among the image's: [n][ctotal][rows][cols].
-template <int NCH, bool YCBCR>
+// MIXED (encode of a mixed-geometry batch): g is the bounding geometry, which sets the grid and the slot of
+// ctotal * rows * cols bytes per image; image z starts at pixels + px_off[z] and is averaged with its own geometry
+// from `md`, its planes [ctotal][rows][cols] of that geometry at the start of its slot.  Blocks outside it, and
+// images with dims out of bounds, are idle.
+template <int NCH, bool YCBCR, bool MIXED = false>
 __global__ void __launch_bounds__(kTile) k_lowres_avg(const uint8_t *__restrict__ pixels, Geom g,
-                                                      uint8_t *__restrict__ avg, int cbase, int ctotal) {
+                                                      uint8_t *__restrict__ avg, int cbase, int ctotal, MixedDims md = {},
+                                                      const unsigned long long *__restrict__ px_off = nullptr) {
   __shared__ int sB[NCH][kTile + 1];
   const int v = blockIdx.y, t0 = blockIdx.x * kTile, u = t0 + threadIdx.x;
-  const uint8_t *img = pixels + (size_t)blockIdx.z * g.img_bytes;
+  const Geom gb = g;  // bounding geometry (slot strides)
+  if (MIXED && (!image_geom(md, blockIdx.z, g) || t0 >= g.cols || v >= g.rows)) return;  // (uniform per CTA)
+  const uint8_t *img = MIXED ? pixels + px_off[blockIdx.z] : pixels + (size_t)blockIdx.z * g.img_bytes;
   const int y0 = max(0, 8 * v - 3), y1 = min(g.h - 1, 8 * v + 4);
   int A[NCH], B[NCH];
 #pragma unroll
@@ -136,7 +143,11 @@ __global__ void __launch_bounds__(kTile) k_lowres_avg(const uint8_t *__restrict_
 #pragma unroll
     for (int c = 0; c < NCH; ++c) {
       const int s = A[c] + sB[c][threadIdx.x];
-      avg[(((size_t)blockIdx.z * ctotal + cbase + c) * g.rows + v) * g.cols + u] = (uint8_t)((s + (cnt >> 1)) / cnt);
+      if (MIXED)
+        avg[(size_t)blockIdx.z * ctotal * gb.rows * gb.cols + ((size_t)(cbase + c) * g.rows + v) * g.cols + u] =
+            (uint8_t)((s + (cnt >> 1)) / cnt);
+      else
+        avg[(((size_t)blockIdx.z * ctotal + cbase + c) * g.rows + v) * g.cols + u] = (uint8_t)((s + (cnt >> 1)) / cnt);
     }
   }
 }
@@ -146,10 +157,21 @@ __global__ void __launch_bounds__(kTile) k_lowres_avg(const uint8_t *__restrict_
 // kCompRows consecutive rows and computes every row blend once (the lower blend of row v is the upper
 // blend of row v+1); 32-bit indices only (a 64-bit division per sample was most of the first version).
 // grid (planes, ceil(rows / kCompRows)), any block size (threads stride over the columns).
+// MIXED: rows x cols is the bounding geometry and plane p is channel p % md.nch of image p / md.nch, laid out with
+// that image's rows and cols inside its slot of md.nch * rows * cols bytes (as k_lowres_avg<.., true> writes it).
 constexpr int kCompRows = 4;
+template <bool MIXED = false>
 __global__ void k_lowres_comp(const uint8_t *__restrict__ avg, int planes, int rows, int cols,
-                              uint8_t *__restrict__ L) {
-  const size_t base = (size_t)blockIdx.x * rows * cols;
+                              uint8_t *__restrict__ L, MixedDims md = {}) {
+  size_t base = (size_t)blockIdx.x * rows * cols;
+  if (MIXED) {
+    const int img = blockIdx.x / md.nch, c = blockIdx.x - img * md.nch;
+    Geom gi;
+    if (!image_geom(md, img, gi) || (int)blockIdx.y * kCompRows >= gi.rows) return;
+    base = (size_t)img * md.nch * rows * cols + (size_t)c * gi.rows * gi.cols;
+    rows = gi.rows;
+    cols = gi.cols;
+  }
   const uint8_t *a = avg + base;
   uint8_t *o = L + base;
   const int v0 = blockIdx.y * kCompRows;
@@ -193,7 +215,7 @@ struct LowResTables {
 
 constexpr int kLresWarps = 4;
 
-// MIXED (decode of a mixed-geometry batch): g is the bounding geometry, which sets the grid and the slot strides
+// MIXED (mixed-geometry batch, encode or decode): g is the bounding geometry, which sets the grid and the slot strides
 // (lres_stride and nch * rows * cols bytes per image); image img's macroblocks and its layout inside the slots are
 // those of its own geometry from `md`.  Macroblocks outside it, and images with dims out of bounds, are idle.
 template <bool ENCODE, bool MIXED = false>
@@ -203,7 +225,6 @@ __global__ void __launch_bounds__(kLresWarps * 32)
                 uint8_t *__restrict__ Rout,        // DECODE: R [n][nch][rows][cols]
                 Geom g, int n, const uint8_t *__restrict__ map_lut, const int16_t *__restrict__ unmap,
                 unsigned long long unmap_stride, MixedDims md = {}) {
-  static_assert(!(ENCODE && MIXED), "mixed geometry is decode only");
   __shared__ uint8_t sL[kLresWarps * 2][16][16];
   __shared__ uint8_t sR[kLresWarps * 2][16][17];
   // The codes of a macroblock are contiguous in memory but the wavefront touches them along
@@ -350,11 +371,15 @@ __device__ __forceinline__ LowCorners load_corners(const uint8_t *__restrict__ X
 // quantize.cpp:127-151, mapper.cpp:159-182).  grid (ceil(cols/kTile), rows, n), block kTile.
 // Algorithmic traffic: nch bytes read + nch bytes written per pixel.
 // ---------------------------------------------------------------------------------------------
-template <int NCH, bool YCBCR>
+// MIXED (encode of a mixed-geometry batch): g is the bounding geometry (grid; slots of planes_bytes in `planes` and
+// of ctotal * rows * cols in L); image z starts at pixels + px_off[z], and its blocks, edges, low-res planes and
+// segments (gi.seg bytes each, from the start of its slot) are those of its own geometry from `md`.
+template <int NCH, bool YCBCR, bool MIXED = false>
 __global__ void __launch_bounds__(kTile)
     k_forward(const uint8_t *__restrict__ pixels, const uint8_t *__restrict__ L, Geom g,
               const __grid_constant__ QuantParams qp, const uint8_t *__restrict__ map_lut,
-              uint8_t *__restrict__ planes, int cbase, int ctotal) {
+              uint8_t *__restrict__ planes, int cbase, int ctotal, MixedDims md = {},
+              const unsigned long long *__restrict__ px_off = nullptr) {
   __shared__ uint8_t sLut[7616];
   {
     const uint4 *src = reinterpret_cast<const uint4 *>(map_lut);
@@ -363,11 +388,17 @@ __global__ void __launch_bounds__(kTile)
   }
   __syncthreads();
   const int v = blockIdx.y, u = blockIdx.x * kTile + threadIdx.x;
+  const Geom gb = g;  // bounding geometry (slot strides)
+  const uint8_t *img;
+  if (MIXED) {
+    if (!image_geom(md, blockIdx.z, g) || v >= g.rows) return;
+    img = pixels + px_off[blockIdx.z];
+  }
   if (u >= g.cols) return;
-  const uint8_t *img = pixels + (size_t)blockIdx.z * g.img_bytes;
+  if (!MIXED) img = pixels + (size_t)blockIdx.z * g.img_bytes;
   const bool fast = row_fast_ok<NCH>(img, g, u);
   const int bh = min(8, g.h - 8 * v);
-  uint8_t *seg = planes + (size_t)blockIdx.z * g.planes_bytes + (size_t)v * g.seg;
+  uint8_t *seg = planes + (size_t)blockIdx.z * gb.planes_bytes + (size_t)v * g.seg;
 
 #pragma unroll 1
   for (int c = 0; c < NCH; ++c) {
@@ -401,7 +432,9 @@ __global__ void __launch_bounds__(kTile)
     }
     // ---- subtract the interpolated low-res patch (un-quantised L: SURVEY A.4-5)
     {
-      const LowCorners k = load_corners(L + ((size_t)blockIdx.z * ctotal + cbase + c) * g.rows * g.cols, g, u, v);
+      const uint8_t *Lp = MIXED ? L + (size_t)blockIdx.z * ctotal * gb.rows * gb.cols + (size_t)(cbase + c) * g.rows * g.cols
+                                : L + ((size_t)blockIdx.z * ctotal + cbase + c) * g.rows * g.cols;
+      const LowCorners k = load_corners(Lp, g, u, v);
       int lf[9], rt[9];
       nine(k.x11, k.x21, lf);
       nine(k.x12, k.x22, rt);

@@ -146,6 +146,26 @@ int himgcu_decode_batch_region_mixed(himgcu_ctx *ctx, const uint8_t *d_himg, con
                                      int max_height, int num_channels, int flags, const int32_t *d_origins,
                                      int rw, int rh, uint8_t *d_pixels_out, int32_t *d_status);
 
+/* The encoder's side of the call above: n images of one channel count, each of its own size, in one call.
+ * Image i is [h_i][w_i][num_channels], tightly packed at d_pixels + d_pixel_offsets[i] (no alignment
+ * required), with d_dims[2i] = w_i and d_dims[2i+1] = h_i; offsets and dims are in DEVICE memory.
+ * max_width x max_height (host) bounds every image and sizes the workspace (HIMGCU_ERR_UNSUPPORTED if it
+ * is not a shape himgcu_encode_batch takes).  One quality and one use_ycbcr for the batch (YCbCr iff
+ * use_ycbcr && num_channels >= 3).  Output as in himgcu_encode_batch: image i's stream at d_out +
+ * i*out_stride, its size in d_sizes[i]; asynchronous on the context's stream.  Image i's bytes and size are
+ * exactly those of himgcu_encode (or himgcu_encode_batch with n = 1) on that image alone, and a batch whose
+ * dims are all equal gives what himgcu_encode_batch gives.  Per image, without effect on the others:
+ * dims < 1 or above the bounds give size 0 and nothing is written to its output slot (himgcu_encode_status
+ * then reports HIMGCU_ERR_ARG, unless a worse error of the same call outranks it); a stream that does not
+ * fit out_stride gives size 0 and HIMGCU_ERR_CAPACITY.  Null pointers and n < 0 are HIMGCU_ERR_ARG; n = 0
+ * does nothing.  The transforms are always the generic (one block per thread) kernels, and the option
+ * "force_generic" does not change the entropy coder of this call: the first-generation coder it selects
+ * elsewhere has no variant for images of their own sizes. */
+int himgcu_encode_batch_mixed(himgcu_ctx *ctx, const uint8_t *d_pixels, const uint64_t *d_pixel_offsets,
+                              const int32_t *d_dims, int n, int max_width, int max_height, int num_channels,
+                              int quality, int use_ycbcr, uint8_t *d_out, size_t out_stride,
+                              uint32_t *d_sizes);
+
 /* ---- batch, HOST pointers (what a file/stream based caller uses; basis of the e2e figure) ----
  * Same work as the device batch calls with the transfers included: pixels (or bitstreams) are
  * copied host->device in sub-batches, coded, and the results copied back.  Pinned host memory

@@ -219,6 +219,37 @@ class Context:
                                                               _ptr(status)))
         return out, status
 
+    def decode_batch_mixed(self, himg, offsets, sizes, dims, nch, max_w, max_h, flags=STRICT, out=None, pixel_offsets=None,
+                           status=None):
+        """decode_batch of streams with their own sizes: dims is a CUDA int32 [n][2] tensor of (w_i, h_i), each at most
+        max_w x max_h.  Image i is written as [h_i][w_i][nch] at byte pixel_offsets[i] (int64 [n]) of the flat uint8
+        buffer out.  When pixel_offsets is None they are the exclusive prefix sum of w_i * h_i * nch (0 for dims out of
+        bounds), computed on the device; when out is None it is allocated for the spans, which reads their total back
+        to the host (one synchronisation).  Returns (out, pixel_offsets, status); status[i] is REJECT where the stream is rejected or its
+        shape is not dims[i] x nch, and ERR_ARG where dims[i] is < 1 or exceeds the bounds (nothing of it is written)."""
+        import torch
+
+        n = offsets.numel()
+        if dims.dtype != torch.int32 or dims.numel() != 2 * n:
+            raise ValueError("dims must be an int32 tensor [n][2]")
+        if pixel_offsets is not None and (pixel_offsets.dtype != torch.int64 or pixel_offsets.numel() != n):
+            raise ValueError("pixel_offsets must be an int64 tensor [n]")
+        self._bind(himg, offsets, sizes, dims, out, pixel_offsets, status)
+        if pixel_offsets is None or out is None:  # (an image with dims out of bounds gets an empty span)
+            wh = dims.reshape(n, 2).to(torch.int64)
+            ok = (wh >= 1).all(dim=1) & (wh[:, 0] <= max_w) & (wh[:, 1] <= max_h)
+            spans = torch.where(ok, wh[:, 0] * wh[:, 1] * nch, 0)
+        if pixel_offsets is None:
+            pixel_offsets = torch.cumsum(spans, 0) - spans
+        if out is None:
+            total = int(spans.sum()) if n else 0
+            out = torch.empty((max(total, 1),), dtype=torch.uint8, device=himg.device)
+        if status is None:
+            status = torch.empty((n,), dtype=torch.int32, device=himg.device)
+        self._check(self.lib.himgcu_decode_batch_mixed(self.h, _ptr(himg), _ptr(offsets), _ptr(sizes), n, _ptr(dims), max_w,
+                                                       max_h, nch, flags, _ptr(pixel_offsets), _ptr(out), _ptr(status)))
+        return out, pixel_offsets, status
+
     def encode_batch_mixed(self, pixels, offsets, dims, nch, max_w, max_h, quality=50, use_ycbcr=True, out=None, sizes=None):
         """encode_batch of images with their own sizes: pixels is a flat CUDA uint8 buffer holding image i as
         [h_i][w_i][nch] at byte offsets[i] (int64 [n]), dims a CUDA int32 [n][2] tensor of (w_i, h_i), each at most

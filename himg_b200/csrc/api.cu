@@ -491,10 +491,17 @@ int stage_forward(himgcu_ctx *ctx, const uint8_t *d_pixels, const uint8_t *d_L, 
   return rc;
 }
 
+// With `md` the batch has mixed geometry (g is the bounding one) and image i is written at d_pixels + px_off[i].
 template <int NCH>
 int launch_inv(himgcu_ctx *ctx, const uint8_t *d_planes, const uint8_t *d_R, int n, const Geom &g,
-               const DecTables *d_tabs, unsigned long long tab_stride, uint8_t *d_pixels, int cbase = 0, int ctotal = NCH) {
+               const DecTables *d_tabs, unsigned long long tab_stride, uint8_t *d_pixels, int cbase = 0, int ctotal = NCH,
+               const MixedDims *md = nullptr, const unsigned long long *px_off = nullptr) {
   dim3 grid((g.cols + kTile - 1) / kTile, g.rows, n);
+  if (md) {
+    LAUNCH("k_inverse", (k_inverse<NCH, true>), grid, kTile, 0, d_planes, d_R, g, d_tabs, tab_stride, d_pixels, cbase, ctotal,
+           *md, px_off);
+    return HIMGCU_OK;
+  }
   LAUNCH("k_inverse", (k_inverse<NCH>), grid, kTile, 0, d_planes, d_R, g, d_tabs, tab_stride, d_pixels, cbase, ctotal);
   return HIMGCU_OK;
 }
@@ -532,16 +539,18 @@ int launch_inv4(himgcu_ctx *ctx, const uint8_t *d_planes, const uint8_t *d_R, in
   return HIMGCU_OK;
 }
 
+// With `md` the batch has mixed geometry (see launch_inv) and takes the generic kernel.
 int stage_inverse(himgcu_ctx *ctx, const uint8_t *d_planes, const uint8_t *d_R, int n, const Geom &g,
-                  const DecTables *d_tabs, unsigned long long tab_stride, uint8_t *d_pixels) {
+                  const DecTables *d_tabs, unsigned long long tab_stride, uint8_t *d_pixels, const MixedDims *md = nullptr,
+                  const unsigned long long *px_off = nullptr) {
   // lane-pair fast path: two blocks per thread, flat tiles, 16-byte pixel stores
-  if (!ctx->force_generic && !(ctx->xform_variant & 1) && (g.h % 8) == 0 && (g.cols % 16) == 0 && (g.w % 16) == 0 &&
+  if (!md && !ctx->force_generic && !(ctx->xform_variant & 1) && (g.h % 8) == 0 && (g.cols % 16) == 0 && (g.w % 16) == 0 &&
       (g.nch == 1 || g.nch == 3) && (reinterpret_cast<uintptr_t>(d_planes) & 15) == 0 &&
       (reinterpret_cast<uintptr_t>(d_pixels) & 15) == 0 && (reinterpret_cast<uintptr_t>(d_R) & 1) == 0) {
     if (g.nch == 1) return launch_inv4<1>(ctx, d_planes, d_R, n, g, d_tabs, tab_stride, d_pixels);
     return launch_inv4<3>(ctx, d_planes, d_R, n, g, d_tabs, tab_stride, d_pixels);
   }
-  if (!ctx->force_generic && (g.w % 8) == 0 && (g.h % 8) == 0 && (g.cols % 16) == 0 &&
+  if (!md && !ctx->force_generic && (g.w % 8) == 0 && (g.h % 8) == 0 && (g.cols % 16) == 0 &&
       (reinterpret_cast<uintptr_t>(d_planes) & 15) == 0 && (reinterpret_cast<uintptr_t>(d_pixels) & 7) == 0 &&
       (((size_t)g.w * g.nch) & 7) == 0) {
     switch (g.nch) {
@@ -552,14 +561,15 @@ int stage_inverse(himgcu_ctx *ctx, const uint8_t *d_planes, const uint8_t *d_R, 
     }
   }
   switch (g.nch) {
-    case 1: return launch_inv<1>(ctx, d_planes, d_R, n, g, d_tabs, tab_stride, d_pixels);
-    case 2: return launch_inv<2>(ctx, d_planes, d_R, n, g, d_tabs, tab_stride, d_pixels);
-    case 3: return launch_inv<3>(ctx, d_planes, d_R, n, g, d_tabs, tab_stride, d_pixels);
-    case 4: return launch_inv<4>(ctx, d_planes, d_R, n, g, d_tabs, tab_stride, d_pixels);
+    case 1: return launch_inv<1>(ctx, d_planes, d_R, n, g, d_tabs, tab_stride, d_pixels, 0, 1, md, px_off);
+    case 2: return launch_inv<2>(ctx, d_planes, d_R, n, g, d_tabs, tab_stride, d_pixels, 0, 2, md, px_off);
+    case 3: return launch_inv<3>(ctx, d_planes, d_R, n, g, d_tabs, tab_stride, d_pixels, 0, 3, md, px_off);
+    case 4: return launch_inv<4>(ctx, d_planes, d_R, n, g, d_tabs, tab_stride, d_pixels, 0, 4, md, px_off);
     default: break;
   }
-  int rc = launch_inv<3>(ctx, d_planes, d_R, n, g, d_tabs, tab_stride, d_pixels, 0, g.nch);
-  for (int c = 3; c < g.nch && !rc; ++c) rc = launch_inv<1>(ctx, d_planes, d_R, n, g, d_tabs, tab_stride, d_pixels, c, g.nch);
+  int rc = launch_inv<3>(ctx, d_planes, d_R, n, g, d_tabs, tab_stride, d_pixels, 0, g.nch, md, px_off);
+  for (int c = 3; c < g.nch && !rc; ++c)
+    rc = launch_inv<1>(ctx, d_planes, d_R, n, g, d_tabs, tab_stride, d_pixels, c, g.nch, md, px_off);
   return rc;
 }
 
@@ -943,14 +953,16 @@ int decode_front(himgcu_ctx *ctx, const uint8_t *d_himg, const unsigned long lon
   return rc_l;
 }
 
-// Whole-image decode of n streams resident on the device.
+// Whole-image decode of n streams resident on the device.  With `md` the batch has mixed geometry: g is its bounding
+// geometry, and image i is written at d_pixels + px_off[i] with its own size (see MixedDims).
 int decode_device(himgcu_ctx *ctx, const uint8_t *d_himg, const unsigned long long *d_offsets,
-                  const uint32_t *d_sizes, int n, const Geom &g, int flags, uint8_t *d_pixels, int *d_status) {
+                  const uint32_t *d_sizes, int n, const Geom &g, int flags, uint8_t *d_pixels, int *d_status,
+                  const MixedDims *md = nullptr, const unsigned long long *px_off = nullptr) {
   const int lenient = (flags & HIMGCU_LENIENT) ? 1 : 0;
   uint8_t *d_planes;
   ENSURE("planes", (size_t)n * g.planes_bytes, d_planes);
   DecFront f;
-  int rc = decode_front(ctx, d_himg, d_offsets, d_sizes, n, g, lenient, d_status, &f);
+  int rc = decode_front(ctx, d_himg, d_offsets, d_sizes, n, g, lenient, d_status, &f, md);
   if (rc) return rc;
   const ChunkDesc *d_fcd = f.fcd;
   const DecTree *d_ftree = f.ftree;
@@ -962,6 +974,18 @@ int decode_device(himgcu_ctx *ctx, const uint8_t *d_himg, const unsigned long lo
   const unsigned nb = (unsigned)((n + 127) / 128);
   // a warp per block row when the batch alone fills the GPU, wider teams for few streams
   const int fres_team = decode_team((long long)n * g.rows, g.seg, kParFresThreads);
+  if (md) {  // (no inline walk; block rows past an image's own are idle in the stream decoder)
+    LAUNCH("k_dec_segtab", k_dec_segtab_mixed, nb, 128, 0, d_himg, d_fcd, d_ftree, n, g.rows, lenient, d_fseg, d_status, *md);
+    if (fres_team == 32) {
+      LAUNCH("k_dec_stream_fres", (k_dec_stream_par<true, 1, kMixWhole>), dim3((g.rows + kParWarpTeams - 1) / kParWarpTeams, n),
+             32 * kParWarpTeams, 0, d_himg, d_fcd, d_ftree, d_fseg, g.rows, g.seg, d_planes, g.planes_bytes, d_status, 0, 0, *md);
+    } else {
+      LAUNCH("k_dec_stream_fres", (k_dec_stream_par<false, 1, kMixWhole>), dim3(g.rows, n), fres_team, 0, d_himg, d_fcd, d_ftree,
+             d_fseg, g.rows, g.seg, d_planes, g.planes_bytes, d_status, 0, 0, *md);
+    }
+    if (fork) CK(cudaStreamWaitEvent(main_stream, ctx->ev_join, 0));
+    return stage_inverse(ctx, d_planes, d_R, n, g, d_tabs, sizeof(DecTables), d_pixels, md, px_off);
+  }
   // Few streams (single images): the serial walk over the segment headers runs inside the decode kernel
   // and the rows decode as soon as their entry is published (all CTAs of such a grid are resident at once)
   const bool inline_walk = fres_team > 32 && !ctx->force_generic && (long long)n * (g.rows + 1) * fres_team <= 148LL * 2048;
@@ -1586,6 +1610,30 @@ int himgcu_decode_batch(himgcu_ctx *ctx, const uint8_t *d_himg, const uint64_t *
     const int m = std::min(sub, n - i0);
     int rc = decode_device(ctx, d_himg, reinterpret_cast<const unsigned long long *>(d_offsets) + i0, d_sizes + i0, m,
                            g, flags, d_pixels_out + (size_t)i0 * g.out_img_bytes, d_status + i0);
+    if (rc) return rc;
+  }
+  return HIMGCU_OK;
+}
+
+int himgcu_decode_batch_mixed(himgcu_ctx *ctx, const uint8_t *d_himg, const uint64_t *d_offsets, const uint32_t *d_sizes, int n,
+                              const int32_t *d_dims, int max_width, int max_height, int nch, int flags,
+                              const uint64_t *d_pixel_offsets, uint8_t *d_pixels_out, int32_t *d_status) {
+  if (!ctx || !d_himg || !d_offsets || !d_sizes || !d_dims || !d_pixel_offsets || !d_pixels_out || !d_status || n < 0)
+    return fail(ctx, HIMGCU_ERR_ARG, "bad argument");
+  if (!shape_ok(max_width, max_height, nch))
+    return fail(ctx, HIMGCU_ERR_UNSUPPORTED, "unsupported bounding shape %dx%dx%d", max_width, max_height, nch);
+  if (n == 0) return HIMGCU_OK;
+  CK(cudaSetDevice(ctx->device));
+  // every per-image scratch slot has the bounding geometry's size; the kernels lay each image out in its own
+  const Geom g = make_geom(max_width, max_height, nch, nch);
+  const size_t per = per_image_encode_ws(g) + sizeof(DecTables) + 2 * sizeof(DecTree);
+  int sub = (int)std::min<size_t>((size_t)n, std::max<size_t>(1, ctx->max_workspace / per));
+  sub = std::min(sub, 65535);
+  for (int i0 = 0; i0 < n; i0 += sub) {
+    const int m = std::min(sub, n - i0);
+    const MixedDims md{d_dims + 2 * (size_t)i0, max_width, max_height, nch};
+    int rc = decode_device(ctx, d_himg, reinterpret_cast<const unsigned long long *>(d_offsets) + i0, d_sizes + i0, m, g, flags,
+                           d_pixels_out, d_status + i0, &md, reinterpret_cast<const unsigned long long *>(d_pixel_offsets) + i0);
     if (rc) return rc;
   }
   return HIMGCU_OK;

@@ -526,6 +526,20 @@ __global__ void k_dec_segtab(const uint8_t *__restrict__ data, const ChunkDesc *
   segtab_walk<false>(data, cd[i], trees + i, nseg, seg_size, mode, lenient, segs + (size_t)i * nseg, status + i);
 }
 
+// Whole-image FRES segment table of a mixed-geometry batch: image i's header chain is walked for its own gi.rows
+// segments of gi.seg bytes (so the framing decision is the image's own), into a table of `stride` (the bounding
+// geometry's rows) entries per image.  Entries past gi.rows are left alone: k_dec_stream_par<..., kMixWhole> never
+// reads them.  A separate kernel, so that k_dec_segtab keeps its code.
+__global__ void k_dec_segtab_mixed(const uint8_t *__restrict__ data, const ChunkDesc *__restrict__ cd,
+                                   const DecTree *__restrict__ trees, int n, int stride, int lenient,
+                                   SegRef *__restrict__ segs, int *__restrict__ status, MixedDims md) {
+  const int i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= n) return;
+  Geom gi;
+  image_geom(md, i, gi);  // (dims out of bounds: the chunk is invalid, and the walk only marks entry 0 invalid)
+  segtab_walk<false>(data, cd[i], trees + i, gi.rows, gi.seg, 1, lenient, segs + (size_t)i * stride, status + i);
+}
+
 // Region decode (framed FRES chunk): the segment table of the block rows r0 = y / 8 .. r1 = (y + rh - 1) / 8 that
 // image i's rectangle touches, compacted to kr entries per image: entry k is row min(r0 + k, r1), so a rectangle
 // that touches fewer than kr rows decodes its last row again instead of needing a "skip" entry.  The header
@@ -675,8 +689,10 @@ constexpr int kParWarpTeams = 8;  // WARP_TEAMS: streams (one warp each) per CTA
 //   cluster barriers.  This is what a single large image needs: its low-res chunk is ONE stream,
 //   and one CTA (one SM) was the whole machine for it.
 // MIX (mixed-geometry batches, one CTA per stream or warp teams, no inline walk): the output size of a stream is
-//   its image's own (from `md`): the low-res chunk (kMixLres) or a block row (kMixFres); out_seg is unused.
-constexpr int kMixLres = 1, kMixFres = 2;
+//   its image's own (from `md`): the low-res chunk (kMixLres) or a block row (kMixFres, kMixWhole); out_seg is unused.
+//   kMixWhole (whole-image decode): nseg is the bounding geometry's rows, and block rows b >= gi.rows of an image
+//   are idle (no status, nothing written): a CTA whose streams all lie past them exits before staging the tree.
+constexpr int kMixLres = 1, kMixFres = 2, kMixWhole = 3;
 template <bool WARP_TEAMS, int CL = 1, int MIX = 0>
 __global__ void k_dec_stream_par(const uint8_t *__restrict__ data, const ChunkDesc *__restrict__ cd,
                                  const DecTree *__restrict__ trees, SegRef *__restrict__ segs, int nseg,
@@ -696,11 +712,13 @@ __global__ void k_dec_stream_par(const uint8_t *__restrict__ data, const ChunkDe
   static_assert(MIX == 0 || CL == 1, "mixed geometry has no cluster decode");
   namespace cg = cooperative_groups;
   const int item = blockIdx.y;
+  int mix_rows = 0;  // kMixWhole: block rows of the item's image
   if (MIX) {  // (an image with dims out of bounds has an invalid chunk: its tree is not ok and nothing is written)
     Geom gi;
     image_geom(md, item, gi);
     out_seg = MIX == kMixLres ? gi.lres_size : gi.seg;
     inline_walk = 0;
+    mix_rows = gi.rows;
   }
   // inline_walk (one CTA per stream only): CTA 0 of every item walks the segment headers of the framed
   // chunk and publishes the table (see segtab_walk); the stream of CTA x is segment x - 1
@@ -730,6 +748,7 @@ __global__ void k_dec_stream_par(const uint8_t *__restrict__ data, const ChunkDe
     }
     return any;
   };
+  if (MIX == kMixWhole && (WARP_TEAMS ? (int)blockIdx.x * kParWarpTeams : b) >= mix_rows) return;  // (the whole CTA)
   const DecTree *T = trees + item;
   if (T->ok) {  // the whole CTA stages the image's LUT and tree
     const uint4 *l2 = reinterpret_cast<const uint4 *>(T->lut2);
@@ -742,6 +761,7 @@ __global__ void k_dec_stream_par(const uint8_t *__restrict__ data, const ChunkDe
   }
   __syncthreads();
   if (WARP_TEAMS && b >= nseg) return;
+  if (MIX == kMixWhole && b >= mix_rows) return;
   SegRef sr;
   if (!WARP_TEAMS && CL == 1 && inline_walk) {
     // ONE thread polls (a whole grid of polling threads slowed the walker's own dependent loads down)

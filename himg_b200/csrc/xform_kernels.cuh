@@ -482,14 +482,20 @@ __global__ void __launch_bounds__(kTile)
 // hadamard.cpp:90-103, ycbcr.cpp:54-82).  Same grid as K-fwd; same algorithmic traffic.
 // Width % 8 != 0 is undefined in the reference; here the block is cropped.
 // ---------------------------------------------------------------------------------------------
-template <int NCH>
+// MIXED (whole-image decode of a mixed-geometry batch): g is the bounding geometry (grid; slots of planes_bytes in
+// `planes` and of ctotal * rows * cols in R); image z is written at pixels + px_off[z], and its blocks, segments,
+// low-res planes and edges are those of its own geometry from `md`.  An image with dims out of bounds is not written.
+template <int NCH, bool MIXED = false>
 __global__ void __launch_bounds__(kTile)
     k_inverse(const uint8_t *__restrict__ planes, const uint8_t *__restrict__ R, Geom g,
               const DecTables *__restrict__ tabs, unsigned long long tab_stride,
-              uint8_t *__restrict__ pixels, int cbase, int ctotal) {
+              uint8_t *__restrict__ pixels, int cbase, int ctotal, MixedDims md = {},
+              const unsigned long long *__restrict__ px_off = nullptr) {
   __shared__ int16_t sUn[256];
   __shared__ uint8_t sShift[2][64];
   __shared__ uint32_t sOut[NCH][kTile][17];  // per channel: 64 result bytes per thread (+1 pad)
+  const Geom gb = g;  // bounding geometry (slot strides)
+  if (MIXED && (!image_geom(md, blockIdx.z, g) || (int)blockIdx.y >= g.rows || (int)blockIdx.x * kTile >= g.cols)) return;
   const DecTables *T = reinterpret_cast<const DecTables *>(reinterpret_cast<const char *>(tabs) + (size_t)blockIdx.z * tab_stride);
   for (int i = threadIdx.x; i < 256; i += blockDim.x) sUn[i] = T->full_unmap[i];
   for (int i = threadIdx.x; i < 128; i += blockDim.x) sShift[i >> 6][i & 63] = T->shift[i >> 6][i & 63];
@@ -498,8 +504,8 @@ __global__ void __launch_bounds__(kTile)
   const int v = blockIdx.y, u = blockIdx.x * kTile + threadIdx.x;
   if (u >= g.cols) return;
   const int bh = min(8, g.h - 8 * v), bw = min(8, g.w - 8 * u);
-  const uint8_t *seg = planes + (size_t)blockIdx.z * g.planes_bytes + (size_t)v * g.seg;
-  uint8_t *img = pixels + (size_t)blockIdx.z * g.out_img_bytes;
+  const uint8_t *seg = planes + (size_t)blockIdx.z * gb.planes_bytes + (size_t)v * g.seg;
+  uint8_t *img = MIXED ? pixels + px_off[blockIdx.z] : pixels + (size_t)blockIdx.z * g.out_img_bytes;
 
 #pragma unroll 1
   for (int c = 0; c < NCH; ++c) {
@@ -526,7 +532,9 @@ __global__ void __launch_bounds__(kTile)
       for (int i = 0; i < 8; ++i) x[i * 8 + q] >>= 3;
     }
     {
-      const LowCorners k = load_corners(R + ((size_t)blockIdx.z * ctotal + cbase + c) * g.rows * g.cols, g, u, v);
+      const uint8_t *Rp = MIXED ? R + (size_t)blockIdx.z * ctotal * gb.rows * gb.cols + (size_t)(cbase + c) * g.rows * g.cols
+                                : R + ((size_t)blockIdx.z * ctotal + cbase + c) * g.rows * g.cols;
+      const LowCorners k = load_corners(Rp, g, u, v);
       int lf[9], rt[9];
       nine(k.x11, k.x21, lf);
       nine(k.x12, k.x22, rt);

@@ -166,6 +166,24 @@ int himgcu_encode_batch_mixed(himgcu_ctx *ctx, const uint8_t *d_pixels, const ui
                               int quality, int use_ycbcr, uint8_t *d_out, size_t out_stride,
                               uint32_t *d_sizes);
 
+/* Whole-image decode of n streams of one channel count, each of its own size: the decoder's side of
+ * himgcu_encode_batch_mixed.  Inputs as in himgcu_decode_batch_region_mixed without the rectangle: d_dims[2i]
+ * = width, d_dims[2i+1] = height of image i (DEVICE memory), bounded by max_width x max_height (host;
+ * HIMGCU_ERR_UNSUPPORTED if it is not a shape himgcu_decode_batch takes).  Image i is written as
+ * [h_i][w_i][num_channels], tightly packed, at d_pixels_out + d_pixel_offsets[i] (DEVICE memory, no alignment
+ * required); the caller sizes the buffer and keeps the spans from overlapping.  Image i's pixels and status are
+ * exactly those of himgcu_decode on its stream alone with the same flags, and a batch whose dims are all equal,
+ * with offsets i*w*h*num_channels, gives what himgcu_decode_batch gives.  d_status[i], without effect on the
+ * other images: HIMGCU_OK; HIMGCU_REJECT where the stream is rejected, including a FRMT shape other than its dims
+ * and num_channels; HIMGCU_ERR_ARG when its dims are < 1 or exceed the bounds (nothing of it is written).  An
+ * image with a non-OK status writes nothing outside its own span.  Null pointers and n < 0 are HIMGCU_ERR_ARG;
+ * n = 0 does nothing.  Asynchronous on the context's stream.  The inverse transform is always the generic (one
+ * block per thread) kernel. */
+int himgcu_decode_batch_mixed(himgcu_ctx *ctx, const uint8_t *d_himg, const uint64_t *d_offsets,
+                              const uint32_t *d_sizes, int n, const int32_t *d_dims, int max_width,
+                              int max_height, int num_channels, int flags,
+                              const uint64_t *d_pixel_offsets, uint8_t *d_pixels_out, int32_t *d_status);
+
 /* ---- batch, HOST pointers (what a file/stream based caller uses; basis of the e2e figure) ----
  * Same work as the device batch calls with the transfers included: pixels (or bitstreams) are
  * copied host->device in sub-batches, coded, and the results copied back.  Pinned host memory

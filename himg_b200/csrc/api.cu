@@ -196,10 +196,18 @@ void resolve_profile(himgcu_ctx *ctx) {
   ctx->pending.clear();
 }
 
+// A block row (FRES segment) holds at most kMaxSegBytes = 2^26 bytes, i.e. 8 * ceil(w / 8) * nch <= 2^23.  A token
+// covers at least one byte and takes at most a 32-bit code plus 14 extra bits, so a segment codes to fewer than
+// 46 * 2^26 < 2^32 bits: the segment sizes and the 32-bit bit counts and positions of the entropy kernels cannot
+// overflow, and Geom::seg fits an int.
+constexpr long long kMaxSegBytes = 1ll << 26;
+
 bool shape_ok(int w, int h, int nch) {
   if (w < 1 || h < 1 || nch < 1 || nch > 255) return false;  // (the container stores the channel count in one byte)
+  // (64-bit rounding: w + 7 and h + 7 overflow an int near 2^31)
   const unsigned long long px = (unsigned long long)w * h * nch;
-  return px < (1ull << 31) && ((h + 7) >> 3) <= 65535;
+  const long long rows = ((long long)h + 7) >> 3, seg = (((long long)w + 7) >> 3) * 64 * nch;
+  return px < (1ull << 31) && rows <= 65535 && seg <= kMaxSegBytes;
 }
 
 int upload_full_lut(himgcu_ctx *ctx) {
@@ -534,8 +542,7 @@ int launch_inv4(himgcu_ctx *ctx, const uint8_t *d_planes, const uint8_t *d_R, in
   dim3 grid((total_pairs + TP - 1) / TP, 1, n);
   const int smem = NCH * 64 * 2 * TP + kInvTableBytes;
   CK(cudaFuncSetAttribute((k_inverse4<NCH, TP>), cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
-  const uint32_t pr_magic = (uint32_t)((1ull << 32) / (unsigned)(g.cols / 2)) + 1u;  // (cols >= 16 here)
-  LAUNCH("k_inverse", (k_inverse4<NCH, TP>), grid, TP, smem, d_planes, d_R, g, d_inv, inv_stride, d_pixels, 1u, pr_magic);
+  LAUNCH("k_inverse", (k_inverse4<NCH, TP>), grid, TP, smem, d_planes, d_R, g, d_inv, inv_stride, d_pixels, 1u);
   return HIMGCU_OK;
 }
 
@@ -796,12 +803,12 @@ int encode_device(himgcu_ctx *ctx, const uint8_t *d_pixels, int n, const Geom &g
   if (rc) return rc;
   HuffChunkArgs ch[2];
   ch[0].d_in = d_lres;
-  ch[0].hg = HuffGeom{g.lres_size, g.lres_size, 1, g.lres_stride, 1, g.lres_size};
+  ch[0].hg = HuffGeom{g.lres_size, 1, g.lres_stride, 1, g.lres_size};
   ch[0].tag = "lres";
   ch[0].prefix = ct.head;
   ch[0].size_patch = (int)ct.head.size() - 4;
   ch[1].d_in = d_planes;
-  ch[1].hg = HuffGeom{(int)g.planes_bytes, g.seg, g.rows, g.planes_bytes, 1, g.seg};
+  ch[1].hg = HuffGeom{g.seg, g.rows, g.planes_bytes, 1, g.seg};
   ch[1].tag = "fres";
   ch[1].prefix = ct.mid;
   ch[1].size_patch = (int)ct.mid.size() - 4;
@@ -2015,10 +2022,11 @@ int himgcu_stage_huff_compress(himgcu_ctx *ctx, const uint8_t *d_in, size_t in_s
   if (block_size < 1) block_size = in_size;
   if (in_size % block_size) return fail(ctx, HIMGCU_ERR_ARG, "in_size is not a multiple of block_size");
   if (in_size / block_size > 65535) return fail(ctx, HIMGCU_ERR_UNSUPPORTED, "too many segments");
+  if (block_size > kMaxSegBytes) return fail(ctx, HIMGCU_ERR_UNSUPPORTED, "segment larger than 2^26 bytes");
   CK(cudaSetDevice(ctx->device));
   HuffChunkArgs ch;
   ch.d_in = d_in;
-  ch.hg = HuffGeom{in_size, block_size, in_size / block_size, (unsigned long long)in_stride, 1, block_size};
+  ch.hg = HuffGeom{block_size, in_size / block_size, (unsigned long long)in_stride, 1, block_size};
   ch.tag = "stage";
   ch.size_patch = -1;
   return huff_encode_items(ctx, n, &ch, 1, false, d_out, out_stride, d_sizes);
@@ -2033,6 +2041,7 @@ int himgcu_stage_huff_uncompress(himgcu_ctx *ctx, const uint8_t *d_in, size_t in
   const int seg = whole ? out_size : block_size;
   if (out_size % seg || (seg & 3)) return fail(ctx, HIMGCU_ERR_ARG, "segment size must divide out_size and be a multiple of 4");
   if (out_stride & 3) return fail(ctx, HIMGCU_ERR_ARG, "out_stride must be a multiple of 4");
+  if (seg > kMaxSegBytes) return fail(ctx, HIMGCU_ERR_UNSUPPORTED, "segment larger than 2^26 bytes");
   const int nseg = out_size / seg;
   CK(cudaSetDevice(ctx->device));
   ChunkDesc *d_cd;

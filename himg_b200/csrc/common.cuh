@@ -17,7 +17,7 @@ struct Geom {
   int w, h, nch, pstride;  // pstride = bytes between pixels of the INPUT (>= nch)
   int rows, cols;          // 8x8 blocks
   int mrows, mcols;        // 16x16 macroblocks of the low-res image
-  int seg;                 // FRES segment = one block row of all channels = cols*64*nch bytes
+  int seg;                 // FRES segment = one block row of all channels = cols*64*nch bytes (<= 2^26: shape_ok)
   int lres_ch;             // mrows*mcols + rows*cols
   int lres_size;           // lres_ch * nch
   unsigned long long img_bytes;     // w*h*pstride

@@ -446,6 +446,10 @@ __global__ void __launch_bounds__(kDecTreeThreads)
 // acquire theirs, so the decode of the first rows overlaps the rest of the walk.  Entries start as
 // kSegNotReady (host memset) and always end up valid or invalid (0xffffffff).
 constexpr uint32_t kSegNotReady = 0xfefefefeu;
+// A segment (framed or not) of this many packed bytes or more is rejected.  No valid stream has one (a block row codes
+// to fewer than 46 * 2^26 bits, see shape_ok), and the bound keeps PBits' 32-bit bit positions (8 * size) exact and
+// every size clear of kSegNotReady on corrupt streams.
+constexpr uint32_t kMaxSegPacked = 1u << 29;
 
 // An entry is ONE aligned 8-byte word (offset | size << 32): a single store publishes it and a single
 // load takes it, no fence (a release store per entry tripled the time of the walk).
@@ -484,7 +488,7 @@ __device__ void segtab_walk(const uint8_t *__restrict__ data, const ChunkDesc d,
   if (mode == 0) {
     // HuffmanDec(in, size, 0): block size = packed size => never framed; an empty payload can
     // only produce an empty output (huffman_dec.cpp:278-279).
-    if (start >= d.size) return fail();
+    if (start >= d.size || d.size - start >= kMaxSegPacked) return fail();
     seg_store<PUBLISH>(S, start, d.size - start);
     done = 1;
     for (int b = done; b < nseg; ++b) seg_store<PUBLISH>(S + b, 0, 0xffffffffu);
@@ -495,6 +499,7 @@ __device__ void segtab_walk(const uint8_t *__restrict__ data, const ChunkDesc d,
   const bool framed = lenient ? (nseg > 1) : ((uint32_t)seg_size < d.size);
   if (!framed) {
     if (!lenient || start >= d.size) return fail();  // UncompressBlock refuses unframed data (:265)
+    if (d.size - start >= kMaxSegPacked) return fail();
     seg_store<PUBLISH>(S, start, d.size - start);
     done = 1;
     for (int b = done; b < nseg; ++b) seg_store<PUBLISH>(S + b, 0, 0xffffffffu);
@@ -511,7 +516,7 @@ __device__ void segtab_walk(const uint8_t *__restrict__ data, const ChunkDesc d,
       sz = (sz & 0x7fffu) | (((uint32_t)p[pos] | ((uint32_t)p[pos + 1] << 8)) << 15);
       pos += 2;
     }
-    if ((unsigned long long)pos + sz > d.size || sz == kSegNotReady) return fail();
+    if ((unsigned long long)pos + sz > d.size || sz >= kMaxSegPacked) return fail();
     seg_store<PUBLISH>(S + b, pos, sz);
     done = b + 1;
     pos += sz;

@@ -31,8 +31,7 @@ constexpr int kWinWords = 8192;                          // bit window: 32 KiB +
 constexpr int kWinBits = kWinWords * 32;
 
 struct HuffGeom {
-  int in_size;   // unpacked bytes per chunk
-  int seg_size;  // bytes per segment (== in_size when the chunk is unframed)
+  int seg_size;  // bytes per segment (the whole chunk when it is unframed)
   int nseg;
   unsigned long long in_stride;  // bytes between the chunks of consecutive items
   // A segment may be coded by `nsub` CTAs, each taking `sub_size` bytes (a multiple of the 8 KiB
@@ -59,9 +58,8 @@ __device__ __forceinline__ bool mixed_chunk(const MixedHuff &m, int item, HuffGe
   if (m.fres) {
     hg.seg_size = hg.sub_size = gi.seg;
     hg.nseg = gi.rows;
-    hg.in_size = gi.rows * gi.seg;
   } else {
-    hg.seg_size = hg.sub_size = hg.in_size = gi.lres_size;
+    hg.seg_size = hg.sub_size = gi.lres_size;
     hg.nseg = 1;
   }
   return ok;

@@ -401,8 +401,7 @@ __device__ __forceinline__ void inv4_compute(uint8_t *col, const uint8_t *sDq, c
 template <int NCH, int TP>
 __global__ void __launch_bounds__(TP, NCH == 1 ? 3 : 2)
     k_inverse4(const uint8_t *__restrict__ planes, const uint8_t *__restrict__ R, Geom g,
-               const InvTables *__restrict__ tabs, unsigned long long tab_stride, uint8_t *__restrict__ pixels, uint32_t one,
-               uint32_t pr_magic) {
+               const InvTables *__restrict__ tabs, unsigned long long tab_stride, uint8_t *__restrict__ pixels, uint32_t one) {
   extern __shared__ __align__(128) uint8_t sPl[];
   constexpr int PITCH = 2 * TP, CPR = TP / 8;  // bytes per tile row, 16-byte chunks per tile row
   static_assert(TP % 32 == 0 && TP == 8 * CPR, "a CTA is 8 groups of one thread per chunk of a tile row");
@@ -418,8 +417,8 @@ __global__ void __launch_bounds__(TP, NCH == 1 ? 3 : 2)
   const InvTables *T = reinterpret_cast<const InvTables *>(reinterpret_cast<const char *>(tabs) + (size_t)blockIdx.z * tab_stride);
   // block row / first pair of the tile's first element: one division per CTA, everything else by
   // carrying (a tile spans few block rows unless the image is very narrow)
-  // (pr_magic = floor(2^32 / PR) + 1 from the host: the quotient is exact for f0 < 2^32 / PR, i.e. any image)
-  const int v0 = (int)__umulhi((uint32_t)f0, pr_magic), p0 = f0 - v0 * PR;
+  // (a true division: a 32-bit reciprocal of PR is not exact for every tile start of every accepted shape)
+  const int v0 = (int)((uint32_t)f0 / (uint32_t)PR), p0 = f0 - v0 * PR;
   auto locate = [&](int k, int &v, int &p) {  // element f0 + k of the image -> block row, pair in the row
     if (PR >= 32) {
       v = v0;

@@ -11,6 +11,18 @@
  *
  * Threading: a context owns one CUDA stream and its device scratch; use one context per host
  * thread (distinct contexts may run concurrently).
+ *
+ * Accepted shapes (every entry point, including the bounds of the mixed batch calls and the FRMT
+ * shape of a stream being decoded; anything else is HIMGCU_ERR_UNSUPPORTED, and encode_bound /
+ * lres_size / lres_stride return 0):
+ *   1 <= num_channels <= 255;
+ *   width * height * num_channels < 2^31 pixel bytes;
+ *   ceil(height / 8) <= 65535 block rows;
+ *   8 * ceil(width / 8) * num_channels <= 2^23, i.e. a block row of at most 2^26 coefficient bytes
+ *   (width * num_channels <= 8 388 608 when width is a multiple of 8).  Such a row codes to fewer
+ *   than 2^32 bits, which keeps the entropy coder's bit counts 32-bit.
+ * A decoded stream with a coded segment (a framed FRES segment, or a whole unframed chunk) of 2^29
+ * bytes or more is rejected.
  */
 #ifndef HIMG_CUDA_H_
 #define HIMG_CUDA_H_

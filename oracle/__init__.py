@@ -41,11 +41,16 @@ class _Port:
         L.ho_fnv1a64.argtypes = [_u8p, C.c_size_t]
         L.ho_synth_image.argtypes = [_u8p, C.c_int, C.c_int, C.c_int, C.c_uint32, C.c_uint32]
         L.ho_synth_image.restype = None
-        L.ho_encode.argtypes = [_u8p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, _u8p, C.c_int]
-        L.ho_decode.argtypes = [_u8p, C.c_int, C.c_int, _u8p, C.c_int, _ip, _ip, _ip]
-        L.ho_huff_compress.argtypes = [_u8p, C.c_int, _u8p, C.c_int, C.c_int]
-        L.ho_huff_uncompress.argtypes = [_u8p, C.c_int, C.c_int, C.c_int, _u8p, C.c_int, C.c_int, C.c_int]
-        L.ho_huff_histogram.argtypes = [_u8p, C.c_int, C.c_int, _u32p]
+        # (sizes of images, streams and buffers are 64-bit: they may exceed 2 GiB)
+        L.ho_encode_bound.restype = C.c_size_t
+        L.ho_encode_bound.argtypes = [C.c_int, C.c_int, C.c_int]
+        L.ho_encode.restype = C.c_longlong
+        L.ho_encode.argtypes = [_u8p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, _u8p, C.c_size_t]
+        L.ho_decode.argtypes = [_u8p, C.c_size_t, C.c_int, _u8p, C.c_size_t, _ip, _ip, _ip]
+        L.ho_huff_compress.restype = C.c_longlong
+        L.ho_huff_compress.argtypes = [_u8p, C.c_size_t, _u8p, C.c_size_t, C.c_size_t]
+        L.ho_huff_uncompress.argtypes = [_u8p, C.c_size_t, C.c_size_t, C.c_int, _u8p, C.c_size_t, C.c_int, C.c_size_t]
+        L.ho_huff_histogram.argtypes = [_u8p, C.c_size_t, C.c_size_t, _u32p]
         L.ho_huff_histogram.restype = None
         L.ho_huff_tree.argtypes = [_u32p, C.c_int, _u32p, _u8p, _u8p]
         L.ho_shift_table.argtypes = [C.c_int, C.c_int, _u8p]
@@ -115,7 +120,8 @@ class _Port:
                 continue
             if r == 0:
                 return None
-            return out[: w.value * h.value * n.value].reshape(h.value, w.value, n.value).copy()
+            img = out[: w.value * h.value * n.value].reshape(h.value, w.value, n.value)
+            return img if img.size == cap else img.copy()
 
     # -- stages ----------------------------------------------------------------------------
     def shift_table(self, quality, chroma) -> np.ndarray:

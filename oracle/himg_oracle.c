@@ -533,7 +533,7 @@ enum { SYM_Z2 = 256, SYM_Z6 = 257, SYM_Z22 = 258, SYM_Z278 = 259, SYM_Z16662 = 2
 
 /* Token at position k of a segment: returns symbol, sets *adv (bytes consumed), *extra / *nextra.
  * huffman_enc.cpp:105-141 == :296-336. */
-static int next_token(const uint8_t *seg, int k, int seg_size, int *adv, uint32_t *extra, int *nextra) {
+static int next_token(const uint8_t *seg, size_t k, size_t seg_size, int *adv, uint32_t *extra, int *nextra) {
   *extra = 0;
   *nextra = 0;
   if (seg[k] != 0) {
@@ -566,11 +566,11 @@ static int next_token(const uint8_t *seg, int k, int seg_size, int *adv, uint32_
 }
 
 /* huffman_enc.cpp:98-144 */
-void ho_huff_histogram(const uint8_t *in, int in_size, int block_size, uint32_t hist[HO_NUM_SYMBOLS]) {
+void ho_huff_histogram(const uint8_t *in, size_t in_size, size_t block_size, uint32_t hist[HO_NUM_SYMBOLS]) {
   memset(hist, 0, sizeof(uint32_t) * HO_NUM_SYMBOLS);
   if (block_size < 1) block_size = in_size;
-  for (int base = 0; base < in_size; base += block_size)
-    for (int k = 0; k < block_size;) {
+  for (size_t base = 0; base < in_size; base += block_size)
+    for (size_t k = 0; k < block_size;) {
       int adv, nx;
       uint32_t ex;
       hist[next_token(in + base, k, block_size, &adv, &ex, &nx)]++;
@@ -741,11 +741,11 @@ int ho_huff_tree(const uint32_t hist[HO_NUM_SYMBOLS], int fast, uint32_t code[HO
 }
 
 /* huffman_enc.cpp:242-244 */
-int ho_huff_max_size(int n) { return n + ((2 + 9) * HO_NUM_SYMBOLS + 7) / 8; }
+size_t ho_huff_max_size(size_t n) { return n + ((2 + 9) * HO_NUM_SYMBOLS + 7) / 8; }
 
 /* huffman_enc.cpp:246-363.  Returns the packed size, 0 for the reference's "nothing to do"
  * cases, -1 if `out_cap` is too small. */
-int ho_huff_compress(uint8_t *out, int out_cap, const uint8_t *in, int in_size, int block_size) {
+long long ho_huff_compress(uint8_t *out, size_t out_cap, const uint8_t *in, size_t in_size, size_t block_size) {
   if (in_size < 1) return 0;
   if (block_size < 1) block_size = in_size;
   int framed = block_size < in_size;
@@ -758,15 +758,15 @@ int ho_huff_compress(uint8_t *out, int out_cap, const uint8_t *in, int in_size, 
   if (tree_bits < 0) return 0;
   size_t pos = (size_t)(tree_bits + 7) / 8;
 
-  int nseg = in_size / block_size;
+  size_t nseg = in_size / block_size;
   size_t *seg_bits = (size_t *)malloc(sizeof(size_t) * nseg);
   size_t *seg_pos = (size_t *)malloc(sizeof(size_t) * nseg);
   /* pass 1: bit length of every segment -> layout */
   size_t total = pos;
-  for (int b = 0; b < nseg; ++b) {
-    const uint8_t *seg = in + (size_t)b * block_size;
+  for (size_t b = 0; b < nseg; ++b) {
+    const uint8_t *seg = in + b * block_size;
     size_t bits = 0;
-    for (int k = 0; k < block_size;) {
+    for (size_t k = 0; k < block_size;) {
       int adv, nx;
       uint32_t ex;
       int s = next_token(seg, k, block_size, &adv, &ex, &nx);
@@ -777,15 +777,15 @@ int ho_huff_compress(uint8_t *out, int out_cap, const uint8_t *in, int in_size, 
     size_t size = (bits + 7) / 8;
     total += size + (framed ? (size <= 0x7fff ? 2 : 4) : 0);
   }
-  if (total > (size_t)out_cap) {
+  if (total > out_cap) {
     free(seg_bits);
     free(seg_pos);
     return -1;
   }
   memcpy(out, tree, pos);
   /* pass 2: emit */
-  for (int b = 0; b < nseg; ++b) {
-    const uint8_t *seg = in + (size_t)b * block_size;
+  for (size_t b = 0; b < nseg; ++b) {
+    const uint8_t *seg = in + b * block_size;
     size_t bits = seg_bits[b], size = (bits + 7) / 8;
     if (framed) { /* :340-352 */
       if (size <= 0x7fff) {
@@ -801,7 +801,7 @@ int ho_huff_compress(uint8_t *out, int out_cap, const uint8_t *in, int in_size, 
     }
     memset(out + pos, 0, size);
     BitW w = {out + pos, 0};
-    for (int k = 0; k < block_size;) {
+    for (size_t k = 0; k < block_size;) {
       int adv, nx;
       uint32_t ex;
       int s = next_token(seg, k, block_size, &adv, &ex, &nx);
@@ -813,7 +813,7 @@ int ho_huff_compress(uint8_t *out, int out_cap, const uint8_t *in, int in_size, 
     /* Stale padding bits (SURVEY A.3 step 5): each padding bit position p of this segment takes
      * the value that the most recent earlier segment with more than p bits WROTE there. */
     for (size_t p = bits; p < 8 * size; ++p)
-      for (int e = b - 1; e >= 0; --e)
+      for (size_t e = b; e-- > 0;)
         if (seg_bits[e] > p) {
           if ((out[seg_pos[e] + (p >> 3)] >> (p & 7)) & 1u) out[pos + (p >> 3)] |= (uint8_t)(1u << (p & 7));
           break;
@@ -822,7 +822,7 @@ int ho_huff_compress(uint8_t *out, int out_cap, const uint8_t *in, int in_size, 
   }
   free(seg_bits);
   free(seg_pos);
-  return (int)pos;
+  return (long long)pos;
 }
 
 typedef struct {
@@ -886,10 +886,10 @@ static int parse_tree(BitR *r, DTree *t) {
 }
 
 /* huffman_dec.cpp:274-418.  Fully checked (hostile streams are rejected, never over-read). */
-static int decode_stream(const DTree *t, const uint8_t *p, size_t size, uint8_t *out, int out_size,
+static int decode_stream(const DTree *t, const uint8_t *p, size_t size, uint8_t *out, size_t out_size,
                          int strict) {
   BitR r = {p, 0, size * 8, 0};
-  int n = 0;
+  size_t n = 0;
   while (n < out_size) {
     int k = 0;
     while (t->sym[k] < 0) {
@@ -908,17 +908,17 @@ static int decode_stream(const DTree *t, const uint8_t *p, size_t size, uint8_t 
       out[n++] = (uint8_t)s;
       continue;
     }
-    int z;
+    size_t z;
     switch (s) {
       case SYM_Z2: z = 2; break;
-      case SYM_Z6: z = (int)get_bits(&r, 2) + 3; break;
-      case SYM_Z22: z = (int)get_bits(&r, 4) + 7; break;
-      case SYM_Z278: z = (int)get_bits(&r, 8) + 23; break;
-      case SYM_Z16662: z = (int)get_bits(&r, 14) + 279; break;
+      case SYM_Z6: z = get_bits(&r, 2) + 3; break;
+      case SYM_Z22: z = get_bits(&r, 4) + 7; break;
+      case SYM_Z278: z = get_bits(&r, 8) + 23; break;
+      case SYM_Z16662: z = get_bits(&r, 14) + 279; break;
       default: return 0;
     }
     if (r.fail || n + z > out_size) return 0;
-    memset(out + n, 0, (size_t)z);
+    memset(out + n, 0, z);
     n += z;
   }
   /* BitStream::AtTheEnd, huffman_dec.cpp:140-145: the read position must lie in the last byte
@@ -926,15 +926,14 @@ static int decode_stream(const DTree *t, const uint8_t *p, size_t size, uint8_t 
   return size == 0 ? r.bit == 0 : (r.bit > 8 * (size - 1) && r.bit <= 8 * size);
 }
 
-int ho_huff_uncompress(const uint8_t *in, int in_size, int block_size, int block_no, uint8_t *out,
-                       int out_size, int strict, int unpacked_total) {
-  if (in_size < 0) return 0;
-  BitR r = {in, 0, (size_t)in_size * 8, 0};
+int ho_huff_uncompress(const uint8_t *in, size_t in_size, size_t block_size, int block_no, uint8_t *out,
+                       size_t out_size, int strict, size_t unpacked_total) {
+  BitR r = {in, 0, in_size * 8, 0};
   DTree *t = (DTree *)malloc(sizeof(DTree));
   int ok = 0;
   if (!parse_tree(&r, t)) goto done;
   size_t pos = (r.bit + 7) / 8;
-  int bs = block_size > 0 ? block_size : in_size;
+  size_t bs = block_size > 0 ? block_size : in_size;
   /* huffman_dec.cpp:215-219: the reference compares the UNPACKED block size with the PACKED
    * chunk size (SURVEY A.4-6); lenient mode uses what the encoder did. */
   int framed = strict ? bs < in_size : (block_size > 0 && block_size < unpacked_total);
@@ -942,25 +941,25 @@ int ho_huff_uncompress(const uint8_t *in, int in_size, int block_size, int block
   if (!strict && !framed && block_no == 0) block_no = -1;
   if (block_no < 0) {
     if (framed) goto done;
-    if (pos == (size_t)in_size) { /* :278-279 */
+    if (pos == in_size) { /* :278-279 */
       ok = out_size == 0;
       goto done;
     }
-    ok = decode_stream(t, in + pos, (size_t)in_size - pos, out, out_size, strict);
+    ok = decode_stream(t, in + pos, in_size - pos, out, out_size, strict);
     goto done;
   }
   if (!framed) goto done; /* UncompressBlock refuses, huffman_dec.cpp:265 */
   for (int b = 0;; ++b) { /* :233-248 */
-    if (pos == (size_t)in_size) goto done; /* table ended before block_no */
-    if (pos + 2 > (size_t)in_size) goto done;
+    if (pos == in_size) goto done; /* table ended before block_no */
+    if (pos + 2 > in_size) goto done;
     size_t sz = in[pos] | ((size_t)in[pos + 1] << 8);
     pos += 2;
     if (sz & 0x8000) {
-      if (pos + 2 > (size_t)in_size) goto done;
+      if (pos + 2 > in_size) goto done;
       sz = (sz & 0x7fff) | ((size_t)(in[pos] | (in[pos + 1] << 8)) << 15);
       pos += 2;
     }
-    if (pos + sz > (size_t)in_size) goto done;
+    if (pos + sz > in_size) goto done;
     if (b == block_no) {
       ok = decode_stream(t, in + pos, sz, out, out_size, strict);
       goto done;
@@ -993,16 +992,16 @@ static size_t put_chunk_hdr(uint8_t *out, size_t pos, const char *fourcc, uint32
   return pos + 8;
 }
 
-int ho_encode_bound(int w, int h, int nch) {
-  int rows = (h + 7) >> 3, cols = (w + 7) >> 3;
-  long lres = (long)ho_lowres_channel_size(rows, cols) * nch;
-  long fres = (long)rows * cols * 64 * nch;
-  return (int)(12 + 19 + 136 + 8 + 72 + 188 + 8 + ho_huff_max_size((int)lres) + ho_huff_max_size((int)fres));
+size_t ho_encode_bound(int w, int h, int nch) {
+  size_t rows = (size_t)(h + 7) >> 3, cols = (size_t)(w + 7) >> 3;
+  size_t lres = (size_t)ho_lowres_channel_size((int)rows, (int)cols) * nch;
+  size_t fres = rows * cols * 64 * nch;
+  return 12 + 19 + 136 + 8 + 72 + 188 + 8 + ho_huff_max_size(lres) + ho_huff_max_size(fres);
 }
 
 /* encoder.cpp:59-109 (container layout: SURVEY A.1) */
-int ho_encode(const uint8_t *data, int w, int h, int pixel_stride, int nch, int quality,
-              int use_ycbcr, uint8_t *out, int out_cap) {
+long long ho_encode(const uint8_t *data, int w, int h, int pixel_stride, int nch, int quality,
+                    int use_ycbcr, uint8_t *out, size_t out_cap) {
   int ycbcr = use_ycbcr && nch >= 3;
   int rows = (h + 7) >> 3, cols = (w + 7) >> 3;
   size_t npix = (size_t)w * h;
@@ -1048,7 +1047,7 @@ int ho_encode(const uint8_t *data, int w, int h, int pixel_stride, int nch, int 
     pos += (size_t)n;
   }
   {
-    int n = ho_huff_compress(tmp + pos + 8, (int)(tmp_cap - pos - 8), lres, chsz * nch, 0);
+    long long n = ho_huff_compress(tmp + pos + 8, tmp_cap - pos - 8, lres, (size_t)chsz * nch, 0);
     if (n < 0) n = 0;
     pos = put_chunk_hdr(tmp, pos, "LRES", (uint32_t)n) + (size_t)n;
   }
@@ -1067,12 +1066,12 @@ int ho_encode(const uint8_t *data, int w, int h, int pixel_stride, int nch, int 
     pos += (size_t)n;
   }
   {
-    int n = ho_huff_compress(tmp + pos + 8, (int)(tmp_cap - pos - 8 - 512), planes, (int)fres_n, cols * nch * 64);
+    long long n = ho_huff_compress(tmp + pos + 8, tmp_cap - pos - 8 - 512, planes, fres_n, (size_t)cols * nch * 64);
     if (n < 0) n = 0;
     pos = put_chunk_hdr(tmp, pos, "FRES", (uint32_t)n) + (size_t)n;
   }
   put_u32(tmp + 4, (uint32_t)(pos - 8));
-  int ret = pos <= (size_t)out_cap ? (int)pos : -1;
+  long long ret = pos <= out_cap ? (long long)pos : -1;
   if (ret > 0) memcpy(out, tmp, pos);
   free(tmp);
   free(planes);
@@ -1083,15 +1082,15 @@ int ho_encode(const uint8_t *data, int w, int h, int pixel_stride, int nch, int 
 }
 
 /* decoder.cpp:428-461 */
-static int find_chunk(const uint8_t *p, int size, int *idx, const char *fourcc, int *chunk_size) {
+static int find_chunk(const uint8_t *p, size_t size, size_t *idx, const char *fourcc, size_t *chunk_size) {
   for (;;) {
     if (*idx + 8 > size) return 0;
     uint32_t cc = get_u32(p + *idx);
     int32_t sz = (int32_t)get_u32(p + *idx + 4);
     *idx += 8;
-    if (sz < 0 || (long)*idx + sz > size) return 0;
+    if (sz < 0 || *idx + (size_t)sz > size) return 0;
     if (cc == get_u32((const uint8_t *)fourcc)) {
-      *chunk_size = sz;
+      *chunk_size = (size_t)sz;
       return 1;
     }
     *idx += sz;
@@ -1099,11 +1098,11 @@ static int find_chunk(const uint8_t *p, int size, int *idx, const char *fourcc, 
 }
 
 /* decoder.cpp:87-138 */
-int ho_decode(const uint8_t *packed, int size, int strict, uint8_t *out, int out_cap, int *w,
+int ho_decode(const uint8_t *packed, size_t size, int strict, uint8_t *out, size_t out_cap, int *w,
               int *h, int *nch) {
   if (size < 12 || memcmp(packed, "RIFF", 4) || memcmp(packed + 8, "HIMG", 4)) return 0;
-  if ((int32_t)get_u32(packed + 4) + 8 != size) return 0;
-  int idx = 12, cs;
+  if ((long long)(int32_t)get_u32(packed + 4) + 8 != (long long)size) return 0;
+  size_t idx = 12, cs;
   if (!find_chunk(packed, size, &idx, "FRMT", &cs) || cs < 11) return 0;
   const uint8_t *c = packed + idx;
   idx += cs;
@@ -1126,7 +1125,7 @@ int ho_decode(const uint8_t *packed, int size, int strict, uint8_t *out, int out
   uint8_t *R = (uint8_t *)malloc((size_t)rows * cols * N);
   uint8_t *planes = NULL;
   int ret = 0;
-  if (!ho_huff_uncompress(packed + idx, cs, 0, -1, lres, chsz * N, strict, chsz * N)) goto done;
+  if (!ho_huff_uncompress(packed + idx, cs, 0, -1, lres, (size_t)chsz * N, strict, (size_t)chsz * N)) goto done;
   idx += cs;
   for (int k = 0; k < N; ++k)
     ho_lowres_decode(lres + (size_t)k * chsz, rows, cols, lun, R + (size_t)k * rows * cols);
@@ -1147,12 +1146,12 @@ int ho_decode(const uint8_t *packed, int size, int strict, uint8_t *out, int out
   idx += cs;
 
   if (!find_chunk(packed, size, &idx, "FRES", &cs)) goto done;
-  if ((size_t)W * H * N > (size_t)out_cap) {
+  if ((size_t)W * H * N > out_cap) {
     ret = -1;
     goto done;
   }
-  int seg = cols * 64 * N;
-  planes = (uint8_t *)malloc((size_t)seg * rows);
+  size_t seg = (size_t)cols * 64 * N;
+  planes = (uint8_t *)malloc(seg * rows);
   for (int v = 0; v < rows; ++v)
     if (!ho_huff_uncompress(packed + idx, cs, seg, v, planes + (size_t)v * seg, seg, strict, seg * rows))
       goto done;

@@ -132,6 +132,22 @@ class Context:
                                                 C.byref(h), C.byref(n)), allow=(_native.REJECT,))
         return None if rc == _native.REJECT else out
 
+    def decode_scaled(self, data: bytes, factor: int, flags=STRICT):
+        """The image at 1/factor size (factor 1, 2, 4 or 8): the [ceil(h/f)][ceil(w/f)][nch] array of rounded box
+        averages of decode(data) over f x f windows (clipped at the right and bottom edges), or None where the stream
+        is rejected.  Raises HimgError (ERR_ARG) for another factor."""
+        buf = np.frombuffer(data, np.uint8)
+        w, h, n = C.c_int(), C.c_int(), C.c_int()
+        if self.lib.himgcu_decode_info(_ptr(buf), buf.size, C.byref(w), C.byref(h), C.byref(n)) != _native.OK:
+            return None
+        if w.value < 1 or h.value < 1 or n.value < 1:
+            return None
+        f = max(int(factor), 1)
+        out = np.empty((-(-h.value // f), -(-w.value // f), n.value), np.uint8)
+        rc = self._check(self.lib.himgcu_decode_scaled(self.h, _ptr(buf), buf.size, flags, factor, _ptr(out), out.size,
+                                                       C.byref(w), C.byref(h), C.byref(n)), allow=(_native.REJECT,))
+        return None if rc == _native.REJECT else out
+
     def decode_region(self, data: bytes, x: int, y: int, w: int, h: int, flags=STRICT):
         """Rectangle [x, x+w) x [y, y+h) of the image: the [h][w][nch] array equal to decode(data)[y:y+h, x:x+w],
         or None where the stream is rejected.  Raises HimgError for an empty rectangle or one outside the image."""
@@ -248,6 +264,55 @@ class Context:
             status = torch.empty((n,), dtype=torch.int32, device=himg.device)
         self._check(self.lib.himgcu_decode_batch_mixed(self.h, _ptr(himg), _ptr(offsets), _ptr(sizes), n, _ptr(dims), max_w,
                                                        max_h, nch, flags, _ptr(pixel_offsets), _ptr(out), _ptr(status)))
+        return out, pixel_offsets, status
+
+    def decode_batch_scaled(self, himg, offsets, sizes, w, h, nch, factor, flags=STRICT, out=None, status=None):
+        """decode_batch at 1/factor size (factor 1, 2, 4 or 8, see decode_scaled).  Returns (pixels
+        [n][ceil(h/f)][ceil(w/f)][nch], status)."""
+        import torch
+
+        n = offsets.numel()
+        self._bind(himg, offsets, sizes, out, status)
+        if out is None:
+            f = max(int(factor), 1)
+            out = torch.empty((n, -(-h // f), -(-w // f), nch), dtype=torch.uint8, device=himg.device)
+        if status is None:
+            status = torch.empty((n,), dtype=torch.int32, device=himg.device)
+        self._check(self.lib.himgcu_decode_batch_scaled(self.h, _ptr(himg), _ptr(offsets), _ptr(sizes), n, w, h, nch, flags,
+                                                        factor, _ptr(out), _ptr(status)))
+        return out, status
+
+    def decode_batch_mixed_scaled(self, himg, offsets, sizes, dims, nch, max_w, max_h, factor, flags=STRICT, out=None,
+                                  pixel_offsets=None, status=None):
+        """decode_batch_mixed at 1/factor size (factor 1, 2, 4 or 8, see decode_scaled): image i is written as
+        [ceil(h_i/f)][ceil(w_i/f)][nch] at byte pixel_offsets[i] of the flat uint8 buffer out.  When pixel_offsets is
+        None they are the exclusive prefix sum of those spans (0 for dims out of bounds), computed on the device; when
+        out is None it is allocated for the spans (one synchronisation).  Returns (out, pixel_offsets, status), with
+        the statuses of decode_batch_mixed."""
+        import torch
+
+        n = offsets.numel()
+        if dims.dtype != torch.int32 or dims.numel() != 2 * n:
+            raise ValueError("dims must be an int32 tensor [n][2]")
+        if pixel_offsets is not None and (pixel_offsets.dtype != torch.int64 or pixel_offsets.numel() != n):
+            raise ValueError("pixel_offsets must be an int64 tensor [n]")
+        self._bind(himg, offsets, sizes, dims, out, pixel_offsets, status)
+        if pixel_offsets is None or out is None:  # (an image with dims out of bounds gets an empty span)
+            f = max(int(factor), 1)
+            wh = dims.reshape(n, 2).to(torch.int64)
+            ok = (wh >= 1).all(dim=1) & (wh[:, 0] <= max_w) & (wh[:, 1] <= max_h)
+            swh = torch.div(wh + (f - 1), f, rounding_mode="floor")
+            spans = torch.where(ok, swh[:, 0] * swh[:, 1] * nch, 0)
+        if pixel_offsets is None:
+            pixel_offsets = torch.cumsum(spans, 0) - spans
+        if out is None:
+            total = int(spans.sum()) if n else 0
+            out = torch.empty((max(total, 1),), dtype=torch.uint8, device=himg.device)
+        if status is None:
+            status = torch.empty((n,), dtype=torch.int32, device=himg.device)
+        self._check(self.lib.himgcu_decode_batch_mixed_scaled(self.h, _ptr(himg), _ptr(offsets), _ptr(sizes), n, _ptr(dims),
+                                                              max_w, max_h, nch, flags, factor, _ptr(pixel_offsets), _ptr(out),
+                                                              _ptr(status)))
         return out, pixel_offsets, status
 
     def encode_batch_mixed(self, pixels, offsets, dims, nch, max_w, max_h, quality=50, use_ycbcr=True, out=None, sizes=None):

@@ -546,10 +546,76 @@ int launch_inv4(himgcu_ctx *ctx, const uint8_t *d_planes, const uint8_t *d_R, in
   return HIMGCU_OK;
 }
 
-// With `md` the batch has mixed geometry (see launch_inv) and takes the generic kernel.
+// Scaled decode by 2^lf (lf in 1..3), generic kernel: any shape, channel group [cbase, cbase + NCH) of ctotal channels.
+template <int NCH>
+int launch_inv_scaled(himgcu_ctx *ctx, const uint8_t *d_planes, const uint8_t *d_R, int n, const Geom &g,
+                      const DecTables *d_tabs, unsigned long long tab_stride, uint8_t *d_pixels, int cbase, int ctotal, int lf,
+                      const MixedDims *md, const unsigned long long *px_off) {
+  dim3 grid((g.cols + kTile - 1) / kTile, g.rows, n);
+  if (md) {
+    LAUNCH("k_inverse_scaled", (k_inverse_scaled<NCH, true>), grid, kTile, 0, d_planes, d_R, g, d_tabs, tab_stride, d_pixels, cbase,
+           ctotal, lf, *md, px_off);
+    return HIMGCU_OK;
+  }
+  LAUNCH("k_inverse_scaled", (k_inverse_scaled<NCH>), grid, kTile, 0, d_planes, d_R, g, d_tabs, tab_stride, d_pixels, cbase, ctotal, lf);
+  return HIMGCU_OK;
+}
+
+// Scaled decode by 2^LF, lane-pair kernel: the shapes and tiles of launch_inv4.
+template <int NCH, int LF>
+int launch_inv4_scaled(himgcu_ctx *ctx, const uint8_t *d_planes, const uint8_t *d_R, int n, const Geom &g,
+                       const DecTables *d_tabs, unsigned long long tab_stride, uint8_t *d_pixels) {
+  const int ntab = tab_stride ? n : 1;
+  InvTables *d_inv;
+  ENSURE("inv_tables", (size_t)ntab * sizeof(InvTables), d_inv);
+  LAUNCH("k_inv_tables", k_inv_tables, ntab, 256, 0, d_tabs, tab_stride, d_inv);
+  const unsigned long long inv_stride = tab_stride ? sizeof(InvTables) : 0;
+  const int total_pairs = g.rows * (g.cols / 2);
+  constexpr int TP = NCH == 1 ? kInv4ThreadsGray : kInv4ThreadsRgb;
+  dim3 grid((total_pairs + TP - 1) / TP, 1, n);
+  const int smem = NCH * 64 * 2 * TP + kInvTableBytes;
+  CK(cudaFuncSetAttribute((k_inverse4_scaled<NCH, TP, LF>), cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
+  LAUNCH("k_inverse4_scaled", (k_inverse4_scaled<NCH, TP, LF>), grid, TP, smem, d_planes, d_R, g, d_inv, inv_stride, d_pixels, 1u);
+  return HIMGCU_OK;
+}
+
+// K-inv of a decode scaled by 2^lf (lf in 1..3): image i is [ceil(h / 2^lf)][ceil(w / 2^lf)][nch], at d_pixels plus i times
+// that size, or with `md` at d_pixels + px_off[i] (see launch_inv).
+int stage_inverse_scaled(himgcu_ctx *ctx, const uint8_t *d_planes, const uint8_t *d_R, int n, const Geom &g,
+                         const DecTables *d_tabs, unsigned long long tab_stride, uint8_t *d_pixels, int lf,
+                         const MixedDims *md, const unsigned long long *px_off) {
+  // lane-pair path: the shapes k_inverse4 takes (every window is whole); its stores are 16 >> lf bytes wide
+  if (!md && !ctx->force_generic && !(ctx->xform_variant & 1) && (g.h % 8) == 0 && (g.cols % 16) == 0 && (g.w % 16) == 0 &&
+      (g.nch == 1 || g.nch == 3) && (reinterpret_cast<uintptr_t>(d_planes) & 15) == 0 &&
+      (reinterpret_cast<uintptr_t>(d_pixels) & ((16u >> lf) - 1)) == 0 && (reinterpret_cast<uintptr_t>(d_R) & 1) == 0) {
+    switch (g.nch * 4 + lf) {
+      case 1 * 4 + 1: return launch_inv4_scaled<1, 1>(ctx, d_planes, d_R, n, g, d_tabs, tab_stride, d_pixels);
+      case 1 * 4 + 2: return launch_inv4_scaled<1, 2>(ctx, d_planes, d_R, n, g, d_tabs, tab_stride, d_pixels);
+      case 1 * 4 + 3: return launch_inv4_scaled<1, 3>(ctx, d_planes, d_R, n, g, d_tabs, tab_stride, d_pixels);
+      case 3 * 4 + 1: return launch_inv4_scaled<3, 1>(ctx, d_planes, d_R, n, g, d_tabs, tab_stride, d_pixels);
+      case 3 * 4 + 2: return launch_inv4_scaled<3, 2>(ctx, d_planes, d_R, n, g, d_tabs, tab_stride, d_pixels);
+      default: return launch_inv4_scaled<3, 3>(ctx, d_planes, d_R, n, g, d_tabs, tab_stride, d_pixels);
+    }
+  }
+  switch (g.nch) {
+    case 1: return launch_inv_scaled<1>(ctx, d_planes, d_R, n, g, d_tabs, tab_stride, d_pixels, 0, 1, lf, md, px_off);
+    case 2: return launch_inv_scaled<2>(ctx, d_planes, d_R, n, g, d_tabs, tab_stride, d_pixels, 0, 2, lf, md, px_off);
+    case 3: return launch_inv_scaled<3>(ctx, d_planes, d_R, n, g, d_tabs, tab_stride, d_pixels, 0, 3, lf, md, px_off);
+    case 4: return launch_inv_scaled<4>(ctx, d_planes, d_R, n, g, d_tabs, tab_stride, d_pixels, 0, 4, lf, md, px_off);
+    default: break;
+  }
+  int rc = launch_inv_scaled<3>(ctx, d_planes, d_R, n, g, d_tabs, tab_stride, d_pixels, 0, g.nch, lf, md, px_off);
+  for (int c = 3; c < g.nch && !rc; ++c)
+    rc = launch_inv_scaled<1>(ctx, d_planes, d_R, n, g, d_tabs, tab_stride, d_pixels, c, g.nch, lf, md, px_off);
+  return rc;
+}
+
+// With `md` the batch has mixed geometry (see launch_inv) and takes the generic kernel.  lf > 0: the decode is scaled by
+// 2^lf (stage_inverse_scaled).
 int stage_inverse(himgcu_ctx *ctx, const uint8_t *d_planes, const uint8_t *d_R, int n, const Geom &g,
                   const DecTables *d_tabs, unsigned long long tab_stride, uint8_t *d_pixels, const MixedDims *md = nullptr,
-                  const unsigned long long *px_off = nullptr) {
+                  const unsigned long long *px_off = nullptr, int lf = 0) {
+  if (lf) return stage_inverse_scaled(ctx, d_planes, d_R, n, g, d_tabs, tab_stride, d_pixels, lf, md, px_off);
   // lane-pair fast path: two blocks per thread, flat tiles, 16-byte pixel stores
   if (!md && !ctx->force_generic && !(ctx->xform_variant & 1) && (g.h % 8) == 0 && (g.cols % 16) == 0 && (g.w % 16) == 0 &&
       (g.nch == 1 || g.nch == 3) && (reinterpret_cast<uintptr_t>(d_planes) & 15) == 0 &&
@@ -961,10 +1027,11 @@ int decode_front(himgcu_ctx *ctx, const uint8_t *d_himg, const unsigned long lon
 }
 
 // Whole-image decode of n streams resident on the device.  With `md` the batch has mixed geometry: g is its bounding
-// geometry, and image i is written at d_pixels + px_off[i] with its own size (see MixedDims).
+// geometry, and image i is written at d_pixels + px_off[i] with its own size (see MixedDims).  lf > 0: every image is
+// written scaled by 2^lf (stage_inverse_scaled); everything before the inverse transform is the same.
 int decode_device(himgcu_ctx *ctx, const uint8_t *d_himg, const unsigned long long *d_offsets,
                   const uint32_t *d_sizes, int n, const Geom &g, int flags, uint8_t *d_pixels, int *d_status,
-                  const MixedDims *md = nullptr, const unsigned long long *px_off = nullptr) {
+                  const MixedDims *md = nullptr, const unsigned long long *px_off = nullptr, int lf = 0) {
   const int lenient = (flags & HIMGCU_LENIENT) ? 1 : 0;
   uint8_t *d_planes;
   ENSURE("planes", (size_t)n * g.planes_bytes, d_planes);
@@ -991,7 +1058,7 @@ int decode_device(himgcu_ctx *ctx, const uint8_t *d_himg, const unsigned long lo
              d_fseg, g.rows, g.seg, d_planes, g.planes_bytes, d_status, 0, 0, *md);
     }
     if (fork) CK(cudaStreamWaitEvent(main_stream, ctx->ev_join, 0));
-    return stage_inverse(ctx, d_planes, d_R, n, g, d_tabs, sizeof(DecTables), d_pixels, md, px_off);
+    return stage_inverse(ctx, d_planes, d_R, n, g, d_tabs, sizeof(DecTables), d_pixels, md, px_off, lf);
   }
   // Few streams (single images): the serial walk over the segment headers runs inside the decode kernel
   // and the rows decode as soon as their entry is published (all CTAs of such a grid are resident at once)
@@ -1001,7 +1068,7 @@ int decode_device(himgcu_ctx *ctx, const uint8_t *d_himg, const unsigned long lo
     LAUNCH("k_dec_stream_fres", k_dec_stream_par<false>, dim3(g.rows + 1, n), fres_team, 0, d_himg, d_fcd, d_ftree, d_fseg,
            g.rows, g.seg, d_planes, g.planes_bytes, d_status, 1, lenient);
     if (fork) CK(cudaStreamWaitEvent(main_stream, ctx->ev_join, 0));
-    return stage_inverse(ctx, d_planes, d_R, n, g, d_tabs, sizeof(DecTables), d_pixels);
+    return stage_inverse(ctx, d_planes, d_R, n, g, d_tabs, sizeof(DecTables), d_pixels, nullptr, nullptr, lf);
   }
   LAUNCH("k_dec_segtab", k_dec_segtab, nb, 128, 0, d_himg, d_fcd, d_ftree, n, g.rows, g.seg, 1, lenient, d_fseg,
          d_status);
@@ -1013,7 +1080,7 @@ int decode_device(himgcu_ctx *ctx, const uint8_t *d_himg, const unsigned long lo
            g.rows, g.seg, d_planes, g.planes_bytes, d_status);
   }
   if (fork) CK(cudaStreamWaitEvent(main_stream, ctx->ev_join, 0));
-  return stage_inverse(ctx, d_planes, d_R, n, g, d_tabs, sizeof(DecTables), d_pixels);
+  return stage_inverse(ctx, d_planes, d_R, n, g, d_tabs, sizeof(DecTables), d_pixels, nullptr, nullptr, lf);
 }
 
 // Compact block rows a region decode keeps per image: the most a rectangle of rh rows can touch.
@@ -1538,6 +1605,116 @@ int copy_to_host(himgcu_ctx *ctx, void *dst, const void *src, size_t bytes) {
   return HIMGCU_OK;
 }
 
+// log2 of the factor of a scaled decode: 0 to 3 for 1, 2, 4, 8; -1 for any other factor.
+int scale_log2(int factor) {
+  switch (factor) {
+    case 1: return 0;
+    case 2: return 1;
+    case 4: return 2;
+    case 8: return 3;
+    default: return -1;
+  }
+}
+
+// Bytes of one image of g decoded at 1 / 2^lf size: [ceil(h / 2^lf)][ceil(w / 2^lf)][nch].
+size_t scaled_bytes(const Geom &g, int lf) {
+  const int f = 1 << lf;
+  return (size_t)((g.w + f - 1) >> lf) * (size_t)((g.h + f - 1) >> lf) * (size_t)g.nch;
+}
+
+// himgcu_decode_batch, and with lf > 0 himgcu_decode_batch_scaled: image i goes to d_pixels_out + i * scaled_bytes(g, lf).
+int decode_batch_lf(himgcu_ctx *ctx, const uint8_t *d_himg, const uint64_t *d_offsets, const uint32_t *d_sizes, int n, int w,
+                    int h, int nch, int flags, int lf, uint8_t *d_pixels_out, int32_t *d_status) {
+  if (!ctx || !d_himg || !d_offsets || !d_sizes || !d_pixels_out || !d_status || n < 0)
+    return fail(ctx, HIMGCU_ERR_ARG, "bad argument");
+  if (!shape_ok(w, h, nch)) return fail(ctx, HIMGCU_ERR_UNSUPPORTED, "unsupported shape %dx%dx%d", w, h, nch);
+  if (n == 0) return HIMGCU_OK;
+  CK(cudaSetDevice(ctx->device));
+  const Geom g = make_geom(w, h, nch, nch);
+  const size_t per = per_image_encode_ws(g) + sizeof(DecTables) + 2 * sizeof(DecTree);
+  int sub = (int)std::min<size_t>((size_t)n, std::max<size_t>(1, ctx->max_workspace / per));
+  sub = std::min(sub, 65535);
+  for (int i0 = 0; i0 < n; i0 += sub) {
+    const int m = std::min(sub, n - i0);
+    int rc = decode_device(ctx, d_himg, reinterpret_cast<const unsigned long long *>(d_offsets) + i0, d_sizes + i0, m,
+                           g, flags, d_pixels_out + (size_t)i0 * scaled_bytes(g, lf), d_status + i0, nullptr, nullptr, lf);
+    if (rc) return rc;
+  }
+  return HIMGCU_OK;
+}
+
+// himgcu_decode_batch_mixed, and with lf > 0 himgcu_decode_batch_mixed_scaled.
+int decode_batch_mixed_lf(himgcu_ctx *ctx, const uint8_t *d_himg, const uint64_t *d_offsets, const uint32_t *d_sizes, int n,
+                          const int32_t *d_dims, int max_width, int max_height, int nch, int flags, int lf,
+                          const uint64_t *d_pixel_offsets, uint8_t *d_pixels_out, int32_t *d_status) {
+  if (!ctx || !d_himg || !d_offsets || !d_sizes || !d_dims || !d_pixel_offsets || !d_pixels_out || !d_status || n < 0)
+    return fail(ctx, HIMGCU_ERR_ARG, "bad argument");
+  if (!shape_ok(max_width, max_height, nch))
+    return fail(ctx, HIMGCU_ERR_UNSUPPORTED, "unsupported bounding shape %dx%dx%d", max_width, max_height, nch);
+  if (n == 0) return HIMGCU_OK;
+  CK(cudaSetDevice(ctx->device));
+  // every per-image scratch slot has the bounding geometry's size; the kernels lay each image out in its own
+  const Geom g = make_geom(max_width, max_height, nch, nch);
+  const size_t per = per_image_encode_ws(g) + sizeof(DecTables) + 2 * sizeof(DecTree);
+  int sub = (int)std::min<size_t>((size_t)n, std::max<size_t>(1, ctx->max_workspace / per));
+  sub = std::min(sub, 65535);
+  for (int i0 = 0; i0 < n; i0 += sub) {
+    const int m = std::min(sub, n - i0);
+    const MixedDims md{d_dims + 2 * (size_t)i0, max_width, max_height, nch};
+    int rc = decode_device(ctx, d_himg, reinterpret_cast<const unsigned long long *>(d_offsets) + i0, d_sizes + i0, m, g, flags,
+                           d_pixels_out, d_status + i0, &md, reinterpret_cast<const unsigned long long *>(d_pixel_offsets) + i0, lf);
+    if (rc) return rc;
+  }
+  return HIMGCU_OK;
+}
+
+// himgcu_decode, and with lf > 0 himgcu_decode_scaled (out_cap is checked against the scaled size).
+int decode_single_lf(himgcu_ctx *ctx, const uint8_t *himg, size_t size, int flags, int lf, uint8_t *out, size_t out_cap, int *w,
+                     int *h, int *nch) {
+  if (!ctx || !himg || !out) return fail(ctx, HIMGCU_ERR_ARG, "bad argument");
+  int W = 0, H = 0, N = 0;
+  if (himgcu_decode_info(himg, size, &W, &H, &N) != HIMGCU_OK) return fail(ctx, HIMGCU_REJECT, "not a HIMG stream");
+  if (w) *w = W;
+  if (h) *h = H;
+  if (nch) *nch = N;
+  if (W < 1 || H < 1 || N < 1) return fail(ctx, HIMGCU_REJECT, "bad dimensions");
+  if (!shape_ok(W, H, N)) return fail(ctx, HIMGCU_ERR_UNSUPPORTED, "unsupported shape %dx%dx%d", W, H, N);
+  if (size > 0xffffffffull) return fail(ctx, HIMGCU_ERR_UNSUPPORTED, "stream too large");
+  CK(cudaSetDevice(ctx->device));
+  const Geom g = make_geom(W, H, N, N);
+  const size_t out_bytes = scaled_bytes(g, lf);
+  if (out_bytes > out_cap) return fail(ctx, HIMGCU_ERR_CAPACITY, "output buffer too small");
+  uint8_t *d_in, *d_px;
+  unsigned long long *d_off;
+  uint32_t *d_sz;
+  int *d_status;
+  ENSURE("single_in", size + 16, d_in);
+  ENSURE("single_px", out_bytes, d_px);
+  ENSURE("single_off", sizeof(unsigned long long), d_off);
+  ENSURE("single_size", sizeof(uint32_t), d_sz);
+  ENSURE("single_status", sizeof(int), d_status);
+  int rc = ensure_pinned(ctx, 64);
+  if (rc) return rc;
+  // offset / size / status travel through the context's page-locked scratch (truly asynchronous copies)
+  unsigned long long *h_off = reinterpret_cast<unsigned long long *>(ctx->pinned);
+  uint32_t *h_sz = reinterpret_cast<uint32_t *>(h_off + 1);
+  int *h_status = reinterpret_cast<int *>(h_off + 2);
+  CK(cudaStreamSynchronize(ctx->stream));  // (the scratch words of the previous call are no longer in flight)
+  *h_off = 0;
+  *h_sz = (uint32_t)size;
+  if ((rc = copy_to_device(ctx, d_in, himg, size))) return rc;
+  CK(cudaMemcpyAsync(d_off, h_off, sizeof(*h_off), cudaMemcpyHostToDevice, ctx->stream));
+  CK(cudaMemcpyAsync(d_sz, h_sz, sizeof(*h_sz), cudaMemcpyHostToDevice, ctx->stream));
+  rc = decode_device(ctx, d_in, d_off, d_sz, 1, g, flags, d_px, d_status, nullptr, nullptr, lf);
+  if (rc) return rc;
+  // The pixels follow the status on the same stream without a round trip in between: a rejected stream
+  // costs one wasted copy, an accepted one (the common case) saves a synchronisation.
+  CK(cudaMemcpyAsync(h_status, d_status, sizeof(int), cudaMemcpyDeviceToHost, ctx->stream));
+  if ((rc = copy_to_host(ctx, out, d_px, out_bytes))) return rc;
+  if (*h_status) return fail(ctx, HIMGCU_REJECT, "stream rejected");
+  return HIMGCU_OK;
+}
+
 }  // namespace
 
 extern "C" {
@@ -1604,91 +1781,42 @@ int himgcu_decode_info(const uint8_t *p, size_t size, int *w, int *h, int *nch) 
 
 int himgcu_decode_batch(himgcu_ctx *ctx, const uint8_t *d_himg, const uint64_t *d_offsets, const uint32_t *d_sizes,
                         int n, int w, int h, int nch, int flags, uint8_t *d_pixels_out, int32_t *d_status) {
-  if (!ctx || !d_himg || !d_offsets || !d_sizes || !d_pixels_out || !d_status || n < 0)
-    return fail(ctx, HIMGCU_ERR_ARG, "bad argument");
-  if (!shape_ok(w, h, nch)) return fail(ctx, HIMGCU_ERR_UNSUPPORTED, "unsupported shape %dx%dx%d", w, h, nch);
-  if (n == 0) return HIMGCU_OK;
-  CK(cudaSetDevice(ctx->device));
-  const Geom g = make_geom(w, h, nch, nch);
-  const size_t per = per_image_encode_ws(g) + sizeof(DecTables) + 2 * sizeof(DecTree);
-  int sub = (int)std::min<size_t>((size_t)n, std::max<size_t>(1, ctx->max_workspace / per));
-  sub = std::min(sub, 65535);
-  for (int i0 = 0; i0 < n; i0 += sub) {
-    const int m = std::min(sub, n - i0);
-    int rc = decode_device(ctx, d_himg, reinterpret_cast<const unsigned long long *>(d_offsets) + i0, d_sizes + i0, m,
-                           g, flags, d_pixels_out + (size_t)i0 * g.out_img_bytes, d_status + i0);
-    if (rc) return rc;
-  }
-  return HIMGCU_OK;
+  return decode_batch_lf(ctx, d_himg, d_offsets, d_sizes, n, w, h, nch, flags, 0, d_pixels_out, d_status);
+}
+
+int himgcu_decode_batch_scaled(himgcu_ctx *ctx, const uint8_t *d_himg, const uint64_t *d_offsets, const uint32_t *d_sizes,
+                               int n, int w, int h, int nch, int flags, int factor, uint8_t *d_pixels_out, int32_t *d_status) {
+  const int lf = scale_log2(factor);
+  if (lf < 0) return fail(ctx, HIMGCU_ERR_ARG, "scale factor %d is not 1, 2, 4 or 8", factor);
+  return decode_batch_lf(ctx, d_himg, d_offsets, d_sizes, n, w, h, nch, flags, lf, d_pixels_out, d_status);
 }
 
 int himgcu_decode_batch_mixed(himgcu_ctx *ctx, const uint8_t *d_himg, const uint64_t *d_offsets, const uint32_t *d_sizes, int n,
                               const int32_t *d_dims, int max_width, int max_height, int nch, int flags,
                               const uint64_t *d_pixel_offsets, uint8_t *d_pixels_out, int32_t *d_status) {
-  if (!ctx || !d_himg || !d_offsets || !d_sizes || !d_dims || !d_pixel_offsets || !d_pixels_out || !d_status || n < 0)
-    return fail(ctx, HIMGCU_ERR_ARG, "bad argument");
-  if (!shape_ok(max_width, max_height, nch))
-    return fail(ctx, HIMGCU_ERR_UNSUPPORTED, "unsupported bounding shape %dx%dx%d", max_width, max_height, nch);
-  if (n == 0) return HIMGCU_OK;
-  CK(cudaSetDevice(ctx->device));
-  // every per-image scratch slot has the bounding geometry's size; the kernels lay each image out in its own
-  const Geom g = make_geom(max_width, max_height, nch, nch);
-  const size_t per = per_image_encode_ws(g) + sizeof(DecTables) + 2 * sizeof(DecTree);
-  int sub = (int)std::min<size_t>((size_t)n, std::max<size_t>(1, ctx->max_workspace / per));
-  sub = std::min(sub, 65535);
-  for (int i0 = 0; i0 < n; i0 += sub) {
-    const int m = std::min(sub, n - i0);
-    const MixedDims md{d_dims + 2 * (size_t)i0, max_width, max_height, nch};
-    int rc = decode_device(ctx, d_himg, reinterpret_cast<const unsigned long long *>(d_offsets) + i0, d_sizes + i0, m, g, flags,
-                           d_pixels_out, d_status + i0, &md, reinterpret_cast<const unsigned long long *>(d_pixel_offsets) + i0);
-    if (rc) return rc;
-  }
-  return HIMGCU_OK;
+  return decode_batch_mixed_lf(ctx, d_himg, d_offsets, d_sizes, n, d_dims, max_width, max_height, nch, flags, 0, d_pixel_offsets,
+                               d_pixels_out, d_status);
+}
+
+int himgcu_decode_batch_mixed_scaled(himgcu_ctx *ctx, const uint8_t *d_himg, const uint64_t *d_offsets, const uint32_t *d_sizes,
+                                     int n, const int32_t *d_dims, int max_width, int max_height, int nch, int flags, int factor,
+                                     const uint64_t *d_pixel_offsets, uint8_t *d_pixels_out, int32_t *d_status) {
+  const int lf = scale_log2(factor);
+  if (lf < 0) return fail(ctx, HIMGCU_ERR_ARG, "scale factor %d is not 1, 2, 4 or 8", factor);
+  return decode_batch_mixed_lf(ctx, d_himg, d_offsets, d_sizes, n, d_dims, max_width, max_height, nch, flags, lf, d_pixel_offsets,
+                               d_pixels_out, d_status);
 }
 
 int himgcu_decode(himgcu_ctx *ctx, const uint8_t *himg, size_t size, int flags, uint8_t *out, size_t out_cap, int *w,
                   int *h, int *nch) {
-  if (!ctx || !himg || !out) return fail(ctx, HIMGCU_ERR_ARG, "bad argument");
-  int W = 0, H = 0, N = 0;
-  if (himgcu_decode_info(himg, size, &W, &H, &N) != HIMGCU_OK) return fail(ctx, HIMGCU_REJECT, "not a HIMG stream");
-  if (w) *w = W;
-  if (h) *h = H;
-  if (nch) *nch = N;
-  if (W < 1 || H < 1 || N < 1) return fail(ctx, HIMGCU_REJECT, "bad dimensions");
-  if (!shape_ok(W, H, N)) return fail(ctx, HIMGCU_ERR_UNSUPPORTED, "unsupported shape %dx%dx%d", W, H, N);
-  if (size > 0xffffffffull) return fail(ctx, HIMGCU_ERR_UNSUPPORTED, "stream too large");
-  CK(cudaSetDevice(ctx->device));
-  const Geom g = make_geom(W, H, N, N);
-  if (g.out_img_bytes > out_cap) return fail(ctx, HIMGCU_ERR_CAPACITY, "output buffer too small");
-  uint8_t *d_in, *d_px;
-  unsigned long long *d_off;
-  uint32_t *d_sz;
-  int *d_status;
-  ENSURE("single_in", size + 16, d_in);
-  ENSURE("single_px", g.out_img_bytes, d_px);
-  ENSURE("single_off", sizeof(unsigned long long), d_off);
-  ENSURE("single_size", sizeof(uint32_t), d_sz);
-  ENSURE("single_status", sizeof(int), d_status);
-  int rc = ensure_pinned(ctx, 64);
-  if (rc) return rc;
-  // offset / size / status travel through the context's page-locked scratch (truly asynchronous copies)
-  unsigned long long *h_off = reinterpret_cast<unsigned long long *>(ctx->pinned);
-  uint32_t *h_sz = reinterpret_cast<uint32_t *>(h_off + 1);
-  int *h_status = reinterpret_cast<int *>(h_off + 2);
-  CK(cudaStreamSynchronize(ctx->stream));  // (the scratch words of the previous call are no longer in flight)
-  *h_off = 0;
-  *h_sz = (uint32_t)size;
-  if ((rc = copy_to_device(ctx, d_in, himg, size))) return rc;
-  CK(cudaMemcpyAsync(d_off, h_off, sizeof(*h_off), cudaMemcpyHostToDevice, ctx->stream));
-  CK(cudaMemcpyAsync(d_sz, h_sz, sizeof(*h_sz), cudaMemcpyHostToDevice, ctx->stream));
-  rc = decode_device(ctx, d_in, d_off, d_sz, 1, g, flags, d_px, d_status);
-  if (rc) return rc;
-  // The pixels follow the status on the same stream without a round trip in between: a rejected stream
-  // costs one wasted copy, an accepted one (the common case) saves a synchronisation.
-  CK(cudaMemcpyAsync(h_status, d_status, sizeof(int), cudaMemcpyDeviceToHost, ctx->stream));
-  if ((rc = copy_to_host(ctx, out, d_px, g.out_img_bytes))) return rc;
-  if (*h_status) return fail(ctx, HIMGCU_REJECT, "stream rejected");
-  return HIMGCU_OK;
+  return decode_single_lf(ctx, himg, size, flags, 0, out, out_cap, w, h, nch);
+}
+
+int himgcu_decode_scaled(himgcu_ctx *ctx, const uint8_t *himg, size_t size, int flags, int factor, uint8_t *out, size_t out_cap,
+                         int *w, int *h, int *nch) {
+  const int lf = scale_log2(factor);
+  if (lf < 0) return fail(ctx, HIMGCU_ERR_ARG, "scale factor %d is not 1, 2, 4 or 8", factor);
+  return decode_single_lf(ctx, himg, size, flags, lf, out, out_cap, w, h, nch);
 }
 
 int himgcu_decode_batch_region(himgcu_ctx *ctx, const uint8_t *d_himg, const uint64_t *d_offsets, const uint32_t *d_sizes, int n,

@@ -248,11 +248,40 @@ struct Inv4Store16 {
   }
 };
 
+// Output row wy of a block pair's 1 / 2^LF scaled decode (p: the (8 >> LF) * NCH pooled lane pairs, pixel-major,
+// channel-minor; low lanes block A, high lanes block B) to dst0 + wy * row_bytes: the K bytes of block A, then those of
+// block B, as NCH stores of 16 >> LF bytes each (8, 4 or 2: the pair's output row starts at a multiple of that).
+template <int NCH, int LF>
+struct Inv4StorePooled {
+  uint8_t *dst0;
+  size_t row_bytes;
+  __device__ __forceinline__ void operator()(int wy, const uint32_t (&p)[(8 >> LF) * NCH]) const {
+    constexpr int K = (8 >> LF) * NCH, UB = 16 >> LF;  // bytes per block, bytes per store
+    // byte b of the pair's output row (every lane holds a byte value)
+    auto byte = [&](int b) -> uint32_t { return b < K ? (p[b] & 0xffu) : (p[b - K] >> 16); };
+    uint8_t *dst = dst0 + (size_t)wy * row_bytes;
+    uint32_t wd[(2 * K + 3) / 4];
+#pragma unroll
+    for (int k = 0; k < (2 * K + 3) / 4; ++k) {
+      wd[k] = 0u;
+#pragma unroll
+      for (int j = 0; j < 4; ++j)
+        if (4 * k + j < 2 * K) wd[k] |= byte(4 * k + j) << (8 * j);
+    }
+#pragma unroll
+    for (int q = 0; q < NCH; ++q) {
+      if (UB == 8) reinterpret_cast<uint2 *>(dst)[q] = make_uint2(wd[2 * q], wd[2 * q + 1]);
+      else if (UB == 4) reinterpret_cast<uint32_t *>(dst)[q] = wd[q];
+      else reinterpret_cast<uint16_t *>(dst)[q] = (uint16_t)(wd[q >> 1] >> (16 * (q & 1)));
+    }
+  }
+};
+
 // The inverse proper for ONE thread = one block pair: codes in the thread's two byte columns `col` of a
 // shared-memory tile whose rows
 // (scan positions, channel-major) are PITCH bytes apart; the image's tables in sDq / sTab; pixel row y of
 // the pair goes out through store(y, ...) (active threads only).  No barrier inside.
-template <int NCH, int PITCH, class STORE = Inv4Store16<NCH>>
+template <int NCH, int PITCH, class STORE = Inv4Store16<NCH>, int LF = 0>
 __device__ __forceinline__ void inv4_compute(uint8_t *col, const uint8_t *sDq, const uint32_t *sTab, int pre, int tab_bias,
                                              bool overflow, bool ycbcr, bool active, const uint32_t (&top)[NCH],
                                              const uint32_t (&bot)[NCH], const STORE &store, uint32_t one) {
@@ -352,6 +381,7 @@ __device__ __forceinline__ void inv4_compute(uint8_t *col, const uint8_t *sDq, c
     uint32_t bias[NCH];
 #pragma unroll
     for (int c = 0; c < NCH; ++c) bias[c] = !do_colour ? 0u : c == 0 ? 0x02u : c == 1 ? 0x01u : 0u;
+    uint32_t pool[LF ? (8 >> LF) * NCH : 1];  // (LF > 0) window sums of the output row in progress, per channel
 #pragma unroll
     for (int y = 0; y < 8; ++y) {
       uint32_t s[8 * NCH];  // lane pairs in memory order: pixel-major, channel-minor
@@ -373,16 +403,37 @@ __device__ __forceinline__ void inv4_compute(uint8_t *col, const uint8_t *sDq, c
           ch[NCH >= 3 ? 2 : 0] = __viaddmin_s16x2_relu(Gp, cb, 0x00ff00ffu);
         }
       }
-      // words of block A and of block B: four consecutive lane pairs -> one word each (every lane is a
-      // byte value, so s1 * 256 + s0 = A0 | A1 << 8 | B0 << 16 | B1 << 24)
-      uint32_t wa[2 * NCH], wb[2 * NCH];
+      if constexpr (LF == 0) {
+        // words of block A and of block B: four consecutive lane pairs -> one word each (every lane is a
+        // byte value, so s1 * 256 + s0 = A0 | A1 << 8 | B0 << 16 | B1 << 24)
+        uint32_t wa[2 * NCH], wb[2 * NCH];
 #pragma unroll
-      for (int m = 0; m < 2 * NCH; ++m) {
-        const uint32_t pq = s[4 * m + 1] * k256 + s[4 * m], q = s[4 * m + 3] * k256 + s[4 * m + 2];
-        wa[m] = __byte_perm(pq, q, 0x5410);
-        wb[m] = __byte_perm(pq, q, 0x7632);
+        for (int m = 0; m < 2 * NCH; ++m) {
+          const uint32_t pq = s[4 * m + 1] * k256 + s[4 * m], q = s[4 * m + 3] * k256 + s[4 * m + 2];
+          wa[m] = __byte_perm(pq, q, 0x5410);
+          wb[m] = __byte_perm(pq, q, 0x7632);
+        }
+        if (active) store(y, wa, wb);
+      } else {
+        // scaled decode: box sums of the F x F windows on the lanes (at most 64 * 255 = 16320 per lane), then
+        // (S + F * F / 2) >> 2 LF per lane; output row y >> LF goes out after the window's last pixel row
+        constexpr int F = 1 << LF, OW = 8 >> LF;
+        if ((y & (F - 1)) == 0) {
+#pragma unroll
+          for (int m = 0; m < OW * NCH; ++m) pool[m] = 0u;
+        }
+#pragma unroll
+        for (int wx = 0; wx < OW; ++wx)
+#pragma unroll
+          for (int i = 0; i < F; ++i)
+#pragma unroll
+            for (int c = 0; c < NCH; ++c) pool[wx * NCH + c] += s[(wx * F + i) * NCH + c];
+        if ((y & (F - 1)) == F - 1) {
+#pragma unroll
+          for (int m = 0; m < OW * NCH; ++m) pool[m] = ((pool[m] + (F * F / 2) * 0x00010001u) >> (2 * LF)) & 0x00ff00ffu;
+          if (active) store(y >> LF, pool);
+        }
       }
-      if (active) store(y, wa, wb);
     }
   }
 }
@@ -464,6 +515,79 @@ __global__ void __launch_bounds__(TP, NCH == 1 ? 3 : 2)
   __syncthreads();  // the only barrier: from here on a thread touches its own two byte columns only
   inv4_compute<NCH, PITCH>(sPl + 2 * t, sDq, sTab, pre, tab_bias, overflow, ycbcr, active, top, bot,
                            Inv4Store16<NCH>{img + ((size_t)(8 * v) * g.w + (size_t)u * 8) * NCH, (size_t)g.w * NCH}, one);
+}
+
+// Scaled decode by F = 2^LF (LF in 1..3): k_inverse4 with the pooled output phase of inv4_compute.  Image z's output is
+// [h >> LF][w >> LF][NCH] (every window is whole on these shapes) at pixels + z * its size, each pixel the rounded box
+// average of its F x F window; the stores are 16 >> LF bytes wide.  Grid, block, shared memory and tiles as k_inverse4.
+template <int NCH, int TP, int LF>
+__global__ void __launch_bounds__(TP, NCH == 1 ? 3 : 2)
+    k_inverse4_scaled(const uint8_t *__restrict__ planes, const uint8_t *__restrict__ R, Geom g, const InvTables *__restrict__ tabs,
+                      unsigned long long tab_stride, uint8_t *__restrict__ pixels, uint32_t one) {
+  extern __shared__ __align__(128) uint8_t sPl[];
+  constexpr int PITCH = 2 * TP, CPR = TP / 8;  // bytes per tile row, 16-byte chunks per tile row
+  static_assert(TP % 32 == 0 && TP == 8 * CPR, "a CTA is 8 groups of one thread per chunk of a tile row");
+  uint8_t *sDq = sPl + NCH * 64 * PITCH;
+  uint32_t *sTab = reinterpret_cast<uint32_t *>(sDq + kInvSlots * 256 * 2);
+
+  const int t = threadIdx.x;
+  const int PR = g.cols >> 1, total = g.rows * PR;
+  const int f0 = blockIdx.x * TP;
+  const int nact = min(TP, total - f0);
+  const uint8_t *ipl = planes + (size_t)blockIdx.z * g.planes_bytes;
+  const size_t ow = (size_t)(g.w >> LF);  // (w % 16 == 0, h % 8 == 0: every window is whole)
+  uint8_t *img = pixels + (size_t)blockIdx.z * (ow * (size_t)(g.h >> LF) * NCH);
+  const InvTables *T = reinterpret_cast<const InvTables *>(reinterpret_cast<const char *>(tabs) + (size_t)blockIdx.z * tab_stride);
+  // block row / first pair of the tile's first element: one division per CTA, everything else by
+  // carrying (a tile spans few block rows unless the image is very narrow)
+  // (a true division: a 32-bit reciprocal of PR is not exact for every tile start of every accepted shape)
+  const int v0 = (int)((uint32_t)f0 / (uint32_t)PR), p0 = f0 - v0 * PR;
+  auto locate = [&](int k, int &v, int &p) {  // element f0 + k of the image -> block row, pair in the row
+    if (PR >= 32) {
+      v = v0;
+      p = p0 + k;
+      while (p >= PR) {
+        p -= PR;
+        ++v;
+      }
+    } else {
+      v = (f0 + k) / PR;
+      p = f0 + k - v * PR;
+    }
+  };
+  {
+    // the image's tables, then the tile: thread -> 16-byte chunk t % CPR (8 pairs of ONE block row:
+    // cols % 16 == 0) of the tile rows t / CPR + 8 i; the threads of a row copy 2 * TP contiguous bytes
+    const uint4 *tsrc = reinterpret_cast<const uint4 *>(T);
+    for (int i = t; i < kInvTableBytes / 16; i += TP) cp_async16(sDq + 16 * i, tsrc + i);
+    const int cq = t % CPR, r0 = t / CPR;
+    if (8 * cq < nact) {
+      int vl, pl;
+      locate(8 * cq, vl, pl);
+      const uint8_t *src = ipl + (size_t)vl * g.seg + 2 * pl + (size_t)r0 * g.cols;
+      uint8_t *dst = sPl + r0 * PITCH + cq * 16;
+      const size_t rstep = (size_t)8 * g.cols;
+#pragma unroll 8
+      for (int i = 0; i < NCH * 8; ++i) {
+        cp_async16(dst + i * 8 * PITCH, src);
+        src += rstep;
+      }
+    }
+  }
+  const int pre = T->pre, tab_bias = T->bias;
+  const bool overflow = T->overflow != 0;
+  const bool ycbcr = T->ycbcr != 0;
+  const bool active = t < nact;
+  int v, p;
+  locate(active ? t : 0, v, p);
+  const int u = 2 * p;
+  uint32_t top[NCH], bot[NCH];
+  inv4_corners<NCH>(R, blockIdx.z, g, v, u, top, bot);
+  cp_async_wait_all();
+  __syncthreads();  // the only barrier: from here on a thread touches its own two byte columns only
+  inv4_compute<NCH, PITCH, Inv4StorePooled<NCH, LF>, LF>(
+      sPl + 2 * t, sDq, sTab, pre, tab_bias, overflow, ycbcr, active, top, bot,
+      Inv4StorePooled<NCH, LF>{img + ((size_t)(v << (3 - LF)) * ow + ((size_t)u << (3 - LF))) * NCH, ow * NCH}, one);
 }
 
 }  // namespace himgcu

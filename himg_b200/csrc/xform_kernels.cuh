@@ -599,6 +599,118 @@ __global__ void __launch_bounds__(kTile)
   }
 }
 
+// ---------------------------------------------------------------------------------------------
+// K-inv of a scaled decode (factor F = 2^lf, lf in 1..3): k_inverse's transform, then the final pixels of the thread's
+// block (after the clamp and the inverse colour map) are box-averaged over the F x F windows that start at multiples
+// of F -- each lies inside one block, so no thread needs another's pixels.  Windows on the right and bottom image
+// edges are clipped: out = (S + n / 2) / n over the n pixels inside the image (1 <= n <= 64).
+// Image z's output is [ceil(h / F)][ceil(w / F)][ctotal] at pixels + z * its size, or, with MIXED, at
+// pixels + px_off[z] with its own geometry.  Grid, channel groups (cbase / ctotal) and MIXED as k_inverse.
+// ---------------------------------------------------------------------------------------------
+template <int NCH, bool MIXED = false>
+__global__ void __launch_bounds__(kTile)
+    k_inverse_scaled(const uint8_t *__restrict__ planes, const uint8_t *__restrict__ R, Geom g,
+                     const DecTables *__restrict__ tabs, unsigned long long tab_stride, uint8_t *__restrict__ pixels,
+                     int cbase, int ctotal, int lf, MixedDims md = {}, const unsigned long long *__restrict__ px_off = nullptr) {
+  __shared__ int16_t sUn[256];
+  __shared__ uint8_t sShift[2][64];
+  __shared__ uint32_t sOut[NCH][kTile][17];  // per channel: the 64 pixel bytes of each thread's block (+1 pad)
+  const Geom gb = g;  // bounding geometry (slot strides)
+  if (MIXED && (!image_geom(md, blockIdx.z, g) || (int)blockIdx.y >= g.rows || (int)blockIdx.x * kTile >= g.cols)) return;
+  const DecTables *T = reinterpret_cast<const DecTables *>(reinterpret_cast<const char *>(tabs) + (size_t)blockIdx.z * tab_stride);
+  for (int i = threadIdx.x; i < 256; i += blockDim.x) sUn[i] = T->full_unmap[i];
+  for (int i = threadIdx.x; i < 128; i += blockDim.x) sShift[i >> 6][i & 63] = T->shift[i >> 6][i & 63];
+  const bool YCBCR = T->ycbcr != 0 && cbase == 0;  // (only the first three channels of an image are colour mapped)
+  __syncthreads();
+  const int v = blockIdx.y, u = blockIdx.x * kTile + threadIdx.x;
+  if (u >= g.cols) return;
+  const int bh = min(8, g.h - 8 * v), bw = min(8, g.w - 8 * u);
+  const uint8_t *seg = planes + (size_t)blockIdx.z * gb.planes_bytes + (size_t)v * g.seg;
+
+  // ---- the transform of k_inverse, clamped samples to sOut
+#pragma unroll 1
+  for (int c = 0; c < NCH; ++c) {
+    int x[64];
+    const uint8_t *src = seg + (size_t)(cbase + c) * g.cols * 64 + u;
+    const uint8_t *sh = sShift[(YCBCR && NCH >= 3 && (c == 1 || c == 2)) ? 1 : 0];
+#pragma unroll
+    for (int j = 0; j < 64; ++j) {
+      const int code = __ldg(src + (size_t)scan_pos(j) * g.cols);
+      x[j] = (int)(short)(sUn[code] * (1 << sh[j]));
+    }
+#pragma unroll
+    for (int r = 0; r < 8; ++r) {
+      wht8(x[r * 8 + 0], x[r * 8 + 1], x[r * 8 + 2], x[r * 8 + 3], x[r * 8 + 4], x[r * 8 + 5], x[r * 8 + 6], x[r * 8 + 7]);
+#pragma unroll
+      for (int i = 0; i < 8; ++i) x[r * 8 + i] >>= 3;
+    }
+#pragma unroll
+    for (int q = 0; q < 8; ++q) {
+      wht8(x[q], x[8 + q], x[16 + q], x[24 + q], x[32 + q], x[40 + q], x[48 + q], x[56 + q]);
+#pragma unroll
+      for (int i = 0; i < 8; ++i) x[i * 8 + q] >>= 3;
+    }
+    {
+      const uint8_t *Rp = MIXED ? R + (size_t)blockIdx.z * ctotal * gb.rows * gb.cols + (size_t)(cbase + c) * g.rows * g.cols
+                                : R + ((size_t)blockIdx.z * ctotal + cbase + c) * g.rows * g.cols;
+      const LowCorners k = load_corners(Rp, g, u, v);
+      int lf9[9], rt9[9];
+      nine(k.x11, k.x21, lf9);
+      nine(k.x12, k.x22, rt9);
+#pragma unroll
+      for (int y = 0; y < 8; ++y) {
+        int t[9];
+        nine(lf9[y], rt9[y], t);
+#pragma unroll
+        for (int i = 0; i < 8; ++i) x[y * 8 + i] = clamp255((int)(short)(x[y * 8 + i] + t[i]));
+      }
+    }
+#pragma unroll
+    for (int k = 0; k < 16; ++k) {
+      const uint32_t lo = __byte_perm((uint32_t)x[4 * k], (uint32_t)x[4 * k + 1], 0x0040);
+      const uint32_t hi = __byte_perm((uint32_t)x[4 * k + 2], (uint32_t)x[4 * k + 3], 0x0040);
+      sOut[c][threadIdx.x][k] = __byte_perm(lo, hi, 0x5410);
+    }
+  }
+
+  // ---- inverse colour map in place (a thread only touches its own block's bytes)
+  uint8_t *px[NCH];  // pixel p = 8 * row + column of channel c: px[c][p]
+#pragma unroll
+  for (int c = 0; c < NCH; ++c) px[c] = reinterpret_cast<uint8_t *>(&sOut[c][threadIdx.x][0]);
+  if (NCH >= 3 && YCBCR) {
+#pragma unroll 4
+    for (int p = 0; p < 64; ++p) {
+      const int Y = px[0][p], cb = 2 * px[1][p] - 255, cr = 2 * px[NCH >= 3 ? 2 : 0][p] - 255;
+      const int G = Y - ((cb + cr + 2) >> 2);
+      px[0][p] = (uint8_t)clamp255(G + cr);
+      px[1][p] = (uint8_t)clamp255(G);
+      px[NCH >= 3 ? 2 : 0][p] = (uint8_t)clamp255(G + cb);
+    }
+  }
+
+  // ---- box averages of the windows inside the image
+  const int f = 1 << lf;
+  const size_t ow = (size_t)((g.w + f - 1) >> lf), oh = (size_t)((g.h + f - 1) >> lf);
+  uint8_t *img = MIXED ? pixels + px_off[blockIdx.z] : pixels + (size_t)blockIdx.z * ow * oh * ctotal;
+  const int nwy = (bh + f - 1) >> lf, nwx = (bw + f - 1) >> lf;
+#pragma unroll 1
+  for (int wy = 0; wy < nwy; ++wy) {
+    const int ny = min(f, bh - wy * f);
+    uint8_t *row = img + (((size_t)(8 * v >> lf) + wy) * ow + (size_t)(8 * u >> lf)) * ctotal + cbase;
+#pragma unroll 1
+    for (int wx = 0; wx < nwx; ++wx) {
+      const int nx = min(f, bw - wx * f), n = nx * ny, p0 = wy * f * 8 + wx * f;
+#pragma unroll
+      for (int c = 0; c < NCH; ++c) {
+        int S = 0;
+        for (int yy = 0; yy < ny; ++yy)
+          for (int xx = 0; xx < nx; ++xx) S += px[c][p0 + yy * 8 + xx];
+        row[(size_t)wx * ctotal + c] = (uint8_t)((S + (n >> 1)) / n);
+      }
+    }
+  }
+}
+
 }  // namespace himgcu
 
 #endif  // HIMG_B200_XFORM_KERNELS_CUH_

@@ -196,6 +196,38 @@ int himgcu_decode_batch_mixed(himgcu_ctx *ctx, const uint8_t *d_himg, const uint
                               int max_height, int num_channels, int flags,
                               const uint64_t *d_pixel_offsets, uint8_t *d_pixels_out, int32_t *d_status);
 
+/* ---- scaled decode: the image at 1/factor size, averaged inside the inverse transform -----------
+ * For factor f in {1, 2, 4, 8} and D = what himgcu_decode gives for the stream with the same flags
+ * ([H][W][num_channels]), the output is [ceil(H/f)][ceil(W/f)][num_channels], tightly packed, with
+ *     out[y][x][c] = (S + n/2) / n     (integer division)
+ * where S is the sum of D[yy][xx][c] over yy in [f*y, min(f*y + f, H)), xx in [f*x, min(f*x + f, W)) and n is the
+ * number of pixels of that window inside the image (edge windows are clipped).  The average is taken of the final
+ * pixels, after the clamp and the inverse colour map, without a full-size buffer.  Every FRES segment is still
+ * entropy-decoded, so statuses and accept/reject decisions are those of the unscaled call; f = 1 gives exactly the
+ * unscaled call's output.  Any other factor is HIMGCU_ERR_ARG.  The pixels of an image with a non-OK status are
+ * unspecified, but nothing is written outside its own output.
+ *
+ * Single image, host buffers (as himgcu_decode): width / height / num_channels receive the stream's FULL shape;
+ * out_cap is checked against the scaled size (HIMGCU_ERR_CAPACITY if smaller). */
+int himgcu_decode_scaled(himgcu_ctx *ctx, const uint8_t *himg, size_t size, int flags, int factor,
+                         uint8_t *out, size_t out_cap, int *width, int *height, int *num_channels);
+
+/* himgcu_decode_batch at 1/factor size: image i goes to d_pixels_out + i * ceil(w/f)*ceil(h/f)*num_channels.
+ * Arguments, statuses and host-side checks as himgcu_decode_batch, plus HIMGCU_ERR_ARG for a bad factor. */
+int himgcu_decode_batch_scaled(himgcu_ctx *ctx, const uint8_t *d_himg, const uint64_t *d_offsets,
+                               const uint32_t *d_sizes, int n, int width, int height, int num_channels,
+                               int flags, int factor, uint8_t *d_pixels_out, int32_t *d_status);
+
+/* himgcu_decode_batch_mixed at 1/factor size: image i is written as [ceil(h_i/f)][ceil(w_i/f)][num_channels] at
+ * d_pixels_out + d_pixel_offsets[i] (no alignment required).  Arguments, per-image statuses (HIMGCU_ERR_ARG for dims
+ * out of bounds, HIMGCU_REJECT for a FRMT shape other than the dims) and host-side checks as
+ * himgcu_decode_batch_mixed, plus HIMGCU_ERR_ARG for a bad factor.  A batch whose dims are all equal gives what
+ * himgcu_decode_batch_scaled gives.  The inverse transform is always the generic kernel. */
+int himgcu_decode_batch_mixed_scaled(himgcu_ctx *ctx, const uint8_t *d_himg, const uint64_t *d_offsets,
+                                     const uint32_t *d_sizes, int n, const int32_t *d_dims, int max_width,
+                                     int max_height, int num_channels, int flags, int factor,
+                                     const uint64_t *d_pixel_offsets, uint8_t *d_pixels_out, int32_t *d_status);
+
 /* ---- batch, HOST pointers (what a file/stream based caller uses; basis of the e2e figure) ----
  * Same work as the device batch calls with the transfers included: pixels (or bitstreams) are
  * copied host->device in sub-batches, coded, and the results copied back.  Pinned host memory

@@ -119,48 +119,37 @@ class Context:
                                            C.byref(n)))
         return out[: n.value].tobytes()
 
-    def decode(self, data: bytes, flags=STRICT):
-        """Returns the decoded [h][w][nch] array, or None where the reference decoder returns false."""
+    def _decode_single(self, data: bytes, shape, fn, *args):
+        """Body of decode, decode_scaled and decode_region: probes the header, allocates shape(w, h, nch) and calls the
+        C entry point fn with args after the stream.  None where the stream is rejected."""
         buf = np.frombuffer(data, np.uint8)
         w, h, n = C.c_int(), C.c_int(), C.c_int()
         if self.lib.himgcu_decode_info(_ptr(buf), buf.size, C.byref(w), C.byref(h), C.byref(n)) != _native.OK:
             return None
         if w.value < 1 or h.value < 1 or n.value < 1:
             return None
-        out = np.empty((h.value, w.value, n.value), np.uint8)
-        rc = self._check(self.lib.himgcu_decode(self.h, _ptr(buf), buf.size, flags, _ptr(out), out.size, C.byref(w),
-                                                C.byref(h), C.byref(n)), allow=(_native.REJECT,))
+        out = np.empty(shape(w.value, h.value, n.value), np.uint8)
+        rc = self._check(fn(self.h, _ptr(buf), buf.size, *args, _ptr(out), out.size, C.byref(w), C.byref(h), C.byref(n)),
+                         allow=(_native.REJECT,))
         return None if rc == _native.REJECT else out
+
+    def decode(self, data: bytes, flags=STRICT):
+        """Returns the decoded [h][w][nch] array, or None where the reference decoder returns false."""
+        return self._decode_single(data, lambda w, h, n: (h, w, n), self.lib.himgcu_decode, flags)
 
     def decode_scaled(self, data: bytes, factor: int, flags=STRICT):
         """The image at 1/factor size (factor 1, 2, 4 or 8): the [ceil(h/f)][ceil(w/f)][nch] array of rounded box
         averages of decode(data) over f x f windows (clipped at the right and bottom edges), or None where the stream
         is rejected.  Raises HimgError (ERR_ARG) for another factor."""
-        buf = np.frombuffer(data, np.uint8)
-        w, h, n = C.c_int(), C.c_int(), C.c_int()
-        if self.lib.himgcu_decode_info(_ptr(buf), buf.size, C.byref(w), C.byref(h), C.byref(n)) != _native.OK:
-            return None
-        if w.value < 1 or h.value < 1 or n.value < 1:
-            return None
         f = max(int(factor), 1)
-        out = np.empty((-(-h.value // f), -(-w.value // f), n.value), np.uint8)
-        rc = self._check(self.lib.himgcu_decode_scaled(self.h, _ptr(buf), buf.size, flags, factor, _ptr(out), out.size,
-                                                       C.byref(w), C.byref(h), C.byref(n)), allow=(_native.REJECT,))
-        return None if rc == _native.REJECT else out
+        return self._decode_single(data, lambda w, h, n: (-(-h // f), -(-w // f), n), self.lib.himgcu_decode_scaled, flags,
+                                   factor)
 
     def decode_region(self, data: bytes, x: int, y: int, w: int, h: int, flags=STRICT):
         """Rectangle [x, x+w) x [y, y+h) of the image: the [h][w][nch] array equal to decode(data)[y:y+h, x:x+w],
         or None where the stream is rejected.  Raises HimgError for an empty rectangle or one outside the image."""
-        buf = np.frombuffer(data, np.uint8)
-        W, H, n = C.c_int(), C.c_int(), C.c_int()
-        if self.lib.himgcu_decode_info(_ptr(buf), buf.size, C.byref(W), C.byref(H), C.byref(n)) != _native.OK:
-            return None
-        if n.value < 1:
-            return None
-        out = np.empty((max(h, 1), max(w, 1), n.value), np.uint8)
-        rc = self._check(self.lib.himgcu_decode_region(self.h, _ptr(buf), buf.size, flags, x, y, w, h, _ptr(out), out.size,
-                                                       C.byref(W), C.byref(H), C.byref(n)), allow=(_native.REJECT,))
-        return None if rc == _native.REJECT else out
+        return self._decode_single(data, lambda W, H, n: (max(h, 1), max(w, 1), n), self.lib.himgcu_decode_region, flags, x, y,
+                                   w, h)
 
     # ---- batch, device tensors --------------------------------------------------------------
     def encode_batch(self, pixels, quality=50, use_ycbcr=True, out=None, sizes=None):
@@ -180,19 +169,23 @@ class Context:
                                                  out.stride(0), _ptr(sizes)))
         return out, sizes
 
-    def decode_batch(self, himg, offsets, sizes, w, h, nch, flags=STRICT, out=None, status=None):
-        """himg: CUDA uint8 buffer; offsets int64 [n], sizes int32 [n] (device).  Returns (pixels, status)."""
+    def _decode_batch(self, fn, himg, offsets, sizes, w, h, nch, factor, out, status, *args):
+        """Body of decode_batch and decode_batch_scaled: fn is the C entry point, args its arguments after nch."""
         import torch
 
         n = offsets.numel()
         self._bind(himg, offsets, sizes, out, status)
         if out is None:
-            out = torch.empty((n, h, w, nch), dtype=torch.uint8, device=himg.device)
+            f = max(int(factor), 1)
+            out = torch.empty((n, -(-h // f), -(-w // f), nch), dtype=torch.uint8, device=himg.device)
         if status is None:
             status = torch.empty((n,), dtype=torch.int32, device=himg.device)
-        self._check(self.lib.himgcu_decode_batch(self.h, _ptr(himg), _ptr(offsets), _ptr(sizes), n, w, h, nch, flags,
-                                                 _ptr(out), _ptr(status)))
+        self._check(fn(self.h, _ptr(himg), _ptr(offsets), _ptr(sizes), n, w, h, nch, *args, _ptr(out), _ptr(status)))
         return out, status
+
+    def decode_batch(self, himg, offsets, sizes, w, h, nch, flags=STRICT, out=None, status=None):
+        """himg: CUDA uint8 buffer; offsets int64 [n], sizes int32 [n] (device).  Returns (pixels, status)."""
+        return self._decode_batch(self.lib.himgcu_decode_batch, himg, offsets, sizes, w, h, nch, 1, out, status, flags)
 
     def decode_batch_region(self, himg, offsets, sizes, w, h, nch, origins, crop_w, crop_h, flags=STRICT, out=None,
                             status=None):
@@ -235,14 +228,9 @@ class Context:
                                                               _ptr(status)))
         return out, status
 
-    def decode_batch_mixed(self, himg, offsets, sizes, dims, nch, max_w, max_h, flags=STRICT, out=None, pixel_offsets=None,
-                           status=None):
-        """decode_batch of streams with their own sizes: dims is a CUDA int32 [n][2] tensor of (w_i, h_i), each at most
-        max_w x max_h.  Image i is written as [h_i][w_i][nch] at byte pixel_offsets[i] (int64 [n]) of the flat uint8
-        buffer out.  When pixel_offsets is None they are the exclusive prefix sum of w_i * h_i * nch (0 for dims out of
-        bounds), computed on the device; when out is None it is allocated for the spans, which reads their total back
-        to the host (one synchronisation).  Returns (out, pixel_offsets, status); status[i] is REJECT where the stream is rejected or its
-        shape is not dims[i] x nch, and ERR_ARG where dims[i] is < 1 or exceeds the bounds (nothing of it is written)."""
+    def _decode_batch_mixed(self, fn, himg, offsets, sizes, dims, nch, max_w, max_h, factor, out, pixel_offsets, status, *args):
+        """Body of decode_batch_mixed (factor None) and decode_batch_mixed_scaled: fn is the C entry point, args its
+        arguments after nch."""
         import torch
 
         n = offsets.numel()
@@ -254,6 +242,9 @@ class Context:
         if pixel_offsets is None or out is None:  # (an image with dims out of bounds gets an empty span)
             wh = dims.reshape(n, 2).to(torch.int64)
             ok = (wh >= 1).all(dim=1) & (wh[:, 0] <= max_w) & (wh[:, 1] <= max_h)
+            if factor is not None:
+                f = max(int(factor), 1)
+                wh = torch.div(wh + (f - 1), f, rounding_mode="floor")
             spans = torch.where(ok, wh[:, 0] * wh[:, 1] * nch, 0)
         if pixel_offsets is None:
             pixel_offsets = torch.cumsum(spans, 0) - spans
@@ -262,25 +253,26 @@ class Context:
             out = torch.empty((max(total, 1),), dtype=torch.uint8, device=himg.device)
         if status is None:
             status = torch.empty((n,), dtype=torch.int32, device=himg.device)
-        self._check(self.lib.himgcu_decode_batch_mixed(self.h, _ptr(himg), _ptr(offsets), _ptr(sizes), n, _ptr(dims), max_w,
-                                                       max_h, nch, flags, _ptr(pixel_offsets), _ptr(out), _ptr(status)))
+        self._check(fn(self.h, _ptr(himg), _ptr(offsets), _ptr(sizes), n, _ptr(dims), max_w, max_h, nch, *args, _ptr(pixel_offsets),
+                       _ptr(out), _ptr(status)))
         return out, pixel_offsets, status
+
+    def decode_batch_mixed(self, himg, offsets, sizes, dims, nch, max_w, max_h, flags=STRICT, out=None, pixel_offsets=None,
+                           status=None):
+        """decode_batch of streams with their own sizes: dims is a CUDA int32 [n][2] tensor of (w_i, h_i), each at most
+        max_w x max_h.  Image i is written as [h_i][w_i][nch] at byte pixel_offsets[i] (int64 [n]) of the flat uint8
+        buffer out.  When pixel_offsets is None they are the exclusive prefix sum of w_i * h_i * nch (0 for dims out of
+        bounds), computed on the device; when out is None it is allocated for the spans, which reads their total back
+        to the host (one synchronisation).  Returns (out, pixel_offsets, status); status[i] is REJECT where the stream is rejected or its
+        shape is not dims[i] x nch, and ERR_ARG where dims[i] is < 1 or exceeds the bounds (nothing of it is written)."""
+        return self._decode_batch_mixed(self.lib.himgcu_decode_batch_mixed, himg, offsets, sizes, dims, nch, max_w, max_h, None, out,
+                                        pixel_offsets, status, flags)
 
     def decode_batch_scaled(self, himg, offsets, sizes, w, h, nch, factor, flags=STRICT, out=None, status=None):
         """decode_batch at 1/factor size (factor 1, 2, 4 or 8, see decode_scaled).  Returns (pixels
         [n][ceil(h/f)][ceil(w/f)][nch], status)."""
-        import torch
-
-        n = offsets.numel()
-        self._bind(himg, offsets, sizes, out, status)
-        if out is None:
-            f = max(int(factor), 1)
-            out = torch.empty((n, -(-h // f), -(-w // f), nch), dtype=torch.uint8, device=himg.device)
-        if status is None:
-            status = torch.empty((n,), dtype=torch.int32, device=himg.device)
-        self._check(self.lib.himgcu_decode_batch_scaled(self.h, _ptr(himg), _ptr(offsets), _ptr(sizes), n, w, h, nch, flags,
-                                                        factor, _ptr(out), _ptr(status)))
-        return out, status
+        return self._decode_batch(self.lib.himgcu_decode_batch_scaled, himg, offsets, sizes, w, h, nch, factor, out, status, flags,
+                                  factor)
 
     def decode_batch_mixed_scaled(self, himg, offsets, sizes, dims, nch, max_w, max_h, factor, flags=STRICT, out=None,
                                   pixel_offsets=None, status=None):
@@ -289,31 +281,8 @@ class Context:
         None they are the exclusive prefix sum of those spans (0 for dims out of bounds), computed on the device; when
         out is None it is allocated for the spans (one synchronisation).  Returns (out, pixel_offsets, status), with
         the statuses of decode_batch_mixed."""
-        import torch
-
-        n = offsets.numel()
-        if dims.dtype != torch.int32 or dims.numel() != 2 * n:
-            raise ValueError("dims must be an int32 tensor [n][2]")
-        if pixel_offsets is not None and (pixel_offsets.dtype != torch.int64 or pixel_offsets.numel() != n):
-            raise ValueError("pixel_offsets must be an int64 tensor [n]")
-        self._bind(himg, offsets, sizes, dims, out, pixel_offsets, status)
-        if pixel_offsets is None or out is None:  # (an image with dims out of bounds gets an empty span)
-            f = max(int(factor), 1)
-            wh = dims.reshape(n, 2).to(torch.int64)
-            ok = (wh >= 1).all(dim=1) & (wh[:, 0] <= max_w) & (wh[:, 1] <= max_h)
-            swh = torch.div(wh + (f - 1), f, rounding_mode="floor")
-            spans = torch.where(ok, swh[:, 0] * swh[:, 1] * nch, 0)
-        if pixel_offsets is None:
-            pixel_offsets = torch.cumsum(spans, 0) - spans
-        if out is None:
-            total = int(spans.sum()) if n else 0
-            out = torch.empty((max(total, 1),), dtype=torch.uint8, device=himg.device)
-        if status is None:
-            status = torch.empty((n,), dtype=torch.int32, device=himg.device)
-        self._check(self.lib.himgcu_decode_batch_mixed_scaled(self.h, _ptr(himg), _ptr(offsets), _ptr(sizes), n, _ptr(dims),
-                                                              max_w, max_h, nch, flags, factor, _ptr(pixel_offsets), _ptr(out),
-                                                              _ptr(status)))
-        return out, pixel_offsets, status
+        return self._decode_batch_mixed(self.lib.himgcu_decode_batch_mixed_scaled, himg, offsets, sizes, dims, nch, max_w, max_h,
+                                        factor, out, pixel_offsets, status, flags, factor)
 
     def encode_batch_mixed(self, pixels, offsets, dims, nch, max_w, max_h, quality=50, use_ycbcr=True, out=None, sizes=None):
         """encode_batch of images with their own sizes: pixels is a flat CUDA uint8 buffer holding image i as

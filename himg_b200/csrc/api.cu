@@ -12,6 +12,7 @@
 #include <mutex>
 #include <string>
 #include <thread>
+#include <type_traits>
 #include <vector>
 
 #include "../../include/himg_cuda.h"
@@ -313,25 +314,31 @@ QuantParams make_quant(const EncodeTables &t) {
 }
 
 // ---- stage launchers (device pointers, asynchronous) -------------------------------------------
+//
+// The stage functions are instantiated for uniform batches (MIXED = false) and for batches of mixed geometry
+// (MIXED = true, see MixedDims): g is then the bounding geometry, which sizes the scratch, `md` holds the images' own
+// sizes, and image i's pixels start at d_pixels + px_off[i].  Uniform calls leave md and px_off at the kernels' own
+// defaults.  A mixed batch always takes the generic kernels.
 
-// cbase / ctotal: the channel group [cbase, cbase + NCH) of an image with ctotal channels (see k_lowres_avg);
-// d_pixels points at the group's first channel.  With `md` the batch has mixed geometry (g is the bounding one) and
-// image i starts at d_pixels + px_off[i].
-template <int NCH>
-int launch_avg(himgcu_ctx *ctx, const uint8_t *d_pixels, int n, const Geom &g, bool ycbcr, uint8_t *d_avg, int cbase = 0,
-               int ctotal = NCH, const MixedDims *md = nullptr, const unsigned long long *px_off = nullptr) {
-  dim3 grid((g.cols + kTile - 1) / kTile, g.rows, n);
-  if (md) {
-    if (ycbcr) LAUNCH("k_lowres_avg", (k_lowres_avg<NCH, true, true>), grid, kTile, 0, d_pixels, g, d_avg, cbase, ctotal, *md, px_off);
-    else LAUNCH("k_lowres_avg", (k_lowres_avg<NCH, false, true>), grid, kTile, 0, d_pixels, g, d_avg, cbase, ctotal, *md, px_off);
-    return HIMGCU_OK;
+template <int N>
+using Nch = std::integral_constant<int, N>;
+
+// Calls launch(Nch<NCH>(), cbase, ctotal, ycbcr) for every channel group [cbase, cbase + NCH) of an nch-channel image:
+// up to four channels are one group, more are the first three and then one group per further channel.  Only the group
+// at channel 0 carries the colour map.
+template <class F>
+int for_channel_groups(int nch, bool ycbcr, F &&launch) {
+  switch (nch) {
+    case 1: return launch(Nch<1>(), 0, 1, false);
+    case 2: return launch(Nch<2>(), 0, 2, false);
+    case 3: return launch(Nch<3>(), 0, 3, ycbcr);
+    case 4: return launch(Nch<4>(), 0, 4, ycbcr);
+    default: break;
   }
-  if (ycbcr) LAUNCH("k_lowres_avg", (k_lowres_avg<NCH, true>), grid, kTile, 0, d_pixels, g, d_avg, cbase, ctotal);
-  else LAUNCH("k_lowres_avg", (k_lowres_avg<NCH, false>), grid, kTile, 0, d_pixels, g, d_avg, cbase, ctotal);
-  return HIMGCU_OK;
+  int rc = launch(Nch<3>(), 0, nch, ycbcr);
+  for (int c = 3; c < nch && !rc; ++c) rc = launch(Nch<1>(), c, nch, false);
+  return rc;
 }
-
-void make_colour(int nch, bool ycbcr, ColourW *cw);
 
 template <int NCH>
 int launch_avg2(himgcu_ctx *ctx, const uint8_t *d_pixels, int n, const Geom &g, bool ycbcr, uint8_t *d_avg) {
@@ -342,15 +349,15 @@ int launch_avg2(himgcu_ctx *ctx, const uint8_t *d_pixels, int n, const Geom &g, 
   return HIMGCU_OK;
 }
 
-// With `md` the batch has mixed geometry (see launch_avg) and takes the generic kernels.
+template <bool MIXED = false>
 int stage_lowres(himgcu_ctx *ctx, const uint8_t *d_pixels, int n, const Geom &g, bool ycbcr, uint8_t *d_L,
-                 const MixedDims *md = nullptr, const unsigned long long *px_off = nullptr) {
+                 const MixedDims &md = {}, const unsigned long long *px_off = nullptr) {
   uint8_t *d_avg;
   const size_t nlow = (size_t)n * g.nch * g.rows * g.cols;
   ENSURE("avg", nlow, d_avg);
   int rc;
   // lane-pair fast path: whole 16-pixel block pairs, tightly packed pixels, 16-byte aligned rows
-  const bool fast = !md && !ctx->force_generic && !(ctx->xform_variant & 1) && g.pstride == g.nch && (g.w % 16) == 0 &&
+  const bool fast = !MIXED && !ctx->force_generic && !(ctx->xform_variant & 1) && g.pstride == g.nch && (g.w % 16) == 0 &&
                     (reinterpret_cast<uintptr_t>(d_pixels) & 15) == 0 && (g.img_bytes & 15) == 0 &&
                     (reinterpret_cast<uintptr_t>(d_avg) & 1) == 0 && (g.nch == 1 || g.nch == 3 || g.nch == 4);
   if (fast) {
@@ -359,22 +366,24 @@ int stage_lowres(himgcu_ctx *ctx, const uint8_t *d_pixels, int n, const Geom &g,
       case 3: rc = launch_avg2<3>(ctx, d_pixels, n, g, ycbcr, d_avg); break;
       default: rc = launch_avg2<4>(ctx, d_pixels, n, g, ycbcr, d_avg); break;
     }
-  } else
-  switch (g.nch) {
-    case 1: rc = launch_avg<1>(ctx, d_pixels, n, g, false, d_avg, 0, 1, md, px_off); break;
-    case 2: rc = launch_avg<2>(ctx, d_pixels, n, g, false, d_avg, 0, 2, md, px_off); break;
-    case 3: rc = launch_avg<3>(ctx, d_pixels, n, g, ycbcr, d_avg, 0, 3, md, px_off); break;
-    case 4: rc = launch_avg<4>(ctx, d_pixels, n, g, ycbcr, d_avg, 0, 4, md, px_off); break;
-    default:  // more than four channels: the first three, then one launch per further channel
-      rc = launch_avg<3>(ctx, d_pixels, n, g, ycbcr, d_avg, 0, g.nch, md, px_off);
-      for (int c = 3; c < g.nch && !rc; ++c) rc = launch_avg<1>(ctx, d_pixels + c, n, g, false, d_avg, c, g.nch, md, px_off);
-      break;
+  } else {
+    // cbase / ctotal: the channel group [cbase, cbase + NCH) of an image with ctotal channels (see k_lowres_avg)
+    rc = for_channel_groups(g.nch, ycbcr, [&](auto nc, int cbase, int ctotal, bool yc) -> int {
+      constexpr int NCH = decltype(nc)::value;
+      const dim3 grid((g.cols + kTile - 1) / kTile, g.rows, n);
+      if (yc)
+        LAUNCH("k_lowres_avg", (k_lowres_avg<NCH, true, MIXED>), grid, kTile, 0, d_pixels + cbase, g, d_avg, cbase, ctotal, md,
+               px_off);
+      else
+        LAUNCH("k_lowres_avg", (k_lowres_avg<NCH, false, MIXED>), grid, kTile, 0, d_pixels + cbase, g, d_avg, cbase, ctotal, md,
+               px_off);
+      return HIMGCU_OK;
+    });
   }
   if (rc) return rc;
   const int threads = std::min(256, (g.cols + 31) & ~31);
   const dim3 grid((unsigned)(n * g.nch), (g.rows + kCompRows - 1) / kCompRows);
-  if (md) LAUNCH("k_lowres_comp", k_lowres_comp<true>, grid, threads, 0, d_avg, n * g.nch, g.rows, g.cols, d_L, *md);
-  else LAUNCH("k_lowres_comp", k_lowres_comp<false>, grid, threads, 0, d_avg, n * g.nch, g.rows, g.cols, d_L);
+  LAUNCH("k_lowres_comp", k_lowres_comp<MIXED>, grid, threads, 0, d_avg, n * g.nch, g.rows, g.cols, d_L, md);
   return HIMGCU_OK;
 }
 
@@ -401,38 +410,16 @@ int upload_lowres_tables(himgcu_ctx *ctx, const EncodeTables *enc, const int16_t
   return HIMGCU_OK;
 }
 
+template <bool MIXED = false>
 int stage_lres_encode(himgcu_ctx *ctx, const uint8_t *d_L, int n, const Geom &g, const EncodeTables &t, uint8_t *d_lres,
-                      const MixedDims *md = nullptr) {
+                      const MixedDims &md = {}) {
   LowResTables *d_tabs;
   int rc = upload_lowres_tables(ctx, &t, nullptr, &d_tabs);
   if (rc) return rc;
   const long long nmb = (long long)n * g.nch * g.mrows * g.mcols;
   const unsigned blocks = (unsigned)((nmb + kLresWarps * 2 - 1) / (kLresWarps * 2));
-  if (md) {
-    LAUNCH("k_lres_dpcm_enc", (k_lres_dpcm<true, true>), blocks, kLresWarps * 32, 0, d_L, d_lres, (uint8_t *)nullptr, g, n,
-           d_tabs->map_lut, d_tabs->unmap, (unsigned long long)0, *md);
-    return HIMGCU_OK;
-  }
-  LAUNCH("k_lres_dpcm_enc", (k_lres_dpcm<true>), blocks, kLresWarps * 32, 0, d_L, d_lres, (uint8_t *)nullptr, g, n,
-         d_tabs->map_lut, d_tabs->unmap, (unsigned long long)0);
-  return HIMGCU_OK;
-}
-
-template <int NCH>
-int launch_fwd(himgcu_ctx *ctx, const uint8_t *d_pixels, const uint8_t *d_L, int n, const Geom &g, bool ycbcr,
-               const QuantParams &qp, uint8_t *d_planes, int cbase = 0, int ctotal = NCH, const MixedDims *md = nullptr,
-               const unsigned long long *px_off = nullptr) {
-  dim3 grid((g.cols + kTile - 1) / kTile, g.rows, n);
-  const uint8_t *lut = (const uint8_t *)ctx->full_lut.p;
-  if (md) {
-    if (ycbcr)
-      LAUNCH("k_forward", (k_forward<NCH, true, true>), grid, kTile, 0, d_pixels, d_L, g, qp, lut, d_planes, cbase, ctotal, *md, px_off);
-    else
-      LAUNCH("k_forward", (k_forward<NCH, false, true>), grid, kTile, 0, d_pixels, d_L, g, qp, lut, d_planes, cbase, ctotal, *md, px_off);
-    return HIMGCU_OK;
-  }
-  if (ycbcr) LAUNCH("k_forward", (k_forward<NCH, true>), grid, kTile, 0, d_pixels, d_L, g, qp, lut, d_planes, cbase, ctotal);
-  else LAUNCH("k_forward", (k_forward<NCH, false>), grid, kTile, 0, d_pixels, d_L, g, qp, lut, d_planes, cbase, ctotal);
+  LAUNCH("k_lres_dpcm_enc", (k_lres_dpcm<true, MIXED>), blocks, kLresWarps * 32, 0, d_L, d_lres, (uint8_t *)nullptr, g, n,
+         d_tabs->map_lut, d_tabs->unmap, (unsigned long long)0, md);
   return HIMGCU_OK;
 }
 
@@ -459,12 +446,12 @@ int launch_fwd3(himgcu_ctx *ctx, const uint8_t *d_pixels, const uint8_t *d_L, in
   return HIMGCU_OK;
 }
 
-// With `md` the batch has mixed geometry (see launch_avg) and takes the generic kernels.
+template <bool MIXED = false>
 int stage_forward(himgcu_ctx *ctx, const uint8_t *d_pixels, const uint8_t *d_L, int n, const Geom &g,
-                  const EncodeTables &t, uint8_t *d_planes, const MixedDims *md = nullptr,
+                  const EncodeTables &t, uint8_t *d_planes, const MixedDims &md = {},
                   const unsigned long long *px_off = nullptr) {
   // fast path: whole 16-pixel-wide block pairs, tightly packed pixels, 16-byte aligned rows
-  if (!md && !ctx->force_generic && !(ctx->xform_variant & 1) && g.pstride == g.nch && (g.w % 16) == 0 && (g.h % 8) == 0 &&
+  if (!MIXED && !ctx->force_generic && !(ctx->xform_variant & 1) && g.pstride == g.nch && (g.w % 16) == 0 && (g.h % 8) == 0 &&
       (reinterpret_cast<uintptr_t>(d_pixels) & 15) == 0 && (reinterpret_cast<uintptr_t>(d_L) & 1) == 0 &&
       (g.nch == 1 || g.nch == 3 || g.nch == 4)) {
     Fwd3Params P;
@@ -486,32 +473,18 @@ int stage_forward(himgcu_ctx *ctx, const uint8_t *d_pixels, const uint8_t *d_L, 
   int rc = upload_full_lut(ctx);
   if (rc) return rc;
   const QuantParams qp = make_quant(t);
-  switch (g.nch) {
-    case 1: return launch_fwd<1>(ctx, d_pixels, d_L, n, g, false, qp, d_planes, 0, 1, md, px_off);
-    case 2: return launch_fwd<2>(ctx, d_pixels, d_L, n, g, false, qp, d_planes, 0, 2, md, px_off);
-    case 3: return launch_fwd<3>(ctx, d_pixels, d_L, n, g, t.ycbcr, qp, d_planes, 0, 3, md, px_off);
-    case 4: return launch_fwd<4>(ctx, d_pixels, d_L, n, g, t.ycbcr, qp, d_planes, 0, 4, md, px_off);
-    default: break;
-  }
-  rc = launch_fwd<3>(ctx, d_pixels, d_L, n, g, t.ycbcr, qp, d_planes, 0, g.nch, md, px_off);
-  for (int c = 3; c < g.nch && !rc; ++c)
-    rc = launch_fwd<1>(ctx, d_pixels + c, d_L, n, g, false, qp, d_planes, c, g.nch, md, px_off);
-  return rc;
-}
-
-// With `md` the batch has mixed geometry (g is the bounding one) and image i is written at d_pixels + px_off[i].
-template <int NCH>
-int launch_inv(himgcu_ctx *ctx, const uint8_t *d_planes, const uint8_t *d_R, int n, const Geom &g,
-               const DecTables *d_tabs, unsigned long long tab_stride, uint8_t *d_pixels, int cbase = 0, int ctotal = NCH,
-               const MixedDims *md = nullptr, const unsigned long long *px_off = nullptr) {
-  dim3 grid((g.cols + kTile - 1) / kTile, g.rows, n);
-  if (md) {
-    LAUNCH("k_inverse", (k_inverse<NCH, true>), grid, kTile, 0, d_planes, d_R, g, d_tabs, tab_stride, d_pixels, cbase, ctotal,
-           *md, px_off);
+  const uint8_t *lut = (const uint8_t *)ctx->full_lut.p;
+  return for_channel_groups(g.nch, t.ycbcr, [&](auto nc, int cbase, int ctotal, bool yc) -> int {
+    constexpr int NCH = decltype(nc)::value;
+    const dim3 grid((g.cols + kTile - 1) / kTile, g.rows, n);
+    if (yc)
+      LAUNCH("k_forward", (k_forward<NCH, true, MIXED>), grid, kTile, 0, d_pixels + cbase, d_L, g, qp, lut, d_planes, cbase, ctotal,
+             md, px_off);
+    else
+      LAUNCH("k_forward", (k_forward<NCH, false, MIXED>), grid, kTile, 0, d_pixels + cbase, d_L, g, qp, lut, d_planes, cbase,
+             ctotal, md, px_off);
     return HIMGCU_OK;
-  }
-  LAUNCH("k_inverse", (k_inverse<NCH>), grid, kTile, 0, d_planes, d_R, g, d_tabs, tab_stride, d_pixels, cbase, ctotal);
-  return HIMGCU_OK;
+  });
 }
 
 template <int NCH>
@@ -528,102 +501,67 @@ int launch_inv2(himgcu_ctx *ctx, const uint8_t *d_planes, const uint8_t *d_R, in
   return HIMGCU_OK;
 }
 
-template <int NCH>
+// Dequantisation tables of the lane-pair kernels: one set per image of d_tabs (tab_stride apart), ntab of them.
+int launch_inv_tables(himgcu_ctx *ctx, const DecTables *d_tabs, int ntab, unsigned long long tab_stride, InvTables **d_inv) {
+  InvTables *d;
+  ENSURE("inv_tables", (size_t)ntab * sizeof(InvTables), d);
+  LAUNCH("k_inv_tables", k_inv_tables, ntab, 256, 0, d_tabs, tab_stride, d);
+  *d_inv = d;
+  return HIMGCU_OK;
+}
+
+// Lane-pair inverse: k_inverse4, or at LF > 0 k_inverse4_scaled (a decode scaled by 2^LF, same shapes and tiles).
+template <int NCH, int LF>
 int launch_inv4(himgcu_ctx *ctx, const uint8_t *d_planes, const uint8_t *d_R, int n, const Geom &g,
                 const DecTables *d_tabs, unsigned long long tab_stride, uint8_t *d_pixels) {
   // per-image dequantisation tables first (the tables travel in-band); one set when the caller has one
-  const int ntab = tab_stride ? n : 1;
   InvTables *d_inv;
-  ENSURE("inv_tables", (size_t)ntab * sizeof(InvTables), d_inv);
-  LAUNCH("k_inv_tables", k_inv_tables, ntab, 256, 0, d_tabs, tab_stride, d_inv);
+  int rc = launch_inv_tables(ctx, d_tabs, tab_stride ? n : 1, tab_stride, &d_inv);
+  if (rc) return rc;
   const unsigned long long inv_stride = tab_stride ? sizeof(InvTables) : 0;
   const int total_pairs = g.rows * (g.cols / 2);
   constexpr int TP = NCH == 1 ? kInv4ThreadsGray : kInv4ThreadsRgb;
   dim3 grid((total_pairs + TP - 1) / TP, 1, n);
   const int smem = NCH * 64 * 2 * TP + kInvTableBytes;
-  CK(cudaFuncSetAttribute((k_inverse4<NCH, TP>), cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
-  LAUNCH("k_inverse", (k_inverse4<NCH, TP>), grid, TP, smem, d_planes, d_R, g, d_inv, inv_stride, d_pixels, 1u);
-  return HIMGCU_OK;
-}
-
-// Scaled decode by 2^lf (lf in 1..3), generic kernel: any shape, channel group [cbase, cbase + NCH) of ctotal channels.
-template <int NCH>
-int launch_inv_scaled(himgcu_ctx *ctx, const uint8_t *d_planes, const uint8_t *d_R, int n, const Geom &g,
-                      const DecTables *d_tabs, unsigned long long tab_stride, uint8_t *d_pixels, int cbase, int ctotal, int lf,
-                      const MixedDims *md, const unsigned long long *px_off) {
-  dim3 grid((g.cols + kTile - 1) / kTile, g.rows, n);
-  if (md) {
-    LAUNCH("k_inverse_scaled", (k_inverse_scaled<NCH, true>), grid, kTile, 0, d_planes, d_R, g, d_tabs, tab_stride, d_pixels, cbase,
-           ctotal, lf, *md, px_off);
-    return HIMGCU_OK;
+  if constexpr (LF == 0) {
+    CK(cudaFuncSetAttribute((k_inverse4<NCH, TP>), cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
+    LAUNCH("k_inverse", (k_inverse4<NCH, TP>), grid, TP, smem, d_planes, d_R, g, d_inv, inv_stride, d_pixels, 1u);
+  } else {
+    CK(cudaFuncSetAttribute((k_inverse4_scaled<NCH, TP, LF>), cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
+    LAUNCH("k_inverse4_scaled", (k_inverse4_scaled<NCH, TP, LF>), grid, TP, smem, d_planes, d_R, g, d_inv, inv_stride, d_pixels,
+           1u);
   }
-  LAUNCH("k_inverse_scaled", (k_inverse_scaled<NCH>), grid, kTile, 0, d_planes, d_R, g, d_tabs, tab_stride, d_pixels, cbase, ctotal, lf);
   return HIMGCU_OK;
 }
 
-// Scaled decode by 2^LF, lane-pair kernel: the shapes and tiles of launch_inv4.
-template <int NCH, int LF>
-int launch_inv4_scaled(himgcu_ctx *ctx, const uint8_t *d_planes, const uint8_t *d_R, int n, const Geom &g,
-                       const DecTables *d_tabs, unsigned long long tab_stride, uint8_t *d_pixels) {
-  const int ntab = tab_stride ? n : 1;
-  InvTables *d_inv;
-  ENSURE("inv_tables", (size_t)ntab * sizeof(InvTables), d_inv);
-  LAUNCH("k_inv_tables", k_inv_tables, ntab, 256, 0, d_tabs, tab_stride, d_inv);
-  const unsigned long long inv_stride = tab_stride ? sizeof(InvTables) : 0;
-  const int total_pairs = g.rows * (g.cols / 2);
-  constexpr int TP = NCH == 1 ? kInv4ThreadsGray : kInv4ThreadsRgb;
-  dim3 grid((total_pairs + TP - 1) / TP, 1, n);
-  const int smem = NCH * 64 * 2 * TP + kInvTableBytes;
-  CK(cudaFuncSetAttribute((k_inverse4_scaled<NCH, TP, LF>), cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
-  LAUNCH("k_inverse4_scaled", (k_inverse4_scaled<NCH, TP, LF>), grid, TP, smem, d_planes, d_R, g, d_inv, inv_stride, d_pixels, 1u);
-  return HIMGCU_OK;
+// The shapes the lane-pair kernels of a whole-image decode take, for pixel stores store_bytes wide.
+bool lane_pair_ok(const himgcu_ctx *ctx, const Geom &g, const uint8_t *d_planes, const uint8_t *d_R, const uint8_t *d_pixels,
+                  unsigned store_bytes) {
+  return !ctx->force_generic && !(ctx->xform_variant & 1) && (g.h % 8) == 0 && (g.cols % 16) == 0 && (g.w % 16) == 0 &&
+         (g.nch == 1 || g.nch == 3) && (reinterpret_cast<uintptr_t>(d_planes) & 15) == 0 &&
+         (reinterpret_cast<uintptr_t>(d_pixels) & (store_bytes - 1)) == 0 && (reinterpret_cast<uintptr_t>(d_R) & 1) == 0;
 }
 
-// K-inv of a decode scaled by 2^lf (lf in 1..3): image i is [ceil(h / 2^lf)][ceil(w / 2^lf)][nch], at d_pixels plus i times
-// that size, or with `md` at d_pixels + px_off[i] (see launch_inv).
-int stage_inverse_scaled(himgcu_ctx *ctx, const uint8_t *d_planes, const uint8_t *d_R, int n, const Geom &g,
-                         const DecTables *d_tabs, unsigned long long tab_stride, uint8_t *d_pixels, int lf,
-                         const MixedDims *md, const unsigned long long *px_off) {
-  // lane-pair path: the shapes k_inverse4 takes (every window is whole); its stores are 16 >> lf bytes wide
-  if (!md && !ctx->force_generic && !(ctx->xform_variant & 1) && (g.h % 8) == 0 && (g.cols % 16) == 0 && (g.w % 16) == 0 &&
-      (g.nch == 1 || g.nch == 3) && (reinterpret_cast<uintptr_t>(d_planes) & 15) == 0 &&
-      (reinterpret_cast<uintptr_t>(d_pixels) & ((16u >> lf) - 1)) == 0 && (reinterpret_cast<uintptr_t>(d_R) & 1) == 0) {
+// K-inv of a whole-image decode.  lf > 0 (1..3): the decode is scaled by 2^lf, and image i is
+// [ceil(h / 2^lf)][ceil(w / 2^lf)][nch] at d_pixels plus i times that size (or at d_pixels + px_off[i] when MIXED).
+template <bool MIXED = false>
+int stage_inverse(himgcu_ctx *ctx, const uint8_t *d_planes, const uint8_t *d_R, int n, const Geom &g,
+                  const DecTables *d_tabs, unsigned long long tab_stride, uint8_t *d_pixels, int lf = 0,
+                  const MixedDims &md = {}, const unsigned long long *px_off = nullptr) {
+  // lane-pair fast path: two blocks per thread, flat tiles, pixel stores 16 >> lf bytes wide
+  if (!MIXED && lane_pair_ok(ctx, g, d_planes, d_R, d_pixels, 16u >> lf)) {
     switch (g.nch * 4 + lf) {
-      case 1 * 4 + 1: return launch_inv4_scaled<1, 1>(ctx, d_planes, d_R, n, g, d_tabs, tab_stride, d_pixels);
-      case 1 * 4 + 2: return launch_inv4_scaled<1, 2>(ctx, d_planes, d_R, n, g, d_tabs, tab_stride, d_pixels);
-      case 1 * 4 + 3: return launch_inv4_scaled<1, 3>(ctx, d_planes, d_R, n, g, d_tabs, tab_stride, d_pixels);
-      case 3 * 4 + 1: return launch_inv4_scaled<3, 1>(ctx, d_planes, d_R, n, g, d_tabs, tab_stride, d_pixels);
-      case 3 * 4 + 2: return launch_inv4_scaled<3, 2>(ctx, d_planes, d_R, n, g, d_tabs, tab_stride, d_pixels);
-      default: return launch_inv4_scaled<3, 3>(ctx, d_planes, d_R, n, g, d_tabs, tab_stride, d_pixels);
+      case 1 * 4 + 0: return launch_inv4<1, 0>(ctx, d_planes, d_R, n, g, d_tabs, tab_stride, d_pixels);
+      case 1 * 4 + 1: return launch_inv4<1, 1>(ctx, d_planes, d_R, n, g, d_tabs, tab_stride, d_pixels);
+      case 1 * 4 + 2: return launch_inv4<1, 2>(ctx, d_planes, d_R, n, g, d_tabs, tab_stride, d_pixels);
+      case 1 * 4 + 3: return launch_inv4<1, 3>(ctx, d_planes, d_R, n, g, d_tabs, tab_stride, d_pixels);
+      case 3 * 4 + 0: return launch_inv4<3, 0>(ctx, d_planes, d_R, n, g, d_tabs, tab_stride, d_pixels);
+      case 3 * 4 + 1: return launch_inv4<3, 1>(ctx, d_planes, d_R, n, g, d_tabs, tab_stride, d_pixels);
+      case 3 * 4 + 2: return launch_inv4<3, 2>(ctx, d_planes, d_R, n, g, d_tabs, tab_stride, d_pixels);
+      default: return launch_inv4<3, 3>(ctx, d_planes, d_R, n, g, d_tabs, tab_stride, d_pixels);
     }
   }
-  switch (g.nch) {
-    case 1: return launch_inv_scaled<1>(ctx, d_planes, d_R, n, g, d_tabs, tab_stride, d_pixels, 0, 1, lf, md, px_off);
-    case 2: return launch_inv_scaled<2>(ctx, d_planes, d_R, n, g, d_tabs, tab_stride, d_pixels, 0, 2, lf, md, px_off);
-    case 3: return launch_inv_scaled<3>(ctx, d_planes, d_R, n, g, d_tabs, tab_stride, d_pixels, 0, 3, lf, md, px_off);
-    case 4: return launch_inv_scaled<4>(ctx, d_planes, d_R, n, g, d_tabs, tab_stride, d_pixels, 0, 4, lf, md, px_off);
-    default: break;
-  }
-  int rc = launch_inv_scaled<3>(ctx, d_planes, d_R, n, g, d_tabs, tab_stride, d_pixels, 0, g.nch, lf, md, px_off);
-  for (int c = 3; c < g.nch && !rc; ++c)
-    rc = launch_inv_scaled<1>(ctx, d_planes, d_R, n, g, d_tabs, tab_stride, d_pixels, c, g.nch, lf, md, px_off);
-  return rc;
-}
-
-// With `md` the batch has mixed geometry (see launch_inv) and takes the generic kernel.  lf > 0: the decode is scaled by
-// 2^lf (stage_inverse_scaled).
-int stage_inverse(himgcu_ctx *ctx, const uint8_t *d_planes, const uint8_t *d_R, int n, const Geom &g,
-                  const DecTables *d_tabs, unsigned long long tab_stride, uint8_t *d_pixels, const MixedDims *md = nullptr,
-                  const unsigned long long *px_off = nullptr, int lf = 0) {
-  if (lf) return stage_inverse_scaled(ctx, d_planes, d_R, n, g, d_tabs, tab_stride, d_pixels, lf, md, px_off);
-  // lane-pair fast path: two blocks per thread, flat tiles, 16-byte pixel stores
-  if (!md && !ctx->force_generic && !(ctx->xform_variant & 1) && (g.h % 8) == 0 && (g.cols % 16) == 0 && (g.w % 16) == 0 &&
-      (g.nch == 1 || g.nch == 3) && (reinterpret_cast<uintptr_t>(d_planes) & 15) == 0 &&
-      (reinterpret_cast<uintptr_t>(d_pixels) & 15) == 0 && (reinterpret_cast<uintptr_t>(d_R) & 1) == 0) {
-    if (g.nch == 1) return launch_inv4<1>(ctx, d_planes, d_R, n, g, d_tabs, tab_stride, d_pixels);
-    return launch_inv4<3>(ctx, d_planes, d_R, n, g, d_tabs, tab_stride, d_pixels);
-  }
-  if (!md && !ctx->force_generic && (g.w % 8) == 0 && (g.h % 8) == 0 && (g.cols % 16) == 0 &&
+  if (!MIXED && !lf && !ctx->force_generic && (g.w % 8) == 0 && (g.h % 8) == 0 && (g.cols % 16) == 0 &&
       (reinterpret_cast<uintptr_t>(d_planes) & 15) == 0 && (reinterpret_cast<uintptr_t>(d_pixels) & 7) == 0 &&
       (((size_t)g.w * g.nch) & 7) == 0) {
     switch (g.nch) {
@@ -633,17 +571,17 @@ int stage_inverse(himgcu_ctx *ctx, const uint8_t *d_planes, const uint8_t *d_R, 
       default: break;
     }
   }
-  switch (g.nch) {
-    case 1: return launch_inv<1>(ctx, d_planes, d_R, n, g, d_tabs, tab_stride, d_pixels, 0, 1, md, px_off);
-    case 2: return launch_inv<2>(ctx, d_planes, d_R, n, g, d_tabs, tab_stride, d_pixels, 0, 2, md, px_off);
-    case 3: return launch_inv<3>(ctx, d_planes, d_R, n, g, d_tabs, tab_stride, d_pixels, 0, 3, md, px_off);
-    case 4: return launch_inv<4>(ctx, d_planes, d_R, n, g, d_tabs, tab_stride, d_pixels, 0, 4, md, px_off);
-    default: break;
-  }
-  int rc = launch_inv<3>(ctx, d_planes, d_R, n, g, d_tabs, tab_stride, d_pixels, 0, g.nch, md, px_off);
-  for (int c = 3; c < g.nch && !rc; ++c)
-    rc = launch_inv<1>(ctx, d_planes, d_R, n, g, d_tabs, tab_stride, d_pixels, c, g.nch, md, px_off);
-  return rc;
+  return for_channel_groups(g.nch, false, [&](auto nc, int cbase, int ctotal, bool) -> int {
+    constexpr int NCH = decltype(nc)::value;
+    const dim3 grid((g.cols + kTile - 1) / kTile, g.rows, n);
+    if (lf)
+      LAUNCH("k_inverse_scaled", (k_inverse_scaled<NCH, MIXED>), grid, kTile, 0, d_planes, d_R, g, d_tabs, tab_stride, d_pixels,
+             cbase, ctotal, lf, md, px_off);
+    else
+      LAUNCH("k_inverse", (k_inverse<NCH, MIXED>), grid, kTile, 0, d_planes, d_R, g, d_tabs, tab_stride, d_pixels, cbase, ctotal,
+             md, px_off);
+    return HIMGCU_OK;
+  });
 }
 
 // One Huffman chunk per item, or (image mode) LRES + FRES with the container around them.
@@ -655,12 +593,13 @@ struct HuffChunkArgs {
   int size_patch;
 };
 
-// With `md` the items are the images of a mixed-geometry batch (chunk 0 LRES, chunk 1 FRES, each HuffGeom the
+// With MIXED the items are the images of a mixed-geometry batch (chunk 0 LRES, chunk 1 FRES, each HuffGeom the
 // bounding one; see MixedHuff).  Their chunks have no parts, and force_generic does not apply: the first-generation
 // coder has no mixed variant.
+template <bool MIXED = false>
 int huff_encode_items(himgcu_ctx *ctx, int n, HuffChunkArgs *chunks, int nchunks, bool riff, uint8_t *d_out,
-                      size_t out_stride, uint32_t *d_sizes, const MixedDims *md = nullptr) {
-  const bool generic = ctx->force_generic && !md;
+                      size_t out_stride, uint32_t *d_sizes, const MixedDims &md = {}) {
+  const bool generic = ctx->force_generic && !MIXED;
   // Device error flag of the encoder (5: code longer than 32 bits, 4: output does not fit, 99: internal
   // mismatch, kEncErrDims: dims out of bounds in a mixed batch).  Sticky per context: cleared when it is read (take_enc_err), not per call, so that an
   // error in an earlier sub-batch of an asynchronous call is not lost.
@@ -699,8 +638,10 @@ int huff_encode_items(himgcu_ctx *ctx, int n, HuffChunkArgs *chunks, int nchunks
   memset(&TP, 0, sizeof(TP));
   ItemLists lists[2];
   bool teams[2] = {false, false};
+  MixedHuff mh[2] = {};  // (the uniform kernels take the default)
   for (int k = 0; k < nchunks; ++k) {
     HuffGeom &hg = chunks[k].hg;
+    if (MIXED) mh[k] = MixedHuff{md, k};
     // Parts per segment: only worth it when the segments alone cannot fill the GPU (the low-res chunk
     // of an image is ONE unframed segment: one CTA per image otherwise).  Parts of >= 8 KiB.
     hg.nsub = 1;
@@ -709,7 +650,7 @@ int huff_encode_items(himgcu_ctx *ctx, int n, HuffChunkArgs *chunks, int nchunks
     // CTA per block row and only get parts when even those are few (measured: more parts cost more
     // in the layout and look-back steps than they gain)
     const long long ctas = (long long)n * hg.nseg, fill = hg.nseg == 1 ? 148 * 8 : 148 * 2;
-    if (!generic && !md && ctas < fill && hg.seg_size > 2 * kTokPiece) {
+    if (!generic && !MIXED && ctas < fill && hg.seg_size > 2 * kTokPiece) {
       const int want = (int)std::min<long long>(64, (fill + ctas - 1) / ctas);
       const int sub = (int)((((long long)hg.seg_size + want - 1) / want + kTokPiece - 1) / kTokPiece) * kTokPiece;
       hg.sub_size = sub;
@@ -746,15 +687,10 @@ int huff_encode_items(himgcu_ctx *ctx, int n, HuffChunkArgs *chunks, int nchunks
       CK(cudaMemsetAsync(d_total, 0, (size_t)n * kSyms * sizeof(uint32_t), ctx->stream));
     }
     const dim3 team_grid((hg.nseg + kTeamWarps - 1) / kTeamWarps, n);
-    if (md) {
-      const MixedHuff mh{*md, k};
-      if (teams[k])
-        LAUNCH("k_huff_hist", k_huff_hist4<true>, team_grid, kTeamThreads, 0, chunks[k].d_in, hg, d_seghist[k], il, d_total, mh);
-      else LAUNCH("k_huff_hist", k_huff_hist2<true>, grid, kTokThreads, 0, chunks[k].d_in, hg, d_seghist[k], il, d_total, mh);
-    } else if (generic) LAUNCH("k_huff_hist", k_huff_hist, grid, kHuffThreads, 0, chunks[k].d_in, hg, d_seghist[k]);
+    if (generic) LAUNCH("k_huff_hist", k_huff_hist, grid, kHuffThreads, 0, chunks[k].d_in, hg, d_seghist[k]);
     else if (teams[k])
-      LAUNCH("k_huff_hist", k_huff_hist4<false>, team_grid, kTeamThreads, 0, chunks[k].d_in, hg, d_seghist[k], il, d_total);
-    else LAUNCH("k_huff_hist", k_huff_hist2<false>, grid, kTokThreads, 0, chunks[k].d_in, hg, d_seghist[k], il, d_total);
+      LAUNCH("k_huff_hist", k_huff_hist4<MIXED>, team_grid, kTeamThreads, 0, chunks[k].d_in, hg, d_seghist[k], il, d_total, mh[k]);
+    else LAUNCH("k_huff_hist", k_huff_hist2<MIXED>, grid, kTokThreads, 0, chunks[k].d_in, hg, d_seghist[k], il, d_total, mh[k]);
     TP.total[k] = d_total;
     TP.seghist[k] = d_seghist[k];
     TP.trees[k] = d_trees[k];
@@ -779,48 +715,39 @@ int huff_encode_items(himgcu_ctx *ctx, int n, HuffChunkArgs *chunks, int nchunks
     const int rows = chunks[k].hg.nseg * chunks[k].hg.nsub;
     LAUNCH("k_huff_layout", k_huff_segbits, dim3((rows + 7) / 8, n), 256, 0, d_seghist[k], d_trees[k], rows, d_pbits[k]);
   }
-  if (md) LAUNCH("k_huff_layout", k_huff_layout_mixed, n, kLayoutThreads, 0, P, *md, ContainerTemplate::kDimsAt);
+  if (MIXED) LAUNCH("k_huff_layout", k_huff_layout_mixed, n, kLayoutThreads, 0, P, md, ContainerTemplate::kDimsAt);
   else LAUNCH("k_huff_layout", k_huff_layout, n, kLayoutThreads, 0, P);
   const size_t win_bytes = (kWinWords + 2) * sizeof(uint32_t);
   if (generic)  // static + dynamic shared memory of the first-generation packer exceed 48 KiB
     CK(cudaFuncSetAttribute(k_huff_pack, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)win_bytes));
-  if (teams[0] || teams[1]) {
-    if (md) CK(cudaFuncSetAttribute(k_huff_pack4<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, kP4Smem));
-    else CK(cudaFuncSetAttribute(k_huff_pack4<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, kP4Smem));
-  }
+  if (teams[0] || teams[1]) CK(cudaFuncSetAttribute(k_huff_pack4<MIXED>, cudaFuncAttributeMaxDynamicSharedMemorySize, kP4Smem));
   for (int k = 0; k < nchunks; ++k) {
     const HuffGeom &hg = chunks[k].hg;
     dim3 grid(hg.nseg * hg.nsub, n);
-    if (md) {
-      const MixedHuff mh{*md, k};
-      if (teams[k])
-        LAUNCH("k_huff_pack", k_huff_pack4<true>, dim3((hg.nseg + kTeamWarps - 1) / kTeamWarps, n), kTeamThreads, kP4Smem,
-               chunks[k].d_in, hg, d_trees[k], d_bits[k], d_pos[k], d_sizes, d_out, (unsigned long long)out_stride, d_err, lists[k],
-               mh);
-      else
-        LAUNCH("k_huff_pack", k_huff_pack3<true>, grid, kTokThreads, 0, chunks[k].d_in, hg, d_trees[k], d_bits[k], d_pos[k],
-               d_part[k], d_sizes, d_out, (unsigned long long)out_stride, d_err, lists[k], mh);
-      if (hg.nseg > 1)
-        LAUNCH("k_huff_stale", k_huff_stale<true>, dim3((hg.nseg + 255) / 256, n), 256, 0, n, hg.nseg, d_bits[k], d_pos[k], d_sizes,
-               d_out, (unsigned long long)out_stride, *md);
-      continue;
-    }
     if (generic)
       LAUNCH("k_huff_pack", k_huff_pack, grid, kHuffThreads, win_bytes, chunks[k].d_in, hg, d_trees[k], d_bits[k],
              d_pos[k], d_sizes, d_out, (unsigned long long)out_stride, d_err);
     else if (teams[k])
-      LAUNCH("k_huff_pack", k_huff_pack4<false>, dim3((hg.nseg + kTeamWarps - 1) / kTeamWarps, n), kTeamThreads, kP4Smem, chunks[k].d_in,
-             hg, d_trees[k], d_bits[k], d_pos[k], d_sizes, d_out, (unsigned long long)out_stride, d_err, lists[k]);
+      LAUNCH("k_huff_pack", k_huff_pack4<MIXED>, dim3((hg.nseg + kTeamWarps - 1) / kTeamWarps, n), kTeamThreads, kP4Smem,
+             chunks[k].d_in, hg, d_trees[k], d_bits[k], d_pos[k], d_sizes, d_out, (unsigned long long)out_stride, d_err, lists[k],
+             mh[k]);
     else
-      LAUNCH("k_huff_pack", k_huff_pack3<false>, grid, kTokThreads, 0, chunks[k].d_in, hg, d_trees[k], d_bits[k], d_pos[k],
-             d_part[k], d_sizes, d_out, (unsigned long long)out_stride, d_err, lists[k]);
-    if (hg.nseg > 1) {
-      LAUNCH("k_huff_stale", k_huff_stale<false>, dim3((hg.nseg + 255) / 256, n), 256, 0, n, hg.nseg, d_bits[k], d_pos[k], d_sizes,
-             d_out, (unsigned long long)out_stride);
-    }
+      LAUNCH("k_huff_pack", k_huff_pack3<MIXED>, grid, kTokThreads, 0, chunks[k].d_in, hg, d_trees[k], d_bits[k], d_pos[k],
+             d_part[k], d_sizes, d_out, (unsigned long long)out_stride, d_err, lists[k], mh[k]);
+    if (hg.nseg > 1)
+      LAUNCH("k_huff_stale", k_huff_stale<MIXED>, dim3((hg.nseg + 255) / 256, n), 256, 0, n, hg.nseg, d_bits[k], d_pos[k], d_sizes,
+             d_out, (unsigned long long)out_stride, md);
   }
   return HIMGCU_OK;
 }
+// Instantiated here, before the stages that encode_device calls ahead of it: the module's extern shared arrays are
+// declared in instantiation order, and where k_forward3's 128-byte aligned one comes before k_huff_pack4's 16-byte
+// aligned window, ptxas starts that window 80 bytes later (0x880 instead of 0x830) and allocates k_huff_pack4's
+// registers differently.
+template int huff_encode_items<false>(himgcu_ctx *, int, HuffChunkArgs *, int, bool, uint8_t *, size_t, uint32_t *,
+                                      const MixedDims &);
+template int huff_encode_items<true>(himgcu_ctx *, int, HuffChunkArgs *, int, bool, uint8_t *, size_t, uint32_t *,
+                                     const MixedDims &);
 
 int read_err_flag(himgcu_ctx *ctx, const char *name, int *value) {
   int *d_err;
@@ -848,10 +775,10 @@ size_t per_image_encode_ws(const Geom &g) {
              (kItemCap * 3 + 4);
 }
 
-// Whole-image encode of a sub-batch already resident on the device.  With `md` the batch has mixed geometry: g is
-// the bounding geometry, image i starts at d_pixels + px_off[i] and has its own size (see MixedDims).
+// Whole-image encode of a sub-batch already resident on the device.
+template <bool MIXED = false>
 int encode_device(himgcu_ctx *ctx, const uint8_t *d_pixels, int n, const Geom &g, int quality, bool ycbcr,
-                  uint8_t *d_out, size_t out_stride, uint32_t *d_sizes, const MixedDims *md = nullptr,
+                  uint8_t *d_out, size_t out_stride, uint32_t *d_sizes, const MixedDims &md = {},
                   const unsigned long long *px_off = nullptr) {
   EncodeTables t;
   BuildEncodeTables(quality, ycbcr, &t);
@@ -861,11 +788,11 @@ int encode_device(himgcu_ctx *ctx, const uint8_t *d_pixels, int n, const Geom &g
   ENSURE("L", (size_t)n * g.nch * g.rows * g.cols, d_L);
   ENSURE("lres", (size_t)n * g.lres_stride, d_lres);
   ENSURE("planes", (size_t)n * g.planes_bytes, d_planes);
-  int rc = stage_lowres(ctx, d_pixels, n, g, ycbcr, d_L, md, px_off);
+  int rc = stage_lowres<MIXED>(ctx, d_pixels, n, g, ycbcr, d_L, md, px_off);
   if (rc) return rc;
-  rc = stage_lres_encode(ctx, d_L, n, g, t, d_lres, md);
+  rc = stage_lres_encode<MIXED>(ctx, d_L, n, g, t, d_lres, md);
   if (rc) return rc;
-  rc = stage_forward(ctx, d_pixels, d_L, n, g, t, d_planes, md, px_off);
+  rc = stage_forward<MIXED>(ctx, d_pixels, d_L, n, g, t, d_planes, md, px_off);
   if (rc) return rc;
   HuffChunkArgs ch[2];
   ch[0].d_in = d_lres;
@@ -878,7 +805,7 @@ int encode_device(himgcu_ctx *ctx, const uint8_t *d_pixels, int n, const Geom &g
   ch[1].tag = "fres";
   ch[1].prefix = ct.mid;
   ch[1].size_patch = (int)ct.mid.size() - 4;
-  return huff_encode_items(ctx, n, ch, 2, true, d_out, out_stride, d_sizes, md);
+  return huff_encode_items<MIXED>(ctx, n, ch, 2, true, d_out, out_stride, d_sizes, md);
 }
 
 // Threads per stream for k_dec_stream_par: grow the team until ~128k threads are in flight, but keep
@@ -930,6 +857,21 @@ int launch_stream_cluster(himgcu_ctx *ctx, const char *name, int n, const uint8_
   return HIMGCU_OK;
 }
 
+// nseg framed segments per item from a segment table: a warp per segment (kParWarpTeams per CTA) when team == 32,
+// otherwise a CTA of `team` threads per segment.  MIX: the mixed-geometry mode of k_dec_stream_par (0 = uniform).
+template <int MIX = 0>
+int launch_stream_segments(himgcu_ctx *ctx, const char *name, int team, int n, const uint8_t *d_in, const ChunkDesc *d_cd,
+                           const DecTree *d_tree, SegRef *d_seg, int nseg, int out_seg, uint8_t *d_out,
+                           unsigned long long out_stride, int *d_status, const MixedDims &md = {}) {
+  if (team == 32)
+    LAUNCH(name, (k_dec_stream_par<true, 1, MIX>), dim3((nseg + kParWarpTeams - 1) / kParWarpTeams, n), 32 * kParWarpTeams, 0,
+           d_in, d_cd, d_tree, d_seg, nseg, out_seg, d_out, out_stride, d_status, 0, 0, md);
+  else
+    LAUNCH(name, (k_dec_stream_par<false, 1, MIX>), dim3(nseg, n), team, 0, d_in, d_cd, d_tree, d_seg, nseg, out_seg, d_out,
+           out_stride, d_status, 0, 0, md);
+  return HIMGCU_OK;
+}
+
 // Device scratch of a decode (whole image or region) that decode_front fills.
 struct DecFront {
   const ChunkDesc *fcd;
@@ -943,10 +885,10 @@ struct DecFront {
 // What every decode does before the coefficient planes: container, tables and both trees of n streams, then
 // the low-res branch (segment table, stream, DPCM into R).  The caller ensures its planes buffer before: a
 // workspace that grows is freed after a stream synchronisation, which must not happen while the two branches
-// of a single image run on two streams.  With `md` the batch has mixed geometry (see MixedDims): g is then the
-// bounding geometry, which sizes the scratch, and the low-res stream of an image is never given to a cluster.
+// of a single image run on two streams.  With MIXED the low-res stream of an image is never given to a cluster.
+template <bool MIXED = false>
 int decode_front(himgcu_ctx *ctx, const uint8_t *d_himg, const unsigned long long *d_offsets, const uint32_t *d_sizes, int n,
-                 const Geom &g, int lenient, int *d_status, DecFront *f, const MixedDims *md = nullptr) {
+                 const Geom &g, int lenient, int *d_status, DecFront *f, const MixedDims &md = {}) {
   ChunkDesc *d_lcd, *d_fcd;
   DecTables *d_tabs;
   DecTree *d_ltree, *d_ftree;
@@ -963,13 +905,8 @@ int decode_front(himgcu_ctx *ctx, const uint8_t *d_himg, const unsigned long lon
   ENSURE("L", (size_t)n * g.nch * g.rows * g.cols, d_R);
   *f = DecFront{d_fcd, d_ftree, d_tabs, d_fseg, d_R, n == 1 && !ctx->profile};
   const unsigned nb = (unsigned)((n + 127) / 128);
-  if (md) {
-    LAUNCH("k_dec_parse", k_dec_parse<true>, (unsigned)((n + 3) / 4), 128, 0, d_himg, d_offsets, d_sizes, n, g.w, g.h, g.nch, d_lcd,
-           d_fcd, d_tabs, d_status, *md);
-  } else {
-    LAUNCH("k_dec_parse", k_dec_parse, (unsigned)((n + 3) / 4), 128, 0, d_himg, d_offsets, d_sizes, n, g.w, g.h, g.nch, d_lcd,
-           d_fcd, d_tabs, d_status);
-  }
+  LAUNCH("k_dec_parse", k_dec_parse<MIXED>, (unsigned)((n + 3) / 4), 128, 0, d_himg, d_offsets, d_sizes, n, g.w, g.h, g.nch, d_lcd,
+         d_fcd, d_tabs, d_status, md);
   LAUNCH("k_dec_tree", k_dec_tree, dim3(n, 2), kDecTreeThreads, 0, d_himg, d_lcd, d_fcd, lenient, d_ltree, d_ftree, d_status);
   // A single image is a chain of latency-bound kernels: its two branches (low-res stream -> DPCM, and
   // segment table -> coefficient planes) share nothing until the inverse transform, so they run on
@@ -994,27 +931,18 @@ int decode_front(himgcu_ctx *ctx, const uint8_t *d_himg, const unsigned long lon
     // wider teams (or a cluster of CTAs) when there are few streams (single images).
     const int lres_team = decode_team(n, g.lres_size, kParLresThreads);
     bool clustered = false;
-    if (!md && use_decode_cluster(n, g.lres_size) && !ctx->force_generic) {
+    if (!MIXED && use_decode_cluster(n, g.lres_size) && !ctx->force_generic) {
       int rc = launch_stream_cluster(ctx, "k_dec_stream_lres", n, d_himg, d_lcd, d_ltree, d_lseg, g.lres_size, d_lres,
                                      (unsigned long long)g.lres_stride, d_status, &clustered);
       if (rc) return rc;
     }
-    if (md) {
-      LAUNCH("k_dec_stream_lres", (k_dec_stream_par<false, 1, kMixLres>), dim3(1, n), lres_team, 0, d_himg, d_lcd, d_ltree, d_lseg,
-             1, g.lres_size, d_lres, g.lres_stride, d_status, 0, 0, *md);
-    } else if (!clustered) {
-      LAUNCH("k_dec_stream_lres", k_dec_stream_par<false>, dim3(1, n), lres_team, 0, d_himg, d_lcd, d_ltree, d_lseg, 1,
-             g.lres_size, d_lres, g.lres_stride, d_status);
-    }
+    if (!clustered)
+      LAUNCH("k_dec_stream_lres", (k_dec_stream_par<false, 1, MIXED ? kMixLres : 0>), dim3(1, n), lres_team, 0, d_himg, d_lcd,
+             d_ltree, d_lseg, 1, g.lres_size, d_lres, g.lres_stride, d_status, 0, 0, md);
     const long long nmb = (long long)n * g.nch * g.mrows * g.mcols;
     const unsigned blocks = (unsigned)((nmb + kLresWarps * 2 - 1) / (kLresWarps * 2));
-    if (md) {
-      LAUNCH("k_lres_dpcm_dec", (k_lres_dpcm<false, true>), blocks, kLresWarps * 32, 0, (const uint8_t *)nullptr, d_lres, d_R,
-             g, n, (const uint8_t *)nullptr, d_tabs->low_unmap, (unsigned long long)sizeof(DecTables), *md);
-    } else {
-      LAUNCH("k_lres_dpcm_dec", (k_lres_dpcm<false>), blocks, kLresWarps * 32, 0, (const uint8_t *)nullptr, d_lres, d_R,
-             g, n, (const uint8_t *)nullptr, d_tabs->low_unmap, (unsigned long long)sizeof(DecTables));
-    }
+    LAUNCH("k_lres_dpcm_dec", (k_lres_dpcm<false, MIXED>), blocks, kLresWarps * 32, 0, (const uint8_t *)nullptr, d_lres, d_R, g, n,
+           (const uint8_t *)nullptr, d_tabs->low_unmap, (unsigned long long)sizeof(DecTables), md);
     return HIMGCU_OK;
   };
   int rc_l = lres_branch();
@@ -1026,83 +954,57 @@ int decode_front(himgcu_ctx *ctx, const uint8_t *d_himg, const unsigned long lon
   return rc_l;
 }
 
-// Whole-image decode of n streams resident on the device.  With `md` the batch has mixed geometry: g is its bounding
-// geometry, and image i is written at d_pixels + px_off[i] with its own size (see MixedDims).  lf > 0: every image is
-// written scaled by 2^lf (stage_inverse_scaled); everything before the inverse transform is the same.
-int decode_device(himgcu_ctx *ctx, const uint8_t *d_himg, const unsigned long long *d_offsets,
-                  const uint32_t *d_sizes, int n, const Geom &g, int flags, uint8_t *d_pixels, int *d_status,
-                  const MixedDims *md = nullptr, const unsigned long long *px_off = nullptr, int lf = 0) {
+// Whole-image decode of n streams resident on the device.  lf > 0: every image is written scaled by 2^lf (see
+// stage_inverse); everything before the inverse transform is the same.
+template <bool MIXED = false>
+int decode_device(himgcu_ctx *ctx, const uint8_t *d_himg, const unsigned long long *d_offsets, const uint32_t *d_sizes, int n,
+                  const Geom &g, int flags, uint8_t *d_pixels, int *d_status, int lf = 0, const MixedDims &md = {},
+                  const unsigned long long *px_off = nullptr) {
   const int lenient = (flags & HIMGCU_LENIENT) ? 1 : 0;
   uint8_t *d_planes;
   ENSURE("planes", (size_t)n * g.planes_bytes, d_planes);
   DecFront f;
-  int rc = decode_front(ctx, d_himg, d_offsets, d_sizes, n, g, lenient, d_status, &f, md);
+  int rc = decode_front<MIXED>(ctx, d_himg, d_offsets, d_sizes, n, g, lenient, d_status, &f, md);
   if (rc) return rc;
-  const ChunkDesc *d_fcd = f.fcd;
-  const DecTree *d_ftree = f.ftree;
-  const DecTables *d_tabs = f.tabs;
-  SegRef *d_fseg = f.fseg;
-  const uint8_t *d_R = f.R;
-  const bool fork = f.fork;
-  cudaStream_t main_stream = ctx->stream;
-  const unsigned nb = (unsigned)((n + 127) / 128);
   // a warp per block row when the batch alone fills the GPU, wider teams for few streams
   const int fres_team = decode_team((long long)n * g.rows, g.seg, kParFresThreads);
-  if (md) {  // (no inline walk; block rows past an image's own are idle in the stream decoder)
-    LAUNCH("k_dec_segtab", k_dec_segtab_mixed, nb, 128, 0, d_himg, d_fcd, d_ftree, n, g.rows, lenient, d_fseg, d_status, *md);
-    if (fres_team == 32) {
-      LAUNCH("k_dec_stream_fres", (k_dec_stream_par<true, 1, kMixWhole>), dim3((g.rows + kParWarpTeams - 1) / kParWarpTeams, n),
-             32 * kParWarpTeams, 0, d_himg, d_fcd, d_ftree, d_fseg, g.rows, g.seg, d_planes, g.planes_bytes, d_status, 0, 0, *md);
-    } else {
-      LAUNCH("k_dec_stream_fres", (k_dec_stream_par<false, 1, kMixWhole>), dim3(g.rows, n), fres_team, 0, d_himg, d_fcd, d_ftree,
-             d_fseg, g.rows, g.seg, d_planes, g.planes_bytes, d_status, 0, 0, *md);
-    }
-    if (fork) CK(cudaStreamWaitEvent(main_stream, ctx->ev_join, 0));
-    return stage_inverse(ctx, d_planes, d_R, n, g, d_tabs, sizeof(DecTables), d_pixels, md, px_off, lf);
-  }
   // Few streams (single images): the serial walk over the segment headers runs inside the decode kernel
-  // and the rows decode as soon as their entry is published (all CTAs of such a grid are resident at once)
-  const bool inline_walk = fres_team > 32 && !ctx->force_generic && (long long)n * (g.rows + 1) * fres_team <= 148LL * 2048;
+  // and the rows decode as soon as their entry is published (all CTAs of such a grid are resident at once).
+  // A mixed batch has no inline walk; block rows past an image's own are idle in its stream decoder.
+  const bool inline_walk =
+      !MIXED && fres_team > 32 && !ctx->force_generic && (long long)n * (g.rows + 1) * fres_team <= 148LL * 2048;
   if (inline_walk) {
-    CK(cudaMemsetAsync(d_fseg, 0xfe, (size_t)n * g.rows * sizeof(SegRef), ctx->stream));  // kSegNotReady
-    LAUNCH("k_dec_stream_fres", k_dec_stream_par<false>, dim3(g.rows + 1, n), fres_team, 0, d_himg, d_fcd, d_ftree, d_fseg,
+    CK(cudaMemsetAsync(f.fseg, 0xfe, (size_t)n * g.rows * sizeof(SegRef), ctx->stream));  // kSegNotReady
+    LAUNCH("k_dec_stream_fres", k_dec_stream_par<false>, dim3(g.rows + 1, n), fres_team, 0, d_himg, f.fcd, f.ftree, f.fseg,
            g.rows, g.seg, d_planes, g.planes_bytes, d_status, 1, lenient);
-    if (fork) CK(cudaStreamWaitEvent(main_stream, ctx->ev_join, 0));
-    return stage_inverse(ctx, d_planes, d_R, n, g, d_tabs, sizeof(DecTables), d_pixels, nullptr, nullptr, lf);
-  }
-  LAUNCH("k_dec_segtab", k_dec_segtab, nb, 128, 0, d_himg, d_fcd, d_ftree, n, g.rows, g.seg, 1, lenient, d_fseg,
-         d_status);
-  if (fres_team == 32) {
-    LAUNCH("k_dec_stream_fres", k_dec_stream_par<true>, dim3((g.rows + kParWarpTeams - 1) / kParWarpTeams, n),
-           32 * kParWarpTeams, 0, d_himg, d_fcd, d_ftree, d_fseg, g.rows, g.seg, d_planes, g.planes_bytes, d_status);
   } else {
-    LAUNCH("k_dec_stream_fres", k_dec_stream_par<false>, dim3(g.rows, n), fres_team, 0, d_himg, d_fcd, d_ftree, d_fseg,
-           g.rows, g.seg, d_planes, g.planes_bytes, d_status);
+    const unsigned nb = (unsigned)((n + 127) / 128);
+    if (MIXED)
+      LAUNCH("k_dec_segtab", k_dec_segtab_mixed, nb, 128, 0, d_himg, f.fcd, f.ftree, n, g.rows, lenient, f.fseg, d_status, md);
+    else
+      LAUNCH("k_dec_segtab", k_dec_segtab, nb, 128, 0, d_himg, f.fcd, f.ftree, n, g.rows, g.seg, 1, lenient, f.fseg, d_status);
+    rc = launch_stream_segments<MIXED ? kMixWhole : 0>(ctx, "k_dec_stream_fres", fres_team, n, d_himg, f.fcd, f.ftree, f.fseg,
+                                                        g.rows, g.seg, d_planes, g.planes_bytes, d_status, md);
+    if (rc) return rc;
   }
-  if (fork) CK(cudaStreamWaitEvent(main_stream, ctx->ev_join, 0));
-  return stage_inverse(ctx, d_planes, d_R, n, g, d_tabs, sizeof(DecTables), d_pixels, nullptr, nullptr, lf);
+  if (f.fork) CK(cudaStreamWaitEvent(ctx->stream, ctx->ev_join, 0));
+  return stage_inverse<MIXED>(ctx, d_planes, f.R, n, g, f.tabs, sizeof(DecTables), d_pixels, lf, md, px_off);
 }
 
 // Compact block rows a region decode keeps per image: the most a rectangle of rh rows can touch.
 int region_rows(const Geom &g, int rh) { return std::min((rh + 14) / 8, g.rows); }
 
-// K-inv of a region decode (xform_region.cuh) from the compact planes [n][kr][seg].  A mixed-geometry batch (md) takes
-// the generic kernel.
+// K-inv of a region decode (xform_region.cuh) from the compact planes [n][kr][seg].
+template <bool MIXED = false>
 int stage_inverse_region(himgcu_ctx *ctx, const uint8_t *d_planes, const uint8_t *d_R, int n, const Geom &g,
                          const DecTables *d_tabs, const int32_t *d_origins, int rw, int rh, int kr, uint8_t *d_pixels,
-                         const MixedDims *md = nullptr) {
-  const int kb = (rw + 14) / 8;
-  if (md) {
-    LAUNCH("k_inverse_region", k_inverse_region<true>, dim3((kb + kTile - 1) / kTile, kr, n), kTile, 0, d_planes, d_R, g, d_tabs,
-           (unsigned long long)sizeof(DecTables), d_origins, rw, rh, kr, d_pixels, *md);
-    return HIMGCU_OK;
-  }
+                         const MixedDims &md = {}) {
   // lane-pair fast path: the shapes k_inverse4 takes, except that the rectangle clips rows and columns
-  if (!ctx->force_generic && (g.cols % 16) == 0 && (g.nch == 1 || g.nch == 3) && (reinterpret_cast<uintptr_t>(d_planes) & 15) == 0 &&
-      (reinterpret_cast<uintptr_t>(d_R) & 1) == 0) {
+  if (!MIXED && !ctx->force_generic && (g.cols % 16) == 0 && (g.nch == 1 || g.nch == 3) &&
+      (reinterpret_cast<uintptr_t>(d_planes) & 15) == 0 && (reinterpret_cast<uintptr_t>(d_R) & 1) == 0) {
     InvTables *d_inv;
-    ENSURE("inv_tables", (size_t)n * sizeof(InvTables), d_inv);
-    LAUNCH("k_inv_tables", k_inv_tables, n, 256, 0, d_tabs, (unsigned long long)sizeof(DecTables), d_inv);
+    int rc = launch_inv_tables(ctx, d_tabs, n, (unsigned long long)sizeof(DecTables), &d_inv);
+    if (rc) return rc;
     const int span = region_span_pairs(rw, g.cols);
     constexpr int TP = kInv4ThreadsRgb;
     static_assert(kInv4ThreadsGray == TP, "one tile width for both channel counts");
@@ -1119,17 +1021,18 @@ int stage_inverse_region(himgcu_ctx *ctx, const uint8_t *d_planes, const uint8_t
     }
     return HIMGCU_OK;
   }
-  LAUNCH("k_inverse_region", k_inverse_region, dim3((kb + kTile - 1) / kTile, kr, n), kTile, 0, d_planes, d_R, g, d_tabs,
-         (unsigned long long)sizeof(DecTables), d_origins, rw, rh, kr, d_pixels);
+  const int kb = (rw + 14) / 8;
+  LAUNCH("k_inverse_region", k_inverse_region<MIXED>, dim3((kb + kTile - 1) / kTile, kr, n), kTile, 0, d_planes, d_R, g, d_tabs,
+         (unsigned long long)sizeof(DecTables), d_origins, rw, rh, kr, d_pixels, md);
   return HIMGCU_OK;
 }
 
 // Region decode of n streams resident on the device: image i's rectangle rw x rh at (d_origins[2i], d_origins[2i+1])
 // to d_pixels + i * rw * rh * nch.  Only the FRES segments of the block rows the rectangle touches are decoded.
-// With `md` the batch has mixed geometry and g is its bounding geometry (see MixedDims).
+template <bool MIXED = false>
 int decode_region_device(himgcu_ctx *ctx, const uint8_t *d_himg, const unsigned long long *d_offsets, const uint32_t *d_sizes,
                          int n, const Geom &g, int flags, const int32_t *d_origins, int rw, int rh, uint8_t *d_pixels,
-                         int *d_status, const MixedDims *md = nullptr) {
+                         int *d_status, const MixedDims &md = {}) {
   const int lenient = (flags & HIMGCU_LENIENT) ? 1 : 0;
   const int kr = region_rows(g, rh);
   uint8_t *d_planes;
@@ -1137,34 +1040,29 @@ int decode_region_device(himgcu_ctx *ctx, const uint8_t *d_himg, const unsigned 
   ENSURE("planes", (size_t)n * kr * g.seg, d_planes);
   ENSURE("dec_rseg", (size_t)n * kr * sizeof(SegRef), d_rseg);
   DecFront f;
-  int rc = decode_front(ctx, d_himg, d_offsets, d_sizes, n, g, lenient, d_status, &f, md);
+  int rc = decode_front<MIXED>(ctx, d_himg, d_offsets, d_sizes, n, g, lenient, d_status, &f, md);
   if (rc) return rc;
-  const unsigned long long stride = (unsigned long long)kr * g.seg;
+  LAUNCH("k_dec_segtab_region", k_dec_segtab_region<MIXED>, (unsigned)((n + 127) / 128), 128, 0, d_himg, f.fcd, f.ftree, n, g,
+         lenient, d_origins, rw, rh, kr, f.fseg, d_rseg, d_status, md);
   const int team = decode_team((long long)n * kr, g.seg, kParFresThreads);
-  if (md) {
-    LAUNCH("k_dec_segtab_region", k_dec_segtab_region<true>, (unsigned)((n + 127) / 128), 128, 0, d_himg, f.fcd, f.ftree, n, g,
-           lenient, d_origins, rw, rh, kr, f.fseg, d_rseg, d_status, *md);
-    if (team == 32) {
-      LAUNCH("k_dec_stream_fres", (k_dec_stream_par<true, 1, kMixFres>), dim3((kr + kParWarpTeams - 1) / kParWarpTeams, n),
-             32 * kParWarpTeams, 0, d_himg, f.fcd, f.ftree, d_rseg, kr, g.seg, d_planes, stride, d_status, 0, 0, *md);
-    } else {
-      LAUNCH("k_dec_stream_fres", (k_dec_stream_par<false, 1, kMixFres>), dim3(kr, n), team, 0, d_himg, f.fcd, f.ftree, d_rseg, kr,
-             g.seg, d_planes, stride, d_status, 0, 0, *md);
-    }
-    if (f.fork) CK(cudaStreamWaitEvent(ctx->stream, ctx->ev_join, 0));
-    return stage_inverse_region(ctx, d_planes, f.R, n, g, f.tabs, d_origins, rw, rh, kr, d_pixels, md);
-  }
-  LAUNCH("k_dec_segtab_region", k_dec_segtab_region, (unsigned)((n + 127) / 128), 128, 0, d_himg, f.fcd, f.ftree, n, g, lenient,
-         d_origins, rw, rh, kr, f.fseg, d_rseg, d_status);
-  if (team == 32) {
-    LAUNCH("k_dec_stream_fres", k_dec_stream_par<true>, dim3((kr + kParWarpTeams - 1) / kParWarpTeams, n), 32 * kParWarpTeams, 0,
-           d_himg, f.fcd, f.ftree, d_rseg, kr, g.seg, d_planes, stride, d_status);
-  } else {
-    LAUNCH("k_dec_stream_fres", k_dec_stream_par<false>, dim3(kr, n), team, 0, d_himg, f.fcd, f.ftree, d_rseg, kr, g.seg,
-           d_planes, stride, d_status);
-  }
+  rc = launch_stream_segments<MIXED ? kMixFres : 0>(ctx, "k_dec_stream_fres", team, n, d_himg, f.fcd, f.ftree, d_rseg, kr, g.seg,
+                                                     d_planes, (unsigned long long)kr * g.seg, d_status, md);
+  if (rc) return rc;
   if (f.fork) CK(cudaStreamWaitEvent(ctx->stream, ctx->ev_join, 0));
-  return stage_inverse_region(ctx, d_planes, f.R, n, g, f.tabs, d_origins, rw, rh, kr, d_pixels);
+  return stage_inverse_region<MIXED>(ctx, d_planes, f.R, n, g, f.tabs, d_origins, rw, rh, kr, d_pixels, md);
+}
+
+// Runs body(i0, m) over the sub-batches [i0, i0 + m) of n images: as many images as fit max_workspace_bytes at `per`
+// workspace bytes each, at least one and at most 65535.
+template <class F>
+int for_sub_batches(himgcu_ctx *ctx, int n, size_t per, F &&body) {
+  int sub = (int)std::min<size_t>((size_t)n, std::max<size_t>(1, ctx->max_workspace / per));
+  sub = std::min(sub, 65535);
+  for (int i0 = 0; i0 < n; i0 += sub) {
+    const int rc = body(i0, std::min(sub, n - i0));
+    if (rc) return rc;
+  }
+  return HIMGCU_OK;
 }
 
 }  // namespace
@@ -1492,16 +1390,10 @@ int himgcu_encode_batch(himgcu_ctx *ctx, const uint8_t *d_pixels, int n, int w, 
   CK(cudaSetDevice(ctx->device));
   const Geom g = make_geom(w, h, nch, nch);
   const bool ycbcr = use_ycbcr && nch >= 3;
-  const size_t per = per_image_encode_ws(g);
-  int sub = (int)std::min<size_t>((size_t)n, std::max<size_t>(1, ctx->max_workspace / per));
-  sub = std::min(sub, 65535);
-  for (int i0 = 0; i0 < n; i0 += sub) {
-    const int m = std::min(sub, n - i0);
-    int rc = encode_device(ctx, d_pixels + (size_t)i0 * g.img_bytes, m, g, quality, ycbcr,
-                           d_out + (size_t)i0 * out_stride, out_stride, d_sizes + i0);
-    if (rc) return rc;
-  }
-  return HIMGCU_OK;
+  return for_sub_batches(ctx, n, per_image_encode_ws(g), [&](int i0, int m) -> int {
+    return encode_device(ctx, d_pixels + (size_t)i0 * g.img_bytes, m, g, quality, ycbcr, d_out + (size_t)i0 * out_stride,
+                         out_stride, d_sizes + i0);
+  });
 }
 
 int himgcu_encode_batch_mixed(himgcu_ctx *ctx, const uint8_t *d_pixels, const uint64_t *d_pixel_offsets, const int32_t *d_dims,
@@ -1515,17 +1407,11 @@ int himgcu_encode_batch_mixed(himgcu_ctx *ctx, const uint8_t *d_pixels, const ui
   // every per-image scratch slot has the bounding geometry's size; the kernels lay each image out in its own
   const Geom g = make_geom(max_width, max_height, nch, nch);
   const bool ycbcr = use_ycbcr && nch >= 3;
-  const size_t per = per_image_encode_ws(g);
-  int sub = (int)std::min<size_t>((size_t)n, std::max<size_t>(1, ctx->max_workspace / per));
-  sub = std::min(sub, 65535);
-  for (int i0 = 0; i0 < n; i0 += sub) {
-    const int m = std::min(sub, n - i0);
+  return for_sub_batches(ctx, n, per_image_encode_ws(g), [&](int i0, int m) -> int {
     const MixedDims md{d_dims + 2 * (size_t)i0, max_width, max_height, nch};
-    int rc = encode_device(ctx, d_pixels, m, g, quality, ycbcr, d_out + (size_t)i0 * out_stride, out_stride, d_sizes + i0, &md,
-                           reinterpret_cast<const unsigned long long *>(d_pixel_offsets) + i0);
-    if (rc) return rc;
-  }
-  return HIMGCU_OK;
+    return encode_device<true>(ctx, d_pixels, m, g, quality, ycbcr, d_out + (size_t)i0 * out_stride, out_stride, d_sizes + i0, md,
+                               reinterpret_cast<const unsigned long long *>(d_pixel_offsets) + i0);
+  });
 }
 
 }  // extern "C"
@@ -1622,55 +1508,66 @@ size_t scaled_bytes(const Geom &g, int lf) {
   return (size_t)((g.w + f - 1) >> lf) * (size_t)((g.h + f - 1) >> lf) * (size_t)g.nch;
 }
 
-// himgcu_decode_batch, and with lf > 0 himgcu_decode_batch_scaled: image i goes to d_pixels_out + i * scaled_bytes(g, lf).
-int decode_batch_lf(himgcu_ctx *ctx, const uint8_t *d_himg, const uint64_t *d_offsets, const uint32_t *d_sizes, int n, int w,
-                    int h, int nch, int flags, int lf, uint8_t *d_pixels_out, int32_t *d_status) {
-  if (!ctx || !d_himg || !d_offsets || !d_sizes || !d_pixels_out || !d_status || n < 0)
+// himgcu_decode_batch(_scaled), and with MIXED himgcu_decode_batch_mixed(_scaled), whose w x h are the bounds of the
+// images: image i goes to d_pixels_out + i * scaled_bytes(g, lf), or with MIXED to d_pixels_out + d_pixel_offsets[i].
+template <bool MIXED>
+int decode_batch_lf(himgcu_ctx *ctx, const uint8_t *d_himg, const uint64_t *d_offsets, const uint32_t *d_sizes, int n,
+                    const int32_t *d_dims, int w, int h, int nch, int flags, int lf, const uint64_t *d_pixel_offsets,
+                    uint8_t *d_pixels_out, int32_t *d_status) {
+  if (!ctx || !d_himg || !d_offsets || !d_sizes || (MIXED && (!d_dims || !d_pixel_offsets)) || !d_pixels_out || !d_status || n < 0)
     return fail(ctx, HIMGCU_ERR_ARG, "bad argument");
-  if (!shape_ok(w, h, nch)) return fail(ctx, HIMGCU_ERR_UNSUPPORTED, "unsupported shape %dx%dx%d", w, h, nch);
+  if (!shape_ok(w, h, nch))
+    return fail(ctx, HIMGCU_ERR_UNSUPPORTED, "unsupported %sshape %dx%dx%d", MIXED ? "bounding " : "", w, h, nch);
+  if (n == 0) return HIMGCU_OK;
+  CK(cudaSetDevice(ctx->device));
+  // with MIXED every per-image scratch slot has the bounding geometry's size; the kernels lay each image out in its own
+  const Geom g = make_geom(w, h, nch, nch);
+  const size_t per = per_image_encode_ws(g) + sizeof(DecTables) + 2 * sizeof(DecTree);
+  return for_sub_batches(ctx, n, per, [&](int i0, int m) -> int {
+    const MixedDims md = MIXED ? MixedDims{d_dims + 2 * (size_t)i0, w, h, nch} : MixedDims{};
+    const unsigned long long *px_off = MIXED ? reinterpret_cast<const unsigned long long *>(d_pixel_offsets) + i0 : nullptr;
+    uint8_t *out = MIXED ? d_pixels_out : d_pixels_out + (size_t)i0 * scaled_bytes(g, lf);
+    return decode_device<MIXED>(ctx, d_himg, reinterpret_cast<const unsigned long long *>(d_offsets) + i0, d_sizes + i0, m, g, flags,
+                                out, d_status + i0, lf, md, px_off);
+  });
+}
+
+// himgcu_decode_batch_region, and with MIXED himgcu_decode_batch_region_mixed, whose w x h are the bounds of the images.
+template <bool MIXED>
+int decode_batch_region(himgcu_ctx *ctx, const uint8_t *d_himg, const uint64_t *d_offsets, const uint32_t *d_sizes, int n,
+                        const int32_t *d_dims, int w, int h, int nch, int flags, const int32_t *d_origins, int rw, int rh,
+                        uint8_t *d_pixels_out, int32_t *d_status) {
+  if (!ctx || !d_himg || !d_offsets || !d_sizes || (MIXED && !d_dims) || !d_origins || !d_pixels_out || !d_status || n < 0)
+    return fail(ctx, HIMGCU_ERR_ARG, "bad argument");
+  if (!shape_ok(w, h, nch))
+    return fail(ctx, HIMGCU_ERR_UNSUPPORTED, "unsupported %sshape %dx%dx%d", MIXED ? "bounding " : "", w, h, nch);
+  if (rw < 1 || rh < 1 || rw > w || rh > h)
+    return fail(ctx, HIMGCU_ERR_ARG, MIXED ? "region %dx%d does not fit the %dx%d bounds" : "region %dx%d does not fit a %dx%d image",
+                rw, rh, w, h);
   if (n == 0) return HIMGCU_OK;
   CK(cudaSetDevice(ctx->device));
   const Geom g = make_geom(w, h, nch, nch);
-  const size_t per = per_image_encode_ws(g) + sizeof(DecTables) + 2 * sizeof(DecTree);
-  int sub = (int)std::min<size_t>((size_t)n, std::max<size_t>(1, ctx->max_workspace / per));
-  sub = std::min(sub, 65535);
-  for (int i0 = 0; i0 < n; i0 += sub) {
-    const int m = std::min(sub, n - i0);
-    int rc = decode_device(ctx, d_himg, reinterpret_cast<const unsigned long long *>(d_offsets) + i0, d_sizes + i0, m,
-                           g, flags, d_pixels_out + (size_t)i0 * scaled_bytes(g, lf), d_status + i0, nullptr, nullptr, lf);
-    if (rc) return rc;
-  }
-  return HIMGCU_OK;
+  const int kr = region_rows(g, rh);
+  const size_t out_bytes = (size_t)rw * rh * nch;
+  // (the uniform count includes the tables of the lane-pair inverse, which a mixed batch does not take)
+  const size_t per = per_image_encode_ws(g) - g.planes_bytes + (size_t)kr * (g.seg + sizeof(SegRef)) + sizeof(DecTables) +
+                     2 * sizeof(DecTree) + (MIXED ? 0 : sizeof(InvTables));
+  return for_sub_batches(ctx, n, per, [&](int i0, int m) -> int {
+    const MixedDims md = MIXED ? MixedDims{d_dims + 2 * (size_t)i0, w, h, nch} : MixedDims{};
+    return decode_region_device<MIXED>(ctx, d_himg, reinterpret_cast<const unsigned long long *>(d_offsets) + i0, d_sizes + i0, m,
+                                       g, flags, d_origins + 2 * (size_t)i0, rw, rh, d_pixels_out + (size_t)i0 * out_bytes,
+                                       d_status + i0, md);
+  });
 }
 
-// himgcu_decode_batch_mixed, and with lf > 0 himgcu_decode_batch_mixed_scaled.
-int decode_batch_mixed_lf(himgcu_ctx *ctx, const uint8_t *d_himg, const uint64_t *d_offsets, const uint32_t *d_sizes, int n,
-                          const int32_t *d_dims, int max_width, int max_height, int nch, int flags, int lf,
-                          const uint64_t *d_pixel_offsets, uint8_t *d_pixels_out, int32_t *d_status) {
-  if (!ctx || !d_himg || !d_offsets || !d_sizes || !d_dims || !d_pixel_offsets || !d_pixels_out || !d_status || n < 0)
-    return fail(ctx, HIMGCU_ERR_ARG, "bad argument");
-  if (!shape_ok(max_width, max_height, nch))
-    return fail(ctx, HIMGCU_ERR_UNSUPPORTED, "unsupported bounding shape %dx%dx%d", max_width, max_height, nch);
-  if (n == 0) return HIMGCU_OK;
-  CK(cudaSetDevice(ctx->device));
-  // every per-image scratch slot has the bounding geometry's size; the kernels lay each image out in its own
-  const Geom g = make_geom(max_width, max_height, nch, nch);
-  const size_t per = per_image_encode_ws(g) + sizeof(DecTables) + 2 * sizeof(DecTree);
-  int sub = (int)std::min<size_t>((size_t)n, std::max<size_t>(1, ctx->max_workspace / per));
-  sub = std::min(sub, 65535);
-  for (int i0 = 0; i0 < n; i0 += sub) {
-    const int m = std::min(sub, n - i0);
-    const MixedDims md{d_dims + 2 * (size_t)i0, max_width, max_height, nch};
-    int rc = decode_device(ctx, d_himg, reinterpret_cast<const unsigned long long *>(d_offsets) + i0, d_sizes + i0, m, g, flags,
-                           d_pixels_out, d_status + i0, &md, reinterpret_cast<const unsigned long long *>(d_pixel_offsets) + i0, lf);
-    if (rc) return rc;
-  }
-  return HIMGCU_OK;
-}
+struct Rect {
+  int x, y, w, h;
+};
 
-// himgcu_decode, and with lf > 0 himgcu_decode_scaled (out_cap is checked against the scaled size).
-int decode_single_lf(himgcu_ctx *ctx, const uint8_t *himg, size_t size, int flags, int lf, uint8_t *out, size_t out_cap, int *w,
-                     int *h, int *nch) {
+// himgcu_decode, himgcu_decode_scaled (lf > 0, out_cap is checked against the scaled size) and, with `rect`,
+// himgcu_decode_region.
+int decode_single(himgcu_ctx *ctx, const uint8_t *himg, size_t size, int flags, int lf, const Rect *rect, uint8_t *out,
+                  size_t out_cap, int *w, int *h, int *nch) {
   if (!ctx || !himg || !out) return fail(ctx, HIMGCU_ERR_ARG, "bad argument");
   int W = 0, H = 0, N = 0;
   if (himgcu_decode_info(himg, size, &W, &H, &N) != HIMGCU_OK) return fail(ctx, HIMGCU_REJECT, "not a HIMG stream");
@@ -1680,32 +1577,47 @@ int decode_single_lf(himgcu_ctx *ctx, const uint8_t *himg, size_t size, int flag
   if (W < 1 || H < 1 || N < 1) return fail(ctx, HIMGCU_REJECT, "bad dimensions");
   if (!shape_ok(W, H, N)) return fail(ctx, HIMGCU_ERR_UNSUPPORTED, "unsupported shape %dx%dx%d", W, H, N);
   if (size > 0xffffffffull) return fail(ctx, HIMGCU_ERR_UNSUPPORTED, "stream too large");
+  if (rect && (rect->w < 1 || rect->h < 1 || rect->x < 0 || rect->y < 0 || rect->x > W - rect->w || rect->y > H - rect->h))
+    return fail(ctx, HIMGCU_ERR_ARG, "region %dx%d at (%d, %d) is empty or outside the %dx%d image", rect->w, rect->h, rect->x,
+                rect->y, W, H);
   CK(cudaSetDevice(ctx->device));
   const Geom g = make_geom(W, H, N, N);
-  const size_t out_bytes = scaled_bytes(g, lf);
+  const size_t out_bytes = rect ? (size_t)rect->w * rect->h * N : scaled_bytes(g, lf);
   if (out_bytes > out_cap) return fail(ctx, HIMGCU_ERR_CAPACITY, "output buffer too small");
   uint8_t *d_in, *d_px;
   unsigned long long *d_off;
   uint32_t *d_sz;
   int *d_status;
+  int32_t *d_org = nullptr;
   ENSURE("single_in", size + 16, d_in);
-  ENSURE("single_px", out_bytes, d_px);
+  ENSURE(rect ? "single_rpx" : "single_px", out_bytes, d_px);
   ENSURE("single_off", sizeof(unsigned long long), d_off);
   ENSURE("single_size", sizeof(uint32_t), d_sz);
   ENSURE("single_status", sizeof(int), d_status);
+  if (rect) ENSURE("single_origin", 2 * sizeof(int32_t), d_org);
   int rc = ensure_pinned(ctx, 64);
   if (rc) return rc;
-  // offset / size / status travel through the context's page-locked scratch (truly asynchronous copies)
+  // offset / size / status / origin travel through the context's page-locked scratch (truly asynchronous copies)
   unsigned long long *h_off = reinterpret_cast<unsigned long long *>(ctx->pinned);
   uint32_t *h_sz = reinterpret_cast<uint32_t *>(h_off + 1);
   int *h_status = reinterpret_cast<int *>(h_off + 2);
+  int32_t *h_org = reinterpret_cast<int32_t *>(h_off + 3);
   CK(cudaStreamSynchronize(ctx->stream));  // (the scratch words of the previous call are no longer in flight)
   *h_off = 0;
   *h_sz = (uint32_t)size;
+  if (rect) {
+    h_org[0] = rect->x;
+    h_org[1] = rect->y;
+  }
   if ((rc = copy_to_device(ctx, d_in, himg, size))) return rc;
   CK(cudaMemcpyAsync(d_off, h_off, sizeof(*h_off), cudaMemcpyHostToDevice, ctx->stream));
   CK(cudaMemcpyAsync(d_sz, h_sz, sizeof(*h_sz), cudaMemcpyHostToDevice, ctx->stream));
-  rc = decode_device(ctx, d_in, d_off, d_sz, 1, g, flags, d_px, d_status, nullptr, nullptr, lf);
+  if (rect) {
+    CK(cudaMemcpyAsync(d_org, h_org, 2 * sizeof(int32_t), cudaMemcpyHostToDevice, ctx->stream));
+    rc = decode_region_device(ctx, d_in, d_off, d_sz, 1, g, flags, d_org, rect->w, rect->h, d_px, d_status);
+  } else {
+    rc = decode_device(ctx, d_in, d_off, d_sz, 1, g, flags, d_px, d_status, lf);
+  }
   if (rc) return rc;
   // The pixels follow the status on the same stream without a round trip in between: a rejected stream
   // costs one wasted copy, an accepted one (the common case) saves a synchronisation.
@@ -1781,20 +1693,20 @@ int himgcu_decode_info(const uint8_t *p, size_t size, int *w, int *h, int *nch) 
 
 int himgcu_decode_batch(himgcu_ctx *ctx, const uint8_t *d_himg, const uint64_t *d_offsets, const uint32_t *d_sizes,
                         int n, int w, int h, int nch, int flags, uint8_t *d_pixels_out, int32_t *d_status) {
-  return decode_batch_lf(ctx, d_himg, d_offsets, d_sizes, n, w, h, nch, flags, 0, d_pixels_out, d_status);
+  return decode_batch_lf<false>(ctx, d_himg, d_offsets, d_sizes, n, nullptr, w, h, nch, flags, 0, nullptr, d_pixels_out, d_status);
 }
 
 int himgcu_decode_batch_scaled(himgcu_ctx *ctx, const uint8_t *d_himg, const uint64_t *d_offsets, const uint32_t *d_sizes,
                                int n, int w, int h, int nch, int flags, int factor, uint8_t *d_pixels_out, int32_t *d_status) {
   const int lf = scale_log2(factor);
   if (lf < 0) return fail(ctx, HIMGCU_ERR_ARG, "scale factor %d is not 1, 2, 4 or 8", factor);
-  return decode_batch_lf(ctx, d_himg, d_offsets, d_sizes, n, w, h, nch, flags, lf, d_pixels_out, d_status);
+  return decode_batch_lf<false>(ctx, d_himg, d_offsets, d_sizes, n, nullptr, w, h, nch, flags, lf, nullptr, d_pixels_out, d_status);
 }
 
 int himgcu_decode_batch_mixed(himgcu_ctx *ctx, const uint8_t *d_himg, const uint64_t *d_offsets, const uint32_t *d_sizes, int n,
                               const int32_t *d_dims, int max_width, int max_height, int nch, int flags,
                               const uint64_t *d_pixel_offsets, uint8_t *d_pixels_out, int32_t *d_status) {
-  return decode_batch_mixed_lf(ctx, d_himg, d_offsets, d_sizes, n, d_dims, max_width, max_height, nch, flags, 0, d_pixel_offsets,
+  return decode_batch_lf<true>(ctx, d_himg, d_offsets, d_sizes, n, d_dims, max_width, max_height, nch, flags, 0, d_pixel_offsets,
                                d_pixels_out, d_status);
 }
 
@@ -1803,127 +1715,40 @@ int himgcu_decode_batch_mixed_scaled(himgcu_ctx *ctx, const uint8_t *d_himg, con
                                      const uint64_t *d_pixel_offsets, uint8_t *d_pixels_out, int32_t *d_status) {
   const int lf = scale_log2(factor);
   if (lf < 0) return fail(ctx, HIMGCU_ERR_ARG, "scale factor %d is not 1, 2, 4 or 8", factor);
-  return decode_batch_mixed_lf(ctx, d_himg, d_offsets, d_sizes, n, d_dims, max_width, max_height, nch, flags, lf, d_pixel_offsets,
+  return decode_batch_lf<true>(ctx, d_himg, d_offsets, d_sizes, n, d_dims, max_width, max_height, nch, flags, lf, d_pixel_offsets,
                                d_pixels_out, d_status);
 }
 
 int himgcu_decode(himgcu_ctx *ctx, const uint8_t *himg, size_t size, int flags, uint8_t *out, size_t out_cap, int *w,
                   int *h, int *nch) {
-  return decode_single_lf(ctx, himg, size, flags, 0, out, out_cap, w, h, nch);
+  return decode_single(ctx, himg, size, flags, 0, nullptr, out, out_cap, w, h, nch);
 }
 
 int himgcu_decode_scaled(himgcu_ctx *ctx, const uint8_t *himg, size_t size, int flags, int factor, uint8_t *out, size_t out_cap,
                          int *w, int *h, int *nch) {
   const int lf = scale_log2(factor);
   if (lf < 0) return fail(ctx, HIMGCU_ERR_ARG, "scale factor %d is not 1, 2, 4 or 8", factor);
-  return decode_single_lf(ctx, himg, size, flags, lf, out, out_cap, w, h, nch);
+  return decode_single(ctx, himg, size, flags, lf, nullptr, out, out_cap, w, h, nch);
 }
 
 int himgcu_decode_batch_region(himgcu_ctx *ctx, const uint8_t *d_himg, const uint64_t *d_offsets, const uint32_t *d_sizes, int n,
                                int w, int h, int nch, int flags, const int32_t *d_origins, int rw, int rh, uint8_t *d_pixels_out,
                                int32_t *d_status) {
-  if (!ctx || !d_himg || !d_offsets || !d_sizes || !d_origins || !d_pixels_out || !d_status || n < 0)
-    return fail(ctx, HIMGCU_ERR_ARG, "bad argument");
-  if (!shape_ok(w, h, nch)) return fail(ctx, HIMGCU_ERR_UNSUPPORTED, "unsupported shape %dx%dx%d", w, h, nch);
-  if (rw < 1 || rh < 1 || rw > w || rh > h) return fail(ctx, HIMGCU_ERR_ARG, "region %dx%d does not fit a %dx%d image", rw, rh, w, h);
-  if (n == 0) return HIMGCU_OK;
-  CK(cudaSetDevice(ctx->device));
-  const Geom g = make_geom(w, h, nch, nch);
-  const int kr = region_rows(g, rh);
-  const size_t out_bytes = (size_t)rw * rh * nch;
-  const size_t per = per_image_encode_ws(g) - g.planes_bytes + (size_t)kr * (g.seg + sizeof(SegRef)) + sizeof(DecTables) +
-                     2 * sizeof(DecTree) + sizeof(InvTables);
-  int sub = (int)std::min<size_t>((size_t)n, std::max<size_t>(1, ctx->max_workspace / per));
-  sub = std::min(sub, 65535);
-  for (int i0 = 0; i0 < n; i0 += sub) {
-    const int m = std::min(sub, n - i0);
-    int rc = decode_region_device(ctx, d_himg, reinterpret_cast<const unsigned long long *>(d_offsets) + i0, d_sizes + i0, m, g,
-                                  flags, d_origins + 2 * (size_t)i0, rw, rh, d_pixels_out + (size_t)i0 * out_bytes, d_status + i0);
-    if (rc) return rc;
-  }
-  return HIMGCU_OK;
+  return decode_batch_region<false>(ctx, d_himg, d_offsets, d_sizes, n, nullptr, w, h, nch, flags, d_origins, rw, rh, d_pixels_out,
+                                    d_status);
 }
 
 int himgcu_decode_batch_region_mixed(himgcu_ctx *ctx, const uint8_t *d_himg, const uint64_t *d_offsets, const uint32_t *d_sizes,
                                      int n, const int32_t *d_dims, int max_width, int max_height, int nch, int flags,
                                      const int32_t *d_origins, int rw, int rh, uint8_t *d_pixels_out, int32_t *d_status) {
-  if (!ctx || !d_himg || !d_offsets || !d_sizes || !d_dims || !d_origins || !d_pixels_out || !d_status || n < 0)
-    return fail(ctx, HIMGCU_ERR_ARG, "bad argument");
-  if (!shape_ok(max_width, max_height, nch))
-    return fail(ctx, HIMGCU_ERR_UNSUPPORTED, "unsupported bounding shape %dx%dx%d", max_width, max_height, nch);
-  if (rw < 1 || rh < 1 || rw > max_width || rh > max_height)
-    return fail(ctx, HIMGCU_ERR_ARG, "region %dx%d does not fit the %dx%d bounds", rw, rh, max_width, max_height);
-  if (n == 0) return HIMGCU_OK;
-  CK(cudaSetDevice(ctx->device));
-  // every per-image scratch slot has the bounding geometry's size; the kernels lay each image out in its own
-  const Geom g = make_geom(max_width, max_height, nch, nch);
-  const int kr = region_rows(g, rh);
-  const size_t out_bytes = (size_t)rw * rh * nch;
-  const size_t per = per_image_encode_ws(g) - g.planes_bytes + (size_t)kr * (g.seg + sizeof(SegRef)) + sizeof(DecTables) +
-                     2 * sizeof(DecTree);
-  int sub = (int)std::min<size_t>((size_t)n, std::max<size_t>(1, ctx->max_workspace / per));
-  sub = std::min(sub, 65535);
-  for (int i0 = 0; i0 < n; i0 += sub) {
-    const int m = std::min(sub, n - i0);
-    const MixedDims md{d_dims + 2 * (size_t)i0, max_width, max_height, nch};
-    int rc = decode_region_device(ctx, d_himg, reinterpret_cast<const unsigned long long *>(d_offsets) + i0, d_sizes + i0, m, g,
-                                  flags, d_origins + 2 * (size_t)i0, rw, rh, d_pixels_out + (size_t)i0 * out_bytes, d_status + i0,
-                                  &md);
-    if (rc) return rc;
-  }
-  return HIMGCU_OK;
+  return decode_batch_region<true>(ctx, d_himg, d_offsets, d_sizes, n, d_dims, max_width, max_height, nch, flags, d_origins, rw, rh,
+                                   d_pixels_out, d_status);
 }
 
 int himgcu_decode_region(himgcu_ctx *ctx, const uint8_t *himg, size_t size, int flags, int x, int y, int rw, int rh, uint8_t *out,
                          size_t out_cap, int *w, int *h, int *nch) {
-  if (!ctx || !himg || !out) return fail(ctx, HIMGCU_ERR_ARG, "bad argument");
-  int W = 0, H = 0, N = 0;
-  if (himgcu_decode_info(himg, size, &W, &H, &N) != HIMGCU_OK) return fail(ctx, HIMGCU_REJECT, "not a HIMG stream");
-  if (w) *w = W;
-  if (h) *h = H;
-  if (nch) *nch = N;
-  if (W < 1 || H < 1 || N < 1) return fail(ctx, HIMGCU_REJECT, "bad dimensions");
-  if (!shape_ok(W, H, N)) return fail(ctx, HIMGCU_ERR_UNSUPPORTED, "unsupported shape %dx%dx%d", W, H, N);
-  if (size > 0xffffffffull) return fail(ctx, HIMGCU_ERR_UNSUPPORTED, "stream too large");
-  if (rw < 1 || rh < 1 || x < 0 || y < 0 || x > W - rw || y > H - rh)
-    return fail(ctx, HIMGCU_ERR_ARG, "region %dx%d at (%d, %d) is empty or outside the %dx%d image", rw, rh, x, y, W, H);
-  CK(cudaSetDevice(ctx->device));
-  const Geom g = make_geom(W, H, N, N);
-  const size_t out_bytes = (size_t)rw * rh * N;
-  if (out_bytes > out_cap) return fail(ctx, HIMGCU_ERR_CAPACITY, "output buffer too small");
-  uint8_t *d_in, *d_px;
-  unsigned long long *d_off;
-  uint32_t *d_sz;
-  int *d_status;
-  int32_t *d_org;
-  ENSURE("single_in", size + 16, d_in);
-  ENSURE("single_rpx", out_bytes, d_px);
-  ENSURE("single_off", sizeof(unsigned long long), d_off);
-  ENSURE("single_size", sizeof(uint32_t), d_sz);
-  ENSURE("single_status", sizeof(int), d_status);
-  ENSURE("single_origin", 2 * sizeof(int32_t), d_org);
-  int rc = ensure_pinned(ctx, 64);
-  if (rc) return rc;
-  // offset / size / status / origin travel through the context's page-locked scratch, as in himgcu_decode
-  unsigned long long *h_off = reinterpret_cast<unsigned long long *>(ctx->pinned);
-  uint32_t *h_sz = reinterpret_cast<uint32_t *>(h_off + 1);
-  int *h_status = reinterpret_cast<int *>(h_off + 2);
-  int32_t *h_org = reinterpret_cast<int32_t *>(h_off + 3);
-  CK(cudaStreamSynchronize(ctx->stream));
-  *h_off = 0;
-  *h_sz = (uint32_t)size;
-  h_org[0] = x;
-  h_org[1] = y;
-  if ((rc = copy_to_device(ctx, d_in, himg, size))) return rc;
-  CK(cudaMemcpyAsync(d_off, h_off, sizeof(*h_off), cudaMemcpyHostToDevice, ctx->stream));
-  CK(cudaMemcpyAsync(d_sz, h_sz, sizeof(*h_sz), cudaMemcpyHostToDevice, ctx->stream));
-  CK(cudaMemcpyAsync(d_org, h_org, 2 * sizeof(int32_t), cudaMemcpyHostToDevice, ctx->stream));
-  rc = decode_region_device(ctx, d_in, d_off, d_sz, 1, g, flags, d_org, rw, rh, d_px, d_status);
-  if (rc) return rc;
-  CK(cudaMemcpyAsync(h_status, d_status, sizeof(int), cudaMemcpyDeviceToHost, ctx->stream));
-  if ((rc = copy_to_host(ctx, out, d_px, out_bytes))) return rc;
-  if (*h_status) return fail(ctx, HIMGCU_REJECT, "stream rejected");
-  return HIMGCU_OK;
+  const Rect rect{x, y, rw, rh};
+  return decode_single(ctx, himg, size, flags, 0, &rect, out, out_cap, w, h, nch);
 }
 
 // ---- batch with host buffers -------------------------------------------------------------------
@@ -2190,14 +2015,8 @@ int himgcu_stage_huff_uncompress(himgcu_ctx *ctx, const uint8_t *d_in, size_t in
                                    d_status, &clustered);
     if (rc || clustered) return rc;
   }
-  if (team == 32) {
-    LAUNCH("k_dec_stream", k_dec_stream_par<true>, dim3((nseg + kParWarpTeams - 1) / kParWarpTeams, n), 32 * kParWarpTeams, 0,
-           d_in, d_cd, d_tree, d_seg, nseg, seg, d_out, (unsigned long long)out_stride, d_status);
-  } else {
-    LAUNCH("k_dec_stream", k_dec_stream_par<false>, dim3(nseg, n), team, 0, d_in, d_cd, d_tree, d_seg, nseg, seg, d_out,
-           (unsigned long long)out_stride, d_status);
-  }
-  return HIMGCU_OK;
+  return launch_stream_segments(ctx, "k_dec_stream", team, n, d_in, d_cd, d_tree, d_seg, nseg, seg, d_out,
+                                (unsigned long long)out_stride, d_status);
 }
 
 int himgcu_stage_lres_decode(himgcu_ctx *ctx, const uint8_t *d_lres, size_t lres_stride, int n, int w, int h, int nch,

@@ -777,7 +777,8 @@ __global__ void k_dec_stream_par(const uint8_t *__restrict__ data, const ChunkDe
   } else {
     sr = segs[(size_t)item * nseg + b];
   }
-  if (!T->ok || sr.size == 0xffffffffu || sr.size == 0) {  // an empty stream cannot produce out_seg > 0 bytes
+  // An empty stream produces out_seg > 0 bytes only through a single-leaf tree's 0-bit codes (strict mode)
+  if (!T->ok || sr.size == 0xffffffffu || (sr.size == 0 && !T->single)) {
     if (t == 0) atomicMax(&status[item], 1);
     return;
   }
@@ -822,7 +823,8 @@ __global__ void k_dec_stream_par(const uint8_t *__restrict__ data, const ChunkDe
         if (lit) o[n] = (uint8_t)lit;
         n += z;
       }
-      if (ok) ok = br.pos > 8u * (sr.size - 1) && br.pos <= total_bits;
+      // BitStream::AtTheEnd: the read position lies in the last byte, or at bit 0 of an empty stream
+      if (ok) ok = sr.size == 0 ? br.pos == 0 : (br.pos > 8u * (sr.size - 1) && br.pos <= total_bits);
       if (!ok) atomicMax(&status[item], 1);
     }
     return;

@@ -120,8 +120,8 @@ class Context:
         return out[: n.value].tobytes()
 
     def _decode_single(self, data: bytes, shape, fn, *args):
-        """Body of decode, decode_scaled and decode_region: probes the header, allocates shape(w, h, nch) and calls the
-        C entry point fn with args after the stream.  None where the stream is rejected."""
+        """Body of decode, decode_scaled, decode_region and decode_region_scaled: probes the header, allocates
+        shape(w, h, nch) and calls the C entry point fn with args after the stream.  None where the stream is rejected."""
         buf = np.frombuffer(data, np.uint8)
         w, h, n = C.c_int(), C.c_int(), C.c_int()
         if self.lib.himgcu_decode_info(_ptr(buf), buf.size, C.byref(w), C.byref(h), C.byref(n)) != _native.OK:
@@ -150,6 +150,14 @@ class Context:
         or None where the stream is rejected.  Raises HimgError for an empty rectangle or one outside the image."""
         return self._decode_single(data, lambda W, H, n: (max(h, 1), max(w, 1), n), self.lib.himgcu_decode_region, flags, x, y,
                                    w, h)
+
+    def decode_region_scaled(self, data: bytes, factor: int, x: int, y: int, w: int, h: int, flags=STRICT):
+        """Rectangle [x, x+w) x [y, y+h) of the image at 1/factor size (factor 1, 2, 4 or 8): the [h][w][nch] array
+        equal to decode_scaled(data, factor)[y:y+h, x:x+w], or None where the stream is rejected.  Only the block rows
+        of the source rectangle are entropy-decoded, so the status is that of decode_region on it.  Raises HimgError
+        (ERR_ARG) for another factor, an empty rectangle or one outside the scaled image."""
+        return self._decode_single(data, lambda W, H, n: (max(h, 1), max(w, 1), n), self.lib.himgcu_decode_region_scaled, flags,
+                                   factor, x, y, w, h)
 
     # ---- batch, device tensors --------------------------------------------------------------
     def encode_batch(self, pixels, quality=50, use_ycbcr=True, out=None, sizes=None):
@@ -187,24 +195,31 @@ class Context:
         """himg: CUDA uint8 buffer; offsets int64 [n], sizes int32 [n] (device).  Returns (pixels, status)."""
         return self._decode_batch(self.lib.himgcu_decode_batch, himg, offsets, sizes, w, h, nch, 1, out, status, flags)
 
+    def _decode_batch_region(self, fn, himg, offsets, sizes, dims, origins, crop_w, crop_h, nch, out, status, *args):
+        """Body of the decode_batch_region calls: fn is the C entry point, args its arguments between n and the origins
+        (dims is None for a uniform batch)."""
+        import torch
+
+        n = offsets.numel()
+        for name, t in (("dims", dims), ("origins", origins)):
+            if t is not None and (t.dtype != torch.int32 or t.numel() != 2 * n):
+                raise ValueError(name + " must be an int32 tensor [n][2]")
+        self._bind(himg, offsets, sizes, dims, origins, out, status)
+        if out is None:
+            out = torch.empty((n, crop_h, crop_w, nch), dtype=torch.uint8, device=himg.device)
+        if status is None:
+            status = torch.empty((n,), dtype=torch.int32, device=himg.device)
+        self._check(fn(self.h, _ptr(himg), _ptr(offsets), _ptr(sizes), n, *args, _ptr(origins), crop_w, crop_h, _ptr(out),
+                       _ptr(status)))
+        return out, status
+
     def decode_batch_region(self, himg, offsets, sizes, w, h, nch, origins, crop_w, crop_h, flags=STRICT, out=None,
                             status=None):
         """decode_batch of a crop_w x crop_h rectangle per image: origins is a CUDA int32 [n][2] tensor of (x, y).
         Returns (pixels [n][crop_h][crop_w][nch], status); status[i] is ERR_ARG where the origin puts the
         rectangle outside the image (that image's pixels are not written)."""
-        import torch
-
-        n = offsets.numel()
-        if origins.dtype != torch.int32 or origins.numel() != 2 * n:
-            raise ValueError("origins must be an int32 tensor [n][2]")
-        self._bind(himg, offsets, sizes, origins, out, status)
-        if out is None:
-            out = torch.empty((n, crop_h, crop_w, nch), dtype=torch.uint8, device=himg.device)
-        if status is None:
-            status = torch.empty((n,), dtype=torch.int32, device=himg.device)
-        self._check(self.lib.himgcu_decode_batch_region(self.h, _ptr(himg), _ptr(offsets), _ptr(sizes), n, w, h, nch, flags,
-                                                        _ptr(origins), crop_w, crop_h, _ptr(out), _ptr(status)))
-        return out, status
+        return self._decode_batch_region(self.lib.himgcu_decode_batch_region, himg, offsets, sizes, None, origins, crop_w, crop_h,
+                                         nch, out, status, w, h, nch, flags)
 
     def decode_batch_region_mixed(self, himg, offsets, sizes, dims, nch, origins, crop_w, crop_h, max_w, max_h, flags=STRICT,
                                   out=None, status=None):
@@ -212,21 +227,24 @@ class Context:
         each at most max_w x max_h, and origins one of (x, y).  Returns (pixels [n][crop_h][crop_w][nch], status);
         status[i] is REJECT where the stream is rejected or its shape is not dims[i] x nch, and ERR_ARG where dims[i]
         is < 1 or exceeds the bounds or the origin puts the rectangle outside the image (those pixels are not written)."""
-        import torch
+        return self._decode_batch_region(self.lib.himgcu_decode_batch_region_mixed, himg, offsets, sizes, dims, origins, crop_w,
+                                         crop_h, nch, out, status, _ptr(dims), max_w, max_h, nch, flags)
 
-        n = offsets.numel()
-        for name, t in (("dims", dims), ("origins", origins)):
-            if t.dtype != torch.int32 or t.numel() != 2 * n:
-                raise ValueError(name + " must be an int32 tensor [n][2]")
-        self._bind(himg, offsets, sizes, dims, origins, out, status)
-        if out is None:
-            out = torch.empty((n, crop_h, crop_w, nch), dtype=torch.uint8, device=himg.device)
-        if status is None:
-            status = torch.empty((n,), dtype=torch.int32, device=himg.device)
-        self._check(self.lib.himgcu_decode_batch_region_mixed(self.h, _ptr(himg), _ptr(offsets), _ptr(sizes), n, _ptr(dims), max_w,
-                                                              max_h, nch, flags, _ptr(origins), crop_w, crop_h, _ptr(out),
-                                                              _ptr(status)))
-        return out, status
+    def decode_batch_region_scaled(self, himg, offsets, sizes, w, h, nch, factor, origins, crop_w, crop_h, flags=STRICT, out=None,
+                                   status=None):
+        """decode_batch_region of the images at 1/factor size (factor 1, 2, 4 or 8, see decode_region_scaled): origins
+        and crop_w x crop_h are in the scaled images' coordinates, and crop_w x crop_h must fit ceil(w/f) x ceil(h/f).
+        Returns (pixels [n][crop_h][crop_w][nch], status) with the statuses of decode_batch_region."""
+        return self._decode_batch_region(self.lib.himgcu_decode_batch_region_scaled, himg, offsets, sizes, None, origins, crop_w,
+                                         crop_h, nch, out, status, w, h, nch, flags, factor)
+
+    def decode_batch_region_mixed_scaled(self, himg, offsets, sizes, dims, nch, factor, origins, crop_w, crop_h, max_w, max_h,
+                                         flags=STRICT, out=None, status=None):
+        """decode_batch_region_mixed of the images at 1/factor size: origins are checked against each image's scaled
+        shape, and crop_w x crop_h against ceil(max_w/f) x ceil(max_h/f).  Returns (pixels [n][crop_h][crop_w][nch],
+        status) with the statuses of decode_batch_region_mixed."""
+        return self._decode_batch_region(self.lib.himgcu_decode_batch_region_mixed_scaled, himg, offsets, sizes, dims, origins,
+                                         crop_w, crop_h, nch, out, status, _ptr(dims), max_w, max_h, nch, flags, factor)
 
     def _decode_batch_mixed(self, fn, himg, offsets, sizes, dims, nch, max_w, max_h, factor, out, pixel_offsets, status, *args):
         """Body of decode_batch_mixed (factor None) and decode_batch_mixed_scaled: fn is the C entry point, args its

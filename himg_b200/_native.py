@@ -51,6 +51,14 @@ SIGNATURES = {
                                              C.c_int, C.c_int, _u8p, C.c_void_p]),
     "himgcu_decode_batch_mixed_scaled": (C.c_int, [C.c_void_p, _u8p, C.c_void_p, C.c_void_p, C.c_int, C.c_void_p, C.c_int,
                                                    C.c_int, C.c_int, C.c_int, C.c_int, C.c_void_p, _u8p, C.c_void_p]),
+    "himgcu_decode_region_scaled": (C.c_int, [C.c_void_p, _u8p, C.c_size_t, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int,
+                                              C.c_int, _u8p, C.c_size_t, C.POINTER(C.c_int), C.POINTER(C.c_int),
+                                              C.POINTER(C.c_int)]),
+    "himgcu_decode_batch_region_scaled": (C.c_int, [C.c_void_p, _u8p, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int,
+                                                    C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_int, C.c_int, _u8p, C.c_void_p]),
+    "himgcu_decode_batch_region_mixed_scaled": (C.c_int, [C.c_void_p, _u8p, C.c_void_p, C.c_void_p, C.c_int, C.c_void_p,
+                                                          C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_int,
+                                                          C.c_int, _u8p, C.c_void_p]),
     "himgcu_host_alloc": (C.c_void_p, [C.c_size_t]),
     "himgcu_host_free": (None, [C.c_void_p]),
     "himgcu_encode_batch_host": (C.c_int, [C.c_void_p, _u8p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, _u8p,

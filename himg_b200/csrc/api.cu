@@ -991,14 +991,51 @@ int decode_device(himgcu_ctx *ctx, const uint8_t *d_himg, const unsigned long lo
   return stage_inverse<MIXED>(ctx, d_planes, f.R, n, g, f.tabs, sizeof(DecTables), d_pixels, lf, md, px_off);
 }
 
-// Compact block rows a region decode keeps per image: the most a rectangle of rh rows can touch.
-int region_rows(const Geom &g, int rh) { return std::min((rh + 14) / 8, g.rows); }
+// Compact block rows a region decode keeps per image: the most a rectangle of rh rows can touch.  Scaled by 2^lf, the
+// rectangle reads at most (rh << lf) source rows from a row that is a multiple of 2^lf.
+int region_rows(const Geom &g, int rh, int lf = 0) { return std::min(((rh << lf) + 15 - (1 << lf)) / 8, g.rows); }
 
-// K-inv of a region decode (xform_region.cuh) from the compact planes [n][kr][seg].
+// Lane-pair inverse of a region decode scaled by 2^LF (LF in 1..3): k_inverse_region4_scaled.
+template <int NCH, int LF>
+int launch_inv_region4_scaled(himgcu_ctx *ctx, const uint8_t *d_planes, const uint8_t *d_R, int n, const Geom &g,
+                              const InvTables *d_inv, const int32_t *d_origins, int rw, int rh, int kr, uint8_t *d_pixels) {
+  constexpr int TP = kInv4ThreadsRgb;
+  const int span = region_span_pairs(rw << LF, g.cols);
+  dim3 grid((unsigned)(((long long)kr * span + TP - 1) / TP), 1, n);
+  const int smem = NCH * 64 * 2 * TP + kInvTableBytes;
+  CK(cudaFuncSetAttribute((k_inverse_region4_scaled<NCH, TP, LF>), cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
+  LAUNCH("k_inverse_region4_scaled", (k_inverse_region4_scaled<NCH, TP, LF>), grid, TP, smem, d_planes, d_R, g, d_inv,
+         (unsigned long long)sizeof(InvTables), d_origins, rw, rh, kr, span, d_pixels, 1u);
+  return HIMGCU_OK;
+}
+
+// K-inv of a region decode (xform_region.cuh) from the compact planes [n][kr][seg].  lf > 0 (1..3): the rectangle is
+// one of the image scaled by 2^lf.
 template <bool MIXED = false>
 int stage_inverse_region(himgcu_ctx *ctx, const uint8_t *d_planes, const uint8_t *d_R, int n, const Geom &g,
                          const DecTables *d_tabs, const int32_t *d_origins, int rw, int rh, int kr, uint8_t *d_pixels,
-                         const MixedDims &md = {}) {
+                         const MixedDims &md = {}, int lf = 0) {
+  if (lf) {
+    // lane-pair fast path: the shapes k_inverse4_scaled takes (every window whole), the rectangle clips rows and columns
+    // (the clipped stores take any output alignment)
+    if (!MIXED && lane_pair_ok(ctx, g, d_planes, d_R, d_pixels, 1u)) {
+      InvTables *d_inv;
+      int rc = launch_inv_tables(ctx, d_tabs, n, (unsigned long long)sizeof(DecTables), &d_inv);
+      if (rc) return rc;
+      switch (g.nch * 4 + lf) {
+        case 1 * 4 + 1: return launch_inv_region4_scaled<1, 1>(ctx, d_planes, d_R, n, g, d_inv, d_origins, rw, rh, kr, d_pixels);
+        case 1 * 4 + 2: return launch_inv_region4_scaled<1, 2>(ctx, d_planes, d_R, n, g, d_inv, d_origins, rw, rh, kr, d_pixels);
+        case 1 * 4 + 3: return launch_inv_region4_scaled<1, 3>(ctx, d_planes, d_R, n, g, d_inv, d_origins, rw, rh, kr, d_pixels);
+        case 3 * 4 + 1: return launch_inv_region4_scaled<3, 1>(ctx, d_planes, d_R, n, g, d_inv, d_origins, rw, rh, kr, d_pixels);
+        case 3 * 4 + 2: return launch_inv_region4_scaled<3, 2>(ctx, d_planes, d_R, n, g, d_inv, d_origins, rw, rh, kr, d_pixels);
+        default: return launch_inv_region4_scaled<3, 3>(ctx, d_planes, d_R, n, g, d_inv, d_origins, rw, rh, kr, d_pixels);
+      }
+    }
+    const int kb = ((rw << lf) + 15 - (1 << lf)) / 8;
+    LAUNCH("k_inverse_region_scaled", k_inverse_region_scaled<MIXED>, dim3((kb + kTile - 1) / kTile, kr, n), kTile, 0, d_planes, d_R,
+           g, d_tabs, (unsigned long long)sizeof(DecTables), d_origins, rw, rh, kr, lf, d_pixels, md);
+    return HIMGCU_OK;
+  }
   // lane-pair fast path: the shapes k_inverse4 takes, except that the rectangle clips rows and columns
   if (!MIXED && !ctx->force_generic && (g.cols % 16) == 0 && (g.nch == 1 || g.nch == 3) &&
       (reinterpret_cast<uintptr_t>(d_planes) & 15) == 0 && (reinterpret_cast<uintptr_t>(d_R) & 1) == 0) {
@@ -1029,12 +1066,13 @@ int stage_inverse_region(himgcu_ctx *ctx, const uint8_t *d_planes, const uint8_t
 
 // Region decode of n streams resident on the device: image i's rectangle rw x rh at (d_origins[2i], d_origins[2i+1])
 // to d_pixels + i * rw * rh * nch.  Only the FRES segments of the block rows the rectangle touches are decoded.
+// lf > 0: the rectangle is one of the image scaled by 2^lf, and the rows are those of the source pixels it reads.
 template <bool MIXED = false>
 int decode_region_device(himgcu_ctx *ctx, const uint8_t *d_himg, const unsigned long long *d_offsets, const uint32_t *d_sizes,
                          int n, const Geom &g, int flags, const int32_t *d_origins, int rw, int rh, uint8_t *d_pixels,
-                         int *d_status, const MixedDims &md = {}) {
+                         int *d_status, const MixedDims &md = {}, int lf = 0) {
   const int lenient = (flags & HIMGCU_LENIENT) ? 1 : 0;
-  const int kr = region_rows(g, rh);
+  const int kr = region_rows(g, rh, lf);
   uint8_t *d_planes;
   SegRef *d_rseg;
   ENSURE("planes", (size_t)n * kr * g.seg, d_planes);
@@ -1042,14 +1080,18 @@ int decode_region_device(himgcu_ctx *ctx, const uint8_t *d_himg, const unsigned 
   DecFront f;
   int rc = decode_front<MIXED>(ctx, d_himg, d_offsets, d_sizes, n, g, lenient, d_status, &f, md);
   if (rc) return rc;
-  LAUNCH("k_dec_segtab_region", k_dec_segtab_region<MIXED>, (unsigned)((n + 127) / 128), 128, 0, d_himg, f.fcd, f.ftree, n, g,
-         lenient, d_origins, rw, rh, kr, f.fseg, d_rseg, d_status, md);
+  if (lf)
+    LAUNCH("k_dec_segtab_region", k_dec_segtab_region_scaled<MIXED>, (unsigned)((n + 127) / 128), 128, 0, d_himg, f.fcd, f.ftree,
+           n, g, lenient, d_origins, rw, rh, kr, lf, f.fseg, d_rseg, d_status, md);
+  else
+    LAUNCH("k_dec_segtab_region", k_dec_segtab_region<MIXED>, (unsigned)((n + 127) / 128), 128, 0, d_himg, f.fcd, f.ftree, n, g,
+           lenient, d_origins, rw, rh, kr, f.fseg, d_rseg, d_status, md);
   const int team = decode_team((long long)n * kr, g.seg, kParFresThreads);
   rc = launch_stream_segments<MIXED ? kMixFres : 0>(ctx, "k_dec_stream_fres", team, n, d_himg, f.fcd, f.ftree, d_rseg, kr, g.seg,
                                                      d_planes, (unsigned long long)kr * g.seg, d_status, md);
   if (rc) return rc;
   if (f.fork) CK(cudaStreamWaitEvent(ctx->stream, ctx->ev_join, 0));
-  return stage_inverse_region<MIXED>(ctx, d_planes, f.R, n, g, f.tabs, d_origins, rw, rh, kr, d_pixels, md);
+  return stage_inverse_region<MIXED>(ctx, d_planes, f.R, n, g, f.tabs, d_origins, rw, rh, kr, d_pixels, md, lf);
 }
 
 // Runs body(i0, m) over the sub-batches [i0, i0 + m) of n images: as many images as fit max_workspace_bytes at `per`
@@ -1532,22 +1574,25 @@ int decode_batch_lf(himgcu_ctx *ctx, const uint8_t *d_himg, const uint64_t *d_of
   });
 }
 
-// himgcu_decode_batch_region, and with MIXED himgcu_decode_batch_region_mixed, whose w x h are the bounds of the images.
+// himgcu_decode_batch_region(_scaled), and with MIXED himgcu_decode_batch_region_mixed(_scaled), whose w x h are the
+// bounds of the images.  lf > 0: the rectangles are those of the images scaled by 2^lf, and rw x rh must fit the
+// scaled bounds.
 template <bool MIXED>
 int decode_batch_region(himgcu_ctx *ctx, const uint8_t *d_himg, const uint64_t *d_offsets, const uint32_t *d_sizes, int n,
-                        const int32_t *d_dims, int w, int h, int nch, int flags, const int32_t *d_origins, int rw, int rh,
+                        const int32_t *d_dims, int w, int h, int nch, int flags, int lf, const int32_t *d_origins, int rw, int rh,
                         uint8_t *d_pixels_out, int32_t *d_status) {
   if (!ctx || !d_himg || !d_offsets || !d_sizes || (MIXED && !d_dims) || !d_origins || !d_pixels_out || !d_status || n < 0)
     return fail(ctx, HIMGCU_ERR_ARG, "bad argument");
   if (!shape_ok(w, h, nch))
     return fail(ctx, HIMGCU_ERR_UNSUPPORTED, "unsupported %sshape %dx%dx%d", MIXED ? "bounding " : "", w, h, nch);
-  if (rw < 1 || rh < 1 || rw > w || rh > h)
+  const int sw = (w + (1 << lf) - 1) >> lf, sh = (h + (1 << lf) - 1) >> lf;  // the (scaled) bounds of a rectangle
+  if (rw < 1 || rh < 1 || rw > sw || rh > sh)
     return fail(ctx, HIMGCU_ERR_ARG, MIXED ? "region %dx%d does not fit the %dx%d bounds" : "region %dx%d does not fit a %dx%d image",
-                rw, rh, w, h);
+                rw, rh, sw, sh);
   if (n == 0) return HIMGCU_OK;
   CK(cudaSetDevice(ctx->device));
   const Geom g = make_geom(w, h, nch, nch);
-  const int kr = region_rows(g, rh);
+  const int kr = region_rows(g, rh, lf);
   const size_t out_bytes = (size_t)rw * rh * nch;
   // (the uniform count includes the tables of the lane-pair inverse, which a mixed batch does not take)
   const size_t per = per_image_encode_ws(g) - g.planes_bytes + (size_t)kr * (g.seg + sizeof(SegRef)) + sizeof(DecTables) +
@@ -1556,7 +1601,7 @@ int decode_batch_region(himgcu_ctx *ctx, const uint8_t *d_himg, const uint64_t *
     const MixedDims md = MIXED ? MixedDims{d_dims + 2 * (size_t)i0, w, h, nch} : MixedDims{};
     return decode_region_device<MIXED>(ctx, d_himg, reinterpret_cast<const unsigned long long *>(d_offsets) + i0, d_sizes + i0, m,
                                        g, flags, d_origins + 2 * (size_t)i0, rw, rh, d_pixels_out + (size_t)i0 * out_bytes,
-                                       d_status + i0, md);
+                                       d_status + i0, md, lf);
   });
 }
 
@@ -1565,7 +1610,7 @@ struct Rect {
 };
 
 // himgcu_decode, himgcu_decode_scaled (lf > 0, out_cap is checked against the scaled size) and, with `rect`,
-// himgcu_decode_region.
+// himgcu_decode_region(_scaled) (a rectangle of the image scaled by 2^lf).
 int decode_single(himgcu_ctx *ctx, const uint8_t *himg, size_t size, int flags, int lf, const Rect *rect, uint8_t *out,
                   size_t out_cap, int *w, int *h, int *nch) {
   if (!ctx || !himg || !out) return fail(ctx, HIMGCU_ERR_ARG, "bad argument");
@@ -1577,9 +1622,10 @@ int decode_single(himgcu_ctx *ctx, const uint8_t *himg, size_t size, int flags, 
   if (W < 1 || H < 1 || N < 1) return fail(ctx, HIMGCU_REJECT, "bad dimensions");
   if (!shape_ok(W, H, N)) return fail(ctx, HIMGCU_ERR_UNSUPPORTED, "unsupported shape %dx%dx%d", W, H, N);
   if (size > 0xffffffffull) return fail(ctx, HIMGCU_ERR_UNSUPPORTED, "stream too large");
-  if (rect && (rect->w < 1 || rect->h < 1 || rect->x < 0 || rect->y < 0 || rect->x > W - rect->w || rect->y > H - rect->h))
+  const int SW = (W + (1 << lf) - 1) >> lf, SH = (H + (1 << lf) - 1) >> lf;  // the scaled image
+  if (rect && (rect->w < 1 || rect->h < 1 || rect->x < 0 || rect->y < 0 || rect->x > SW - rect->w || rect->y > SH - rect->h))
     return fail(ctx, HIMGCU_ERR_ARG, "region %dx%d at (%d, %d) is empty or outside the %dx%d image", rect->w, rect->h, rect->x,
-                rect->y, W, H);
+                rect->y, SW, SH);
   CK(cudaSetDevice(ctx->device));
   const Geom g = make_geom(W, H, N, N);
   const size_t out_bytes = rect ? (size_t)rect->w * rect->h * N : scaled_bytes(g, lf);
@@ -1614,7 +1660,7 @@ int decode_single(himgcu_ctx *ctx, const uint8_t *himg, size_t size, int flags, 
   CK(cudaMemcpyAsync(d_sz, h_sz, sizeof(*h_sz), cudaMemcpyHostToDevice, ctx->stream));
   if (rect) {
     CK(cudaMemcpyAsync(d_org, h_org, 2 * sizeof(int32_t), cudaMemcpyHostToDevice, ctx->stream));
-    rc = decode_region_device(ctx, d_in, d_off, d_sz, 1, g, flags, d_org, rect->w, rect->h, d_px, d_status);
+    rc = decode_region_device(ctx, d_in, d_off, d_sz, 1, g, flags, d_org, rect->w, rect->h, d_px, d_status, {}, lf);
   } else {
     rc = decode_device(ctx, d_in, d_off, d_sz, 1, g, flags, d_px, d_status, lf);
   }
@@ -1734,21 +1780,48 @@ int himgcu_decode_scaled(himgcu_ctx *ctx, const uint8_t *himg, size_t size, int 
 int himgcu_decode_batch_region(himgcu_ctx *ctx, const uint8_t *d_himg, const uint64_t *d_offsets, const uint32_t *d_sizes, int n,
                                int w, int h, int nch, int flags, const int32_t *d_origins, int rw, int rh, uint8_t *d_pixels_out,
                                int32_t *d_status) {
-  return decode_batch_region<false>(ctx, d_himg, d_offsets, d_sizes, n, nullptr, w, h, nch, flags, d_origins, rw, rh, d_pixels_out,
-                                    d_status);
+  return decode_batch_region<false>(ctx, d_himg, d_offsets, d_sizes, n, nullptr, w, h, nch, flags, 0, d_origins, rw, rh,
+                                    d_pixels_out, d_status);
+}
+
+int himgcu_decode_batch_region_scaled(himgcu_ctx *ctx, const uint8_t *d_himg, const uint64_t *d_offsets, const uint32_t *d_sizes,
+                                      int n, int w, int h, int nch, int flags, int factor, const int32_t *d_origins, int rw, int rh,
+                                      uint8_t *d_pixels_out, int32_t *d_status) {
+  const int lf = scale_log2(factor);
+  if (lf < 0) return fail(ctx, HIMGCU_ERR_ARG, "scale factor %d is not 1, 2, 4 or 8", factor);
+  return decode_batch_region<false>(ctx, d_himg, d_offsets, d_sizes, n, nullptr, w, h, nch, flags, lf, d_origins, rw, rh,
+                                    d_pixels_out, d_status);
 }
 
 int himgcu_decode_batch_region_mixed(himgcu_ctx *ctx, const uint8_t *d_himg, const uint64_t *d_offsets, const uint32_t *d_sizes,
                                      int n, const int32_t *d_dims, int max_width, int max_height, int nch, int flags,
                                      const int32_t *d_origins, int rw, int rh, uint8_t *d_pixels_out, int32_t *d_status) {
-  return decode_batch_region<true>(ctx, d_himg, d_offsets, d_sizes, n, d_dims, max_width, max_height, nch, flags, d_origins, rw, rh,
-                                   d_pixels_out, d_status);
+  return decode_batch_region<true>(ctx, d_himg, d_offsets, d_sizes, n, d_dims, max_width, max_height, nch, flags, 0, d_origins, rw,
+                                   rh, d_pixels_out, d_status);
+}
+
+int himgcu_decode_batch_region_mixed_scaled(himgcu_ctx *ctx, const uint8_t *d_himg, const uint64_t *d_offsets,
+                                            const uint32_t *d_sizes, int n, const int32_t *d_dims, int max_width, int max_height,
+                                            int nch, int flags, int factor, const int32_t *d_origins, int rw, int rh,
+                                            uint8_t *d_pixels_out, int32_t *d_status) {
+  const int lf = scale_log2(factor);
+  if (lf < 0) return fail(ctx, HIMGCU_ERR_ARG, "scale factor %d is not 1, 2, 4 or 8", factor);
+  return decode_batch_region<true>(ctx, d_himg, d_offsets, d_sizes, n, d_dims, max_width, max_height, nch, flags, lf, d_origins, rw,
+                                   rh, d_pixels_out, d_status);
 }
 
 int himgcu_decode_region(himgcu_ctx *ctx, const uint8_t *himg, size_t size, int flags, int x, int y, int rw, int rh, uint8_t *out,
                          size_t out_cap, int *w, int *h, int *nch) {
   const Rect rect{x, y, rw, rh};
   return decode_single(ctx, himg, size, flags, 0, &rect, out, out_cap, w, h, nch);
+}
+
+int himgcu_decode_region_scaled(himgcu_ctx *ctx, const uint8_t *himg, size_t size, int flags, int factor, int x, int y, int rw,
+                                int rh, uint8_t *out, size_t out_cap, int *w, int *h, int *nch) {
+  const int lf = scale_log2(factor);
+  if (lf < 0) return fail(ctx, HIMGCU_ERR_ARG, "scale factor %d is not 1, 2, 4 or 8", factor);
+  const Rect rect{x, y, rw, rh};
+  return decode_single(ctx, himg, size, flags, lf, &rect, out, out_cap, w, h, nch);
 }
 
 // ---- batch with host buffers -------------------------------------------------------------------

@@ -107,6 +107,17 @@ __device__ __forceinline__ bool region_origin(const int32_t *__restrict__ origin
   return x >= 0 && y >= 0 && x <= g.w - rw && y <= g.h - rh;
 }
 
+// Scaled region decode (factor 2^lf): origin (x, y) of image i's rw x rh rectangle of the scaled image
+// [ceil(h / 2^lf)][ceil(w / 2^lf)].  The rectangle reads the source pixels [x << lf, min((x + rw) << lf, w)) x
+// [y << lf, min((y + rh) << lf, h)).  False when it does not lie inside the scaled image.
+__device__ __forceinline__ bool region_origin_scaled(const int32_t *__restrict__ origins, int i, const Geom &g, int lf, int rw,
+                                                     int rh, int &x, int &y) {
+  x = origins[2 * i];
+  y = origins[2 * i + 1];
+  const int f = 1 << lf;
+  return x >= 0 && y >= 0 && x <= ((g.w + f - 1) >> lf) - rw && y <= ((g.h + f - 1) >> lf) - rh;
+}
+
 // Sequency-ordered 8-point Walsh-Hadamard butterflies (hadamard.cpp:18-44), in place.
 __device__ __forceinline__ void wht8(int &x0, int &x1, int &x2, int &x3, int &x4, int &x5, int &x6,
                                      int &x7) {

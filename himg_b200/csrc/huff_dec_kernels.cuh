@@ -554,27 +554,48 @@ __global__ void k_dec_segtab_mixed(const uint8_t *__restrict__ data, const Chunk
 // the image makes the image's status 2 (HIMGCU_ERR_ARG) and all its entries invalid.
 // MIXED: g is the bounding geometry (the stride of `full`); image i's header chain and origin are those of its own
 // geometry from `md`, and dims out of bounds are treated as an origin outside the image.
-template <bool MIXED = false>
-__global__ void k_dec_segtab_region(const uint8_t *__restrict__ data, const ChunkDesc *__restrict__ cd,
-                                    const DecTree *__restrict__ trees, int n, Geom g, int lenient,
-                                    const int32_t *__restrict__ origins, int rw, int rh, int kr,
-                                    SegRef *__restrict__ full, SegRef *__restrict__ segs, int *__restrict__ status,
-                                    MixedDims md = {}) {
+// SCALED (k_dec_segtab_region_scaled): the rectangle is one of the image scaled by 2^lf (region_origin_scaled), and
+// the rows are those of the source pixels it reads.
+template <bool MIXED, bool SCALED>
+__device__ __forceinline__ void segtab_region(const uint8_t *__restrict__ data, const ChunkDesc *__restrict__ cd,
+                                              const DecTree *__restrict__ trees, int n, const Geom &g, int lenient,
+                                              const int32_t *__restrict__ origins, int rw, int rh, int kr,
+                                              SegRef *__restrict__ full, SegRef *__restrict__ segs, int *__restrict__ status,
+                                              const MixedDims &md, int lf) {
   const int i = blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= n) return;
   SegRef *S = segs + (size_t)i * kr;
   Geom gi = g;
   const bool dims_ok = !MIXED || image_geom(md, i, gi);
   int x, y;
-  if (!dims_ok || !region_origin(origins, i, gi, rw, rh, x, y)) {
+  if (!dims_ok || !(SCALED ? region_origin_scaled(origins, i, gi, lf, rw, rh, x, y) : region_origin(origins, i, gi, rw, rh, x, y))) {
     for (int k = 0; k < kr; ++k) seg_store<false>(S + k, 0, 0xffffffffu);
     atomicMax(status + i, 2);
     return;
   }
-  const int r0 = y >> 3, r1 = (y + rh - 1) >> 3;
+  const int r0 = SCALED ? (y << lf) >> 3 : y >> 3;
+  const int r1 = SCALED ? (min((y + rh) << lf, gi.h) - 1) >> 3 : (y + rh - 1) >> 3;
   SegRef *F = full + (size_t)i * g.rows;
   segtab_walk<false>(data, cd[i], trees + i, gi.rows > 1 ? max(r1 + 1, 2) : 1, gi.seg, 1, lenient, F, status + i);
   for (int k = 0; k < kr; ++k) S[k] = F[min(r0 + k, r1)];
+}
+
+template <bool MIXED = false>
+__global__ void k_dec_segtab_region(const uint8_t *__restrict__ data, const ChunkDesc *__restrict__ cd,
+                                    const DecTree *__restrict__ trees, int n, Geom g, int lenient,
+                                    const int32_t *__restrict__ origins, int rw, int rh, int kr,
+                                    SegRef *__restrict__ full, SegRef *__restrict__ segs, int *__restrict__ status,
+                                    MixedDims md = {}) {
+  segtab_region<MIXED, false>(data, cd, trees, n, g, lenient, origins, rw, rh, kr, full, segs, status, md, 0);
+}
+
+template <bool MIXED = false>
+__global__ void k_dec_segtab_region_scaled(const uint8_t *__restrict__ data, const ChunkDesc *__restrict__ cd,
+                                           const DecTree *__restrict__ trees, int n, Geom g, int lenient,
+                                           const int32_t *__restrict__ origins, int rw, int rh, int kr, int lf,
+                                           SegRef *__restrict__ full, SegRef *__restrict__ segs, int *__restrict__ status,
+                                           MixedDims md = {}) {
+  segtab_region<MIXED, true>(data, cd, trees, n, g, lenient, origins, rw, rh, kr, full, segs, status, md, lf);
 }
 
 // ---- subsequence-parallel stream decode ---------------------------------------------------------

@@ -228,6 +228,44 @@ int himgcu_decode_batch_mixed_scaled(himgcu_ctx *ctx, const uint8_t *d_himg, con
                                      int max_height, int num_channels, int flags, int factor,
                                      const uint64_t *d_pixel_offsets, uint8_t *d_pixels_out, int32_t *d_status);
 
+/* ---- scaled region decode: a rectangle of the image at 1/factor size ----------------------------
+ * The rectangle [x, x+rw) x [y, y+rh) is given in the coordinates of the SCALED image: for f in {1, 2, 4, 8} and
+ * S = what himgcu_decode_scaled gives for the stream with the same flags and factor ([ceil(H/f)][ceil(W/f)][nch]),
+ *     out[yy][xx][c] = S[y + yy][x + xx][c]
+ * and the output is [rh][rw][num_channels], tightly packed (edge windows are clipped as in the scaled calls).  The
+ * call reads exactly what himgcu_decode_region reads for the source rectangle (f*x, f*y, min(f*rw, W - f*x),
+ * min(f*rh, H - f*y)), and its status is that call's: a stream the whole decode accepts is accepted, and a stream whose
+ * corruption lies only below the rectangle's last block row may decode.  f = 1 is exactly the unscaled region call.
+ * Any other factor is HIMGCU_ERR_ARG.
+ *
+ * Single image, host buffers (as himgcu_decode_region): width / height / num_channels receive the stream's FULL
+ * shape; HIMGCU_ERR_ARG for an empty rectangle or one outside the scaled image; out_cap is checked against
+ * rw*rh*num_channels. */
+int himgcu_decode_region_scaled(himgcu_ctx *ctx, const uint8_t *himg, size_t size, int flags, int factor, int x, int y,
+                                int rw, int rh, uint8_t *out, size_t out_cap, int *width, int *height,
+                                int *num_channels);
+
+/* himgcu_decode_batch_region at 1/factor size: rw x rh is checked here against ceil(width/f) x ceil(height/f)
+ * (HIMGCU_ERR_ARG), and d_status[i] is HIMGCU_ERR_ARG if image i's origin puts the rectangle outside the scaled image
+ * (nothing of it is written).  Image i's rectangle goes to d_pixels_out + i*rw*rh*num_channels.  Otherwise as
+ * himgcu_decode_batch_region, plus HIMGCU_ERR_ARG for a bad factor. */
+int himgcu_decode_batch_region_scaled(himgcu_ctx *ctx, const uint8_t *d_himg, const uint64_t *d_offsets,
+                                      const uint32_t *d_sizes, int n, int width, int height, int num_channels,
+                                      int flags, int factor, const int32_t *d_origins, int rw, int rh,
+                                      uint8_t *d_pixels_out, int32_t *d_status);
+
+/* himgcu_decode_batch_region_mixed at 1/factor size: rw x rh is checked against ceil(max_width/f) x
+ * ceil(max_height/f), origins against image i's scaled shape.  Image i's rectangle goes to d_pixels_out +
+ * i*rw*rh*num_channels.  Per-image statuses (HIMGCU_ERR_ARG for dims out of bounds or an origin outside the scaled
+ * image, HIMGCU_REJECT for a FRMT shape other than the dims) as himgcu_decode_batch_region_mixed, plus HIMGCU_ERR_ARG
+ * for a bad factor.  A batch whose dims are all equal gives what himgcu_decode_batch_region_scaled gives.  The inverse
+ * transform is always the generic kernel. */
+int himgcu_decode_batch_region_mixed_scaled(himgcu_ctx *ctx, const uint8_t *d_himg, const uint64_t *d_offsets,
+                                            const uint32_t *d_sizes, int n, const int32_t *d_dims, int max_width,
+                                            int max_height, int num_channels, int flags, int factor,
+                                            const int32_t *d_origins, int rw, int rh, uint8_t *d_pixels_out,
+                                            int32_t *d_status);
+
 /* ---- batch, HOST pointers (what a file/stream based caller uses; basis of the e2e figure) ----
  * Same work as the device batch calls with the transfers included: pixels (or bitstreams) are
  * copied host->device in sub-batches, coded, and the results copied back.  Pinned host memory

@@ -33,13 +33,15 @@ sys.path.insert(0, ROOT)
 
 
 def compare(a, b):
-    ra = [json.loads(x) for x in open(os.path.join(a, "trace.jsonl"))]
-    rb = [json.loads(x) for x in open(os.path.join(b, "trace.jsonl"))]
-    bad = [x["call"] for x, y in zip(ra, rb) if x != y]
-    if len(ra) != len(rb):
-        bad.append(f"record count {len(ra)} != {len(rb)}")
-    print(json.dumps({"calls": len(ra), "mismatches": bad}))
-    return 1 if bad else 0
+    """Compares the records of the calls both files have.  A call of the first file missing from the second fails, as a
+    mismatch does; calls only the second file has (new entry points) are listed."""
+    ra = {r["call"]: r for r in map(json.loads, open(os.path.join(a, "trace.jsonl")))}
+    rb = {r["call"]: r for r in map(json.loads, open(os.path.join(b, "trace.jsonl")))}
+    both = [k for k in ra if k in rb]
+    bad = [k for k in both if ra[k] != rb[k]]
+    print(json.dumps({"calls": len(both), "mismatches": bad, "only_a": [k for k in ra if k not in rb],
+                      "only_b": [k for k in rb if k not in ra]}))
+    return 1 if bad or any(k not in rb for k in ra) else 0
 
 
 def main():
@@ -119,6 +121,10 @@ def main():
         for f in (2, 4, 8):
             add(f"decode_scaled/{k}/f{f}", lambda ctx, k=k, f=f: ctx.decode_scaled(streams[k], f))
         add(f"decode_region/{k}", lambda ctx, k=k, w=w, h=h: ctx.decode_region(streams[k], w // 5, h // 7, w // 2, h // 3))
+        for f in (1, 2, 4, 8):
+            sw, sh = -(-w // f), -(-h // f)
+            add(f"decode_region_scaled/{k}/f{f}", lambda ctx, k=k, f=f, sw=sw, sh=sh: ctx.decode_region_scaled(
+                streams[k], f, sw // 5, sh // 7, max(1, sw // 2), max(1, sh // 3)))
         add(f"encode/{k}", lambda ctx, k=k: ctx.encode(host_img[k], 50, True))
 
     def decode_batch(ctx, k, n, f=None, off=0):
@@ -150,17 +156,27 @@ def main():
     for f in (1, 2, 4, 8):
         add(f"decode_batch_mixed_scaled/f{f}", lambda ctx, f=f: decode_mixed(ctx, f))
 
-    def region_batch(ctx, k, n):
+    def region_batch(ctx, k, n, f=None):
         w, h, c = shapes[k]
+        if f is not None:  # (a rectangle of the image scaled by f)
+            w, h = -(-w // f), -(-h // f)
         cw, ch = min(224, w // 2), min(224, h // 2)
         himg, offs, sizes = batch(k, n)
         org = torch.tensor([[(37 * i) % (w - cw + 1), (23 * i) % (h - ch + 1)] for i in range(n)], dtype=torch.int32, device=dev)
+        if f is not None:
+            return ctx.decode_batch_region_scaled(himg, offs, sizes, *shapes[k], f, org, cw, ch)
         return ctx.decode_batch_region(himg, offs, sizes, w, h, c, org, cw, ch)
 
     for k, n in (("1080p", 64), ("1080p", 2), ("gray1024", 2), ("rgba512", 2), ("odd", 2), ("ch5", 2)):
         add(f"decode_batch_region/{k}/n{n}", lambda ctx, k=k, n=n: region_batch(ctx, k, n))
     add("decode_batch_region_mixed", lambda ctx: ctx.decode_batch_region_mixed(
         mhimg, mhoffs, msizes, mdims, 3, torch.zeros((len(mixed_dims), 2), dtype=torch.int32, device=dev), 64, 48, 1920, 1080))
+    for f in (1, 2, 4, 8):
+        for k, n in (("1080p", 64), ("1080p", 2), ("gray1024", 2), ("rgba512", 2), ("odd", 2), ("ch5", 2)):
+            add(f"decode_batch_region_scaled/{k}/n{n}/f{f}", lambda ctx, k=k, n=n, f=f: region_batch(ctx, k, n, f))
+        add(f"decode_batch_region_mixed_scaled/f{f}", lambda ctx, f=f: ctx.decode_batch_region_mixed_scaled(
+            mhimg, mhoffs, msizes, mdims, 3, f, torch.zeros((len(mixed_dims), 2), dtype=torch.int32, device=dev), 64 // f, 48 // f,
+            1920, 1080))
 
     for k, n in (("1080p", 64), ("1080p", 2), ("4k", 2), ("8kgray", 1), ("oddw", 2), ("odd", 2), ("ch5", 2), ("rgba512", 2),
                  ("gray1024", 2), ("rgb512", 2)):
@@ -209,6 +225,8 @@ def main():
         "decode/1080p", "decode/gray1024", "decode_scaled/1080p/f2", "decode_region/1080p", "encode/1080p", "encode/gray1024",
         "decode_batch/1080p/n64", "decode_batch/1080p/n2", "decode_batch_scaled/1080p/n64/f2", "decode_batch/rgba512/n2",
         "decode_batch_region/1080p/n64", "decode_batch_region/1080p/n2", "decode_batch_mixed", "decode_batch_region_mixed",
+        "decode_region_scaled/1080p/f2", "decode_batch_region_scaled/1080p/n64/f2", "decode_batch_region_scaled/gray1024/n2/f4",
+        "decode_batch_region_mixed_scaled/f2",
         "encode_batch/1080p/n64", "encode_batch/1080p/n2", "encode_batch/4k/n2", "encode_batch/8kgray/n1", "encode_batch_mixed",
         "stage_lowres/1080p", "stage_forward/1080p", "stage_inverse/1080p", "stage_huff_compress/bs4096",
         "stage_huff_uncompress/bs0", "stage_huff_uncompress/bs4096")]

@@ -340,6 +340,25 @@ int for_channel_groups(int nch, bool ycbcr, F &&launch) {
   return rc;
 }
 
+template <int N>
+using Lf = std::integral_constant<int, N>;
+
+// Calls launch(Nch<NCH>(), Lf<LF>()) for the shapes of the lane-pair kernels: nch 1 or 3, a decode scaled by 2^lf with
+// lf 0..3.
+template <class F>
+int for_lane_pair_shape(int nch, int lf, F &&launch) {
+  switch (nch * 4 + lf) {
+    case 1 * 4 + 0: return launch(Nch<1>(), Lf<0>());
+    case 1 * 4 + 1: return launch(Nch<1>(), Lf<1>());
+    case 1 * 4 + 2: return launch(Nch<1>(), Lf<2>());
+    case 1 * 4 + 3: return launch(Nch<1>(), Lf<3>());
+    case 3 * 4 + 0: return launch(Nch<3>(), Lf<0>());
+    case 3 * 4 + 1: return launch(Nch<3>(), Lf<1>());
+    case 3 * 4 + 2: return launch(Nch<3>(), Lf<2>());
+    default: return launch(Nch<3>(), Lf<3>());
+  }
+}
+
 template <int NCH>
 int launch_avg2(himgcu_ctx *ctx, const uint8_t *d_pixels, int n, const Geom &g, bool ycbcr, uint8_t *d_avg) {
   Avg2Params P;
@@ -510,7 +529,7 @@ int launch_inv_tables(himgcu_ctx *ctx, const DecTables *d_tabs, int ntab, unsign
   return HIMGCU_OK;
 }
 
-// Lane-pair inverse: k_inverse4, or at LF > 0 k_inverse4_scaled (a decode scaled by 2^LF, same shapes and tiles).
+// Lane-pair inverse of a whole-image decode scaled by 2^LF (LF = 0: unscaled): k_inverse4.
 template <int NCH, int LF>
 int launch_inv4(himgcu_ctx *ctx, const uint8_t *d_planes, const uint8_t *d_R, int n, const Geom &g,
                 const DecTables *d_tabs, unsigned long long tab_stride, uint8_t *d_pixels) {
@@ -523,14 +542,9 @@ int launch_inv4(himgcu_ctx *ctx, const uint8_t *d_planes, const uint8_t *d_R, in
   constexpr int TP = NCH == 1 ? kInv4ThreadsGray : kInv4ThreadsRgb;
   dim3 grid((total_pairs + TP - 1) / TP, 1, n);
   const int smem = NCH * 64 * 2 * TP + kInvTableBytes;
-  if constexpr (LF == 0) {
-    CK(cudaFuncSetAttribute((k_inverse4<NCH, TP>), cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
-    LAUNCH("k_inverse", (k_inverse4<NCH, TP>), grid, TP, smem, d_planes, d_R, g, d_inv, inv_stride, d_pixels, 1u);
-  } else {
-    CK(cudaFuncSetAttribute((k_inverse4_scaled<NCH, TP, LF>), cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
-    LAUNCH("k_inverse4_scaled", (k_inverse4_scaled<NCH, TP, LF>), grid, TP, smem, d_planes, d_R, g, d_inv, inv_stride, d_pixels,
-           1u);
-  }
+  CK(cudaFuncSetAttribute((k_inverse4<NCH, TP, LF>), cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
+  LAUNCH(LF == 0 ? "k_inverse" : "k_inverse4_scaled", (k_inverse4<NCH, TP, LF>), grid, TP, smem, d_planes, d_R, g, d_inv,
+         inv_stride, d_pixels, 1u);
   return HIMGCU_OK;
 }
 
@@ -550,16 +564,9 @@ int stage_inverse(himgcu_ctx *ctx, const uint8_t *d_planes, const uint8_t *d_R, 
                   const MixedDims &md = {}, const unsigned long long *px_off = nullptr) {
   // lane-pair fast path: two blocks per thread, flat tiles, pixel stores 16 >> lf bytes wide
   if (!MIXED && lane_pair_ok(ctx, g, d_planes, d_R, d_pixels, 16u >> lf)) {
-    switch (g.nch * 4 + lf) {
-      case 1 * 4 + 0: return launch_inv4<1, 0>(ctx, d_planes, d_R, n, g, d_tabs, tab_stride, d_pixels);
-      case 1 * 4 + 1: return launch_inv4<1, 1>(ctx, d_planes, d_R, n, g, d_tabs, tab_stride, d_pixels);
-      case 1 * 4 + 2: return launch_inv4<1, 2>(ctx, d_planes, d_R, n, g, d_tabs, tab_stride, d_pixels);
-      case 1 * 4 + 3: return launch_inv4<1, 3>(ctx, d_planes, d_R, n, g, d_tabs, tab_stride, d_pixels);
-      case 3 * 4 + 0: return launch_inv4<3, 0>(ctx, d_planes, d_R, n, g, d_tabs, tab_stride, d_pixels);
-      case 3 * 4 + 1: return launch_inv4<3, 1>(ctx, d_planes, d_R, n, g, d_tabs, tab_stride, d_pixels);
-      case 3 * 4 + 2: return launch_inv4<3, 2>(ctx, d_planes, d_R, n, g, d_tabs, tab_stride, d_pixels);
-      default: return launch_inv4<3, 3>(ctx, d_planes, d_R, n, g, d_tabs, tab_stride, d_pixels);
-    }
+    return for_lane_pair_shape(g.nch, lf, [&](auto nc, auto l) -> int {
+      return launch_inv4<decltype(nc)::value, decltype(l)::value>(ctx, d_planes, d_R, n, g, d_tabs, tab_stride, d_pixels);
+    });
   }
   if (!MIXED && !lf && !ctx->force_generic && (g.w % 8) == 0 && (g.h % 8) == 0 && (g.cols % 16) == 0 &&
       (reinterpret_cast<uintptr_t>(d_planes) & 15) == 0 && (reinterpret_cast<uintptr_t>(d_pixels) & 7) == 0 &&
@@ -995,17 +1002,18 @@ int decode_device(himgcu_ctx *ctx, const uint8_t *d_himg, const unsigned long lo
 // rectangle reads at most (rh << lf) source rows from a row that is a multiple of 2^lf.
 int region_rows(const Geom &g, int rh, int lf = 0) { return std::min(((rh << lf) + 15 - (1 << lf)) / 8, g.rows); }
 
-// Lane-pair inverse of a region decode scaled by 2^LF (LF in 1..3): k_inverse_region4_scaled.
+// Lane-pair inverse of a region decode scaled by 2^LF (LF = 0: unscaled): k_inverse_region4.
 template <int NCH, int LF>
-int launch_inv_region4_scaled(himgcu_ctx *ctx, const uint8_t *d_planes, const uint8_t *d_R, int n, const Geom &g,
-                              const InvTables *d_inv, const int32_t *d_origins, int rw, int rh, int kr, uint8_t *d_pixels) {
+int launch_inv_region4(himgcu_ctx *ctx, const uint8_t *d_planes, const uint8_t *d_R, int n, const Geom &g, const InvTables *d_inv,
+                       const int32_t *d_origins, int rw, int rh, int kr, uint8_t *d_pixels) {
   constexpr int TP = kInv4ThreadsRgb;
+  static_assert(kInv4ThreadsGray == TP, "one tile width for both channel counts");
   const int span = region_span_pairs(rw << LF, g.cols);
   dim3 grid((unsigned)(((long long)kr * span + TP - 1) / TP), 1, n);
   const int smem = NCH * 64 * 2 * TP + kInvTableBytes;
-  CK(cudaFuncSetAttribute((k_inverse_region4_scaled<NCH, TP, LF>), cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
-  LAUNCH("k_inverse_region4_scaled", (k_inverse_region4_scaled<NCH, TP, LF>), grid, TP, smem, d_planes, d_R, g, d_inv,
-         (unsigned long long)sizeof(InvTables), d_origins, rw, rh, kr, span, d_pixels, 1u);
+  CK(cudaFuncSetAttribute((k_inverse_region4<NCH, TP, LF>), cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
+  LAUNCH(LF == 0 ? "k_inverse_region4" : "k_inverse_region4_scaled", (k_inverse_region4<NCH, TP, LF>), grid, TP, smem, d_planes,
+         d_R, g, d_inv, (unsigned long long)sizeof(InvTables), d_origins, rw, rh, kr, span, d_pixels, 1u);
   return HIMGCU_OK;
 }
 
@@ -1015,47 +1023,26 @@ template <bool MIXED = false>
 int stage_inverse_region(himgcu_ctx *ctx, const uint8_t *d_planes, const uint8_t *d_R, int n, const Geom &g,
                          const DecTables *d_tabs, const int32_t *d_origins, int rw, int rh, int kr, uint8_t *d_pixels,
                          const MixedDims &md = {}, int lf = 0) {
-  if (lf) {
-    // lane-pair fast path: the shapes k_inverse4_scaled takes (every window whole), the rectangle clips rows and columns
-    // (the clipped stores take any output alignment)
-    if (!MIXED && lane_pair_ok(ctx, g, d_planes, d_R, d_pixels, 1u)) {
-      InvTables *d_inv;
-      int rc = launch_inv_tables(ctx, d_tabs, n, (unsigned long long)sizeof(DecTables), &d_inv);
-      if (rc) return rc;
-      switch (g.nch * 4 + lf) {
-        case 1 * 4 + 1: return launch_inv_region4_scaled<1, 1>(ctx, d_planes, d_R, n, g, d_inv, d_origins, rw, rh, kr, d_pixels);
-        case 1 * 4 + 2: return launch_inv_region4_scaled<1, 2>(ctx, d_planes, d_R, n, g, d_inv, d_origins, rw, rh, kr, d_pixels);
-        case 1 * 4 + 3: return launch_inv_region4_scaled<1, 3>(ctx, d_planes, d_R, n, g, d_inv, d_origins, rw, rh, kr, d_pixels);
-        case 3 * 4 + 1: return launch_inv_region4_scaled<3, 1>(ctx, d_planes, d_R, n, g, d_inv, d_origins, rw, rh, kr, d_pixels);
-        case 3 * 4 + 2: return launch_inv_region4_scaled<3, 2>(ctx, d_planes, d_R, n, g, d_inv, d_origins, rw, rh, kr, d_pixels);
-        default: return launch_inv_region4_scaled<3, 3>(ctx, d_planes, d_R, n, g, d_inv, d_origins, rw, rh, kr, d_pixels);
-      }
-    }
-    const int kb = ((rw << lf) + 15 - (1 << lf)) / 8;
-    LAUNCH("k_inverse_region_scaled", k_inverse_region_scaled<MIXED>, dim3((kb + kTile - 1) / kTile, kr, n), kTile, 0, d_planes, d_R,
-           g, d_tabs, (unsigned long long)sizeof(DecTables), d_origins, rw, rh, kr, lf, d_pixels, md);
-    return HIMGCU_OK;
-  }
-  // lane-pair fast path: the shapes k_inverse4 takes, except that the rectangle clips rows and columns
-  if (!MIXED && !ctx->force_generic && (g.cols % 16) == 0 && (g.nch == 1 || g.nch == 3) &&
-      (reinterpret_cast<uintptr_t>(d_planes) & 15) == 0 && (reinterpret_cast<uintptr_t>(d_R) & 1) == 0) {
+  // lane-pair fast path.  Unscaled: the shapes k_inverse4 takes, except that the rectangle clips rows and columns.
+  // Scaled: the shapes the scaled k_inverse4 takes (every window whole), with the rectangle's clips.  (The clipped
+  // stores take any output alignment.)
+  const bool lane_pair =
+      !MIXED && (lf ? lane_pair_ok(ctx, g, d_planes, d_R, d_pixels, 1u)
+                    : !ctx->force_generic && (g.cols % 16) == 0 && (g.nch == 1 || g.nch == 3) &&
+                          (reinterpret_cast<uintptr_t>(d_planes) & 15) == 0 && (reinterpret_cast<uintptr_t>(d_R) & 1) == 0);
+  if (lane_pair) {
     InvTables *d_inv;
     int rc = launch_inv_tables(ctx, d_tabs, n, (unsigned long long)sizeof(DecTables), &d_inv);
     if (rc) return rc;
-    const int span = region_span_pairs(rw, g.cols);
-    constexpr int TP = kInv4ThreadsRgb;
-    static_assert(kInv4ThreadsGray == TP, "one tile width for both channel counts");
-    dim3 grid((unsigned)(((long long)kr * span + TP - 1) / TP), 1, n);
-    const int smem = g.nch * 64 * 2 * TP + kInvTableBytes;
-    if (g.nch == 1) {
-      CK(cudaFuncSetAttribute((k_inverse_region4<1, TP>), cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
-      LAUNCH("k_inverse_region4", (k_inverse_region4<1, TP>), grid, TP, smem, d_planes, d_R, g, d_inv,
-             (unsigned long long)sizeof(InvTables), d_origins, rw, rh, kr, span, d_pixels, 1u);
-    } else {
-      CK(cudaFuncSetAttribute((k_inverse_region4<3, TP>), cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
-      LAUNCH("k_inverse_region4", (k_inverse_region4<3, TP>), grid, TP, smem, d_planes, d_R, g, d_inv,
-             (unsigned long long)sizeof(InvTables), d_origins, rw, rh, kr, span, d_pixels, 1u);
-    }
+    return for_lane_pair_shape(g.nch, lf, [&](auto nc, auto l) -> int {
+      return launch_inv_region4<decltype(nc)::value, decltype(l)::value>(ctx, d_planes, d_R, n, g, d_inv, d_origins, rw, rh, kr,
+                                                                         d_pixels);
+    });
+  }
+  if (lf) {
+    const int kb = ((rw << lf) + 15 - (1 << lf)) / 8;
+    LAUNCH("k_inverse_region_scaled", k_inverse_region_scaled<MIXED>, dim3((kb + kTile - 1) / kTile, kr, n), kTile, 0, d_planes, d_R,
+           g, d_tabs, (unsigned long long)sizeof(DecTables), d_origins, rw, rh, kr, lf, d_pixels, md);
     return HIMGCU_OK;
   }
   const int kb = (rw + 14) / 8;

@@ -98,20 +98,12 @@ __device__ __forceinline__ bool image_geom(const MixedDims &m, int i, Geom &gi) 
 
 __device__ __forceinline__ int clamp255(int x) { return min(max(x, 0), 255); }
 
-// Region decode: origin (x, y) of image i's rw x rh rectangle (origins [n][2], device memory).  False when the
-// rectangle does not lie inside the image (rw, rh >= 1 are checked on the host).
-__device__ __forceinline__ bool region_origin(const int32_t *__restrict__ origins, int i, const Geom &g, int rw, int rh,
+// Region decode at scale 2^lf (lf = 0: unscaled): origin (x, y) of image i's rw x rh rectangle (origins [n][2], device
+// memory) in the scaled image [ceil(h / 2^lf)][ceil(w / 2^lf)].  The rectangle reads the source pixels
+// [x << lf, min((x + rw) << lf, w)) x [y << lf, min((y + rh) << lf, h)).  False when it does not lie inside the scaled
+// image (rw, rh >= 1 are checked on the host).
+__device__ __forceinline__ bool region_origin(const int32_t *__restrict__ origins, int i, const Geom &g, int lf, int rw, int rh,
                                               int &x, int &y) {
-  x = origins[2 * i];
-  y = origins[2 * i + 1];
-  return x >= 0 && y >= 0 && x <= g.w - rw && y <= g.h - rh;
-}
-
-// Scaled region decode (factor 2^lf): origin (x, y) of image i's rw x rh rectangle of the scaled image
-// [ceil(h / 2^lf)][ceil(w / 2^lf)].  The rectangle reads the source pixels [x << lf, min((x + rw) << lf, w)) x
-// [y << lf, min((y + rh) << lf, h)).  False when it does not lie inside the scaled image.
-__device__ __forceinline__ bool region_origin_scaled(const int32_t *__restrict__ origins, int i, const Geom &g, int lf, int rw,
-                                                     int rh, int &x, int &y) {
   x = origins[2 * i];
   y = origins[2 * i + 1];
   const int f = 1 << lf;

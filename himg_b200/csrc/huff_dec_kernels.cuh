@@ -554,7 +554,7 @@ __global__ void k_dec_segtab_mixed(const uint8_t *__restrict__ data, const Chunk
 // the image makes the image's status 2 (HIMGCU_ERR_ARG) and all its entries invalid.
 // MIXED: g is the bounding geometry (the stride of `full`); image i's header chain and origin are those of its own
 // geometry from `md`, and dims out of bounds are treated as an origin outside the image.
-// SCALED (k_dec_segtab_region_scaled): the rectangle is one of the image scaled by 2^lf (region_origin_scaled), and
+// SCALED (k_dec_segtab_region_scaled): the rectangle is one of the image scaled by 2^lf, and
 // the rows are those of the source pixels it reads.
 template <bool MIXED, bool SCALED>
 __device__ __forceinline__ void segtab_region(const uint8_t *__restrict__ data, const ChunkDesc *__restrict__ cd,
@@ -568,7 +568,7 @@ __device__ __forceinline__ void segtab_region(const uint8_t *__restrict__ data, 
   Geom gi = g;
   const bool dims_ok = !MIXED || image_geom(md, i, gi);
   int x, y;
-  if (!dims_ok || !(SCALED ? region_origin_scaled(origins, i, gi, lf, rw, rh, x, y) : region_origin(origins, i, gi, rw, rh, x, y))) {
+  if (!dims_ok || !region_origin(origins, i, gi, lf, rw, rh, x, y)) {
     for (int k = 0; k < kr; ++k) seg_store<false>(S + k, 0, 0xffffffffu);
     atomicMax(status + i, 2);
     return;

@@ -21,8 +21,10 @@
 //  * low-res add + clamp is one DPX instruction per lane pair, so is every output of the inverse
 //    colour map; finished samples overwrite the thread's own codes in the tile.
 //
+// k_inverse4<NCH, TP, LF> also decodes scaled by 2^LF (LF 1..3), averaging inside the output phase.
+//
 // Preconditions (host checked, else k_inverse2 / k_inverse): cols % 16 == 0, height % 8 == 0,
-// 16-byte aligned planes / pixels, 2-byte aligned low-res image, nch in {1, 3}.
+// 16-byte aligned planes / pixels (LF > 0: 16 >> LF bytes), 2-byte aligned low-res image, nch in {1, 3}.
 #ifndef HIMG_B200_XFORM_INV4_CUH_
 #define HIMG_B200_XFORM_INV4_CUH_
 
@@ -281,7 +283,7 @@ struct Inv4StorePooled {
 // shared-memory tile whose rows
 // (scan positions, channel-major) are PITCH bytes apart; the image's tables in sDq / sTab; pixel row y of
 // the pair goes out through store(y, ...) (active threads only).  No barrier inside.
-template <int NCH, int PITCH, class STORE = Inv4Store16<NCH>, int LF = 0>
+template <int NCH, int PITCH, class STORE, int LF>
 __device__ __forceinline__ void inv4_compute(uint8_t *col, const uint8_t *sDq, const uint32_t *sTab, int pre, int tab_bias,
                                              bool overflow, bool ycbcr, bool active, const uint32_t (&top)[NCH],
                                              const uint32_t (&bot)[NCH], const STORE &store, uint32_t one) {
@@ -449,7 +451,11 @@ __device__ __forceinline__ void inv4_compute(uint8_t *col, const uint8_t *sDq, c
 // (Measured and dropped: several tiles per CTA with the next tile prefetched into L2 or copied early from
 // inside the output phase, and tiles owned by single warps -- all slower than fresh CTAs whose start-up
 // overlaps the other resident CTA.)
-template <int NCH, int TP>
+//
+// LF > 0 (1..3): the decode scaled by F = 2^LF, through the pooled output phase of inv4_compute.  Image z's output is
+// [h >> LF][w >> LF][NCH] at pixels + z * its size (every window is whole on these shapes), each pixel the rounded box
+// average of its F x F window; the stores are 16 >> LF bytes wide.
+template <int NCH, int TP, int LF>
 __global__ void __launch_bounds__(TP, NCH == 1 ? 3 : 2)
     k_inverse4(const uint8_t *__restrict__ planes, const uint8_t *__restrict__ R, Geom g,
                const InvTables *__restrict__ tabs, unsigned long long tab_stride, uint8_t *__restrict__ pixels, uint32_t one) {
@@ -464,7 +470,7 @@ __global__ void __launch_bounds__(TP, NCH == 1 ? 3 : 2)
   const int f0 = blockIdx.x * TP;
   const int nact = min(TP, total - f0);
   const uint8_t *ipl = planes + (size_t)blockIdx.z * g.planes_bytes;
-  uint8_t *img = pixels + (size_t)blockIdx.z * g.out_img_bytes;
+  uint8_t *img = pixels + (size_t)blockIdx.z * (LF ? (size_t)(g.w >> LF) * (size_t)(g.h >> LF) * NCH : g.out_img_bytes);
   const InvTables *T = reinterpret_cast<const InvTables *>(reinterpret_cast<const char *>(tabs) + (size_t)blockIdx.z * tab_stride);
   // block row / first pair of the tile's first element: one division per CTA, everything else by
   // carrying (a tile spans few block rows unless the image is very narrow)
@@ -513,81 +519,11 @@ __global__ void __launch_bounds__(TP, NCH == 1 ? 3 : 2)
   inv4_corners<NCH>(R, blockIdx.z, g, v, u, top, bot);
   cp_async_wait_all();
   __syncthreads();  // the only barrier: from here on a thread touches its own two byte columns only
-  inv4_compute<NCH, PITCH>(sPl + 2 * t, sDq, sTab, pre, tab_bias, overflow, ycbcr, active, top, bot,
-                           Inv4Store16<NCH>{img + ((size_t)(8 * v) * g.w + (size_t)u * 8) * NCH, (size_t)g.w * NCH}, one);
-}
-
-// Scaled decode by F = 2^LF (LF in 1..3): k_inverse4 with the pooled output phase of inv4_compute.  Image z's output is
-// [h >> LF][w >> LF][NCH] (every window is whole on these shapes) at pixels + z * its size, each pixel the rounded box
-// average of its F x F window; the stores are 16 >> LF bytes wide.  Grid, block, shared memory and tiles as k_inverse4.
-template <int NCH, int TP, int LF>
-__global__ void __launch_bounds__(TP, NCH == 1 ? 3 : 2)
-    k_inverse4_scaled(const uint8_t *__restrict__ planes, const uint8_t *__restrict__ R, Geom g, const InvTables *__restrict__ tabs,
-                      unsigned long long tab_stride, uint8_t *__restrict__ pixels, uint32_t one) {
-  extern __shared__ __align__(128) uint8_t sPl[];
-  constexpr int PITCH = 2 * TP, CPR = TP / 8;  // bytes per tile row, 16-byte chunks per tile row
-  static_assert(TP % 32 == 0 && TP == 8 * CPR, "a CTA is 8 groups of one thread per chunk of a tile row");
-  uint8_t *sDq = sPl + NCH * 64 * PITCH;
-  uint32_t *sTab = reinterpret_cast<uint32_t *>(sDq + kInvSlots * 256 * 2);
-
-  const int t = threadIdx.x;
-  const int PR = g.cols >> 1, total = g.rows * PR;
-  const int f0 = blockIdx.x * TP;
-  const int nact = min(TP, total - f0);
-  const uint8_t *ipl = planes + (size_t)blockIdx.z * g.planes_bytes;
-  const size_t ow = (size_t)(g.w >> LF);  // (w % 16 == 0, h % 8 == 0: every window is whole)
-  uint8_t *img = pixels + (size_t)blockIdx.z * (ow * (size_t)(g.h >> LF) * NCH);
-  const InvTables *T = reinterpret_cast<const InvTables *>(reinterpret_cast<const char *>(tabs) + (size_t)blockIdx.z * tab_stride);
-  // block row / first pair of the tile's first element: one division per CTA, everything else by
-  // carrying (a tile spans few block rows unless the image is very narrow)
-  // (a true division: a 32-bit reciprocal of PR is not exact for every tile start of every accepted shape)
-  const int v0 = (int)((uint32_t)f0 / (uint32_t)PR), p0 = f0 - v0 * PR;
-  auto locate = [&](int k, int &v, int &p) {  // element f0 + k of the image -> block row, pair in the row
-    if (PR >= 32) {
-      v = v0;
-      p = p0 + k;
-      while (p >= PR) {
-        p -= PR;
-        ++v;
-      }
-    } else {
-      v = (f0 + k) / PR;
-      p = f0 + k - v * PR;
-    }
-  };
-  {
-    // the image's tables, then the tile: thread -> 16-byte chunk t % CPR (8 pairs of ONE block row:
-    // cols % 16 == 0) of the tile rows t / CPR + 8 i; the threads of a row copy 2 * TP contiguous bytes
-    const uint4 *tsrc = reinterpret_cast<const uint4 *>(T);
-    for (int i = t; i < kInvTableBytes / 16; i += TP) cp_async16(sDq + 16 * i, tsrc + i);
-    const int cq = t % CPR, r0 = t / CPR;
-    if (8 * cq < nact) {
-      int vl, pl;
-      locate(8 * cq, vl, pl);
-      const uint8_t *src = ipl + (size_t)vl * g.seg + 2 * pl + (size_t)r0 * g.cols;
-      uint8_t *dst = sPl + r0 * PITCH + cq * 16;
-      const size_t rstep = (size_t)8 * g.cols;
-#pragma unroll 8
-      for (int i = 0; i < NCH * 8; ++i) {
-        cp_async16(dst + i * 8 * PITCH, src);
-        src += rstep;
-      }
-    }
-  }
-  const int pre = T->pre, tab_bias = T->bias;
-  const bool overflow = T->overflow != 0;
-  const bool ycbcr = T->ycbcr != 0;
-  const bool active = t < nact;
-  int v, p;
-  locate(active ? t : 0, v, p);
-  const int u = 2 * p;
-  uint32_t top[NCH], bot[NCH];
-  inv4_corners<NCH>(R, blockIdx.z, g, v, u, top, bot);
-  cp_async_wait_all();
-  __syncthreads();  // the only barrier: from here on a thread touches its own two byte columns only
-  inv4_compute<NCH, PITCH, Inv4StorePooled<NCH, LF>, LF>(
-      sPl + 2 * t, sDq, sTab, pre, tab_bias, overflow, ycbcr, active, top, bot,
-      Inv4StorePooled<NCH, LF>{img + ((size_t)(v << (3 - LF)) * ow + ((size_t)u << (3 - LF))) * NCH, ow * NCH}, one);
+  using Store = std::conditional_t<LF == 0, Inv4Store16<NCH>, Inv4StorePooled<NCH, LF>>;
+  constexpr int OB = 8 >> LF;  // output pixels of a block per row
+  const size_t ow = (size_t)(g.w >> LF);
+  inv4_compute<NCH, PITCH, Store, LF>(sPl + 2 * t, sDq, sTab, pre, tab_bias, overflow, ycbcr, active, top, bot,
+                                      Store{img + ((size_t)(OB * v) * ow + (size_t)u * OB) * NCH, ow * NCH}, one);
 }
 
 }  // namespace himgcu

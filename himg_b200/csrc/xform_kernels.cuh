@@ -366,6 +366,69 @@ __device__ __forceinline__ LowCorners load_corners(const uint8_t *__restrict__ X
 }
 
 // ---------------------------------------------------------------------------------------------
+// Pieces of the generic inverse kernels: the block reconstruction of k_inverse and k_inverse_scaled, and the inverse
+// colour map of those and of k_inverse_region / k_inverse_region_scaled (xform_region.cuh).
+// ---------------------------------------------------------------------------------------------
+// One channel of block (u, v) of geometry g, in int32: gather the 64 codes (src: the block's column of its coefficient
+// plane, scan positions g.cols bytes apart) and dequantise them through the image's tables sUn / sh, two WHT passes with
+// a floor >> 3 after each, add the low-res patch from the corners of the low-res plane plane(), clamp, and pack the 64
+// samples as bytes (row-major) into sOut[slot][t].  (plane() is evaluated after the transform and t, the thread index,
+// comes from the kernel: an address computed before the transform, or threadIdx.x read here, costs registers.)
+template <class PLANE, int NS>
+__device__ __forceinline__ void inv_block(const uint8_t *__restrict__ src, const int16_t *sUn, const uint8_t *sh, const PLANE &plane,
+                                          const Geom &g, int u, int v, uint32_t (&sOut)[NS][kTile][17], int slot, int t) {
+  int x[64];
+#pragma unroll
+  for (int j = 0; j < 64; ++j) {
+    const int code = __ldg(src + (size_t)scan_pos(j) * g.cols);
+    const int val = sUn[code];
+    // (int16)(Unmap << shift): the narrowing only matters for hostile streams
+    x[j] = (int)(short)(val * (1 << sh[j]));
+  }
+#pragma unroll
+  for (int r = 0; r < 8; ++r) {
+    wht8(x[r * 8 + 0], x[r * 8 + 1], x[r * 8 + 2], x[r * 8 + 3], x[r * 8 + 4], x[r * 8 + 5], x[r * 8 + 6], x[r * 8 + 7]);
+#pragma unroll
+    for (int i = 0; i < 8; ++i) x[r * 8 + i] >>= 3;
+  }
+#pragma unroll
+  for (int q = 0; q < 8; ++q) {
+    wht8(x[q], x[8 + q], x[16 + q], x[24 + q], x[32 + q], x[40 + q], x[48 + q], x[56 + q]);
+#pragma unroll
+    for (int i = 0; i < 8; ++i) x[i * 8 + q] >>= 3;
+  }
+  {
+    const LowCorners k = load_corners(plane(), g, u, v);
+    int lf[9], rt[9];
+    nine(k.x11, k.x21, lf);
+    nine(k.x12, k.x22, rt);
+#pragma unroll
+    for (int y = 0; y < 8; ++y) {
+      int t[9];
+      nine(lf[y], rt[y], t);
+#pragma unroll
+      for (int i = 0; i < 8; ++i) x[y * 8 + i] = clamp255((int)(short)(x[y * 8 + i] + t[i]));
+    }
+  }
+#pragma unroll
+  for (int k = 0; k < 16; ++k) {
+    const uint32_t lo = __byte_perm((uint32_t)x[4 * k], (uint32_t)x[4 * k + 1], 0x0040);
+    const uint32_t hi = __byte_perm((uint32_t)x[4 * k + 2], (uint32_t)x[4 * k + 3], 0x0040);
+    sOut[slot][t][k] = __byte_perm(lo, hi, 0x5410);
+  }
+}
+
+// Inverse colour map of one pixel (ycbcr.cpp:54-82): Y, Cb, Cr in, R, G, B out.
+template <class T>
+__device__ __forceinline__ void inv_colour(T &c0, T &c1, T &c2) {
+  const int Y = c0, cb = 2 * c1 - 255, cr = 2 * c2 - 255;
+  const int G = Y - ((cb + cr + 2) >> 2);
+  c0 = (T)clamp255(G + cr);
+  c1 = (T)clamp255(G);
+  c2 = (T)clamp255(G + cb);
+}
+
+// ---------------------------------------------------------------------------------------------
 // K-fwd (the roofline kernel): colour map + low-res subtract + rows/cols WHT + shift quantise +
 // 8-bit map + coefficient-planar scatter (encoder.cpp:275-328, hadamard.cpp:78-88,
 // quantize.cpp:127-151, mapper.cpp:159-182).  grid (ceil(cols/kTile), rows, n), block kTile.
@@ -509,49 +572,12 @@ __global__ void __launch_bounds__(kTile)
 
 #pragma unroll 1
   for (int c = 0; c < NCH; ++c) {
-    int x[64];
-    const uint8_t *src = seg + (size_t)(cbase + c) * g.cols * 64 + u;
-    const uint8_t *sh = sShift[(YCBCR && NCH >= 3 && (c == 1 || c == 2)) ? 1 : 0];
-#pragma unroll
-    for (int j = 0; j < 64; ++j) {
-      const int code = __ldg(src + (size_t)scan_pos(j) * g.cols);
-      const int val = sUn[code];
-      // (int16)(Unmap << shift): the narrowing only matters for hostile streams
-      x[j] = (int)(short)(val * (1 << sh[j]));
-    }
-#pragma unroll
-    for (int r = 0; r < 8; ++r) {
-      wht8(x[r * 8 + 0], x[r * 8 + 1], x[r * 8 + 2], x[r * 8 + 3], x[r * 8 + 4], x[r * 8 + 5], x[r * 8 + 6], x[r * 8 + 7]);
-#pragma unroll
-      for (int i = 0; i < 8; ++i) x[r * 8 + i] >>= 3;
-    }
-#pragma unroll
-    for (int q = 0; q < 8; ++q) {
-      wht8(x[q], x[8 + q], x[16 + q], x[24 + q], x[32 + q], x[40 + q], x[48 + q], x[56 + q]);
-#pragma unroll
-      for (int i = 0; i < 8; ++i) x[i * 8 + q] >>= 3;
-    }
-    {
-      const uint8_t *Rp = MIXED ? R + (size_t)blockIdx.z * ctotal * gb.rows * gb.cols + (size_t)(cbase + c) * g.rows * g.cols
-                                : R + ((size_t)blockIdx.z * ctotal + cbase + c) * g.rows * g.cols;
-      const LowCorners k = load_corners(Rp, g, u, v);
-      int lf[9], rt[9];
-      nine(k.x11, k.x21, lf);
-      nine(k.x12, k.x22, rt);
-#pragma unroll
-      for (int y = 0; y < 8; ++y) {
-        int t[9];
-        nine(lf[y], rt[y], t);
-#pragma unroll
-        for (int i = 0; i < 8; ++i) x[y * 8 + i] = clamp255((int)(short)(x[y * 8 + i] + t[i]));
-      }
-    }
-#pragma unroll
-    for (int k = 0; k < 16; ++k) {
-      const uint32_t lo = __byte_perm((uint32_t)x[4 * k], (uint32_t)x[4 * k + 1], 0x0040);
-      const uint32_t hi = __byte_perm((uint32_t)x[4 * k + 2], (uint32_t)x[4 * k + 3], 0x0040);
-      sOut[c][threadIdx.x][k] = __byte_perm(lo, hi, 0x5410);
-    }
+    auto plane = [&] {
+      return MIXED ? R + (size_t)blockIdx.z * ctotal * gb.rows * gb.cols + (size_t)(cbase + c) * g.rows * g.cols
+                   : R + ((size_t)blockIdx.z * ctotal + cbase + c) * g.rows * g.cols;
+    };
+    inv_block(seg + (size_t)(cbase + c) * g.cols * 64 + u, sUn, sShift[(YCBCR && NCH >= 3 && (c == 1 || c == 2)) ? 1 : 0], plane,
+              g, u, v, sOut, c, threadIdx.x);
   }
 
   // ---- inverse colour map + interleave + store
@@ -567,13 +593,7 @@ __global__ void __launch_bounds__(kTile)
         int ch[NCH];
 #pragma unroll
         for (int c = 0; c < NCH; ++c) ch[c] = (int)__byte_perm(sOut[c][threadIdx.x][y * 2 + (i >> 2)], 0u, 0x4440u + (i & 3));
-        if (YCBCR && NCH >= 3) {
-          const int Y = ch[0], cb = 2 * ch[1] - 255, cr = 2 * ch[NCH >= 3 ? 2 : 0] - 255;
-          const int G = Y - ((cb + cr + 2) >> 2);
-          ch[0] = clamp255(G + cr);
-          ch[1] = clamp255(G);
-          ch[NCH >= 3 ? 2 : 0] = clamp255(G + cb);
-        }
+        if (YCBCR && NCH >= 3) inv_colour(ch[0], ch[1], ch[NCH >= 3 ? 2 : 0]);
 #pragma unroll
         for (int c = 0; c < NCH; ++c) {
           const int k = i * NCH + c;
@@ -630,47 +650,12 @@ __global__ void __launch_bounds__(kTile)
   // ---- the transform of k_inverse, clamped samples to sOut
 #pragma unroll 1
   for (int c = 0; c < NCH; ++c) {
-    int x[64];
-    const uint8_t *src = seg + (size_t)(cbase + c) * g.cols * 64 + u;
-    const uint8_t *sh = sShift[(YCBCR && NCH >= 3 && (c == 1 || c == 2)) ? 1 : 0];
-#pragma unroll
-    for (int j = 0; j < 64; ++j) {
-      const int code = __ldg(src + (size_t)scan_pos(j) * g.cols);
-      x[j] = (int)(short)(sUn[code] * (1 << sh[j]));
-    }
-#pragma unroll
-    for (int r = 0; r < 8; ++r) {
-      wht8(x[r * 8 + 0], x[r * 8 + 1], x[r * 8 + 2], x[r * 8 + 3], x[r * 8 + 4], x[r * 8 + 5], x[r * 8 + 6], x[r * 8 + 7]);
-#pragma unroll
-      for (int i = 0; i < 8; ++i) x[r * 8 + i] >>= 3;
-    }
-#pragma unroll
-    for (int q = 0; q < 8; ++q) {
-      wht8(x[q], x[8 + q], x[16 + q], x[24 + q], x[32 + q], x[40 + q], x[48 + q], x[56 + q]);
-#pragma unroll
-      for (int i = 0; i < 8; ++i) x[i * 8 + q] >>= 3;
-    }
-    {
-      const uint8_t *Rp = MIXED ? R + (size_t)blockIdx.z * ctotal * gb.rows * gb.cols + (size_t)(cbase + c) * g.rows * g.cols
-                                : R + ((size_t)blockIdx.z * ctotal + cbase + c) * g.rows * g.cols;
-      const LowCorners k = load_corners(Rp, g, u, v);
-      int lf9[9], rt9[9];
-      nine(k.x11, k.x21, lf9);
-      nine(k.x12, k.x22, rt9);
-#pragma unroll
-      for (int y = 0; y < 8; ++y) {
-        int t[9];
-        nine(lf9[y], rt9[y], t);
-#pragma unroll
-        for (int i = 0; i < 8; ++i) x[y * 8 + i] = clamp255((int)(short)(x[y * 8 + i] + t[i]));
-      }
-    }
-#pragma unroll
-    for (int k = 0; k < 16; ++k) {
-      const uint32_t lo = __byte_perm((uint32_t)x[4 * k], (uint32_t)x[4 * k + 1], 0x0040);
-      const uint32_t hi = __byte_perm((uint32_t)x[4 * k + 2], (uint32_t)x[4 * k + 3], 0x0040);
-      sOut[c][threadIdx.x][k] = __byte_perm(lo, hi, 0x5410);
-    }
+    auto plane = [&] {
+      return MIXED ? R + (size_t)blockIdx.z * ctotal * gb.rows * gb.cols + (size_t)(cbase + c) * g.rows * g.cols
+                   : R + ((size_t)blockIdx.z * ctotal + cbase + c) * g.rows * g.cols;
+    };
+    inv_block(seg + (size_t)(cbase + c) * g.cols * 64 + u, sUn, sShift[(YCBCR && NCH >= 3 && (c == 1 || c == 2)) ? 1 : 0], plane,
+              g, u, v, sOut, c, threadIdx.x);
   }
 
   // ---- inverse colour map in place (a thread only touches its own block's bytes)
@@ -679,13 +664,7 @@ __global__ void __launch_bounds__(kTile)
   for (int c = 0; c < NCH; ++c) px[c] = reinterpret_cast<uint8_t *>(&sOut[c][threadIdx.x][0]);
   if (NCH >= 3 && YCBCR) {
 #pragma unroll 4
-    for (int p = 0; p < 64; ++p) {
-      const int Y = px[0][p], cb = 2 * px[1][p] - 255, cr = 2 * px[NCH >= 3 ? 2 : 0][p] - 255;
-      const int G = Y - ((cb + cr + 2) >> 2);
-      px[0][p] = (uint8_t)clamp255(G + cr);
-      px[1][p] = (uint8_t)clamp255(G);
-      px[NCH >= 3 ? 2 : 0][p] = (uint8_t)clamp255(G + cb);
-    }
+    for (int p = 0; p < 64; ++p) inv_colour(px[0][p], px[1][p], px[NCH >= 3 ? 2 : 0][p]);
   }
 
   // ---- box averages of the windows inside the image

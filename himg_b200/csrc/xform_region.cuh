@@ -6,7 +6,8 @@
 // the corner and edge clamps of the interpolation are those of the image, not of the rectangle.
 //
 //   k_inverse_region4  fast path (nch 1 / 3, cols % 16 == 0): k_inverse4's lane pairs and warp tiles over the
-//                      flattened (slot, block pair) space of the staged columns, clipped stores (Inv4StoreClip)
+//                      flattened (slot, block pair) space of the staged columns, clipped stores (Inv4StoreClip); at
+//                      LF > 0 the scaled decode below, with clipped pooled stores (Inv4StorePooledClip)
 //   k_inverse_region   every other shape and force_generic: one block per thread in int32, as k_inverse, with a
 //                      runtime channel count (colour map on channels 0-2)
 #ifndef HIMG_B200_XFORM_REGION_CUH_
@@ -64,6 +65,46 @@ struct Inv4StoreClip {
   }
 };
 
+// Output row wy of a block pair's pooled lanes (see Inv4StorePooled), clipped to the rectangle.  The pair's
+// 2 * (8 >> LF) * NCH bytes of a row are one run in the output at any byte alignment, of which the bytes [b0, b1)
+// lie inside the rectangle: stored as Inv4StoreClip stores a full-size run.
+template <int NCH, int LF>
+struct Inv4StorePooledClip {
+  uint8_t *row0;       // byte 0 of the pair's output row 0 (may lie outside the rectangle)
+  long long row_bytes; // rw * NCH
+  int y0, rh;          // output row 0 of the pair is row y0 of the rectangle
+  int b0, b1;          // bytes of a run inside the rectangle
+  __device__ __forceinline__ void operator()(int wy, const uint32_t (&p)[(8 >> LF) * NCH]) const {
+    if (y0 + wy < 0 || y0 + wy >= rh) return;
+    constexpr int K = (8 >> LF) * NCH, RB = 2 * K, NW = (RB + 3) / 4;  // bytes per block, per run, words of a run
+    auto byte = [&](int b) -> uint32_t { return b < K ? (p[b] & 0xffu) : (p[b - K] >> 16); };
+    uint32_t W[NW];
+#pragma unroll
+    for (int k = 0; k < NW; ++k) {
+      W[k] = 0u;
+#pragma unroll
+      for (int j = 0; j < 4; ++j)
+        if (4 * k + j < RB) W[k] |= byte(4 * k + j) << (8 * j);
+    }
+    const uintptr_t addr = reinterpret_cast<uintptr_t>(row0) + (uintptr_t)((long long)wy * row_bytes);
+    const int a = (int)(addr & 3);
+    uint8_t *base = reinterpret_cast<uint8_t *>(addr - (uintptr_t)a);
+#pragma unroll
+    for (int j = 0; j <= NW; ++j) {
+      const int s = 4 * j - a;  // run byte at the output word's byte 0
+      if (s >= b1 || s + 4 <= b0) continue;
+      const uint32_t v = __funnelshift_rc(j > 0 ? W[j - 1] : 0u, j < NW ? W[j] : 0u, 8 * (4 - a));
+      if (s >= b0 && s + 4 <= b1) {
+        *reinterpret_cast<uint32_t *>(base + 4 * j) = v;
+      } else {
+#pragma unroll
+        for (int t = 0; t < 4; ++t)
+          if (s + t >= b0 && s + t < b1) base[4 * j + t] = (uint8_t)(v >> (8 * t));
+      }
+    }
+  }
+};
+
 // Block pairs of a compact slot staged by k_inverse_region4 for a rectangle of width rw: the columns from the
 // 16-block boundary at or below x / 8 (16-byte aligned cp.async sources) to (x + rw - 1) / 8, for the worst x, in
 // whole 16-byte chunks (8 pairs), at most the image's.
@@ -73,25 +114,27 @@ inline int region_span_pairs(int rw, int cols) {
   return span < cols / 2 ? span : cols / 2;
 }
 
-// grid (ceil(kr * span / TP), 1, n), block TP, dynamic smem as k_inverse4.  A CTA owns TP consecutive elements of
-// the image's flattened [kr][span] space of block pairs; pairs outside the image or the rectangle and repeated
-// slots are computed on whatever the tile holds and not stored.
-template <int NCH, int TP>
+// grid (ceil(kr * span / TP), 1, n) with span = region_span_pairs(rw << LF, cols), block TP, dynamic smem as k_inverse4.
+// A CTA owns TP consecutive elements of the image's flattened [kr][span] space of block pairs; pairs outside the image
+// or the rectangle and repeated slots are computed on whatever the tile holds and not stored.  LF > 0: the rectangle
+// is one of the image scaled by 2^LF (see below), and the pairs are those of its source rectangle.
+template <int NCH, int TP, int LF>
 __global__ void __launch_bounds__(TP, NCH == 1 ? 3 : 2)
     k_inverse_region4(const uint8_t *__restrict__ planes, const uint8_t *__restrict__ R, Geom g,
                       const InvTables *__restrict__ tabs, unsigned long long tab_stride, const int32_t *__restrict__ origins,
                       int rw, int rh, int kr, int span, uint8_t *__restrict__ pixels, uint32_t one) {
   extern __shared__ __align__(128) uint8_t sPl[];
-  constexpr int PITCH = 2 * TP, CPR = TP / 8;
+  constexpr int PITCH = 2 * TP, CPR = TP / 8, OB = 8 >> LF;  // OB: output pixels of a block per row
   static_assert(TP % 32 == 0 && TP == 8 * CPR, "a CTA is 8 groups of one thread per chunk of a tile row");
   uint8_t *sDq = sPl + NCH * 64 * PITCH;
   uint32_t *sTab = reinterpret_cast<uint32_t *>(sDq + kInvSlots * 256 * 2);
   const int item = blockIdx.z;
   int x, y;
-  if (!region_origin(origins, item, g, rw, rh, x, y)) return;  // (the whole CTA)
+  if (!region_origin(origins, item, g, LF, rw, rh, x, y)) return;  // (the whole CTA)
   const int t = threadIdx.x;
-  const int r0 = y >> 3, r1 = (y + rh - 1) >> 3;
-  const int u0 = (x >> 3) & ~15, ul = x >> 3, ur = (x + rw - 1) >> 3;
+  const int sx = x << LF, sy = y << LF;  // (LF > 0: every window is whole, the source rectangle is (rw << LF) x (rh << LF))
+  const int r0 = sy >> 3, r1 = (sy + (rh << LF) - 1) >> 3;
+  const int u0 = (sx >> 3) & ~15, ul = sx >> 3, ur = (sx + (rw << LF) - 1) >> 3;
   const int f0 = blockIdx.x * TP, nact = min(TP, kr * span - f0);
   const uint8_t *ipl = planes + (size_t)item * kr * g.seg;
   const InvTables *T = reinterpret_cast<const InvTables *>(reinterpret_cast<const char *>(tabs) + (size_t)item * tab_stride);
@@ -119,16 +162,16 @@ __global__ void __launch_bounds__(TP, NCH == 1 ? 3 : 2)
   const int v = min(r0 + s, r1);
   uint32_t top[NCH], bot[NCH];
   inv4_corners<NCH>(R, item, g, v, u, top, bot);
-  const int X0 = 8 * u - x;  // rectangle column of the pair's first pixel
-  const Inv4StoreClip<NCH> store{pixels + (size_t)item * rw * rh * NCH + ((long long)(8 * v - y) * rw + X0) * NCH,
-                                 (long long)rw * NCH, 8 * v - y, rh, max(0, -X0) * NCH, min(16, rw - X0) * NCH};
+  const int X0 = OB * u - x;  // rectangle column of the pair's first output pixel
+  using Store = std::conditional_t<LF == 0, Inv4StoreClip<NCH>, Inv4StorePooledClip<NCH, LF>>;
+  const Store store{pixels + (size_t)item * rw * rh * NCH + ((long long)(OB * v - y) * rw + X0) * NCH, (long long)rw * NCH,
+                    OB * v - y, rh, max(0, -X0) * NCH, min(2 * OB, rw - X0) * NCH};
   const int pre = T->pre, tab_bias = T->bias;
   const bool overflow = T->overflow != 0;
   const bool ycbcr = T->ycbcr != 0;
   cp_async_wait_all();
   __syncthreads();
-  inv4_compute<NCH, PITCH, Inv4StoreClip<NCH>>(sPl + 2 * t, sDq, sTab, pre, tab_bias, overflow, ycbcr, active, top, bot, store,
-                                               one);
+  inv4_compute<NCH, PITCH, Store, LF>(sPl + 2 * t, sDq, sTab, pre, tab_bias, overflow, ycbcr, active, top, bot, store, one);
 }
 
 // grid (ceil(kb / kTile), kr, n), block kTile (kb = (rw + 14) / 8 block columns): thread = block column x / 8 + i of
@@ -148,7 +191,7 @@ __global__ void __launch_bounds__(kTile)
   Geom gi = g;  // the image's geometry
   if (MIXED && !image_geom(md, item, gi)) return;
   int x, y;
-  if (!region_origin(origins, item, gi, rw, rh, x, y)) return;  // (the whole CTA)
+  if (!region_origin(origins, item, gi, 0, rw, rh, x, y)) return;  // (the whole CTA)
   const int v = (y >> 3) + slot;
   if (v > (y + rh - 1) >> 3) return;  // a repeated slot
   const DecTables *T = reinterpret_cast<const DecTables *>(reinterpret_cast<const char *>(tabs) + (size_t)item * tab_stride);
@@ -167,6 +210,7 @@ __global__ void __launch_bounds__(kTile)
   const int ngroup = min(nch, 3);
 #pragma unroll 1
   for (int c = 0; c < nch; ++c) {
+    // (inv_block's transform, written out: through inv_block the compiler allocates this kernel's registers differently)
     int xv[64];
     const uint8_t *src = seg + (size_t)c * gi.cols * 64 + u;
     const uint8_t *sh = sShift[(ycbcr && (c == 1 || c == 2)) ? 1 : 0];
@@ -217,13 +261,7 @@ __global__ void __launch_bounds__(kTile)
           int ch[3];
 #pragma unroll
           for (int q = 0; q < 3; ++q) ch[q] = q < ngroup ? sample(q, yy, i) : 0;
-          if (ycbcr) {
-            const int Y = ch[0], cb = 2 * ch[1] - 255, cr = 2 * ch[2] - 255;
-            const int G = Y - ((cb + cr + 2) >> 2);
-            ch[0] = clamp255(G + cr);
-            ch[1] = clamp255(G);
-            ch[2] = clamp255(G + cb);
-          }
+          if (ycbcr) inv_colour(ch[0], ch[1], ch[2]);
           uint8_t *p = out(yy, i);
 #pragma unroll
           for (int q = 0; q < 3; ++q)
@@ -239,110 +277,9 @@ __global__ void __launch_bounds__(kTile)
 // k_inverse_scaled.  Every window lies inside one block, so the blocks computed are those of the source rectangle
 // [F x, min(F (x + rw), w)) x [F y, min(F (y + rh), h)), from the compact planes of k_dec_segtab_region_scaled.
 //
-//   k_inverse_region4_scaled  fast path (nch 1 / 3, w % 16 == 0, h % 8 == 0, cols % 16 == 0: every window whole):
-//                             k_inverse_region4's tiles and inv4_compute's pooled output phase, clipped stores
-//                             (Inv4StorePooledClip)
-//   k_inverse_region_scaled   every other shape, force_generic and the mixed call: k_inverse_region's transform, then
-//                             k_inverse_scaled's exact division per window
-
-// Output row wy of a block pair's pooled lanes (see Inv4StorePooled), clipped to the rectangle.  The pair's
-// 2 * (8 >> LF) * NCH bytes of a row are one run in the output at any byte alignment, of which the bytes [b0, b1)
-// lie inside the rectangle: stored as Inv4StoreClip stores a full-size run.
-template <int NCH, int LF>
-struct Inv4StorePooledClip {
-  uint8_t *row0;       // byte 0 of the pair's output row 0 (may lie outside the rectangle)
-  long long row_bytes; // rw * NCH
-  int y0, rh;          // output row 0 of the pair is row y0 of the rectangle
-  int b0, b1;          // bytes of a run inside the rectangle
-  __device__ __forceinline__ void operator()(int wy, const uint32_t (&p)[(8 >> LF) * NCH]) const {
-    if (y0 + wy < 0 || y0 + wy >= rh) return;
-    constexpr int K = (8 >> LF) * NCH, RB = 2 * K, NW = (RB + 3) / 4;  // bytes per block, per run, words of a run
-    auto byte = [&](int b) -> uint32_t { return b < K ? (p[b] & 0xffu) : (p[b - K] >> 16); };
-    uint32_t W[NW];
-#pragma unroll
-    for (int k = 0; k < NW; ++k) {
-      W[k] = 0u;
-#pragma unroll
-      for (int j = 0; j < 4; ++j)
-        if (4 * k + j < RB) W[k] |= byte(4 * k + j) << (8 * j);
-    }
-    const uintptr_t addr = reinterpret_cast<uintptr_t>(row0) + (uintptr_t)((long long)wy * row_bytes);
-    const int a = (int)(addr & 3);
-    uint8_t *base = reinterpret_cast<uint8_t *>(addr - (uintptr_t)a);
-#pragma unroll
-    for (int j = 0; j <= NW; ++j) {
-      const int s = 4 * j - a;  // run byte at the output word's byte 0
-      if (s >= b1 || s + 4 <= b0) continue;
-      const uint32_t v = __funnelshift_rc(j > 0 ? W[j - 1] : 0u, j < NW ? W[j] : 0u, 8 * (4 - a));
-      if (s >= b0 && s + 4 <= b1) {
-        *reinterpret_cast<uint32_t *>(base + 4 * j) = v;
-      } else {
-#pragma unroll
-        for (int t = 0; t < 4; ++t)
-          if (s + t >= b0 && s + t < b1) base[4 * j + t] = (uint8_t)(v >> (8 * t));
-      }
-    }
-  }
-};
-
-// grid (ceil(kr * span / TP), 1, n) with span = region_span_pairs(rw << LF, cols), block TP, dynamic smem as
-// k_inverse4.  k_inverse_region4 on the source rectangle, with the output phase of k_inverse4_scaled.
-template <int NCH, int TP, int LF>
-__global__ void __launch_bounds__(TP, NCH == 1 ? 3 : 2)
-    k_inverse_region4_scaled(const uint8_t *__restrict__ planes, const uint8_t *__restrict__ R, Geom g,
-                             const InvTables *__restrict__ tabs, unsigned long long tab_stride,
-                             const int32_t *__restrict__ origins, int rw, int rh, int kr, int span, uint8_t *__restrict__ pixels,
-                             uint32_t one) {
-  extern __shared__ __align__(128) uint8_t sPl[];
-  constexpr int PITCH = 2 * TP, CPR = TP / 8, OB = 8 >> LF;  // OB: output pixels of a block per row
-  static_assert(TP % 32 == 0 && TP == 8 * CPR, "a CTA is 8 groups of one thread per chunk of a tile row");
-  uint8_t *sDq = sPl + NCH * 64 * PITCH;
-  uint32_t *sTab = reinterpret_cast<uint32_t *>(sDq + kInvSlots * 256 * 2);
-  const int item = blockIdx.z;
-  int x, y;
-  if (!region_origin_scaled(origins, item, g, LF, rw, rh, x, y)) return;  // (the whole CTA)
-  const int t = threadIdx.x;
-  const int sx = x << LF, sy = y << LF;  // (every window is whole: the source rectangle is (rw << LF) x (rh << LF))
-  const int r0 = sy >> 3, r1 = (sy + (rh << LF) - 1) >> 3;
-  const int u0 = (sx >> 3) & ~15, ul = sx >> 3, ur = (sx + (rw << LF) - 1) >> 3;
-  const int f0 = blockIdx.x * TP, nact = min(TP, kr * span - f0);
-  const uint8_t *ipl = planes + (size_t)item * kr * g.seg;
-  const InvTables *T = reinterpret_cast<const InvTables *>(reinterpret_cast<const char *>(tabs) + (size_t)item * tab_stride);
-  {
-    const uint4 *tsrc = reinterpret_cast<const uint4 *>(T);
-    for (int i = t; i < kInvTableBytes / 16; i += TP) cp_async16(sDq + 16 * i, tsrc + i);
-    // a chunk = 8 pairs of one slot (span % 8 == 0), inside the image or wholly outside it (cols % 16 == 0)
-    const int cq = t % CPR, rt = t / CPR, e = f0 + 8 * cq;
-    const int s = e / span, u = u0 + 2 * (e - s * span);
-    if (8 * cq < nact && u < g.cols) {
-      const uint8_t *src = ipl + (size_t)s * g.seg + u + (size_t)rt * g.cols;
-      uint8_t *dst = sPl + rt * PITCH + cq * 16;
-      const size_t rstep = (size_t)8 * g.cols;
-#pragma unroll 8
-      for (int i = 0; i < NCH * 8; ++i) {
-        cp_async16(dst + i * 8 * PITCH, src);
-        src += rstep;
-      }
-    }
-  }
-  const int e = f0 + t, s = e / span;
-  int u = u0 + 2 * (e - s * span);
-  const bool active = t < nact && r0 + s <= r1 && u < g.cols && u + 1 >= ul && u <= ur;
-  if (!active) u = u0;  // (corner loads inside the image)
-  const int v = min(r0 + s, r1);
-  uint32_t top[NCH], bot[NCH];
-  inv4_corners<NCH>(R, item, g, v, u, top, bot);
-  const int X0 = OB * u - x;  // rectangle column of the pair's first output pixel
-  const Inv4StorePooledClip<NCH, LF> store{pixels + (size_t)item * rw * rh * NCH + ((long long)(OB * v - y) * rw + X0) * NCH,
-                                           (long long)rw * NCH, OB * v - y, rh, max(0, -X0) * NCH, min(2 * OB, rw - X0) * NCH};
-  const int pre = T->pre, tab_bias = T->bias;
-  const bool overflow = T->overflow != 0;
-  const bool ycbcr = T->ycbcr != 0;
-  cp_async_wait_all();
-  __syncthreads();
-  inv4_compute<NCH, PITCH, Inv4StorePooledClip<NCH, LF>, LF>(sPl + 2 * t, sDq, sTab, pre, tab_bias, overflow, ycbcr, active, top,
-                                                              bot, store, one);
-}
+//   k_inverse_region4<.., LF>  fast path (nch 1 / 3, w % 16 == 0, h % 8 == 0, cols % 16 == 0: every window whole)
+//   k_inverse_region_scaled    every other shape, force_generic and the mixed call: k_inverse_region's transform, then
+//                              k_inverse_scaled's exact division per window
 
 // grid (ceil(kb / kTile), kr, n), block kTile (kb = ((rw << lf) + 15 - (1 << lf)) / 8 block columns): thread = block
 // column (x << lf) / 8 + i of compact slot blockIdx.y.  k_inverse_region's transform and MIXED; the colour map is applied
@@ -360,7 +297,7 @@ __global__ void __launch_bounds__(kTile)
   Geom gi = g;  // the image's geometry
   if (MIXED && !image_geom(md, item, gi)) return;
   int x, y;
-  if (!region_origin_scaled(origins, item, gi, lf, rw, rh, x, y)) return;  // (the whole CTA)
+  if (!region_origin(origins, item, gi, lf, rw, rh, x, y)) return;  // (the whole CTA)
   const int f = 1 << lf;
   const int sx = x << lf, sy = y << lf, sx1 = min((x + rw) << lf, gi.w), sy1 = min((y + rh) << lf, gi.h);
   const int v = (sy >> 3) + slot;
@@ -392,6 +329,7 @@ __global__ void __launch_bounds__(kTile)
   const int ngroup = min(nch, 3);
 #pragma unroll 1
   for (int c = 0; c < nch; ++c) {
+    // (inv_block's transform, written out: through inv_block the compiler allocates this kernel's registers differently)
     int xv[64];
     const uint8_t *src = seg + (size_t)c * gi.cols * 64 + u;
     const uint8_t *sh = sShift[(ycbcr && (c == 1 || c == 2)) ? 1 : 0];
@@ -441,13 +379,7 @@ __global__ void __launch_bounds__(kTile)
     } else if (c == ngroup - 1) {  // channels 0 .. ngroup - 1 done: inverse colour map in place, then the averages
       if (ycbcr) {
 #pragma unroll 4
-        for (int p = 0; p < 64; ++p) {
-          const int Y = px[0][p], cb = 2 * px[1][p] - 255, cr = 2 * px[2][p] - 255;
-          const int G = Y - ((cb + cr + 2) >> 2);
-          px[0][p] = (uint8_t)clamp255(G + cr);
-          px[1][p] = (uint8_t)clamp255(G);
-          px[2][p] = (uint8_t)clamp255(G + cb);
-        }
+        for (int p = 0; p < 64; ++p) inv_colour(px[0][p], px[1][p], px[2][p]);
       }
       for (int wy = wya; wy < wyb; ++wy)
         for (int wx = wxa; wx < wxb; ++wx) {

@@ -1,7 +1,7 @@
 """Static SASS instruction counts of a kernel per code section (cut at barriers, votes, calls and exits), by pipe.
 
-    python tools/phase_count.py "k_inverse4<3"            # from himg_b200/_lib/libhimgcu.so
-    python tools/phase_count.py "k_inverse4<3" --file=x.cubin
+    python tools/phase_count.py "k_inverse4<3, 256, 0>"          # from himg_b200/_lib/libhimgcu.so
+    python tools/phase_count.py "k_inverse4<3, 256, 0>" --file=x.cubin
 
 Used to balance the ALU and FMA pipes of K-inv (DESIGN.md 7); compile the kernel with -DHIMG_FORCE_PRE3 to
 count the quality <= 60 path alone."""

@@ -199,6 +199,7 @@ def test_stage_huff_compress(ctx, port):
     for k, (data, bs) in enumerate(_huff_cases()):
         want = port.huff_compress(data, bs)
         out, sizes = ctx.stage_huff_compress(dev(data[None]), bs)
+        ctx.encode_status()
         size = int(sizes.cpu()[0])
         assert size == len(want), f"case {k}: size {size} vs {len(want)}"
         assert_same(out.cpu().numpy()[0, :size], np.frombuffer(want, np.uint8), f"huff case {k} (n={data.size}, bs={bs})")
@@ -210,6 +211,7 @@ def test_stage_huff_compress_batch(ctx, port):
     for i in range(6):
         data[i][rng.random(data.shape[1]) < 0.15 * i] = 0
     out, sizes = ctx.stage_huff_compress(dev(data), 2048)
+    ctx.encode_status()
     out, sizes = out.cpu().numpy(), sizes.cpu().numpy()
     for i in range(6):
         want = port.huff_compress(data[i], 2048)

@@ -42,6 +42,7 @@ def huff_both(ctxs, port, data, bs, what):
     res = {}
     for teams, c in ctxs.items():
         out, sizes = c.stage_huff_compress(dev(data), bs)
+        c.encode_status()  # the device error flag (a packed size that disagrees with the layout, ...)
         res[teams] = (out.cpu().numpy(), sizes.cpu().numpy())
     for i in range(data.shape[0]):
         want = np.frombuffer(port.huff_compress(data[i], bs), np.uint8)
@@ -54,6 +55,7 @@ def encode_both(ctxs, port, imgs, q, what):
     res = {}
     for teams, c in ctxs.items():
         out, sizes = c.encode_batch(dev(imgs), q, True)
+        c.encode_status()
         res[teams] = (out.cpu().numpy(), sizes.cpu().numpy())
     for k in range(imgs.shape[0]):
         want = np.frombuffer(port.encode(imgs[k], q, True), np.uint8)
